@@ -393,6 +393,63 @@ typedef struct trepb_d2_args {
 int trepb_deriv2_batch(trepb_system* sys, const trepb_d2_args* args);
 int trepb_deriv2_batch_dev(trepb_system* sys, const trepb_d2_args* args, void* stream);
 
+/* ---- per-instance physical parameters ------------------------------------------------------
+ * The entry points above run every instance of a batch on the numbers of the one description behind the handle.
+ * The *_varied_batch* entry points take the same arguments plus a trepb_varied: n entries of the description's
+ * numeric tables, and one row of n values per instance, which override those entries for that instance (every
+ * other entry keeps the description's value): Monte Carlo over uncertain masses / lengths / gains, one candidate
+ * parameter set per instance in system identification, K plausible models in robust trajectory optimisation.
+ *   rows       one per instance; trepb_linearize_varied_batch* with traj_len >= 2: one per trajectory r (all
+ *              traj_len - 1 steps of a rollout share its physics).
+ *   entries    only run-time parameters can vary: an entry whose description value is exactly 0, or +-1 in
+ *              frame_se3, is structure (it folds away in the specialised kernels and in trepb_struct_hash), and
+ *              so are the spline x-points of a NonlinearConfigSpring and a Gravity component whose sum over all
+ *              Gravity potentials is 0.  Such an entry, an index out of range or an entry named twice is
+ *              TREPB_ERR_INVALID (trepb_last_error names it).  A varied Gravity component re-forms the
+ *              gravity sum per instance.  A row value of exactly 0 is not checked and keeps the entry's role.
+ *   kernels    specialised and table-driven thread kernels (a handle built for an all-literal instantiation runs
+ *              the run-time-parameter kernels of its structure); cooperative handles are TREPB_ERR_UNSUPPORTED
+ *              (create the handle with TREPB_FLAG_NO_COOP).  No second-derivative entry point varies.
+ * Results equal those of a handle created from each instance's own description, run through the plain entry
+ * point. */
+#define TREPB_PAR_FRAME_VALUE 0   /* index f           */
+#define TREPB_PAR_FRAME_SE3 1     /* index 12 f + k    */
+#define TREPB_PAR_FRAME_MASS 2    /* index 4 f + k     */
+#define TREPB_PAR_POT_D 3         /* index 4 i + k     */
+#define TREPB_PAR_FORCE_D 4       /* index 4 i + k     */
+#define TREPB_PAR_CON_D 5         /* index 4 i + k     */
+#define TREPB_PAR_DPOOL 6         /* index k           */
+typedef struct trepb_varied {
+    int32_t n, _pad;          /* number of varied entries                                                   */
+    const int32_t* table;     /* [n] TREPB_PAR_* (host pointer)                                             */
+    const int32_t* index;     /* [n] flat index into that table (host pointer)                              */
+    const double*  values;    /* [rows][n]: row r = that instance's (trajectory's) values; device pointer for
+                                 the _dev entry points, host pointer otherwise                               */
+} trepb_varied;
+/* Host-only: checks a trepb_varied's entries against a description (values are not read). */
+int trepb_varied_check(const trepb_sysdesc* desc, const trepb_varied* v);
+int trepb_step_varied_batch(trepb_system* sys, const trepb_step_args* args, const trepb_varied* v);
+int trepb_step_varied_batch_dev(trepb_system* sys, const trepb_step_args* args, const trepb_varied* v, void* stream);
+int trepb_linearize_varied_batch(trepb_system* sys, const trepb_lin_args* args, const trepb_varied* v);
+int trepb_linearize_varied_batch_dev(trepb_system* sys, const trepb_lin_args* args, const trepb_varied* v, void* stream);
+int trepb_project_varied_batch(trepb_system* sys, const trepb_project_args* args, const trepb_varied* v);
+int trepb_project_varied_batch_dev(trepb_system* sys, const trepb_project_args* args, const trepb_varied* v, void* stream);
+int trepb_calc_p2_varied_batch(trepb_system* sys, int64_t batch, double dt, const double* q0, const double* q1,
+                               double* p, const trepb_varied* v);
+int trepb_calc_p2_varied_batch_dev(trepb_system* sys, int64_t batch, double dt, const double* q0, const double* q1,
+                                   double* p, const trepb_varied* v, void* stream);
+int trepb_calc_f_varied_batch(trepb_system* sys, int64_t batch, double t1, double t2, const double* q1,
+                              const double* q2, const double* p1, const double* u1, const double* lambda1, double* f,
+                              const trepb_varied* v);
+int trepb_calc_f_varied_batch_dev(trepb_system* sys, int64_t batch, double t1, double t2, const double* q1,
+                                  const double* q2, const double* p1, const double* u1, const double* lambda1,
+                                  double* f, const trepb_varied* v, void* stream);
+int trepb_discrete_fm2_varied_batch(trepb_system* sys, int64_t batch, double t1, double t2, const double* q1,
+                                    const double* q2, const double* u1, double* fm2, const trepb_varied* v);
+int trepb_discrete_fm2_varied_batch_dev(trepb_system* sys, int64_t batch, double t1, double t2, const double* q1,
+                                        const double* q2, const double* u1, double* fm2, const trepb_varied* v,
+                                        void* stream);
+
 /* ---- multi-GPU: one process per GPU ---------------------------------------------------------
  * Instances are independent, so a batch shards over ranks with no exchange during compute (each
  * rank calls the entry points above on its own contiguous block).  The one exchange of the path is

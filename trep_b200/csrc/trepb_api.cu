@@ -122,6 +122,14 @@ struct trepb_system {
     // for the previous such launch - whatever stream that one went to (ScratchGuard).
     cudaEvent_t ev_scratch = nullptr;
     bool scratch_busy = false;
+    // per-instance parameters (trepb_*_varied_batch*): the run-time-parameter kernel set of this structure (the
+    // handle's own, or the one an all-literal handle was matched against), its occupancy, the map and the table-driven
+    // kernels' expanded slots (handle scratch)
+    const KernelSet* vks = nullptr;
+    bool vinit = false;
+    int vbps[4] = {1, 1, 1, 1};
+    int vlin_bps_staged = 0;
+    DevBuf vmap, vslots;
     std::mutex mu;       // serialises launches on this handle
     std::mutex mu_host;  // serialises the host-pointer entry points (they share staging buffers)
 };
@@ -209,6 +217,15 @@ int trepb_system_create(const trepb_sysdesc* desc, int device, int flags, trepb_
                 s->spec_params = std::move(pm.values);
                 break;
             }
+    }
+    s->vks = s->ks;
+    if (s->ks->specialized && s->ks->n_params == 0 && !param_map(s->P).values.empty()) {
+        // all-literal instantiation: the varied calls run the run-time-parameter kernels of the same structure
+        s->vks = nullptr;
+        SpecRegistry& r = spec_registry();
+        const unsigned long long h = struct_hash(s->P);
+        for (int i = 0; i < r.n && !s->vks; ++i)
+            if (r.sets[i]->hash == h && r.sets[i]->n_params == (int)param_map(s->P).values.size()) s->vks = r.sets[i];
     }
     const RtSys& ps = s->P.proto;
     s->ws_doubles = s->wsl.layout(ps.nf, ps.nd, ps.nk, ps.nu, ps.nc);
@@ -314,6 +331,8 @@ void trepb_system_destroy(trepb_system* s) {
     s->ws_hd.release();
     s->ws_du.release();
     s->coop_ext.release();
+    s->vmap.release();
+    s->vslots.release();
     s->d2g.release();
     for (auto& b : s->d2s) b.release();
     for (auto& b : s->hb) b.release();
@@ -463,12 +482,65 @@ struct Timed {
     ~Timed() { cudaEventRecord(s->ev1, st); s->timed = true; }
 };
 
+// Per-instance parameters: checks `v` against the handle's description, uploads its map (trepb_varied.h) to handle
+// scratch and fills va (slots: see varied_slots).  The caller holds s->mu and a ScratchGuard on `stream`.
+int varied_setup(trepb_system* s, const trepb_varied* v, cudaStream_t stream, VariedArgs* va) {
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    if (s->coop)
+        return fail(TREPB_ERR_UNSUPPORTED, "per-instance parameters are not supported by the cooperative kernels (their "
+                                           "link tables are built on the host from the description): create the handle "
+                                           "with TREPB_FLAG_NO_COOP");
+    if (!s->vks) return fail(TREPB_ERR_UNSUPPORTED, "no run-time-parameter kernel set was built for this structure");
+    std::string err;
+    if (!varied_check(s->P, v->n, v->table, v->index, &err)) return fail(TREPB_ERR_INVALID, err);
+    if (v->n > 0 && !v->values) return fail(TREPB_ERR_INVALID, "varied: values is required");
+    if (!s->vinit) {
+        const size_t smem = s->vks->specialized ? 0 : (size_t)s->blob_bytes;
+        for (int w = 0; w < 4; ++w) {
+            int b = 0;
+            CU(s->vks->occupancy_v(w, s->block, smem, &b, nullptr));
+            s->vbps[w] = b > 0 ? b : 1;
+        }
+        if (s->lin_stage_bytes) CU(s->vks->occupancy_v(2, s->block, s->lin_stage_bytes, &s->vlin_bps_staged, nullptr));
+        s->vinit = true;
+    }
+    VariedHost H;
+    varied_map(s->P, v->n, v->table, v->index, s->vks->specialized != 0, &H);
+    // one upload: base, gbase (doubles), then src, gcol (ints)
+    const size_t nb = H.base.size(), ng = H.gbase.size();
+    std::vector<double> buf(nb + ng + (H.src.size() + H.gcol.size() + 1) / 2 + 1, 0.0);
+    memcpy(buf.data(), H.base.data(), nb * sizeof(double));
+    if (ng) memcpy(buf.data() + nb, H.gbase.data(), ng * sizeof(double));
+    int* ib = (int*)(buf.data() + nb + ng);
+    if (!H.src.empty()) memcpy(ib, H.src.data(), H.src.size() * sizeof(int));
+    if (!H.gcol.empty()) memcpy(ib + H.src.size(), H.gcol.data(), H.gcol.size() * sizeof(int));
+    CU(s->vmap.ensure(buf.size() * sizeof(double)));
+    // pageable source: returns once the bytes are staged, so `buf` may go out of scope
+    CU(cudaMemcpyAsync(s->vmap.p, buf.data(), buf.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
+    const double* d = (const double*)s->vmap.p;
+    const int* di = (const int*)(d + nb + ng);
+    va->map = H.view(di, d, di + H.src.size(), d + nb);
+    va->values = v->values;
+    va->slots = nullptr;
+    return TREPB_OK;
+}
+
+// table-driven kernels: one expanded parameter vector per launched thread
+int varied_slots(trepb_system* s, const LaunchCfg& c, VariedArgs* va) {
+    if (s->vks->specialized) return TREPB_OK;
+    CU(s->vslots.ensure((size_t)c.grid * c.block * va->map.n_out * sizeof(double)));
+    va->slots = (double*)s->vslots.p;
+    return TREPB_OK;
+}
+
 }  // namespace
 
 extern "C" {
 
-int trepb_step_batch_dev(trepb_system* s, const trepb_step_args* a, void* stream) {
-    TREPB_NVTX("trepb_step_batch_dev");
+}  // extern "C"
+
+namespace {
+int step_launch(trepb_system* s, const trepb_step_args* a, void* stream, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     const RtSys& ps = s->P.proto;
     if (a->batch < 0 || a->nsteps < 1) return fail(TREPB_ERR_INVALID, "batch must be >= 0 and nsteps >= 1");
@@ -489,6 +561,18 @@ int trepb_step_batch_dev(trepb_system* s, const trepb_step_args* a, void* stream
     p.nsamples = a->sample_every > 0 ? a->nsteps / a->sample_every : 0;
     p.traj_q = a->traj_q; p.traj_p = a->traj_p;
     p.times = a->times;
+    if (v) {
+        ScratchGuard sg(s, (cudaStream_t)stream, true);
+        VariedArgs va;
+        LaunchCfg c;
+        int rc = varied_setup(s, v, (cudaStream_t)stream, &va);
+        if (!rc) rc = make_cfg(s, 0, a->batch, s->vbps[0], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
+        if (!rc) rc = varied_slots(s, c, &va);
+        if (rc) return rc;
+        Timed t(s, c.stream);
+        CU(s->vks->step_v(c, p, va));
+        return TREPB_OK;
+    }
     if (s->coop) {
         CoopLaunch cl;
         make_coop(s, a->batch, (cudaStream_t)stream, &cl, true);
@@ -506,9 +590,25 @@ int trepb_step_batch_dev(trepb_system* s, const trepb_step_args* a, void* stream
     CU(s->ks->step(c, p));
     return TREPB_OK;
 }
+}  // namespace
 
-int trepb_project_batch_dev(trepb_system* s, const trepb_project_args* a, void* stream) {
-    TREPB_NVTX("trepb_project_batch_dev");
+extern "C" {
+
+int trepb_step_batch_dev(trepb_system* s, const trepb_step_args* a, void* stream) {
+    TREPB_NVTX("trepb_step_batch_dev");
+    return step_launch(s, a, stream, nullptr);
+}
+
+int trepb_step_varied_batch_dev(trepb_system* s, const trepb_step_args* a, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_step_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return step_launch(s, a, stream, v);
+}
+
+}  // extern "C"
+
+namespace {
+int project_launch(trepb_system* s, const trepb_project_args* a, void* stream, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     if (a->batch < 0 || a->nsteps < 1) return fail(TREPB_ERR_INVALID, "batch must be >= 0 and nsteps >= 1");
     if (!a->bX || !a->bU || !a->Kfb || !a->X || !a->U || !a->status)
@@ -525,6 +625,18 @@ int trepb_project_batch_dev(trepb_system* s, const trepb_project_args* a, void* 
     p.bX = a->bX; p.bU = a->bU; p.K = a->Kfb; p.k_per_instance = a->k_per_instance; p.use_hint = a->use_hint;
     p.X = a->X; p.U = a->U; p.iters = a->iters; p.status = a->status; p.fail_step = a->fail_step;
     p.times = a->times;
+    if (v) {
+        ScratchGuard sg(s, (cudaStream_t)stream, true);
+        VariedArgs va;
+        LaunchCfg c;
+        int rc = varied_setup(s, v, (cudaStream_t)stream, &va);
+        if (!rc) rc = make_cfg(s, 3, a->batch, s->vbps[3], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
+        if (!rc) rc = varied_slots(s, c, &va);
+        if (rc) return rc;
+        Timed t(s, c.stream);
+        CU(s->vks->proj_v(c, p, va));
+        return TREPB_OK;
+    }
     if (s->coop) {
         CoopLaunch cl;
         make_coop(s, a->batch, (cudaStream_t)stream, &cl, true);
@@ -542,15 +654,41 @@ int trepb_project_batch_dev(trepb_system* s, const trepb_project_args* a, void* 
     CU(s->ks->proj(c, p));
     return TREPB_OK;
 }
+}  // namespace
+
+extern "C" {
+
+int trepb_project_batch_dev(trepb_system* s, const trepb_project_args* a, void* stream) {
+    TREPB_NVTX("trepb_project_batch_dev");
+    return project_launch(s, a, stream, nullptr);
+}
+
+int trepb_project_varied_batch_dev(trepb_system* s, const trepb_project_args* a, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_project_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return project_launch(s, a, stream, v);
+}
 
 }  // extern "C"
 
 namespace {
 // calc_p2 / calc_f / discrete_fm2 share one kernel (P2Params::mode); the caller has validated the pointers
-int eval_launch(trepb_system* s, const P2Params& p, void* stream) {
+int eval_launch(trepb_system* s, const P2Params& p, void* stream, const trepb_varied* v = nullptr) {
     if (p.batch == 0) return TREPB_OK;
     std::lock_guard<std::mutex> lk(s->mu);
     CU(cudaSetDevice(s->device));
+    if (v) {
+        ScratchGuard sg(s, (cudaStream_t)stream, true);
+        VariedArgs va;
+        LaunchCfg c;
+        int rc = varied_setup(s, v, (cudaStream_t)stream, &va);
+        if (!rc) rc = make_cfg(s, 1, p.batch, s->vbps[1], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
+        if (!rc) rc = varied_slots(s, c, &va);
+        if (rc) return rc;
+        Timed t(s, c.stream);
+        CU(s->vks->p2_v(c, p, va));
+        return TREPB_OK;
+    }
     if (s->coop) {
         CoopLaunch cl;
         make_coop(s, p.batch, (cudaStream_t)stream, &cl, true);
@@ -604,11 +742,55 @@ int trepb_discrete_fm2_batch_dev(trepb_system* s, int64_t batch, double t1, doub
     return eval_launch(s, p, stream);
 }
 
+int trepb_calc_p2_varied_batch_dev(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1,
+                                   double* pout, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_calc_p2_varied_batch_dev");
+    if (!s || !q0 || !q1 || !pout || !v) return fail(TREPB_ERR_INVALID, "null argument");
+    if (batch < 0 || !(dt != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or dt");
+    P2Params p{};
+    p.batch = batch; p.dt = dt; p.q0 = q0; p.q1 = q1; p.p = pout; p.mode = 0;
+    return eval_launch(s, p, stream, v);
+}
+
+int trepb_calc_f_varied_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                                  const double* q2, const double* p1, const double* u1, const double* lambda1,
+                                  double* f, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_calc_f_varied_batch_dev");
+    if (!s || !q1 || !q2 || !p1 || !f || !v) return fail(TREPB_ERR_INVALID, "null argument");
+    if (batch < 0 || !(t2 - t1 != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or t2 == t1");
+    P2Params p{};
+    p.batch = batch; p.dt = t2 - t1; p.q0 = q1; p.q1 = q2; p.p = f; p.mode = 1;
+    p.p1 = p1; p.u1 = s->P.proto.nu ? u1 : nullptr; p.lam = s->P.proto.nc ? lambda1 : nullptr;
+    return eval_launch(s, p, stream, v);
+}
+
+int trepb_discrete_fm2_varied_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                                        const double* q2, const double* u1, double* fm2, const trepb_varied* v,
+                                        void* stream) {
+    TREPB_NVTX("trepb_discrete_fm2_varied_batch_dev");
+    if (!s || !q1 || !q2 || !fm2 || !v) return fail(TREPB_ERR_INVALID, "null argument");
+    if (batch < 0 || !(t2 - t1 != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or t2 == t1");
+    P2Params p{};
+    p.batch = batch; p.dt = t2 - t1; p.q0 = q1; p.q1 = q2; p.p = fm2; p.mode = 2;
+    p.u1 = s->P.proto.nu ? u1 : nullptr;
+    return eval_launch(s, p, stream, v);
+}
+
+int trepb_varied_check(const trepb_sysdesc* desc, const trepb_varied* v) {
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    PackedSys P;
+    std::string err;
+    if (!pack_system(desc, &P, &err)) return fail(TREPB_ERR_INVALID, err);
+    if (!varied_check(P, v->n, v->table, v->index, &err)) return fail(TREPB_ERR_INVALID, err);
+    return TREPB_OK;
+}
+
 }  // extern "C"
 
 namespace {
 // validates + launches the linearize kernel; the caller holds s->mu
-int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, double* aux, int aux_size) {
+int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, double* aux, int aux_size,
+               const trepb_varied* v = nullptr) {
     const RtSys& ps = s->P.proto;
     if (a->batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
     if (!a->q1 || !a->p1 || !a->status) return fail(TREPB_ERR_INVALID, "q1, p1 and status are required");
@@ -631,6 +813,26 @@ int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, do
     for (int i = 0; i < 12; ++i) p.raw[i] = raw[i];
     p.aux = aux; p.aux_size = aux_size;
     p.traj_len = a->traj_len;
+    if (v) {
+        ScratchGuard sg(s, stream, true);
+        VariedArgs va;
+        int rc = varied_setup(s, v, stream, &va);
+        if (rc) return rc;
+        const bool stage = s->lin_stage_bytes > 0 && s->vlin_bps_staged > 0 && (p.A || p.B);
+        p.stage = stage ? 1 : 0;
+        LaunchCfg c;
+        const size_t smem = s->ks->specialized ? (stage ? s->lin_stage_bytes : 0) : (size_t)s->blob_bytes;
+        rc = make_cfg(s, 2, a->batch, stage ? s->vlin_bps_staged : s->vbps[2], smem, stream, &c);
+        if (rc) return rc;
+        if (stage) {
+            long long resident = (long long)s->sms * s->vlin_bps_staged;
+            if (c.grid > resident) c.grid = (int)resident;
+        }
+        if ((rc = varied_slots(s, c, &va))) return rc;
+        Timed t(s, c.stream);
+        CU(s->vks->lin_v(c, p, va));
+        return TREPB_OK;
+    }
     if (s->coop) {
         p.stage = 0;
         CoopLaunch cl;
@@ -669,6 +871,13 @@ int trepb_linearize_batch_dev(trepb_system* s, const trepb_lin_args* a, void* st
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> lk(s->mu);
     return lin_launch(s, a, (cudaStream_t)stream, nullptr, 0);
+}
+
+int trepb_linearize_varied_batch_dev(trepb_system* s, const trepb_lin_args* a, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_linearize_varied_batch_dev");
+    if (!s || !a || !v) return fail(TREPB_ERR_INVALID, "null argument");
+    std::lock_guard<std::mutex> lk(s->mu);
+    return lin_launch(s, a, (cudaStream_t)stream, nullptr, 0, v);
 }
 
 int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream_) {
@@ -943,7 +1152,7 @@ struct Pipe {
 
 extern "C" {
 
-static int step_batch_chunked(trepb_system* s, const trepb_step_args* a, int C_) {
+static int step_batch_chunked(trepb_system* s, const trepb_step_args* a, int C_, const trepb_varied* v) {
     const RtSys& ps = s->P.proto;
     const size_t B = (size_t)a->batch, nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc, K = (size_t)a->nsteps;
     const size_t ns = a->sample_every > 0 ? (size_t)(a->nsteps / a->sample_every) : 0;
@@ -954,6 +1163,8 @@ static int step_batch_chunked(trepb_system* s, const trepb_step_args* a, int C_)
     d.q2 = pp.out(a->q2, nq); d.p2 = pp.out(a->p2, nd); d.lambda1 = pp.out(a->lambda1, nc);
     d.iters = pp.out(a->iters, 1); d.status = pp.out(a->status, 1);
     d.traj_q = pp.out(a->traj_q, ns * nq); d.traj_p = pp.out(a->traj_p, ns * nd);
+    trepb_varied dv{};
+    if (v) { dv = *v; dv.values = pp.in(v->values, (size_t)v->n); }   // one row per instance: chunked like q1
     if (pp.err) return pp.err;
     int rc = pp.streams();
     if (rc) return rc;
@@ -973,21 +1184,22 @@ static int step_batch_chunked(trepb_system* s, const trepb_step_args* a, int C_)
         OFF(q1, nq); OFF(p1, nd); OFF(u1, K * nu); OFF(k2, K * nk); OFF(q2_guess, nd); OFF(lambda_guess, nc);
         OFF(q2, nq); OFF(p2, nd); OFF(lambda1, nc); OFF(iters, 1); OFF(status, 1); OFF(traj_q, ns * nq); OFF(traj_p, ns * nd);
 #undef OFF
-        if ((rc = trepb_step_batch_dev(s, &e, st))) return rc;
+        trepb_varied ev = dv;
+        if (ev.values) ev.values += lo * (size_t)v->n;
+        if ((rc = v ? trepb_step_varied_batch_dev(s, &e, &ev, st) : trepb_step_batch_dev(s, &e, st))) return rc;
         if ((rc = pp.download(lo, cnt, st))) return rc;
     }
     return pp.finish();
 }
 
-int trepb_step_batch(trepb_system* s, const trepb_step_args* a) {
-    TREPB_NVTX("trepb_step_batch");
+static int step_host(trepb_system* s, const trepb_step_args* a, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (a->batch < 0 || a->nsteps < 1) return fail(TREPB_ERR_INVALID, "batch must be >= 0 and nsteps >= 1");
     const RtSys& ps = s->P.proto;
     const size_t B = (size_t)a->batch, nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc;
     CU(cudaSetDevice(s->device));
-    if (const int C_ = Pipe::chunks(B); C_ > 1 && a->q1 && a->p1 && a->q2 && a->p2 && a->status) return step_batch_chunked(s, a, C_);
+    if (const int C_ = Pipe::chunks(B); C_ > 1 && a->q1 && a->p1 && a->q2 && a->p2 && a->status) return step_batch_chunked(s, a, C_, v);
     Stager st(s);
     trepb_step_args d = *a;
     d.q1 = st.in(a->q1, B * nq); d.p1 = st.in(a->p1, B * nd);
@@ -998,14 +1210,26 @@ int trepb_step_batch(trepb_system* s, const trepb_step_args* a) {
     const size_t ns = a->sample_every > 0 ? (size_t)(a->nsteps / a->sample_every) : 0;
     d.traj_q = st.out(a->traj_q, B * ns * nq); d.traj_p = st.out(a->traj_p, B * ns * nd);
     d.times = st.in(a->times, (size_t)a->nsteps + 1);
+    trepb_varied dv{};
+    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
     if (st.err) return st.err;
-    int rc = trepb_step_batch_dev(s, &d, nullptr);
+    int rc = v ? trepb_step_varied_batch_dev(s, &d, &dv, nullptr) : trepb_step_batch_dev(s, &d, nullptr);
     if (rc) return rc;
     return st.finish();
 }
 
-int trepb_project_batch(trepb_system* s, const trepb_project_args* a) {
-    TREPB_NVTX("trepb_project_batch");
+int trepb_step_batch(trepb_system* s, const trepb_step_args* a) {
+    TREPB_NVTX("trepb_step_batch");
+    return step_host(s, a, nullptr);
+}
+
+int trepb_step_varied_batch(trepb_system* s, const trepb_step_args* a, const trepb_varied* v) {
+    TREPB_NVTX("trepb_step_varied_batch");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return step_host(s, a, v);
+}
+
+static int project_host(trepb_system* s, const trepb_project_args* a, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (a->batch < 0 || a->nsteps < 1) return fail(TREPB_ERR_INVALID, "batch must be >= 0 and nsteps >= 1");
@@ -1019,14 +1243,27 @@ int trepb_project_batch(trepb_system* s, const trepb_project_args* a) {
     d.X = st.out(a->X, B * (K + 1) * nX); d.U = st.out(a->U, B * K * nU);
     d.iters = st.out(a->iters, B); d.status = st.out(a->status, B); d.fail_step = st.out(a->fail_step, B);
     d.times = st.in(a->times, K + 1);
+    trepb_varied dv{};
+    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
     if (st.err) return st.err;
-    int rc = trepb_project_batch_dev(s, &d, nullptr);
+    int rc = v ? trepb_project_varied_batch_dev(s, &d, &dv, nullptr) : trepb_project_batch_dev(s, &d, nullptr);
     if (rc) return rc;
     return st.finish();
 }
 
-int trepb_calc_p2_batch(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1, double* p) {
-    TREPB_NVTX("trepb_calc_p2_batch");
+int trepb_project_batch(trepb_system* s, const trepb_project_args* a) {
+    TREPB_NVTX("trepb_project_batch");
+    return project_host(s, a, nullptr);
+}
+
+int trepb_project_varied_batch(trepb_system* s, const trepb_project_args* a, const trepb_varied* v) {
+    TREPB_NVTX("trepb_project_varied_batch");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return project_host(s, a, v);
+}
+
+static int calc_p2_host(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1, double* p,
+                        const trepb_varied* v) {
     if (!s) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
@@ -1037,15 +1274,29 @@ int trepb_calc_p2_batch(trepb_system* s, int64_t batch, double dt, const double*
     const double* dq0 = st.in(q0, B * nq);
     const double* dq1 = st.in(q1, B * nq);
     double* dp = st.out(p, B * ps.nd);
+    trepb_varied dv{};
+    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
     if (st.err) return st.err;
-    int rc = trepb_calc_p2_batch_dev(s, batch, dt, dq0, dq1, dp, nullptr);
+    int rc = v ? trepb_calc_p2_varied_batch_dev(s, batch, dt, dq0, dq1, dp, &dv, nullptr)
+               : trepb_calc_p2_batch_dev(s, batch, dt, dq0, dq1, dp, nullptr);
     if (rc) return rc;
     return st.finish();
 }
 
-int trepb_calc_f_batch(trepb_system* s, int64_t batch, double t1, double t2, const double* q1, const double* q2,
-                       const double* p1, const double* u1, const double* lambda1, double* f) {
-    TREPB_NVTX("trepb_calc_f_batch");
+int trepb_calc_p2_batch(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1, double* p) {
+    TREPB_NVTX("trepb_calc_p2_batch");
+    return calc_p2_host(s, batch, dt, q0, q1, p, nullptr);
+}
+
+int trepb_calc_p2_varied_batch(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1,
+                               double* p, const trepb_varied* v) {
+    TREPB_NVTX("trepb_calc_p2_varied_batch");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return calc_p2_host(s, batch, dt, q0, q1, p, v);
+}
+
+static int calc_f_host(trepb_system* s, int64_t batch, double t1, double t2, const double* q1, const double* q2,
+                       const double* p1, const double* u1, const double* lambda1, double* f, const trepb_varied* v) {
     if (!s) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
@@ -1056,15 +1307,31 @@ int trepb_calc_f_batch(trepb_system* s, int64_t batch, double t1, double t2, con
     const double* dq1 = st.in(q1, B * nq); const double* dq2 = st.in(q2, B * nq); const double* dp1 = st.in(p1, B * ps.nd);
     const double* du = st.in(u1, B * ps.nu); const double* dl = st.in(lambda1, B * ps.nc);
     double* df = st.out(f, B * (ps.nd + ps.nc));
+    trepb_varied dv{};
+    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
     if (st.err) return st.err;
-    int rc = trepb_calc_f_batch_dev(s, batch, t1, t2, dq1, dq2, dp1, du, dl, df, nullptr);
+    int rc = v ? trepb_calc_f_varied_batch_dev(s, batch, t1, t2, dq1, dq2, dp1, du, dl, df, &dv, nullptr)
+               : trepb_calc_f_batch_dev(s, batch, t1, t2, dq1, dq2, dp1, du, dl, df, nullptr);
     if (rc) return rc;
     return st.finish();
 }
 
-int trepb_discrete_fm2_batch(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
-                             const double* q2, const double* u1, double* fm2) {
-    TREPB_NVTX("trepb_discrete_fm2_batch");
+int trepb_calc_f_batch(trepb_system* s, int64_t batch, double t1, double t2, const double* q1, const double* q2,
+                       const double* p1, const double* u1, const double* lambda1, double* f) {
+    TREPB_NVTX("trepb_calc_f_batch");
+    return calc_f_host(s, batch, t1, t2, q1, q2, p1, u1, lambda1, f, nullptr);
+}
+
+int trepb_calc_f_varied_batch(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                              const double* q2, const double* p1, const double* u1, const double* lambda1, double* f,
+                              const trepb_varied* v) {
+    TREPB_NVTX("trepb_calc_f_varied_batch");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return calc_f_host(s, batch, t1, t2, q1, q2, p1, u1, lambda1, f, v);
+}
+
+static int discrete_fm2_host(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                             const double* q2, const double* u1, double* fm2, const trepb_varied* v) {
     if (!s) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
@@ -1075,10 +1342,26 @@ int trepb_discrete_fm2_batch(trepb_system* s, int64_t batch, double t1, double t
     const double* dq1 = st.in(q1, B * nq); const double* dq2 = st.in(q2, B * nq);
     const double* du = st.in(u1, B * ps.nu);
     double* df = st.out(fm2, B * ps.nd);
+    trepb_varied dv{};
+    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
     if (st.err) return st.err;
-    int rc = trepb_discrete_fm2_batch_dev(s, batch, t1, t2, dq1, dq2, du, df, nullptr);
+    int rc = v ? trepb_discrete_fm2_varied_batch_dev(s, batch, t1, t2, dq1, dq2, du, df, &dv, nullptr)
+               : trepb_discrete_fm2_batch_dev(s, batch, t1, t2, dq1, dq2, du, df, nullptr);
     if (rc) return rc;
     return st.finish();
+}
+
+int trepb_discrete_fm2_batch(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                             const double* q2, const double* u1, double* fm2) {
+    TREPB_NVTX("trepb_discrete_fm2_batch");
+    return discrete_fm2_host(s, batch, t1, t2, q1, q2, u1, fm2, nullptr);
+}
+
+int trepb_discrete_fm2_varied_batch(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                                    const double* q2, const double* u1, double* fm2, const trepb_varied* v) {
+    TREPB_NVTX("trepb_discrete_fm2_varied_batch");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return discrete_fm2_host(s, batch, t1, t2, q1, q2, u1, fm2, v);
 }
 
 }  // extern "C"
@@ -1139,7 +1422,7 @@ int trepb_deriv2_batch(trepb_system* s, const trepb_d2_args* a) {
 }
 
 // trepb_linearize_batch for a large plain batch (no trajectory rows): chunks alternating between two streams (Pipe)
-static int lin_batch_chunked(trepb_system* s, const trepb_lin_args* a, int C_) {
+static int lin_batch_chunked(trepb_system* s, const trepb_lin_args* a, int C_, const trepb_varied* v) {
     const RtSys& ps = s->P.proto;
     const size_t B = (size_t)a->batch, nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc;
     const size_t nX = 2 * nq, nU = nu + nk;
@@ -1156,6 +1439,8 @@ static int lin_batch_chunked(trepb_system* s, const trepb_lin_args* a, int C_) {
 #define X(f, per) d.f = pp.out(a->f, (per));
     TREPB_LIN_OUT(X)
 #undef X
+    trepb_varied dv{};
+    if (v) { dv = *v; dv.values = pp.in(v->values, (size_t)v->n); }   // one row per instance (no trajectory rows here)
     if (pp.err) return pp.err;
     int rc = pp.streams();
     if (rc) return rc;
@@ -1170,27 +1455,45 @@ static int lin_batch_chunked(trepb_system* s, const trepb_lin_args* a, int C_) {
 #undef X
 #undef TREPB_LIN_IN
 #undef TREPB_LIN_OUT
-        if ((rc = trepb_linearize_batch_dev(s, &e, st))) return rc;
+        trepb_varied ev = dv;
+        if (ev.values) ev.values += lo * (size_t)v->n;
+        if ((rc = v ? trepb_linearize_varied_batch_dev(s, &e, &ev, st) : trepb_linearize_batch_dev(s, &e, st))) return rc;
         if ((rc = pp.download(lo, cnt, st))) return rc;
     }
     return pp.finish();
 }
 
-int trepb_linearize_batch(trepb_system* s, const trepb_lin_args* a) {
-    TREPB_NVTX("trepb_linearize_batch");
+static int lin_host(trepb_system* s, const trepb_lin_args* a, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (a->batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
     CU(cudaSetDevice(s->device));
     if (const int C_ = Pipe::chunks((size_t)a->batch); C_ > 1 && a->traj_len <= 1 && a->q1 && a->p1 && a->status)
-        return lin_batch_chunked(s, a, C_);
+        return lin_batch_chunked(s, a, C_, v);
     Stager st(s);
     trepb_lin_args d;
     stage_lin(st, s, a, &d);
+    trepb_varied dv{};
+    if (v) {
+        const size_t rows = a->traj_len > 1 ? (size_t)a->batch / (size_t)(a->traj_len - 1) : (size_t)a->batch;
+        dv = *v;
+        dv.values = st.in(v->values, rows * v->n);
+    }
     if (st.err) return st.err;
-    int rc = trepb_linearize_batch_dev(s, &d, nullptr);
+    int rc = v ? trepb_linearize_varied_batch_dev(s, &d, &dv, nullptr) : trepb_linearize_batch_dev(s, &d, nullptr);
     if (rc) return rc;
     return st.finish();
+}
+
+int trepb_linearize_batch(trepb_system* s, const trepb_lin_args* a) {
+    TREPB_NVTX("trepb_linearize_batch");
+    return lin_host(s, a, nullptr);
+}
+
+int trepb_linearize_varied_batch(trepb_system* s, const trepb_lin_args* a, const trepb_varied* v) {
+    TREPB_NVTX("trepb_linearize_varied_batch");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return lin_host(s, a, v);
 }
 
 }  // extern "C"

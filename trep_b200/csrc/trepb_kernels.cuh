@@ -18,6 +18,7 @@
 #include <type_traits>
 #include "trepb_hd.h"
 #include "trepb_math.cuh"
+#include "trepb_varied.h"
 
 namespace trepb {
 
@@ -139,6 +140,12 @@ struct KernelSet {
     cudaError_t (*occupancy)(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
     cudaError_t (*d2)(const LaunchCfg&, const WsStridedT<HDG>&, const D2Params&);
     cudaError_t (*d2_occupancy)(int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
+    // per-instance parameters (trepb_*_varied_batch*): the same kernel bodies instantiated with kVaried
+    cudaError_t (*step_v)(const LaunchCfg&, const StepParams&, const VariedArgs&);
+    cudaError_t (*p2_v)(const LaunchCfg&, const P2Params&, const VariedArgs&);
+    cudaError_t (*lin_v)(const LaunchCfg&, const LinParams&, const VariedArgs&);
+    cudaError_t (*proj_v)(const LaunchCfg&, const ProjParams&, const VariedArgs&);
+    cudaError_t (*occupancy_v)(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
 };
 
 // factorizations and tables of deriv1 that the second-derivative kernel reuses (AuxLayout)
@@ -241,10 +248,26 @@ struct Ctx<Sys, false> {
     }
 };
 
-template <class Sys>
-__global__ void __launch_bounds__(128, lb_min<Sys>())
-step_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const StepParams p,
-            const typename Sys::Params par) {
+// kVaried: instance b runs on row `row` of the per-instance parameters (trepb_varied.h).  Specialised: every slot of
+// sys.par with a compile-time index, so that the parameters stay in registers; table-driven: the numeric tables
+// re-pointed at this thread's expanded slot.
+template <class Sys, bool kVaried, class C>
+__device__ __forceinline__ void load_params(C& c, const VariedArgs& va, long row, long tid) {
+    if constexpr (kVaried) {
+        const double* r = va.values + row * va.map.n;
+        if constexpr (Sys::kStatic) {
+#pragma unroll
+            for (int i = 0; i < Sys::kNPAR; ++i) c.sys.par.v[i] = varied_value(va.map, r, i);
+        } else {
+            varied_point(c.sys, va.map, r, va.slots + tid * (long)va.map.n_out);
+        }
+    }
+}
+
+template <class Sys, bool kVaried>
+__device__ __forceinline__ void
+step_body(const RtSys& rsys, const char* dblob, int blob_bytes, const WsStrided& wsp, const StepParams& p,
+          const typename Sys::Params& par, const VariedArgs& va) {
     const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
     const long nth = (long)gridDim.x * blockDim.x;
     Ctx<Sys> c(rsys, dblob, blob_bytes, wsp, tid, nth, par);
@@ -253,6 +276,7 @@ step_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided
     const int nd = sys.ND(), nk = sys.NK(), nq = nd + nk, nu = sys.NU(), nc = sys.NC();
     const double tolT = p.tolT;   // the Newton convergence test needs no square root (sqrt_threshold)
     for (long b = tid; b < p.batch; b += nth) {
+        load_params<Sys, kVaried>(c, va, b, tid);
         TREPB_UNROLL_SYS
         for (int i = 0; i < nq; ++i) {
             const double v = p.q1[b * nq + i];
@@ -310,12 +334,25 @@ step_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided
     }
 }
 
-// DSystem.project / armijo_simulate: X[0] = bX[0]; U[k] = bU[k] - K[k](X[k] - bX[k]); X[k+1] = f(X[k],U[k])
-// (trep/discopt/dsystem.py:426-457), one thread per candidate, the feedback inside the time loop.
 template <class Sys>
 __global__ void __launch_bounds__(128, lb_min<Sys>())
-project_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const ProjParams p,
+step_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const StepParams p,
             const typename Sys::Params par) {
+    step_body<Sys, false>(rsys, dblob, blob_bytes, wsp, p, par, VariedArgs{});
+}
+template <class Sys>
+__global__ void __launch_bounds__(128, lb_min<Sys>())
+step_varied_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const StepParams p,
+                   const VariedArgs va) {
+    step_body<Sys, true>(rsys, dblob, blob_bytes, wsp, p, typename Sys::Params{}, va);
+}
+
+// DSystem.project / armijo_simulate: X[0] = bX[0]; U[k] = bU[k] - K[k](X[k] - bX[k]); X[k+1] = f(X[k],U[k])
+// (trep/discopt/dsystem.py:426-457), one thread per candidate, the feedback inside the time loop.
+template <class Sys, bool kVaried>
+__device__ __forceinline__ void
+project_body(const RtSys& rsys, const char* dblob, int blob_bytes, const WsStrided& wsp, const ProjParams& p,
+             const typename Sys::Params& par, const VariedArgs& va) {
     const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
     const long nth = (long)gridDim.x * blockDim.x;
     Ctx<Sys> c(rsys, dblob, blob_bytes, wsp, tid, nth, par);
@@ -325,6 +362,7 @@ project_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStri
     const double tolT = p.tolT;   // the Newton convergence test needs no square root (sqrt_threshold)
     const int nX = 2 * nq, nU = nu + nk, K = p.nsteps;
     for (long b = tid; b < p.batch; b += nth) {
+        load_params<Sys, kVaried>(c, va, b, tid);
         const double* bX = p.bX + b * (long)(K + 1) * nX;
         const double* bU = p.bU + b * (long)K * nU;
         const double* Kf = p.K + (p.k_per_instance ? b * (long)K * nU * nX : 0);
@@ -377,9 +415,22 @@ project_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStri
 }
 
 template <class Sys>
-__global__ void __launch_bounds__(128)
-p2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const P2Params p,
+__global__ void __launch_bounds__(128, lb_min<Sys>())
+project_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const ProjParams p,
             const typename Sys::Params par) {
+    project_body<Sys, false>(rsys, dblob, blob_bytes, wsp, p, par, VariedArgs{});
+}
+template <class Sys>
+__global__ void __launch_bounds__(128, lb_min<Sys>())
+project_varied_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const ProjParams p,
+                      const VariedArgs va) {
+    project_body<Sys, true>(rsys, dblob, blob_bytes, wsp, p, typename Sys::Params{}, va);
+}
+
+template <class Sys, bool kVaried>
+__device__ __forceinline__ void
+p2_body(const RtSys& rsys, const char* dblob, int blob_bytes, const WsStrided& wsp, const P2Params& p,
+        const typename Sys::Params& par, const VariedArgs& va) {
     const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
     const long nth = (long)gridDim.x * blockDim.x;
     Ctx<Sys> c(rsys, dblob, blob_bytes, wsp, tid, nth, par);
@@ -387,6 +438,7 @@ p2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided w
     auto& ws = c.ws;
     const int nd = sys.ND(), nq = sys.NQ(), nu = sys.NU(), nc = sys.NC();
     for (long b = tid; b < p.batch; b += nth) {
+        load_params<Sys, kVaried>(c, va, b, tid);
         TREPB_UNROLL_SYS
         for (int i = 0; i < nq; ++i) {
             ws.q1(i) = p.q0[b * nq + i];
@@ -413,9 +465,22 @@ p2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided w
 }
 
 template <class Sys>
-__global__ void __launch_bounds__(128, lb_min<Sys, true>())
-lin_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const LinParams p,
+__global__ void __launch_bounds__(128)
+p2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const P2Params p,
             const typename Sys::Params par) {
+    p2_body<Sys, false>(rsys, dblob, blob_bytes, wsp, p, par, VariedArgs{});
+}
+template <class Sys>
+__global__ void __launch_bounds__(128)
+p2_varied_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const P2Params p,
+                 const VariedArgs va) {
+    p2_body<Sys, true>(rsys, dblob, blob_bytes, wsp, p, typename Sys::Params{}, va);
+}
+
+template <class Sys, bool kVaried>
+__device__ __forceinline__ void
+lin_body(const RtSys& rsys, const char* dblob, int blob_bytes, const WsStrided& wsp, const LinParams& p,
+         const typename Sys::Params& par, const VariedArgs& va) {
     const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
     const long nth = (long)gridDim.x * blockDim.x;
     Ctx<Sys> c(rsys, dblob, blob_bytes, wsp, tid, nth, par);
@@ -434,6 +499,7 @@ lin_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided 
         double t1 = 0.0, t2 = 0.0;
         if (live) {
             const long r = p.traj_len > 1 ? b + b / (p.traj_len - 1) : b;   // input row (see trepb_lin_args.traj_len)
+            load_params<Sys, kVaried>(c, va, p.traj_len > 1 ? b / (p.traj_len - 1) : b, tid);   // one row per trajectory
             TREPB_UNROLL_SYS
             for (int i = 0; i < nq; ++i) {
                 const double v = p.q1[r * nq + i];
@@ -533,6 +599,19 @@ lin_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided 
     }
 }
 
+template <class Sys>
+__global__ void __launch_bounds__(128, lb_min<Sys, true>())
+lin_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const LinParams p,
+            const typename Sys::Params par) {
+    lin_body<Sys, false>(rsys, dblob, blob_bytes, wsp, p, par, VariedArgs{});
+}
+template <class Sys>
+__global__ void __launch_bounds__(128, lb_min<Sys, true>())
+lin_varied_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStrided wsp, const LinParams p,
+                  const VariedArgs va) {
+    lin_body<Sys, true>(rsys, dblob, blob_bytes, wsp, p, typename Sys::Params{}, va);
+}
+
 // ---------------------------------------------------------------------------------------------
 template <class Sys>
 struct Launchers {
@@ -579,11 +658,34 @@ struct Launchers {
         project_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, spec_params(c));
         return cudaGetLastError();
     }
+#define TREPB_VLAUNCH(name, kern, P)                                                                            \
+    static cudaError_t name(const LaunchCfg& c, const P& p, const VariedArgs& va) {                           \
+        RtSys rs{};                                                                                           \
+        if (c.sys) rs = *c.sys;                                                                               \
+        cudaError_t e = prep((const void*)kern<Sys>, c.smem);                                                 \
+        if (e != cudaSuccess) return e;                                                                       \
+        kern<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, va);             \
+        return cudaGetLastError();                                                                            \
+    }
+    TREPB_VLAUNCH(step_v, step_varied_kernel, StepParams)
+    TREPB_VLAUNCH(p2_v, p2_varied_kernel, P2Params)
+    TREPB_VLAUNCH(lin_v, lin_varied_kernel, LinParams)
+    TREPB_VLAUNCH(proj_v, project_varied_kernel, ProjParams)
+#undef TREPB_VLAUNCH
     // which: 0 step, 1 p2, 2 lin, 3 project
     static cudaError_t occupancy(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
         const void* fn = which == 0 ? (const void*)step_kernel<Sys>
                        : which == 1 ? (const void*)p2_kernel<Sys>
                        : which == 2 ? (const void*)lin_kernel<Sys> : (const void*)project_kernel<Sys>;
+        return occupancy_of(fn, block, smem, blocks_per_sm, info);
+    }
+    static cudaError_t occupancy_v(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
+        const void* fn = which == 0 ? (const void*)step_varied_kernel<Sys>
+                       : which == 1 ? (const void*)p2_varied_kernel<Sys>
+                       : which == 2 ? (const void*)lin_varied_kernel<Sys> : (const void*)project_varied_kernel<Sys>;
+        return occupancy_of(fn, block, smem, blocks_per_sm, info);
+    }
+    static cudaError_t occupancy_of(const void* fn, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
         cudaFuncAttributes a;
         cudaError_t e = cudaFuncGetAttributes(&a, fn);
         if (e != cudaSuccess) return e;
@@ -617,6 +719,11 @@ KernelSet make_kernelset(const char* name, unsigned long long hash, int speciali
     k.occupancy = &Launchers<Sys>::occupancy;
     k.d2 = &LaunchersD2<Sys>::run;
     k.d2_occupancy = &LaunchersD2<Sys>::occupancy;
+    k.step_v = &Launchers<Sys>::step_v;
+    k.p2_v = &Launchers<Sys>::p2_v;
+    k.lin_v = &Launchers<Sys>::lin_v;
+    k.proj_v = &Launchers<Sys>::proj_v;
+    k.occupancy_v = &Launchers<Sys>::occupancy_v;
     return k;
 }
 #endif  // __CUDACC__

@@ -25,6 +25,9 @@ POT_GRAVITY, POT_LINEAR_SPRING, POT_CONFIG_SPRING, POT_NONLINEAR_CONFIG_SPRING =
 FORCE_DAMPING, FORCE_CONFIG, FORCE_LINEAR_DAMPER, FORCE_BODY_WRENCH, FORCE_HYBRID_WRENCH, FORCE_SPATIAL_WRENCH = range(6)
 # constraint kinds
 CON_DISTANCE, CON_POINT1D, CON_PLANE = range(3)
+# tables a per-instance parameter can come from (TREPB_PAR_*, include/trepb.h)
+PAR_TABLE_NAMES = ["frame_value", "frame_se3", "frame_mass", "pot_d", "force_d", "con_d", "dpool"]
+PAR_TABLES = {n: i for i, n in enumerate(PAR_TABLE_NAMES)}
 
 
 @dataclass
@@ -138,6 +141,36 @@ class SystemDesc:
             h.update(np.ascontiguousarray(a).tobytes())
         h.update(("%d,%d,%d" % (self.nd, self.nk, self.nu)).encode())
         return h.hexdigest()[:16]
+
+    # ---- per-instance parameters (trepb_varied, include/trepb.h) ---------------------------
+    def param_ref(self, table, *idx):
+        """(TREPB_PAR_* id, flat index) of one numeric entry, for per-instance parameters.  table: a key of
+        PAR_TABLES; idx: the entry's index in that array - a frame name or index (+ component) for the frame
+        tables, e.g. param_ref("frame_mass", "Pendulum", 0) or param_ref("pot_d", 0, 2)."""
+        if table not in PAR_TABLES:
+            raise ValueError("unknown parameter table %r (one of %s)" % (table, ", ".join(PAR_TABLES)))
+        idx = list(idx)
+        if table.startswith("frame_") and idx and isinstance(idx[0], str):
+            if idx[0] not in self.frame_names:
+                raise ValueError("no frame named %r" % idx[0])
+            idx[0] = self.frame_names.index(idx[0])
+        a = getattr(self, table)
+        if len(idx) != a.ndim:
+            raise ValueError("%s takes %d index(es)" % (table, a.ndim))
+        return PAR_TABLES[table], int(np.ravel_multi_index(tuple(int(i) for i in idx), a.shape))
+
+    def param_value(self, ref):
+        """The description's value of a param_ref."""
+        t, i = ref
+        return float(getattr(self, PAR_TABLE_NAMES[t]).reshape(-1)[i])
+
+    def with_params(self, refs, values):
+        """A copy with the entries `refs` set to `values` (one row of a per-instance parameter array)."""
+        arrs = {k: getattr(self, k).copy() for k in self._ARRAYS}
+        for (t, i), v in zip(refs, values):
+            arrs[PAR_TABLE_NAMES[t]].reshape(-1)[i] = v
+        return SystemDesc(**arrs, nd=self.nd, nk=self.nk, nu=self.nu, frame_names=list(self.frame_names),
+                          config_names=list(self.config_names), input_names=list(self.input_names), name=self.name)
 
     def equal(self, other):
         if (self.nd, self.nk, self.nu) != (other.nd, other.nk, other.nu):

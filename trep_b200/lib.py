@@ -83,6 +83,28 @@ class D2Args(C.Structure):
                 ("fdxdu", C.c_void_p), ("fdudu", C.c_void_p)]
 
 
+class Varied(C.Structure):
+    """ctypes mirror of trepb_varied: per-instance values of n description entries."""
+    _fields_ = [("n", C.c_int32), ("_pad", C.c_int32), ("table", C.c_void_p), ("index", C.c_void_p),
+                ("values", C.c_void_p)]
+
+
+def _varied(params):
+    """(Varied, keepalive) for params = (refs, values): refs a list of SystemDesc.param_ref results, values
+    [rows][len(refs)] (numpy for the host entry points, anything with data_ptr() for the _dev ones)."""
+    refs, values = params
+    refs = [tuple(r) for r in refs]
+    t = np.ascontiguousarray([r[0] for r in refs], dtype=np.int32)
+    i = np.ascontiguousarray([r[1] for r in refs], dtype=np.int32)
+    if isinstance(values, np.ndarray):
+        values = np.ascontiguousarray(values, dtype=np.float64)
+        if values.ndim != 2 or values.shape[1] != len(refs):
+            raise ValueError("params values must be [rows][%d]" % len(refs))
+    v = Varied(n=len(refs), table=t.ctypes.data if len(refs) else None, index=i.ctypes.data if len(refs) else None,
+               values=_ptr(values))
+    return v, (t, i, values)
+
+
 _lib.trepb_last_error.restype = C.c_char_p
 _lib.trepb_system_kernel_name.restype = C.c_char_p
 _lib.trepb_specialized_name.restype = C.c_char_p
@@ -141,6 +163,22 @@ _lib.trepb_event_elapsed_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
 _lib.trepb_event_pair_destroy.argtypes = [C.c_void_p]
 _lib.trepb_event_pair_destroy.restype = None
 _lib.trepb_measure_fp64_peak.argtypes = [C.c_int, _dp]
+_vp = C.POINTER(Varied)
+_lib.trepb_varied_check.argtypes = [C.c_void_p, _vp]
+_lib.trepb_step_varied_batch.argtypes = [C.c_void_p, C.POINTER(StepArgs), _vp]
+_lib.trepb_step_varied_batch_dev.argtypes = [C.c_void_p, C.POINTER(StepArgs), _vp, C.c_void_p]
+_lib.trepb_project_varied_batch.argtypes = [C.c_void_p, C.POINTER(ProjectArgs), _vp]
+_lib.trepb_project_varied_batch_dev.argtypes = [C.c_void_p, C.POINTER(ProjectArgs), _vp, C.c_void_p]
+_lib.trepb_linearize_varied_batch.argtypes = [C.c_void_p, C.POINTER(LinArgs), _vp]
+_lib.trepb_linearize_varied_batch_dev.argtypes = [C.c_void_p, C.POINTER(LinArgs), _vp, C.c_void_p]
+_lib.trepb_calc_p2_varied_batch.argtypes = [C.c_void_p, C.c_int64, C.c_double] + [C.c_void_p] * 3 + [_vp]
+_lib.trepb_calc_p2_varied_batch_dev.argtypes = [C.c_void_p, C.c_int64, C.c_double] + [C.c_void_p] * 3 + [_vp, C.c_void_p]
+_lib.trepb_calc_f_varied_batch.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 6 + [_vp]
+_lib.trepb_calc_f_varied_batch_dev.argtypes = ([C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 6 +
+                                               [_vp, C.c_void_p])
+_lib.trepb_discrete_fm2_varied_batch.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 4 + [_vp]
+_lib.trepb_discrete_fm2_varied_batch_dev.argtypes = ([C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 4 +
+                                                     [_vp, C.c_void_p])
 _lib.trepb_sincos_batch.argtypes = [C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
 
 EXPORTS = [
@@ -156,6 +194,10 @@ EXPORTS = [
     "trepb_comm_allgather_dev", "trepb_comm_gather_dev", "trepb_ipc_export", "trepb_ipc_open", "trepb_ipc_close",
     "trepb_event_pair_create", "trepb_event_record", "trepb_event_elapsed_ms", "trepb_event_pair_destroy",
     "trepb_synchronize", "trepb_last_kernel_ms", "trepb_measure_fp64_peak", "trepb_sincos_batch",
+    "trepb_varied_check", "trepb_step_varied_batch", "trepb_step_varied_batch_dev", "trepb_linearize_varied_batch",
+    "trepb_linearize_varied_batch_dev", "trepb_project_varied_batch", "trepb_project_varied_batch_dev",
+    "trepb_calc_p2_varied_batch", "trepb_calc_p2_varied_batch_dev", "trepb_calc_f_varied_batch",
+    "trepb_calc_f_varied_batch_dev", "trepb_discrete_fm2_varied_batch", "trepb_discrete_fm2_varied_batch_dev",
 ]
 
 
@@ -312,6 +354,14 @@ def struct_hash(desc):
 def validate(desc):
     cd, keep = D.to_c(desc)
     _check(_lib.trepb_validate(C.byref(cd)))
+
+
+def check_params(desc, refs):
+    """Raises TrepbError (TREPB_ERR_INVALID, the entry named) unless every SystemDesc.param_ref in `refs` may vary
+    per instance (trepb_varied_check: non-zero, not +-1 in frame_se3, not a spline x-point, no repeats)."""
+    cd, keep = D.to_c(desc)
+    v, vkeep = _varied((refs, None))
+    _check(_lib.trepb_varied_check(C.byref(cd), C.byref(v)))
 
 
 def measure_fp64_peak(device=0):
@@ -495,13 +545,20 @@ class System:
     #      anything with data_ptr() => device entry point); the caller owns shapes/dtypes ----------
     def step_raw(self, on_device, batch, nsteps, t0, dt, q1, p1, u1, k2, q2_guess, lambda_guess,
                  q2, p2, lambda1, iters, status, tolerance=1e-10, max_iterations=200,
-                 sample_every=0, traj_q=None, traj_p=None, stream=None, times=None):
+                 sample_every=0, traj_q=None, traj_p=None, stream=None, times=None, params=None):
+        """params: None, or (refs, values [B][len(refs)]) per-instance parameters (trepb_step_varied_batch*)."""
         a = StepArgs(times=_ptr(times), batch=batch, nsteps=nsteps, max_iterations=max_iterations, t0=t0, dt=dt,
                      tolerance=tolerance, q1=_ptr(q1), p1=_ptr(p1), u1=_ptr(u1), k2=_ptr(k2),
                      q2_guess=_ptr(q2_guess), lambda_guess=_ptr(lambda_guess), q2=_ptr(q2),
                      p2=_ptr(p2), lambda1=_ptr(lambda1), iters=_ptr(iters), status=_ptr(status),
                      sample_every=sample_every, traj_q=_ptr(traj_q), traj_p=_ptr(traj_p))
-        if on_device:
+        if params is not None:
+            v, keep = _varied(params)
+            if on_device:
+                _check(_lib.trepb_step_varied_batch_dev(self._h, C.byref(a), C.byref(v), stream))
+            else:
+                _check(_lib.trepb_step_varied_batch(self._h, C.byref(a), C.byref(v)))
+        elif on_device:
             _check(_lib.trepb_step_batch_dev(self._h, C.byref(a), stream))
         else:
             _check(_lib.trepb_step_batch(self._h, C.byref(a)))
@@ -519,9 +576,16 @@ class System:
             setattr(a, n, _ptr(v))
         return a
 
-    def linearize_raw(self, on_device, batch, q1, p1, u1, k2, status, stream=None, **kw):
+    def linearize_raw(self, on_device, batch, q1, p1, u1, k2, status, stream=None, params=None, **kw):
+        """params: None, or (refs, values) with one row per instance, or per trajectory when traj_len >= 2."""
         a = self._lin_args(batch, q1, p1, u1, k2, status, **kw)
-        if on_device:
+        if params is not None:
+            v, keep = _varied(params)
+            if on_device:
+                _check(_lib.trepb_linearize_varied_batch_dev(self._h, C.byref(a), C.byref(v), stream))
+            else:
+                _check(_lib.trepb_linearize_varied_batch(self._h, C.byref(a), C.byref(v)))
+        elif on_device:
             _check(_lib.trepb_linearize_batch_dev(self._h, C.byref(a), stream))
         else:
             _check(_lib.trepb_linearize_batch(self._h, C.byref(a)))
@@ -543,32 +607,58 @@ class System:
 
     def project_raw(self, on_device, batch, nsteps, t0, dt, bX, bU, Kfb, X, U, status, k_per_instance=False,
                     use_hint=True, iters=None, fail_step=None, tolerance=1e-10, max_iterations=200, stream=None,
-                    times=None):
+                    times=None, params=None):
         a = ProjectArgs(times=_ptr(times), batch=batch, nsteps=nsteps, max_iterations=max_iterations, t0=t0, dt=dt, tolerance=tolerance,
                         bX=_ptr(bX), bU=_ptr(bU), Kfb=_ptr(Kfb), k_per_instance=1 if k_per_instance else 0,
                         use_hint=1 if use_hint else 0, X=_ptr(X), U=_ptr(U), iters=_ptr(iters), status=_ptr(status),
                         fail_step=_ptr(fail_step))
-        if on_device:
+        if params is not None:
+            v, keep = _varied(params)
+            if on_device:
+                _check(_lib.trepb_project_varied_batch_dev(self._h, C.byref(a), C.byref(v), stream))
+            else:
+                _check(_lib.trepb_project_varied_batch(self._h, C.byref(a), C.byref(v)))
+        elif on_device:
             _check(_lib.trepb_project_batch_dev(self._h, C.byref(a), stream))
         else:
             _check(_lib.trepb_project_batch(self._h, C.byref(a)))
 
-    def calc_p2_raw(self, on_device, batch, dt, q0, q1, p, stream=None):
-        if on_device:
+    def calc_p2_raw(self, on_device, batch, dt, q0, q1, p, stream=None, params=None):
+        if params is not None:
+            v, keep = _varied(params)
+            if on_device:
+                _check(_lib.trepb_calc_p2_varied_batch_dev(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p), C.byref(v), stream))
+            else:
+                _check(_lib.trepb_calc_p2_varied_batch(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p), C.byref(v)))
+        elif on_device:
             _check(_lib.trepb_calc_p2_batch_dev(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p), stream))
         else:
             _check(_lib.trepb_calc_p2_batch(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p)))
 
-    def calc_f_raw(self, on_device, batch, t1, t2, q1, q2, p1, u1, lambda1, f, stream=None):
-        if on_device:
+    def calc_f_raw(self, on_device, batch, t1, t2, q1, q2, p1, u1, lambda1, f, stream=None, params=None):
+        if params is not None:
+            v, keep = _varied(params)
+            args = (self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(p1), _ptr(u1), _ptr(lambda1), _ptr(f), C.byref(v))
+            if on_device:
+                _check(_lib.trepb_calc_f_varied_batch_dev(*args, stream))
+            else:
+                _check(_lib.trepb_calc_f_varied_batch(*args))
+        elif on_device:
             _check(_lib.trepb_calc_f_batch_dev(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(p1), _ptr(u1),
                                                _ptr(lambda1), _ptr(f), stream))
         else:
             _check(_lib.trepb_calc_f_batch(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(p1), _ptr(u1),
                                            _ptr(lambda1), _ptr(f)))
 
-    def discrete_fm2_raw(self, on_device, batch, t1, t2, q1, q2, u1, fm2, stream=None):
-        if on_device:
+    def discrete_fm2_raw(self, on_device, batch, t1, t2, q1, q2, u1, fm2, stream=None, params=None):
+        if params is not None:
+            v, keep = _varied(params)
+            args = (self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(u1), _ptr(fm2), C.byref(v))
+            if on_device:
+                _check(_lib.trepb_discrete_fm2_varied_batch_dev(*args, stream))
+            else:
+                _check(_lib.trepb_discrete_fm2_varied_batch(*args))
+        elif on_device:
             _check(_lib.trepb_discrete_fm2_batch_dev(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(u1), _ptr(fm2), stream))
         else:
             _check(_lib.trepb_discrete_fm2_batch(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(u1), _ptr(fm2)))
@@ -578,15 +668,22 @@ class System:
         x = np.ascontiguousarray(np.asarray(x, dtype=np.float64))
         return x.reshape(shape)
 
-    def calc_p2(self, dt, q0, q1):
+    def _params(self, params, rows):
+        """params=(refs, values): values as a [rows][len(refs)] float64 array."""
+        if params is None:
+            return None
+        refs, values = params
+        return refs, self._f(values, (rows, len(refs)))
+
+    def calc_p2(self, dt, q0, q1, params=None):
         q0 = np.atleast_2d(np.asarray(q0, float))
         B = q0.shape[0]
         q0, q1 = self._f(q0, (B, self.nq)), self._f(q1, (B, self.nq))
         p = np.empty((B, self.nd))
-        self.calc_p2_raw(False, B, float(dt), q0, q1, p)
+        self.calc_p2_raw(False, B, float(dt), q0, q1, p, params=self._params(params, B))
         return p
 
-    def calc_f(self, t1, t2, q1, q2, p1, u1=None, lambda1=None):
+    def calc_f(self, t1, t2, q1, q2, p1, u1=None, lambda1=None, params=None):
         """Residual of the DEL equation [B][nd+nc] (_MidpointVI._calc_f, midpointvi.c:533-575)."""
         q1 = np.atleast_2d(np.asarray(q1, float))
         B = q1.shape[0]
@@ -594,24 +691,26 @@ class System:
         u1 = None if (u1 is None or self.nu == 0) else self._f(u1, (B, self.nu))
         lam = None if (lambda1 is None or self.nc == 0) else self._f(lambda1, (B, self.nc))
         f = np.empty((B, self.nd + self.nc))
-        self.calc_f_raw(False, B, float(t1), float(t2), q1, q2, p1, u1, lam, f)
+        self.calc_f_raw(False, B, float(t1), float(t2), q1, q2, p1, u1, lam, f, params=self._params(params, B))
         return f
 
-    def discrete_fm2(self, t1, t2, q1, q2, u1=None):
+    def discrete_fm2(self, t1, t2, q1, q2, u1=None, params=None):
         """Discrete forcing (t2 - t1) F(q_mid, dq, u1) [B][nd] (_MidpointVI.discrete_fm2, midpointvi.c:2710-2727)."""
         q1 = np.atleast_2d(np.asarray(q1, float))
         B = q1.shape[0]
         q1, q2 = self._f(q1, (B, self.nq)), self._f(q2, (B, self.nq))
         u1 = None if (u1 is None or self.nu == 0) else self._f(u1, (B, self.nu))
         fm2 = np.empty((B, self.nd))
-        self.discrete_fm2_raw(False, B, float(t1), float(t2), q1, q2, u1, fm2)
+        self.discrete_fm2_raw(False, B, float(t1), float(t2), q1, q2, u1, fm2, params=self._params(params, B))
         return fm2
 
     def step(self, q1, p1, t0, dt, nsteps=1, u1=None, k2=None, q2_guess=None, lambda_guess=None,
-             tolerance=1e-10, max_iterations=200, sample_every=0, times=None):
+             tolerance=1e-10, max_iterations=200, sample_every=0, times=None, params=None):
         """`nsteps` consecutive MidpointVI steps for every instance.  Returns a dict with the
         final q2, p2, lambda1, iters (summed), status and optionally the sampled trajectory.
-        times: optional grid [nsteps+1] shared by the batch (step s runs times[s] -> times[s+1])."""
+        times: optional grid [nsteps+1] shared by the batch (step s runs times[s] -> times[s+1]).
+        params: None, or (refs, values [B][len(refs)]): per-instance values of the SystemDesc.param_ref entries
+        refs (the same keyword on linearize, project, calc_p2, calc_f and discrete_fm2)."""
         if times is not None:
             times = self._f(times, (nsteps + 1,))
         q1 = np.atleast_2d(np.asarray(q1, float))
@@ -635,10 +734,11 @@ class System:
             out["traj_p"] = np.empty((B, ns, self.nd))
         self.step_raw(False, B, nsteps, float(t0), float(dt), q1, p1, u1, k2, q2g, lg, out["q2"],
                       out["p2"], out["lambda1"] if self.nc else None, out["iters"], out["status"],
-                      tolerance, max_iterations, sample_every, out.get("traj_q"), out.get("traj_p"), times=times)
+                      tolerance, max_iterations, sample_every, out.get("traj_q"), out.get("traj_p"), times=times,
+                      params=self._params(params, B))
         return out
 
-    def project(self, bX, bU, Kfb, t0, dt, use_hint=True, tolerance=1e-10, max_iterations=200, times=None):
+    def project(self, bX, bU, Kfb, t0, dt, use_hint=True, tolerance=1e-10, max_iterations=200, times=None, params=None):
         """Closed-loop rollouts X[0] = bX[0], U[k] = bU[k] - K[k](X[k] - bX[k]), X[k+1] = f(X[k], U[k])
         (DSystem.project / DOptimizer.armijo_simulate) for a batch of candidates.
         bX [B,K+1,nX], bU [B,K,nU], Kfb [K,nU,nX] (shared) or [B,K,nU,nX]."""
@@ -656,12 +756,13 @@ class System:
         self.project_raw(False, B, K, float(t0), float(dt), bX, bU, Kfb, out["X"], out["U"], out["status"],
                          k_per_instance=per, use_hint=use_hint, iters=out["iters"], fail_step=out["fail_step"],
                          tolerance=tolerance, max_iterations=max_iterations,
-                         times=None if times is None else self._f(times, (K + 1,)))
+                         times=None if times is None else self._f(times, (K + 1,)), params=self._params(params, B))
         return out
 
     def linearize(self, q1, p1, u1=None, k2=None, t1=0.0, t2=None, dt=None, q2_guess=None,
-                  lambda_guess=None, want_raw=False, tolerance=1e-10, max_iterations=200):
-        """One DSystem-style linearization per instance: solve the step, then A (fdx) and B (fdu)."""
+                  lambda_guess=None, want_raw=False, tolerance=1e-10, max_iterations=200, params=None):
+        """One DSystem-style linearization per instance: solve the step, then A (fdx) and B (fdu).
+        params: None, or (refs, values [B][len(refs)]) per-instance parameters."""
         q1 = np.atleast_2d(np.asarray(q1, float))
         B = q1.shape[0]
         q1, p1 = self._f(q1, (B, self.nq)), self._f(p1, (B, self.nd))
@@ -695,7 +796,7 @@ class System:
                            lambda1=out["lambda1"] if self.nc else None, iters=out["iters"],
                            A=out["A"], B=out["B"] if self.nU else None,
                            raw={k: v for k, v in rawbufs.items() if v.size},
-                           tolerance=tolerance, max_iterations=max_iterations)
+                           tolerance=tolerance, max_iterations=max_iterations, params=self._params(params, B))
         return out
 
     def d2_shapes(self, B):

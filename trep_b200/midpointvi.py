@@ -46,6 +46,27 @@ class MidpointVI:
         self.status = None
         self._lin = None
         self._d2 = None
+        self._params = None
+
+    def set_parameters(self, refs, values):
+        """Per-instance physical parameters for every later initialize_from_*, step, simulate, calc_f,
+        discrete_fm2 and first-derivative call: refs a list of SystemDesc.param_ref entries, values [B][len(refs)]
+        (instance b runs on row b).  set_parameters(None, None) goes back to the description's numbers.  Second
+        derivatives have no per-instance form: they raise while parameters are set."""
+        if refs is None:
+            self._params = None
+        else:
+            refs = [tuple(r) for r in refs]
+            lib.check_params(self.desc, refs)
+            values = np.ascontiguousarray(np.asarray(values, dtype=np.float64).reshape(-1, len(refs)))
+            self._params = (refs, values)
+        self._lin = None
+        self._d2 = None
+
+    def _p(self, B):
+        if self._params is not None and self._params[1].shape[0] != B:
+            raise ValueError("parameters have %d rows for a batch of %d" % (self._params[1].shape[0], B))
+        return self._params
 
     # ---- initialisation (midpointvi.py:138-172) --------------------------------------------------
     def _b(self, x, n):
@@ -68,7 +89,7 @@ class MidpointVI:
         q0, q1 = self._b(q0, self.nq), self._b(q1, self.nq)
         self.t1, self.t2 = float(t0), float(t1)
         self.q1, self.q2 = q0, q1
-        self.p2 = self.sys.calc_p2(self.t2 - self.t1, q0, q1)
+        self.p2 = self.sys.calc_p2(self.t2 - self.t1, q0, q1, params=self._p(q1.shape[0]))
         self.p1 = None
         B = q1.shape[0]
         self.lambda1 = np.zeros((B, self.nc)) if lambda1 is None else self._b(lambda1, self.nc)
@@ -99,7 +120,7 @@ class MidpointVI:
         out = self.sys.step(self.q1, self.p1, t0, float(t2) - t0, nsteps=1,
                             u1=u1[:, None, :] if self.nu else None, k2=k2[:, None, :] if self.nk else None,
                             q2_guess=hint, lambda_guess=lam if self.nc else None,
-                            tolerance=self.tolerance, max_iterations=max_iterations)
+                            tolerance=self.tolerance, max_iterations=max_iterations, params=self._p(B))
         self.t2 = float(t2)
         self.q2, self.p2, self.lambda1 = out["q2"], out["p2"], out["lambda1"]
         self._lin = None
@@ -114,7 +135,8 @@ class MidpointVI:
         Returns dict(iters, traj_q, traj_p) - trajectories only if sample_every > 0."""
         out = self.sys.step(self.q2, self.p2, self.t2, float(dt), nsteps=nsteps, u1=u, k2=k,
                             lambda_guess=self.lambda1 if self.nc else None, tolerance=self.tolerance,
-                            max_iterations=max_iterations, sample_every=sample_every, times=times)
+                            max_iterations=max_iterations, sample_every=sample_every, times=times,
+                            params=self._p(self.batch))
         # state before the last step is only known when a trajectory was captured
         self.q1 = self.p1 = None
         t = self.t2
@@ -134,12 +156,13 @@ class MidpointVI:
         """Residual of the DEL equation at the current (q1, q2, p1, u1, lambda1): [B, nd+nc]
         (_MidpointVI._calc_f, midpointvi.c:567-575)."""
         assert self.q1 is not None and self.p1 is not None, "calc_f needs the state before the step"
-        return self.sys.calc_f(self.t1, self.t2, self.q1, self.q2, self.p1, self.u1, self.lambda1 if self.nc else None)
+        return self.sys.calc_f(self.t1, self.t2, self.q1, self.q2, self.p1, self.u1, self.lambda1 if self.nc else None,
+                               params=self._p(self.batch))
 
     def discrete_fm2(self):
         """Discrete forcing of the current step [B, nd] (_MidpointVI.discrete_fm2, midpointvi.c:2710-2727)."""
         assert self.q1 is not None, "discrete_fm2 needs the configuration before the step"
-        return self.sys.discrete_fm2(self.t1, self.t2, self.q1, self.q2, self.u1)
+        return self.sys.discrete_fm2(self.t1, self.t2, self.q1, self.q2, self.u1, params=self._p(self.batch))
 
     @property
     def v2(self):
@@ -154,7 +177,7 @@ class MidpointVI:
             assert self.q1 is not None and self.p1 is not None, "derivatives need the state before the step"
             out = self.sys.linearize(self.q1, self.p1, self.u1, self.q2[:, self.nd:], t1=self.t1, t2=self.t2,
                                      q2_guess=self.q2[:, :self.nd], lambda_guess=self.lambda1 if self.nc else None,
-                                     want_raw=True, tolerance=self.tolerance)
+                                     want_raw=True, tolerance=self.tolerance, params=self._p(self.batch))
             self._check(out["status"])
             self._lin = out
         return self._lin
@@ -178,6 +201,9 @@ class MidpointVI:
     # ---- second derivatives (midpointvi.py:422-731): the 30 tensors in the reference's storage layout
     #      [B][wrt A][wrt B][out]  (trep.h:439-473), e.g. q2_dq1dq1()[b, i, j, :] = d2 q2 / dq1_i dq1_j
     def _calc_deriv2(self):
+        if self._params is not None:
+            raise NotImplementedError("second derivatives have no per-instance-parameter form: "
+                                      "call set_parameters(None, None) first")
         if getattr(self, "_d2", None) is None or self._lin is None:
             assert self.q1 is not None and self.p1 is not None, "derivatives need the state before the step"
             out = self.sys.deriv2(self.q1, self.p1, self.u1, self.q2[:, self.nd:], t1=self.t1, t2=self.t2,
@@ -205,7 +231,7 @@ class MidpointVI:
 
 
 def monte_carlo_sweep(system, q0, dt, nsteps, q1=None, u=None, k=None, tolerance=1e-10, device=None, group=None,
-                      hist_max=8):
+                      hist_max=8, params=None):
     """Monte-Carlo initial-condition sweep (BASELINE.json config 4): every row of q0 [N, nq] is an
     independent rollout started with ``initialize_from_configs(0, q0, dt, q1 or q0)`` and stepped
     ``nsteps`` times inside one kernel launch.  With a ``trep_b200.dist.Group`` (one process per GPU) the
@@ -213,7 +239,8 @@ def monte_carlo_sweep(system, q0, dt, nsteps, q1=None, u=None, k=None, tolerance
     states (q2, p2: 8 (nq + nd) bytes per rollout), the per-rollout iteration totals and status codes
     are gathered on rank 0, device to device (NCCL).  Returns dict(q2 [N,nq], p2 [N,nd], iters [N],
     status [N], hist) on rank 0 (None elsewhere): ``hist[i]`` = number of rollouts whose mean Newton
-    iterations per step rounds to i."""
+    iterations per step rounds to i.  params=(refs, values [N][len(refs)]): per-rollout physical parameters
+    (SystemDesc.param_ref entries), sharded like q0."""
     from . import dist as D_
     q0 = np.atleast_2d(np.asarray(q0, float))
     n = q0.shape[0]
@@ -228,9 +255,14 @@ def monte_carlo_sweep(system, q0, dt, nsteps, q1=None, u=None, k=None, tolerance
     ks = None if k is None else np.asarray(k, float)[sl]
     mvi = MidpointVI(system, tolerance=tolerance, device=device)
     cnt = hi - lo
+    ps = None
+    if params is not None:
+        refs = [tuple(r) for r in params[0]]
+        ps = (refs, np.ascontiguousarray(np.asarray(params[1], float).reshape(n, len(refs))[sl]))
+        mvi.set_parameters(*ps)
     if world == 1:
         mvi.initialize_from_configs(0.0, q0[sl], dt, q1s)
-        out = mvi.sys.step(mvi.q2, mvi.p2, mvi.t2, float(dt), nsteps=nsteps, u1=us, k2=ks, tolerance=tolerance)
+        out = mvi.sys.step(mvi.q2, mvi.p2, mvi.t2, float(dt), nsteps=nsteps, u1=us, k2=ks, tolerance=tolerance, params=ps)
         q2, p2, iters, status = out["q2"], out["p2"], out["iters"], out["status"]
     else:
         s, nq, nd = mvi.sys, mvi.nq, mvi.nd
@@ -241,9 +273,10 @@ def monte_carlo_sweep(system, q0, dt, nsteps, q1=None, u=None, k=None, tolerance
         m = max(cnt, 1)
         dp = lib.DeviceBuffer(device, (m, nd)); q2d = lib.DeviceBuffer(device, (m, nq)); p2d = lib.DeviceBuffer(device, (m, nd))
         itd = lib.DeviceBuffer(device, (m,), np.int32); std = lib.DeviceBuffer(device, (m,), np.int32)
-        s.calc_p2_raw(True, cnt, float(dt), dq0, dq1, dp)
+        dv = None if ps is None else (ps[0], up(ps[1]) if cnt else None)
+        s.calc_p2_raw(True, cnt, float(dt), dq0, dq1, dp, params=dv)
         s.step_raw(True, cnt, nsteps, float(dt), float(dt), dq1, dp, du, dk, None, None, q2d, p2d, None, itd, std,
-                   tolerance=tolerance)
+                   tolerance=tolerance, params=dv)
         res = []
         for buf, rb, dt_, shape in ((q2d, 8 * nq, np.float64, (n, nq)), (p2d, 8 * nd, np.float64, (n, nd)),
                                     (itd, 4, np.int32, (n,)), (std, 4, np.int32, (n,))):
@@ -251,7 +284,7 @@ def monte_carlo_sweep(system, q0, dt, nsteps, q1=None, u=None, k=None, tolerance
             res.append(None if full is None else full.download()[:n * rb].view(dt_).reshape(shape).copy())
             if full is not None:
                 full.free()
-        for b in (dq0, dq1, du, dk, dp, q2d, p2d, itd, std):
+        for b in (dq0, dq1, du, dk, dp, q2d, p2d, itd, std, None if dv is None else dv[1]):
             if b is not None:
                 b.free()
         if rank != 0:
