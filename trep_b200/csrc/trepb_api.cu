@@ -41,6 +41,12 @@ struct DevBuf {
     }
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
+
+// dynamic shared memory of a cooperative launch: the description blob, rounded up to an even number of doubles,
+// then `teams` workspaces of lay.total doubles
+size_t coop_smem(int blob_bytes, int teams, const trepb::CoopLayout& lay) {
+    return (size_t)(((blob_bytes + 7) / 8 + 1) & ~1) * 8 + (size_t)teams * lay.total * 8;
+}
 }  // namespace
 
 #if defined(TREPB_PHASE_TIMING)
@@ -66,6 +72,13 @@ bool spec_register(const KernelSet* ks, unsigned abi) {
     if (abi != kSpecAbi || r.n >= SpecRegistry::kMax) return false;
     r.sets[r.n++] = ks;
     return true;
+}
+// the first registered kernel set for `hash` that takes n_params run-time parameters, or null
+static const KernelSet* spec_find(unsigned long long hash, int n_params) {
+    const SpecRegistry& r = spec_registry();
+    for (int i = 0; i < r.n; ++i)
+        if (r.sets[i]->hash == hash && r.sets[i]->n_params == n_params) return r.sets[i];
+    return nullptr;
 }
 }  // namespace trepb
 
@@ -201,32 +214,21 @@ int trepb_system_create(const trepb_sysdesc* desc, int device, int flags, trepb_
     s->dview = s->P.view(s->dblob);
     // kernel selection
     s->ks = general_kernels();
+    ParamMap pm = param_map(s->P);
+    const int n_params = (int)pm.values.size();
     if (!(flags & (TREPB_FLAG_NO_SPECIALIZE | TREPB_FLAG_FORCE_COOP))) {
         // an instantiation for exactly this description (every number a literal) if the build made one ...
-        SpecRegistry& r = spec_registry();
-        const unsigned long long hd = desc_hash(s->P);
-        for (int i = 0; i < r.n; ++i)
-            if (r.sets[i]->hash == hd && r.sets[i]->n_params == 0 && !(flags & TREPB_FLAG_NO_LITERAL)) { s->ks = r.sets[i]; break; }
+        const KernelSet* lit = (flags & TREPB_FLAG_NO_LITERAL) ? nullptr : spec_find(desc_hash(s->P), 0);
+        if (lit) s->ks = lit;
         // ... else structure picks the kernel and the numbers travel as its run-time parameters
-        const unsigned long long h = struct_hash(s->P);
-        for (int i = 0; i < r.n && !s->ks->specialized; ++i)
-            if (r.sets[i]->hash == h) {
-                ParamMap pm = param_map(s->P);
-                if ((int)pm.values.size() != r.sets[i]->n_params) continue;   // cannot happen for equal structures
-                s->ks = r.sets[i];
-                s->spec_params = std::move(pm.values);
-                break;
-            }
+        else if (const KernelSet* ks = spec_find(struct_hash(s->P), n_params)) {
+            s->ks = ks;
+            s->spec_params = std::move(pm.values);
+        }
     }
     s->vks = s->ks;
-    if (s->ks->specialized && s->ks->n_params == 0 && !param_map(s->P).values.empty()) {
-        // all-literal instantiation: the varied calls run the run-time-parameter kernels of the same structure
-        s->vks = nullptr;
-        SpecRegistry& r = spec_registry();
-        const unsigned long long h = struct_hash(s->P);
-        for (int i = 0; i < r.n && !s->vks; ++i)
-            if (r.sets[i]->hash == h && r.sets[i]->n_params == (int)param_map(s->P).values.size()) s->vks = r.sets[i];
-    }
+    // all-literal instantiation: the varied calls run the run-time-parameter kernels of the same structure
+    if (s->ks->specialized && s->ks->n_params == 0 && n_params > 0) s->vks = spec_find(struct_hash(s->P), n_params);
     const RtSys& ps = s->P.proto;
     s->ws_doubles = s->wsl.layout(ps.nf, ps.nd, ps.nk, ps.nu, ps.nc);
     // Cooperative kernels for table-driven systems whose per-thread workspace is too large to stay
@@ -239,7 +241,7 @@ int trepb_system_create(const trepb_sysdesc* desc, int device, int flags, trepb_
             s->clay.set(hv, cks->specialized != 0, false, cks->ext != 0);
             s->clay_solve.set(hv, cks->specialized != 0, true, cks->ext != 0);
             s->coop_blob_bytes = (int)s->CP.blob.size();
-            const size_t blob_d = (size_t)(((s->coop_blob_bytes + 7) / 8 + 1) & ~1) * 8;
+            const size_t blob_d = coop_smem(s->coop_blob_bytes, 0, s->clay);
             const size_t ws_b = (size_t)s->clay.total * 8;
             const size_t cap = (size_t)prop.sharedMemPerBlockOptin;
             int warps = cap > blob_d ? (int)((cap - blob_d) / ws_b) : 0;
@@ -278,7 +280,7 @@ int trepb_system_create(const trepb_sysdesc* desc, int device, int flags, trepb_
     if (base_smem > 200 * 1024) { trepb_system_destroy(s); return fail(TREPB_ERR_UNSUPPORTED, "system description exceeds shared memory"); }
     for (int w = 0; w < 4; ++w) {
         int b = 0;
-        CUS(s->ks->occupancy(w, s->block, base_smem, &b, nullptr));
+        CUS(s->ks->occupancy(w, false, s->block, base_smem, &b, nullptr));
         s->bps[w] = b > 0 ? b : 1;
     }
     s->ws_hd_elems = s->wsl_hd.layout(ps.nf, ps.nd, ps.nk, ps.nu, ps.nc, 1);
@@ -310,7 +312,7 @@ int trepb_system_create(const trepb_sysdesc* desc, int device, int flags, trepb_
         const size_t st = (size_t)(nX * nX + nX * nU) * sizeof(double) * s->block;
         if (st <= 160 * 1024) {
             int b = 0;
-            CUS(s->ks->occupancy(2, s->block, st, &b, nullptr));
+            CUS(s->ks->occupancy(2, false, s->block, st, &b, nullptr));
             if (b > 0) { s->lin_stage_bytes = st; s->lin_bps_staged = b; }
         }
     }
@@ -373,12 +375,12 @@ int trepb_kernel_info(trepb_system* s, int which, int32_t* regs, int32_t* local_
         if (local_bytes) *local_bytes = (int32_t)ki.local_bytes;
         if (blocks_per_sm) *blocks_per_sm = 1;
         if (block) *block = 32 * (lin ? s->cks->team_warps : 1) * teams;
-        if (smem_bytes) *smem_bytes = (int32_t)((size_t)(((s->coop_blob_bytes + 7) / 8 + 1) & ~1) * 8 + (size_t)teams * (lin ? s->clay : s->clay_solve).total * 8);
+        if (smem_bytes) *smem_bytes = (int32_t)coop_smem(s->coop_blob_bytes, teams, lin ? s->clay : s->clay_solve);
         return TREPB_OK;
     }
     size_t smem = s->ks->specialized ? 0 : (size_t)s->blob_bytes;
     if (which == 2 && s->lin_stage_bytes) smem = s->lin_stage_bytes;
-    CU(s->ks->occupancy(which, s->block, smem, &b, &ki));
+    CU(s->ks->occupancy(which, false, s->block, smem, &b, &ki));
     if (regs) *regs = ki.regs;
     if (local_bytes) *local_bytes = (int32_t)ki.local_bytes;
     if (blocks_per_sm) *blocks_per_sm = b;
@@ -392,33 +394,42 @@ int trepb_kernel_info(trepb_system* s, int which, int32_t* regs, int32_t* local_
 // ---------------------------------------------------------------------------------------------
 namespace {
 
+// Grid of a launch whose threads each own a column of a workspace slab of `elem_bytes` x `elems` per thread:
+// *grid capped at `resident` CTAs and at ws_grid_cap, and the slab kept within a quarter of the free memory
+// (`reclaim`: bytes of handle buffers this launch may reuse, counted as free).  Sizes `slab` to fit.
+int slab_grid(long long* grid, long long resident, int elems, size_t elem_bytes, int block, size_t reclaim, DevBuf& slab,
+              const char* what) {
+    if (*grid > resident) *grid = resident;
+    if (*grid > ws_grid_cap(elems, block)) *grid = ws_grid_cap(elems, block);
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
+    const size_t per_cta = (size_t)elems * elem_bytes * block;
+    const size_t budget = (free_b + reclaim) / 4;
+    if ((size_t)*grid * per_cta > budget) *grid = (long long)(budget / per_cta);
+    if (*grid < 1) return fail(TREPB_ERR_CUDA, std::string("not enough device memory for the ") + what);
+    CU(slab.ensure((size_t)*grid * per_cta));
+    return TREPB_OK;
+}
+
 // grid for `batch` instances at `bps` resident CTAs per SM; for the general path also sizes the
 // workspace slab (one column per launched thread).
-int make_cfg(trepb_system* s, int which, long long batch, int bps, size_t smem, cudaStream_t stream, LaunchCfg* c) {
+int make_cfg(trepb_system* s, int which, bool varied, long long batch, int bps, size_t smem, cudaStream_t stream,
+             LaunchCfg* c) {
     int block = s->block;
     if (!s->ks->specialized) {
         // small batches of big systems: narrower CTAs so that every SM gets work
         while (block > 32 && (batch + block - 1) / block < 2LL * s->sms) block /= 2;
         if (block != s->block) {
             int b = 0;
-            CU(s->ks->occupancy(which, block, smem, &b, nullptr));
+            CU((varied ? s->vks : s->ks)->occupancy(which, varied, block, smem, &b, nullptr));
             bps = b > 0 ? b : 1;
         }
     }
-    const long long need = (batch + block - 1) / block;
-    long long grid = need;
+    long long grid = (batch + block - 1) / block;
     if (!s->ks->specialized) {
-        long long resident = (long long)s->sms * bps;
-        if (grid > resident) grid = resident;
-        if (grid > ws_grid_cap(s->ws_doubles, block)) grid = ws_grid_cap(s->ws_doubles, block);
-        // keep the slab within a quarter of the free memory
-        size_t free_b = 0, total_b = 0;
-        CU(cudaMemGetInfo(&free_b, &total_b));
-        const size_t per_cta = (size_t)s->ws_doubles * sizeof(double) * block;
-        const size_t budget = (free_b + s->ws.cap) / 4;
-        if ((size_t)grid * per_cta > budget) grid = (long long)(budget / per_cta);
-        if (grid < 1) return fail(TREPB_ERR_CUDA, "not enough device memory for the workspace slab");
-        CU(s->ws.ensure((size_t)grid * per_cta));
+        if (int rc = slab_grid(&grid, (long long)s->sms * bps, s->ws_doubles, sizeof(double), block, s->ws.cap, s->ws,
+                               "workspace slab"))
+            return rc;
     } else {
         if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;
     }
@@ -447,7 +458,7 @@ void make_coop(trepb_system* s, long long batch, cudaStream_t stream, CoopLaunch
     if (grid > s->sms) grid = s->sms;
     c->grid = (int)grid;
     c->warps = warps;
-    c->smem = (size_t)(((s->coop_blob_bytes + 7) / 8 + 1) & ~1) * 8 + (size_t)warps * lay.total * 8;
+    c->smem = coop_smem(s->coop_blob_bytes, warps, lay);
     c->stream = stream;
     c->sys = s->cview;
     c->blob_bytes = s->coop_blob_bytes;
@@ -498,10 +509,10 @@ int varied_setup(trepb_system* s, const trepb_varied* v, cudaStream_t stream, Va
         const size_t smem = s->vks->specialized ? 0 : (size_t)s->blob_bytes;
         for (int w = 0; w < 4; ++w) {
             int b = 0;
-            CU(s->vks->occupancy_v(w, s->block, smem, &b, nullptr));
+            CU(s->vks->occupancy(w, true, s->block, smem, &b, nullptr));
             s->vbps[w] = b > 0 ? b : 1;
         }
-        if (s->lin_stage_bytes) CU(s->vks->occupancy_v(2, s->block, s->lin_stage_bytes, &s->vlin_bps_staged, nullptr));
+        if (s->lin_stage_bytes) CU(s->vks->occupancy(2, true, s->block, s->lin_stage_bytes, &s->vlin_bps_staged, nullptr));
         s->vinit = true;
     }
     VariedHost H;
@@ -533,13 +544,42 @@ int varied_slots(trepb_system* s, const LaunchCfg& c, VariedArgs* va) {
     return TREPB_OK;
 }
 
-}  // namespace
+// Launches one call (which: 0 step, 1 p2, 2 lin, 3 project) on the kernels `v` and the handle select: the
+// run-time-parameter kernels for per-instance parameters, else the cooperative kernels of a cooperative handle,
+// else one thread per instance.  thread(ks, cfg, va) and coop(cl) launch the call's kernel.  stage (linearize with
+// A or B, else null): set to 1 when the outputs are staged through shared memory.  The caller holds s->mu.
+template <class Thread, class Coop>
+int dispatch(trepb_system* s, int which, long long batch, cudaStream_t stream, const trepb_varied* v, int* stage,
+             Thread thread, Coop coop) {
+    if (!v && s->coop) {
+        CoopLaunch cl;
+        make_coop(s, batch, stream, &cl, which != 2);
+        ScratchGuard sg(s, stream, cl.lay.ext != 0);   // ext flavours: slabs owned by the handle
+        if (int rc = attach_slabs(s, &cl)) return rc;
+        Timed t(s, cl.stream);
+        CU(coop(cl));
+        return TREPB_OK;
+    }
+    ScratchGuard sg(s, stream, v || !s->ks->specialized);
+    VariedArgs va;
+    if (v)
+        if (int rc = varied_setup(s, v, stream, &va)) return rc;
+    const int bps_staged = v ? s->vlin_bps_staged : s->lin_bps_staged;
+    const bool staged = stage && s->lin_stage_bytes > 0 && bps_staged > 0;
+    if (stage) *stage = staged ? 1 : 0;
+    const size_t smem = s->ks->specialized ? (staged ? s->lin_stage_bytes : 0) : (size_t)s->blob_bytes;
+    LaunchCfg c;
+    const int bps = staged ? bps_staged : (v ? s->vbps : s->bps)[which];
+    if (int rc = make_cfg(s, which, v != nullptr, batch, bps, smem, stream, &c)) return rc;
+    // persistent-style grid: the staged kernel loops with a warp-uniform bound
+    if (staged && c.grid > (long long)s->sms * bps_staged) c.grid = (int)((long long)s->sms * bps_staged);
+    if (v)
+        if (int rc = varied_slots(s, c, &va)) return rc;
+    Timed t(s, c.stream);
+    CU(thread(v ? s->vks : s->ks, c, v ? &va : nullptr));
+    return TREPB_OK;
+}
 
-extern "C" {
-
-}  // extern "C"
-
-namespace {
 int step_launch(trepb_system* s, const trepb_step_args* a, void* stream, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     const RtSys& ps = s->P.proto;
@@ -561,53 +601,11 @@ int step_launch(trepb_system* s, const trepb_step_args* a, void* stream, const t
     p.nsamples = a->sample_every > 0 ? a->nsteps / a->sample_every : 0;
     p.traj_q = a->traj_q; p.traj_p = a->traj_p;
     p.times = a->times;
-    if (v) {
-        ScratchGuard sg(s, (cudaStream_t)stream, true);
-        VariedArgs va;
-        LaunchCfg c;
-        int rc = varied_setup(s, v, (cudaStream_t)stream, &va);
-        if (!rc) rc = make_cfg(s, 0, a->batch, s->vbps[0], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
-        if (!rc) rc = varied_slots(s, c, &va);
-        if (rc) return rc;
-        Timed t(s, c.stream);
-        CU(s->vks->step_v(c, p, va));
-        return TREPB_OK;
-    }
-    if (s->coop) {
-        CoopLaunch cl;
-        make_coop(s, a->batch, (cudaStream_t)stream, &cl, true);
-        ScratchGuard sg(s, (cudaStream_t)stream, cl.lay.ext != 0);   // ext flavours: slabs owned by the handle
-        if (int rc = attach_slabs(s, &cl)) return rc;
-        Timed t(s, cl.stream);
-        CU(s->cks->step(cl, p));
-        return TREPB_OK;
-    }
-    LaunchCfg c;
-    ScratchGuard sg(s, (cudaStream_t)stream, !s->ks->specialized);
-    int rc = make_cfg(s, 0, a->batch, s->bps[0], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
-    if (rc) return rc;
-    Timed t(s, c.stream);
-    CU(s->ks->step(c, p));
-    return TREPB_OK;
-}
-}  // namespace
-
-extern "C" {
-
-int trepb_step_batch_dev(trepb_system* s, const trepb_step_args* a, void* stream) {
-    TREPB_NVTX("trepb_step_batch_dev");
-    return step_launch(s, a, stream, nullptr);
+    return dispatch(s, 0, a->batch, (cudaStream_t)stream, v, nullptr,
+                    [&](const KernelSet* ks, const LaunchCfg& c, const VariedArgs* va) { return ks->step(c, p, va); },
+                    [&](const CoopLaunch& cl) { return s->cks->step(cl, p); });
 }
 
-int trepb_step_varied_batch_dev(trepb_system* s, const trepb_step_args* a, const trepb_varied* v, void* stream) {
-    TREPB_NVTX("trepb_step_varied_batch_dev");
-    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
-    return step_launch(s, a, stream, v);
-}
-
-}  // extern "C"
-
-namespace {
 int project_launch(trepb_system* s, const trepb_project_args* a, void* stream, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     if (a->batch < 0 || a->nsteps < 1) return fail(TREPB_ERR_INVALID, "batch must be >= 0 and nsteps >= 1");
@@ -625,169 +623,50 @@ int project_launch(trepb_system* s, const trepb_project_args* a, void* stream, c
     p.bX = a->bX; p.bU = a->bU; p.K = a->Kfb; p.k_per_instance = a->k_per_instance; p.use_hint = a->use_hint;
     p.X = a->X; p.U = a->U; p.iters = a->iters; p.status = a->status; p.fail_step = a->fail_step;
     p.times = a->times;
-    if (v) {
-        ScratchGuard sg(s, (cudaStream_t)stream, true);
-        VariedArgs va;
-        LaunchCfg c;
-        int rc = varied_setup(s, v, (cudaStream_t)stream, &va);
-        if (!rc) rc = make_cfg(s, 3, a->batch, s->vbps[3], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
-        if (!rc) rc = varied_slots(s, c, &va);
-        if (rc) return rc;
-        Timed t(s, c.stream);
-        CU(s->vks->proj_v(c, p, va));
-        return TREPB_OK;
-    }
-    if (s->coop) {
-        CoopLaunch cl;
-        make_coop(s, a->batch, (cudaStream_t)stream, &cl, true);
-        ScratchGuard sg(s, (cudaStream_t)stream, cl.lay.ext != 0);   // ext flavours: slabs owned by the handle
-        if (int rc = attach_slabs(s, &cl)) return rc;
-        Timed t(s, cl.stream);
-        CU(s->cks->proj(cl, p));
-        return TREPB_OK;
-    }
-    LaunchCfg c;
-    ScratchGuard sg(s, (cudaStream_t)stream, !s->ks->specialized);
-    int rc = make_cfg(s, 3, a->batch, s->bps[3], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
-    if (rc) return rc;
-    Timed t(s, c.stream);
-    CU(s->ks->proj(c, p));
-    return TREPB_OK;
-}
-}  // namespace
-
-extern "C" {
-
-int trepb_project_batch_dev(trepb_system* s, const trepb_project_args* a, void* stream) {
-    TREPB_NVTX("trepb_project_batch_dev");
-    return project_launch(s, a, stream, nullptr);
+    return dispatch(s, 3, a->batch, (cudaStream_t)stream, v, nullptr,
+                    [&](const KernelSet* ks, const LaunchCfg& c, const VariedArgs* va) { return ks->proj(c, p, va); },
+                    [&](const CoopLaunch& cl) { return s->cks->proj(cl, p); });
 }
 
-int trepb_project_varied_batch_dev(trepb_system* s, const trepb_project_args* a, const trepb_varied* v, void* stream) {
-    TREPB_NVTX("trepb_project_varied_batch_dev");
-    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
-    return project_launch(s, a, stream, v);
-}
-
-}  // extern "C"
-
-namespace {
 // calc_p2 / calc_f / discrete_fm2 share one kernel (P2Params::mode); the caller has validated the pointers
-int eval_launch(trepb_system* s, const P2Params& p, void* stream, const trepb_varied* v = nullptr) {
+int eval_launch(trepb_system* s, const P2Params& p, void* stream, const trepb_varied* v) {
     if (p.batch == 0) return TREPB_OK;
     std::lock_guard<std::mutex> lk(s->mu);
     CU(cudaSetDevice(s->device));
-    if (v) {
-        ScratchGuard sg(s, (cudaStream_t)stream, true);
-        VariedArgs va;
-        LaunchCfg c;
-        int rc = varied_setup(s, v, (cudaStream_t)stream, &va);
-        if (!rc) rc = make_cfg(s, 1, p.batch, s->vbps[1], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
-        if (!rc) rc = varied_slots(s, c, &va);
-        if (rc) return rc;
-        Timed t(s, c.stream);
-        CU(s->vks->p2_v(c, p, va));
-        return TREPB_OK;
-    }
-    if (s->coop) {
-        CoopLaunch cl;
-        make_coop(s, p.batch, (cudaStream_t)stream, &cl, true);
-        ScratchGuard sg(s, (cudaStream_t)stream, cl.lay.ext != 0);   // ext flavours: slabs owned by the handle
-        if (int rc = attach_slabs(s, &cl)) return rc;
-        Timed t(s, cl.stream);
-        CU(s->cks->p2(cl, p));
-        return TREPB_OK;
-    }
-    LaunchCfg c;
-    ScratchGuard sg(s, (cudaStream_t)stream, !s->ks->specialized);
-    int rc = make_cfg(s, 1, p.batch, s->bps[1], s->ks->specialized ? 0 : (size_t)s->blob_bytes, (cudaStream_t)stream, &c);
-    if (rc) return rc;
-    Timed t(s, c.stream);
-    CU(s->ks->p2(c, p));
-    return TREPB_OK;
+    return dispatch(s, 1, p.batch, (cudaStream_t)stream, v, nullptr,
+                    [&](const KernelSet* ks, const LaunchCfg& c, const VariedArgs* va) { return ks->p2(c, p, va); },
+                    [&](const CoopLaunch& cl) { return s->cks->p2(cl, p); });
 }
-}  // namespace
 
-extern "C" {
-
-int trepb_calc_p2_batch_dev(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1,
-                            double* pout, void* stream) {
-    TREPB_NVTX("trepb_calc_p2_batch_dev");
+int calc_p2_dev(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1, double* pout,
+                const trepb_varied* v, void* stream) {
     if (!s || !q0 || !q1 || !pout) return fail(TREPB_ERR_INVALID, "null argument");
     if (batch < 0 || !(dt != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or dt");
     P2Params p{};
     p.batch = batch; p.dt = dt; p.q0 = q0; p.q1 = q1; p.p = pout; p.mode = 0;
-    return eval_launch(s, p, stream);
+    return eval_launch(s, p, stream, v);
 }
 
-int trepb_calc_f_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1, const double* q2,
-                           const double* p1, const double* u1, const double* lambda1, double* f, void* stream) {
-    TREPB_NVTX("trepb_calc_f_batch_dev");
+int calc_f_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1, const double* q2,
+               const double* p1, const double* u1, const double* lambda1, double* f, const trepb_varied* v, void* stream) {
     if (!s || !q1 || !q2 || !p1 || !f) return fail(TREPB_ERR_INVALID, "null argument");
     if (batch < 0 || !(t2 - t1 != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or t2 == t1");
     P2Params p{};
     p.batch = batch; p.dt = t2 - t1; p.q0 = q1; p.q1 = q2; p.p = f; p.mode = 1;
     p.p1 = p1; p.u1 = s->P.proto.nu ? u1 : nullptr; p.lam = s->P.proto.nc ? lambda1 : nullptr;
-    return eval_launch(s, p, stream);
+    return eval_launch(s, p, stream, v);
 }
 
-int trepb_discrete_fm2_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
-                                 const double* q2, const double* u1, double* fm2, void* stream) {
-    TREPB_NVTX("trepb_discrete_fm2_batch_dev");
+int discrete_fm2_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1, const double* q2,
+                     const double* u1, double* fm2, const trepb_varied* v, void* stream) {
     if (!s || !q1 || !q2 || !fm2) return fail(TREPB_ERR_INVALID, "null argument");
     if (batch < 0 || !(t2 - t1 != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or t2 == t1");
     P2Params p{};
     p.batch = batch; p.dt = t2 - t1; p.q0 = q1; p.q1 = q2; p.p = fm2; p.mode = 2;
     p.u1 = s->P.proto.nu ? u1 : nullptr;
-    return eval_launch(s, p, stream);
-}
-
-int trepb_calc_p2_varied_batch_dev(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1,
-                                   double* pout, const trepb_varied* v, void* stream) {
-    TREPB_NVTX("trepb_calc_p2_varied_batch_dev");
-    if (!s || !q0 || !q1 || !pout || !v) return fail(TREPB_ERR_INVALID, "null argument");
-    if (batch < 0 || !(dt != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or dt");
-    P2Params p{};
-    p.batch = batch; p.dt = dt; p.q0 = q0; p.q1 = q1; p.p = pout; p.mode = 0;
     return eval_launch(s, p, stream, v);
 }
 
-int trepb_calc_f_varied_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
-                                  const double* q2, const double* p1, const double* u1, const double* lambda1,
-                                  double* f, const trepb_varied* v, void* stream) {
-    TREPB_NVTX("trepb_calc_f_varied_batch_dev");
-    if (!s || !q1 || !q2 || !p1 || !f || !v) return fail(TREPB_ERR_INVALID, "null argument");
-    if (batch < 0 || !(t2 - t1 != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or t2 == t1");
-    P2Params p{};
-    p.batch = batch; p.dt = t2 - t1; p.q0 = q1; p.q1 = q2; p.p = f; p.mode = 1;
-    p.p1 = p1; p.u1 = s->P.proto.nu ? u1 : nullptr; p.lam = s->P.proto.nc ? lambda1 : nullptr;
-    return eval_launch(s, p, stream, v);
-}
-
-int trepb_discrete_fm2_varied_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
-                                        const double* q2, const double* u1, double* fm2, const trepb_varied* v,
-                                        void* stream) {
-    TREPB_NVTX("trepb_discrete_fm2_varied_batch_dev");
-    if (!s || !q1 || !q2 || !fm2 || !v) return fail(TREPB_ERR_INVALID, "null argument");
-    if (batch < 0 || !(t2 - t1 != 0.0)) return fail(TREPB_ERR_INVALID, "bad batch or t2 == t1");
-    P2Params p{};
-    p.batch = batch; p.dt = t2 - t1; p.q0 = q1; p.q1 = q2; p.p = fm2; p.mode = 2;
-    p.u1 = s->P.proto.nu ? u1 : nullptr;
-    return eval_launch(s, p, stream, v);
-}
-
-int trepb_varied_check(const trepb_sysdesc* desc, const trepb_varied* v) {
-    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
-    PackedSys P;
-    std::string err;
-    if (!pack_system(desc, &P, &err)) return fail(TREPB_ERR_INVALID, err);
-    if (!varied_check(P, v->n, v->table, v->index, &err)) return fail(TREPB_ERR_INVALID, err);
-    return TREPB_OK;
-}
-
-}  // extern "C"
-
-namespace {
 // validates + launches the linearize kernel; the caller holds s->mu
 int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, double* aux, int aux_size,
                const trepb_varied* v = nullptr) {
@@ -813,71 +692,106 @@ int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, do
     for (int i = 0; i < 12; ++i) p.raw[i] = raw[i];
     p.aux = aux; p.aux_size = aux_size;
     p.traj_len = a->traj_len;
-    if (v) {
-        ScratchGuard sg(s, stream, true);
-        VariedArgs va;
-        int rc = varied_setup(s, v, stream, &va);
-        if (rc) return rc;
-        const bool stage = s->lin_stage_bytes > 0 && s->vlin_bps_staged > 0 && (p.A || p.B);
-        p.stage = stage ? 1 : 0;
-        LaunchCfg c;
-        const size_t smem = s->ks->specialized ? (stage ? s->lin_stage_bytes : 0) : (size_t)s->blob_bytes;
-        rc = make_cfg(s, 2, a->batch, stage ? s->vlin_bps_staged : s->vbps[2], smem, stream, &c);
-        if (rc) return rc;
-        if (stage) {
-            long long resident = (long long)s->sms * s->vlin_bps_staged;
-            if (c.grid > resident) c.grid = (int)resident;
-        }
-        if ((rc = varied_slots(s, c, &va))) return rc;
-        Timed t(s, c.stream);
-        CU(s->vks->lin_v(c, p, va));
-        return TREPB_OK;
-    }
-    if (s->coop) {
-        p.stage = 0;
-        CoopLaunch cl;
-        make_coop(s, a->batch, stream, &cl, false);
-        AuxLayout al;
-        al.set(ps.nd, ps.nc);
-        // ext flavours: one slab per team of the persistent grid (handle scratch: ordered across streams)
-        ScratchGuard sg(s, stream, cl.lay.ext != 0);
-        if (int rc = attach_slabs(s, &cl)) return rc;
-        Timed t(s, cl.stream);
-        CU(s->cks->lin(cl, p, al));
-        return TREPB_OK;
-    }
-    const bool stage = s->lin_stage_bytes > 0 && (p.A || p.B);
-    p.stage = stage ? 1 : 0;
-    LaunchCfg c;
-    ScratchGuard sg(s, stream, !s->ks->specialized);
-    const size_t smem = s->ks->specialized ? (stage ? s->lin_stage_bytes : 0) : (size_t)s->blob_bytes;
-    int rc = make_cfg(s, 2, a->batch, stage ? s->lin_bps_staged : s->bps[2], smem, stream, &c);
-    if (rc) return rc;
-    if (stage) {
-        // persistent-style grid: the staged kernel loops with a warp-uniform bound
-        long long resident = (long long)s->sms * s->lin_bps_staged;
-        if (c.grid > resident) c.grid = (int)resident;
-    }
-    Timed t(s, c.stream);
-    CU(s->ks->lin(c, p));
-    return TREPB_OK;
+    p.stage = 0;
+    return dispatch(s, 2, a->batch, stream, v, (p.A || p.B) ? &p.stage : nullptr,
+                    [&](const KernelSet* ks, const LaunchCfg& c, const VariedArgs* va) { return ks->lin(c, p, va); },
+                    [&](const CoopLaunch& cl) {
+                        AuxLayout al;
+                        al.set(ps.nd, ps.nc);
+                        return s->cks->lin(cl, p, al);
+                    });
+}
+
+int lin_dev(trepb_system* s, const trepb_lin_args* a, void* stream, const trepb_varied* v) {
+    if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
+    std::lock_guard<std::mutex> lk(s->mu);
+    return lin_launch(s, a, (cudaStream_t)stream, nullptr, 0, v);
 }
 }  // namespace
 
 extern "C" {
 
+int trepb_step_batch_dev(trepb_system* s, const trepb_step_args* a, void* stream) {
+    TREPB_NVTX("trepb_step_batch_dev");
+    return step_launch(s, a, stream, nullptr);
+}
+
+int trepb_step_varied_batch_dev(trepb_system* s, const trepb_step_args* a, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_step_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return step_launch(s, a, stream, v);
+}
+
+int trepb_project_batch_dev(trepb_system* s, const trepb_project_args* a, void* stream) {
+    TREPB_NVTX("trepb_project_batch_dev");
+    return project_launch(s, a, stream, nullptr);
+}
+
+int trepb_project_varied_batch_dev(trepb_system* s, const trepb_project_args* a, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_project_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return project_launch(s, a, stream, v);
+}
+
+int trepb_calc_p2_batch_dev(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1,
+                            double* pout, void* stream) {
+    TREPB_NVTX("trepb_calc_p2_batch_dev");
+    return calc_p2_dev(s, batch, dt, q0, q1, pout, nullptr, stream);
+}
+
+int trepb_calc_p2_varied_batch_dev(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1,
+                                   double* pout, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_calc_p2_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null argument");
+    return calc_p2_dev(s, batch, dt, q0, q1, pout, v, stream);
+}
+
+int trepb_calc_f_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1, const double* q2,
+                           const double* p1, const double* u1, const double* lambda1, double* f, void* stream) {
+    TREPB_NVTX("trepb_calc_f_batch_dev");
+    return calc_f_dev(s, batch, t1, t2, q1, q2, p1, u1, lambda1, f, nullptr, stream);
+}
+
+int trepb_calc_f_varied_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                                  const double* q2, const double* p1, const double* u1, const double* lambda1,
+                                  double* f, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_calc_f_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null argument");
+    return calc_f_dev(s, batch, t1, t2, q1, q2, p1, u1, lambda1, f, v, stream);
+}
+
+int trepb_discrete_fm2_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                                 const double* q2, const double* u1, double* fm2, void* stream) {
+    TREPB_NVTX("trepb_discrete_fm2_batch_dev");
+    return discrete_fm2_dev(s, batch, t1, t2, q1, q2, u1, fm2, nullptr, stream);
+}
+
+int trepb_discrete_fm2_varied_batch_dev(trepb_system* s, int64_t batch, double t1, double t2, const double* q1,
+                                        const double* q2, const double* u1, double* fm2, const trepb_varied* v,
+                                        void* stream) {
+    TREPB_NVTX("trepb_discrete_fm2_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null argument");
+    return discrete_fm2_dev(s, batch, t1, t2, q1, q2, u1, fm2, v, stream);
+}
+
+int trepb_varied_check(const trepb_sysdesc* desc, const trepb_varied* v) {
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    PackedSys P;
+    std::string err;
+    if (!pack_system(desc, &P, &err)) return fail(TREPB_ERR_INVALID, err);
+    if (!varied_check(P, v->n, v->table, v->index, &err)) return fail(TREPB_ERR_INVALID, err);
+    return TREPB_OK;
+}
+
 int trepb_linearize_batch_dev(trepb_system* s, const trepb_lin_args* a, void* stream) {
     TREPB_NVTX("trepb_linearize_batch_dev");
-    if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
-    std::lock_guard<std::mutex> lk(s->mu);
-    return lin_launch(s, a, (cudaStream_t)stream, nullptr, 0);
+    return lin_dev(s, a, stream, nullptr);
 }
 
 int trepb_linearize_varied_batch_dev(trepb_system* s, const trepb_lin_args* a, const trepb_varied* v, void* stream) {
     TREPB_NVTX("trepb_linearize_varied_batch_dev");
-    if (!s || !a || !v) return fail(TREPB_ERR_INVALID, "null argument");
-    std::lock_guard<std::mutex> lk(s->mu);
-    return lin_launch(s, a, (cudaStream_t)stream, nullptr, 0, v);
+    if (!v) return fail(TREPB_ERR_INVALID, "null argument");
+    return lin_dev(s, a, stream, v);
 }
 
 int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream_) {
@@ -950,14 +864,10 @@ int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream
         if (nb < 1) return fail(TREPB_ERR_CUDA, "not enough device memory for the second-derivative table records");
         if (nb > B) nb = B;
         const int block = s->block;
-        const size_t per_cta = (size_t)s->ws_du_elems * sizeof(Dual) * block;
         long long grid = (nb * p.nx + block - 1) / block;
-        const long long resident = (long long)s->sms * s->bps_d2jac;
-        if (grid > resident) grid = resident;
-        if (grid > ws_grid_cap(s->ws_du_elems, block)) grid = ws_grid_cap(s->ws_du_elems, block);
-        if ((size_t)grid * per_cta > avail / 4) grid = (long long)((avail / 4) / per_cta);
-        if (grid < 1) return fail(TREPB_ERR_CUDA, "not enough device memory for the second-derivative workspace");
-        CU(s->ws_du.ensure((size_t)grid * per_cta));
+        if (int rc = slab_grid(&grid, (long long)s->sms * s->bps_d2jac, s->ws_du_elems, sizeof(Dual), block,
+                               s->ws_du.cap + s->d2g.cap, s->ws_du, "second-derivative workspace"))
+            return rc;
         CU(s->d2g.ensure((size_t)nb * per_inst));
         WsStridedT<Dual> wd = s->wsl_du;
         wd.base = (Dual*)s->ws_du.p; wd.stride = 0;
@@ -983,16 +893,9 @@ int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream
     WsStridedT<HDG> w = s->wsl_hd;
     w.base = nullptr; w.stride = 0;
     if (!s->ks->specialized) {
-        long long resident = (long long)s->sms * s->bps_d2;
-        if (grid > resident) grid = resident;
-        if (grid > ws_grid_cap(s->ws_hd_elems, block)) grid = ws_grid_cap(s->ws_hd_elems, block);
-        size_t free_b = 0, total_b = 0;
-        CU(cudaMemGetInfo(&free_b, &total_b));
-        const size_t per_cta = (size_t)s->ws_hd_elems * sizeof(HDG) * block;
-        const size_t budget = (free_b + s->ws_hd.cap) / 4;
-        if ((size_t)grid * per_cta > budget) grid = (long long)(budget / per_cta);
-        if (grid < 1) return fail(TREPB_ERR_CUDA, "not enough device memory for the second-derivative workspace");
-        CU(s->ws_hd.ensure((size_t)grid * per_cta));
+        if (int rc = slab_grid(&grid, (long long)s->sms * s->bps_d2, s->ws_hd_elems, sizeof(HDG), block, s->ws_hd.cap,
+                               s->ws_hd, "second-derivative workspace"))
+            return rc;
         w.base = (HDG*)s->ws_hd.p;
     } else if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;
     LaunchCfg c;
@@ -1093,6 +996,14 @@ struct Stager {
         outs[nout++] = {host, b.p, bytes};
         return (T*)b.p;
     }
+    // per-instance parameters: `rows` rows of v->n values
+    trepb_varied dv{};
+    const trepb_varied* varied(const trepb_varied* v, size_t rows) {
+        if (!v) return nullptr;
+        dv = *v;
+        dv.values = in(v->values, rows * v->n);
+        return &dv;
+    }
     int finish() {
         for (int i = 0; i < nout; ++i)
             if (outs[i].bytes) CU(cudaMemcpyAsync(outs[i].host, outs[i].dev, outs[i].bytes, cudaMemcpyDeviceToHost, 0));
@@ -1119,8 +1030,10 @@ struct Pipe {
         arr[n++] = {(const char*)hin, (char*)hout, (char*)b.p, per_bytes};
         return (char*)b.p;
     }
-    template <class T> const T* in(const T* host, size_t per) { return host ? (const T*)reg(host, nullptr, per * sizeof(T)) : nullptr; }
-    template <class T> T* out(T* host, size_t per) { return host ? (T*)reg(nullptr, host, per * sizeof(T)) : nullptr; }
+    static constexpr bool kIn = true, kOut = false;
+    template <class T> void field(T*& p, size_t per, bool input) {
+        if (p) p = (T*)reg(input ? (const void*)p : nullptr, input ? nullptr : (void*)p, per * sizeof(T));
+    }
     static int chunks(size_t B) { return B >= 4 * 65536 ? 4 : (B >= 2 * 65536 ? 2 : 1); }
     int streams() {
         for (int i = 0; i < 2; ++i)
@@ -1147,73 +1060,72 @@ struct Pipe {
         for (int i = 0; i < 2; ++i) CU(cudaStreamSynchronize(s->hs[i]));
         return TREPB_OK;
     }
+    // Runs launch(&args, varied, stream) on C_ chunks.  fields(x, f) calls f(x.member, elements per instance,
+    // kIn or kOut) for every per-instance array of x; the parameter rows of v (one per instance) are chunked too.
+    template <class Args, class Fields, class Launch>
+    int run(Args d, const trepb_varied* v, int C_, Fields fields, Launch launch) {
+        fields(d, [&](auto& p, size_t per, bool input) { field(p, per, input); });
+        trepb_varied dv{};
+        if (v) { dv = *v; field(dv.values, (size_t)v->n, kIn); }
+        if (err) return err;
+        int rc = streams();
+        if (rc) return rc;
+        for (int c = 0; c < C_; ++c) {
+            const size_t lo = B * c / C_, hi = B * (c + 1) / C_, cnt = hi - lo;
+            cudaStream_t st = s->hs[c & 1];
+            if ((rc = upload(lo, cnt, st))) return rc;
+            Args e = d;
+            e.batch = (int64_t)cnt;
+            fields(e, [&](auto& p, size_t per, bool) { if (p) p += lo * per; });
+            trepb_varied ev = dv;
+            if (ev.values) ev.values += lo * (size_t)v->n;
+            if ((rc = launch(&e, v ? &ev : nullptr, st))) return rc;
+            if ((rc = download(lo, cnt, st))) return rc;
+        }
+        return finish();
+    }
 };
 }  // namespace
 
 extern "C" {
-
-static int step_batch_chunked(trepb_system* s, const trepb_step_args* a, int C_, const trepb_varied* v) {
-    const RtSys& ps = s->P.proto;
-    const size_t B = (size_t)a->batch, nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc, K = (size_t)a->nsteps;
-    const size_t ns = a->sample_every > 0 ? (size_t)(a->nsteps / a->sample_every) : 0;
-    Pipe pp(s, B);
-    trepb_step_args d = *a;
-    d.q1 = pp.in(a->q1, nq); d.p1 = pp.in(a->p1, nd); d.u1 = pp.in(a->u1, K * nu); d.k2 = pp.in(a->k2, K * nk);
-    d.q2_guess = pp.in(a->q2_guess, nd); d.lambda_guess = pp.in(a->lambda_guess, nc);
-    d.q2 = pp.out(a->q2, nq); d.p2 = pp.out(a->p2, nd); d.lambda1 = pp.out(a->lambda1, nc);
-    d.iters = pp.out(a->iters, 1); d.status = pp.out(a->status, 1);
-    d.traj_q = pp.out(a->traj_q, ns * nq); d.traj_p = pp.out(a->traj_p, ns * nd);
-    trepb_varied dv{};
-    if (v) { dv = *v; dv.values = pp.in(v->values, (size_t)v->n); }   // one row per instance: chunked like q1
-    if (pp.err) return pp.err;
-    int rc = pp.streams();
-    if (rc) return rc;
-    if (a->times) {   // shared by every chunk: up before either stream starts
-        DevBuf& tb = s->hb[pp.k++];
-        CU(tb.ensure((K + 1) * sizeof(double)));
-        CU(cudaMemcpy(tb.p, a->times, (K + 1) * sizeof(double), cudaMemcpyHostToDevice));
-        d.times = (const double*)tb.p;
-    }
-    for (int c = 0; c < C_; ++c) {
-        const size_t lo = B * c / C_, hi = B * (c + 1) / C_, cnt = hi - lo;
-        cudaStream_t st = s->hs[c & 1];
-        if ((rc = pp.upload(lo, cnt, st))) return rc;
-        trepb_step_args e = d;
-        e.batch = (int64_t)cnt;
-#define OFF(f, per) if (e.f) e.f += lo * (per)
-        OFF(q1, nq); OFF(p1, nd); OFF(u1, K * nu); OFF(k2, K * nk); OFF(q2_guess, nd); OFF(lambda_guess, nc);
-        OFF(q2, nq); OFF(p2, nd); OFF(lambda1, nc); OFF(iters, 1); OFF(status, 1); OFF(traj_q, ns * nq); OFF(traj_p, ns * nd);
-#undef OFF
-        trepb_varied ev = dv;
-        if (ev.values) ev.values += lo * (size_t)v->n;
-        if ((rc = v ? trepb_step_varied_batch_dev(s, &e, &ev, st) : trepb_step_batch_dev(s, &e, st))) return rc;
-        if ((rc = pp.download(lo, cnt, st))) return rc;
-    }
-    return pp.finish();
-}
 
 static int step_host(trepb_system* s, const trepb_step_args* a, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (a->batch < 0 || a->nsteps < 1) return fail(TREPB_ERR_INVALID, "batch must be >= 0 and nsteps >= 1");
     const RtSys& ps = s->P.proto;
-    const size_t B = (size_t)a->batch, nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc;
+    const size_t B = (size_t)a->batch, nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc, K = (size_t)a->nsteps;
+    const size_t ns = a->sample_every > 0 ? (size_t)(a->nsteps / a->sample_every) : 0;
     CU(cudaSetDevice(s->device));
-    if (const int C_ = Pipe::chunks(B); C_ > 1 && a->q1 && a->p1 && a->q2 && a->p2 && a->status) return step_batch_chunked(s, a, C_, v);
+    if (const int C_ = Pipe::chunks(B); C_ > 1 && a->q1 && a->p1 && a->q2 && a->p2 && a->status) {
+        Pipe pp(s, B);
+        trepb_step_args d = *a;
+        if (a->times) {   // shared by every chunk: up before either stream starts
+            DevBuf& tb = s->hb[pp.k++];
+            CU(tb.ensure((K + 1) * sizeof(double)));
+            CU(cudaMemcpy(tb.p, a->times, (K + 1) * sizeof(double), cudaMemcpyHostToDevice));
+            d.times = (const double*)tb.p;
+        }
+        constexpr bool kIn = Pipe::kIn, kOut = Pipe::kOut;
+        return pp.run(d, v, C_, [&](trepb_step_args& x, auto&& f) {
+            f(x.q1, nq, kIn); f(x.p1, nd, kIn); f(x.u1, K * nu, kIn); f(x.k2, K * nk, kIn);
+            f(x.q2_guess, nd, kIn); f(x.lambda_guess, nc, kIn);
+            f(x.q2, nq, kOut); f(x.p2, nd, kOut); f(x.lambda1, nc, kOut); f(x.iters, 1, kOut); f(x.status, 1, kOut);
+            f(x.traj_q, ns * nq, kOut); f(x.traj_p, ns * nd, kOut);
+        }, [&](const trepb_step_args* e, const trepb_varied* ev, cudaStream_t st) { return step_launch(s, e, st, ev); });
+    }
     Stager st(s);
     trepb_step_args d = *a;
     d.q1 = st.in(a->q1, B * nq); d.p1 = st.in(a->p1, B * nd);
-    d.u1 = st.in(a->u1, B * a->nsteps * nu); d.k2 = st.in(a->k2, B * a->nsteps * nk);
+    d.u1 = st.in(a->u1, B * K * nu); d.k2 = st.in(a->k2, B * K * nk);
     d.q2_guess = st.in(a->q2_guess, B * nd); d.lambda_guess = st.in(a->lambda_guess, B * nc);
     d.q2 = st.out(a->q2, B * nq); d.p2 = st.out(a->p2, B * nd); d.lambda1 = st.out(a->lambda1, B * nc);
     d.iters = st.out(a->iters, B); d.status = st.out(a->status, B);
-    const size_t ns = a->sample_every > 0 ? (size_t)(a->nsteps / a->sample_every) : 0;
     d.traj_q = st.out(a->traj_q, B * ns * nq); d.traj_p = st.out(a->traj_p, B * ns * nd);
-    d.times = st.in(a->times, (size_t)a->nsteps + 1);
-    trepb_varied dv{};
-    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
+    d.times = st.in(a->times, K + 1);
+    const trepb_varied* dv = st.varied(v, B);
     if (st.err) return st.err;
-    int rc = v ? trepb_step_varied_batch_dev(s, &d, &dv, nullptr) : trepb_step_batch_dev(s, &d, nullptr);
+    int rc = step_launch(s, &d, nullptr, dv);
     if (rc) return rc;
     return st.finish();
 }
@@ -1243,10 +1155,9 @@ static int project_host(trepb_system* s, const trepb_project_args* a, const trep
     d.X = st.out(a->X, B * (K + 1) * nX); d.U = st.out(a->U, B * K * nU);
     d.iters = st.out(a->iters, B); d.status = st.out(a->status, B); d.fail_step = st.out(a->fail_step, B);
     d.times = st.in(a->times, K + 1);
-    trepb_varied dv{};
-    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
+    const trepb_varied* dv = st.varied(v, B);
     if (st.err) return st.err;
-    int rc = v ? trepb_project_varied_batch_dev(s, &d, &dv, nullptr) : trepb_project_batch_dev(s, &d, nullptr);
+    int rc = project_launch(s, &d, nullptr, dv);
     if (rc) return rc;
     return st.finish();
 }
@@ -1274,11 +1185,9 @@ static int calc_p2_host(trepb_system* s, int64_t batch, double dt, const double*
     const double* dq0 = st.in(q0, B * nq);
     const double* dq1 = st.in(q1, B * nq);
     double* dp = st.out(p, B * ps.nd);
-    trepb_varied dv{};
-    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
+    const trepb_varied* dv = st.varied(v, B);
     if (st.err) return st.err;
-    int rc = v ? trepb_calc_p2_varied_batch_dev(s, batch, dt, dq0, dq1, dp, &dv, nullptr)
-               : trepb_calc_p2_batch_dev(s, batch, dt, dq0, dq1, dp, nullptr);
+    int rc = calc_p2_dev(s, batch, dt, dq0, dq1, dp, dv, nullptr);
     if (rc) return rc;
     return st.finish();
 }
@@ -1307,11 +1216,9 @@ static int calc_f_host(trepb_system* s, int64_t batch, double t1, double t2, con
     const double* dq1 = st.in(q1, B * nq); const double* dq2 = st.in(q2, B * nq); const double* dp1 = st.in(p1, B * ps.nd);
     const double* du = st.in(u1, B * ps.nu); const double* dl = st.in(lambda1, B * ps.nc);
     double* df = st.out(f, B * (ps.nd + ps.nc));
-    trepb_varied dv{};
-    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
+    const trepb_varied* dv = st.varied(v, B);
     if (st.err) return st.err;
-    int rc = v ? trepb_calc_f_varied_batch_dev(s, batch, t1, t2, dq1, dq2, dp1, du, dl, df, &dv, nullptr)
-               : trepb_calc_f_batch_dev(s, batch, t1, t2, dq1, dq2, dp1, du, dl, df, nullptr);
+    int rc = calc_f_dev(s, batch, t1, t2, dq1, dq2, dp1, du, dl, df, dv, nullptr);
     if (rc) return rc;
     return st.finish();
 }
@@ -1342,11 +1249,9 @@ static int discrete_fm2_host(trepb_system* s, int64_t batch, double t1, double t
     const double* dq1 = st.in(q1, B * nq); const double* dq2 = st.in(q2, B * nq);
     const double* du = st.in(u1, B * ps.nu);
     double* df = st.out(fm2, B * ps.nd);
-    trepb_varied dv{};
-    if (v) { dv = *v; dv.values = st.in(v->values, B * v->n); }
+    const trepb_varied* dv = st.varied(v, B);
     if (st.err) return st.err;
-    int rc = v ? trepb_discrete_fm2_varied_batch_dev(s, batch, t1, t2, dq1, dq2, du, df, &dv, nullptr)
-               : trepb_discrete_fm2_batch_dev(s, batch, t1, t2, dq1, dq2, du, df, nullptr);
+    int rc = discrete_fm2_dev(s, batch, t1, t2, dq1, dq2, du, df, dv, nullptr);
     if (rc) return rc;
     return st.finish();
 }
@@ -1421,66 +1326,33 @@ int trepb_deriv2_batch(trepb_system* s, const trepb_d2_args* a) {
     return st.finish();
 }
 
-// trepb_linearize_batch for a large plain batch (no trajectory rows): chunks alternating between two streams (Pipe)
-static int lin_batch_chunked(trepb_system* s, const trepb_lin_args* a, int C_, const trepb_varied* v) {
-    const RtSys& ps = s->P.proto;
-    const size_t B = (size_t)a->batch, nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc;
-    const size_t nX = 2 * nq, nU = nu + nk;
-    Pipe pp(s, B);
-    trepb_lin_args d = *a;
-    // (member, elements per instance): inputs first, then outputs
-#define TREPB_LIN_IN(X) X(t1, 1) X(t2, 1) X(q1, nq) X(p1, nd) X(u1, nu) X(k2, nk) X(q2_guess, nd) X(lambda_guess, nc)
-#define TREPB_LIN_OUT(X) X(q2, nq) X(p2, nd) X(lambda1, nc) X(iters, 1) X(status, 1) X(A, nX * nX) X(B, nX * nU) \
-    X(q2_dq1, nq * nd) X(q2_dp1, nd * nd) X(q2_du1, nu * nd) X(q2_dk2, nk * nd) X(p2_dq1, nq * nd) X(p2_dp1, nd * nd) \
-    X(p2_du1, nu * nd) X(p2_dk2, nk * nd) X(l1_dq1, nq * nc) X(l1_dp1, nd * nc) X(l1_du1, nu * nc) X(l1_dk2, nk * nc)
-#define X(f, per) d.f = pp.in(a->f, (per));
-    TREPB_LIN_IN(X)
-#undef X
-#define X(f, per) d.f = pp.out(a->f, (per));
-    TREPB_LIN_OUT(X)
-#undef X
-    trepb_varied dv{};
-    if (v) { dv = *v; dv.values = pp.in(v->values, (size_t)v->n); }   // one row per instance (no trajectory rows here)
-    if (pp.err) return pp.err;
-    int rc = pp.streams();
-    if (rc) return rc;
-    for (int c = 0; c < C_; ++c) {
-        const size_t lo = B * c / C_, hi = B * (c + 1) / C_, cnt = hi - lo;
-        cudaStream_t st = s->hs[c & 1];
-        if ((rc = pp.upload(lo, cnt, st))) return rc;
-        trepb_lin_args e = d;
-        e.batch = (int64_t)cnt;
-#define X(f, per) if (e.f) e.f += lo * (per);
-        TREPB_LIN_IN(X) TREPB_LIN_OUT(X)
-#undef X
-#undef TREPB_LIN_IN
-#undef TREPB_LIN_OUT
-        trepb_varied ev = dv;
-        if (ev.values) ev.values += lo * (size_t)v->n;
-        if ((rc = v ? trepb_linearize_varied_batch_dev(s, &e, &ev, st) : trepb_linearize_batch_dev(s, &e, st))) return rc;
-        if ((rc = pp.download(lo, cnt, st))) return rc;
-    }
-    return pp.finish();
-}
-
 static int lin_host(trepb_system* s, const trepb_lin_args* a, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (a->batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
     CU(cudaSetDevice(s->device));
-    if (const int C_ = Pipe::chunks((size_t)a->batch); C_ > 1 && a->traj_len <= 1 && a->q1 && a->p1 && a->status)
-        return lin_batch_chunked(s, a, C_, v);
+    // a large plain batch (no trajectory rows): chunks alternating between two streams (Pipe)
+    if (const int C_ = Pipe::chunks((size_t)a->batch); C_ > 1 && a->traj_len <= 1 && a->q1 && a->p1 && a->status) {
+        const RtSys& ps = s->P.proto;
+        const size_t nq = ps.nd + ps.nk, nd = ps.nd, nu = ps.nu, nk = ps.nk, nc = ps.nc, nX = 2 * nq, nU = nu + nk;
+        constexpr bool kIn = Pipe::kIn, kOut = Pipe::kOut;
+        return Pipe(s, (size_t)a->batch).run(*a, v, C_, [&](trepb_lin_args& x, auto&& f) {
+            f(x.t1, 1, kIn); f(x.t2, 1, kIn); f(x.q1, nq, kIn); f(x.p1, nd, kIn); f(x.u1, nu, kIn); f(x.k2, nk, kIn);
+            f(x.q2_guess, nd, kIn); f(x.lambda_guess, nc, kIn);
+            f(x.q2, nq, kOut); f(x.p2, nd, kOut); f(x.lambda1, nc, kOut); f(x.iters, 1, kOut); f(x.status, 1, kOut);
+            f(x.A, nX * nX, kOut); f(x.B, nX * nU, kOut);
+            f(x.q2_dq1, nq * nd, kOut); f(x.q2_dp1, nd * nd, kOut); f(x.q2_du1, nu * nd, kOut); f(x.q2_dk2, nk * nd, kOut);
+            f(x.p2_dq1, nq * nd, kOut); f(x.p2_dp1, nd * nd, kOut); f(x.p2_du1, nu * nd, kOut); f(x.p2_dk2, nk * nd, kOut);
+            f(x.l1_dq1, nq * nc, kOut); f(x.l1_dp1, nd * nc, kOut); f(x.l1_du1, nu * nc, kOut); f(x.l1_dk2, nk * nc, kOut);
+        }, [&](const trepb_lin_args* e, const trepb_varied* ev, cudaStream_t st) { return lin_dev(s, e, st, ev); });
+    }
     Stager st(s);
     trepb_lin_args d;
     stage_lin(st, s, a, &d);
-    trepb_varied dv{};
-    if (v) {
-        const size_t rows = a->traj_len > 1 ? (size_t)a->batch / (size_t)(a->traj_len - 1) : (size_t)a->batch;
-        dv = *v;
-        dv.values = st.in(v->values, rows * v->n);
-    }
+    // one row per instance, or per trajectory
+    const trepb_varied* dv = st.varied(v, a->traj_len > 1 ? (size_t)a->batch / (size_t)(a->traj_len - 1) : (size_t)a->batch);
     if (st.err) return st.err;
-    int rc = v ? trepb_linearize_varied_batch_dev(s, &d, &dv, nullptr) : trepb_linearize_batch_dev(s, &d, nullptr);
+    int rc = lin_dev(s, &d, nullptr, dv);
     if (rc) return rc;
     return st.finish();
 }

@@ -132,20 +132,16 @@ struct KernelSet {
     int specialized;
     int nX, nU;
     int n_params;            // specialised: number of run-time parameters the kernels take (param_map order)
-    cudaError_t (*step)(const LaunchCfg&, const StepParams&);
-    cudaError_t (*p2)(const LaunchCfg&, const P2Params&);
-    cudaError_t (*lin)(const LaunchCfg&, const LinParams&);
-    cudaError_t (*proj)(const LaunchCfg&, const ProjParams&);
-    // which: 0 step, 1 p2, 2 lin.  blocks_per_sm at (block, smem).
-    cudaError_t (*occupancy)(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
+    // per-instance parameters (trepb_*_varied_batch*): a non-null VariedArgs launches the same kernel body
+    // instantiated with kVaried (*_varied_kernel)
+    cudaError_t (*step)(const LaunchCfg&, const StepParams&, const VariedArgs*);
+    cudaError_t (*p2)(const LaunchCfg&, const P2Params&, const VariedArgs*);
+    cudaError_t (*lin)(const LaunchCfg&, const LinParams&, const VariedArgs*);
+    cudaError_t (*proj)(const LaunchCfg&, const ProjParams&, const VariedArgs*);
+    // which: 0 step, 1 p2, 2 lin, 3 project, of the *_varied_kernel set when `varied`.  blocks_per_sm at (block, smem).
+    cudaError_t (*occupancy)(int which, bool varied, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
     cudaError_t (*d2)(const LaunchCfg&, const WsStridedT<HDG>&, const D2Params&);
     cudaError_t (*d2_occupancy)(int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
-    // per-instance parameters (trepb_*_varied_batch*): the same kernel bodies instantiated with kVaried
-    cudaError_t (*step_v)(const LaunchCfg&, const StepParams&, const VariedArgs&);
-    cudaError_t (*p2_v)(const LaunchCfg&, const P2Params&, const VariedArgs&);
-    cudaError_t (*lin_v)(const LaunchCfg&, const LinParams&, const VariedArgs&);
-    cudaError_t (*proj_v)(const LaunchCfg&, const ProjParams&, const VariedArgs&);
-    cudaError_t (*occupancy_v)(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
 };
 
 // factorizations and tables of deriv1 that the second-derivative kernel reuses (AuxLayout)
@@ -626,64 +622,25 @@ struct Launchers {
             return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         return cudaSuccess;
     }
-    static cudaError_t step(const LaunchCfg& c, const StepParams& p) {
+    // K for plain launches, KV for per-instance parameters
+    template <class P, void (*K)(RtSys, const char*, int, WsStrided, P, typename Sys::Params),
+              void (*KV)(RtSys, const char*, int, WsStrided, P, VariedArgs)>
+    static cudaError_t launch(const LaunchCfg& c, const P& p, const VariedArgs* va) {
         RtSys rs{};
         if (c.sys) rs = *c.sys;
-        cudaError_t e = prep((const void*)step_kernel<Sys>, c.smem);
+        cudaError_t e = prep(va ? (const void*)KV : (const void*)K, c.smem);
         if (e != cudaSuccess) return e;
-        step_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, spec_params(c));
+        if (va) KV<<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, *va);
+        else K<<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, spec_params(c));
         return cudaGetLastError();
     }
-    static cudaError_t p2(const LaunchCfg& c, const P2Params& p) {
-        RtSys rs{};
-        if (c.sys) rs = *c.sys;
-        cudaError_t e = prep((const void*)p2_kernel<Sys>, c.smem);
-        if (e != cudaSuccess) return e;
-        p2_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, spec_params(c));
-        return cudaGetLastError();
-    }
-    static cudaError_t lin(const LaunchCfg& c, const LinParams& p) {
-        RtSys rs{};
-        if (c.sys) rs = *c.sys;
-        cudaError_t e = prep((const void*)lin_kernel<Sys>, c.smem);
-        if (e != cudaSuccess) return e;
-        lin_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, spec_params(c));
-        return cudaGetLastError();
-    }
-    static cudaError_t proj(const LaunchCfg& c, const ProjParams& p) {
-        RtSys rs{};
-        if (c.sys) rs = *c.sys;
-        cudaError_t e = prep((const void*)project_kernel<Sys>, c.smem);
-        if (e != cudaSuccess) return e;
-        project_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, spec_params(c));
-        return cudaGetLastError();
-    }
-#define TREPB_VLAUNCH(name, kern, P)                                                                            \
-    static cudaError_t name(const LaunchCfg& c, const P& p, const VariedArgs& va) {                           \
-        RtSys rs{};                                                                                           \
-        if (c.sys) rs = *c.sys;                                                                               \
-        cudaError_t e = prep((const void*)kern<Sys>, c.smem);                                                 \
-        if (e != cudaSuccess) return e;                                                                       \
-        kern<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, c.ws, p, va);             \
-        return cudaGetLastError();                                                                            \
-    }
-    TREPB_VLAUNCH(step_v, step_varied_kernel, StepParams)
-    TREPB_VLAUNCH(p2_v, p2_varied_kernel, P2Params)
-    TREPB_VLAUNCH(lin_v, lin_varied_kernel, LinParams)
-    TREPB_VLAUNCH(proj_v, project_varied_kernel, ProjParams)
-#undef TREPB_VLAUNCH
-    // which: 0 step, 1 p2, 2 lin, 3 project
-    static cudaError_t occupancy(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
-        const void* fn = which == 0 ? (const void*)step_kernel<Sys>
-                       : which == 1 ? (const void*)p2_kernel<Sys>
-                       : which == 2 ? (const void*)lin_kernel<Sys> : (const void*)project_kernel<Sys>;
-        return occupancy_of(fn, block, smem, blocks_per_sm, info);
-    }
-    static cudaError_t occupancy_v(int which, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
-        const void* fn = which == 0 ? (const void*)step_varied_kernel<Sys>
-                       : which == 1 ? (const void*)p2_varied_kernel<Sys>
-                       : which == 2 ? (const void*)lin_varied_kernel<Sys> : (const void*)project_varied_kernel<Sys>;
-        return occupancy_of(fn, block, smem, blocks_per_sm, info);
+    static cudaError_t occupancy(int which, bool varied, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
+        const void* const fn[2][4] = {
+            {(const void*)step_kernel<Sys>, (const void*)p2_kernel<Sys>, (const void*)lin_kernel<Sys>,
+             (const void*)project_kernel<Sys>},
+            {(const void*)step_varied_kernel<Sys>, (const void*)p2_varied_kernel<Sys>, (const void*)lin_varied_kernel<Sys>,
+             (const void*)project_varied_kernel<Sys>}};
+        return occupancy_of(fn[varied][which], block, smem, blocks_per_sm, info);
     }
     static cudaError_t occupancy_of(const void* fn, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
         cudaFuncAttributes a;
@@ -712,18 +669,14 @@ KernelSet make_kernelset(const char* name, unsigned long long hash, int speciali
     KernelSet k;
     k.name = name; k.hash = hash; k.specialized = specialized; k.nX = nX; k.nU = nU;
     k.n_params = Sys::kNPAR;
-    k.step = &Launchers<Sys>::step;
-    k.p2 = &Launchers<Sys>::p2;
-    k.lin = &Launchers<Sys>::lin;
-    k.proj = &Launchers<Sys>::proj;
-    k.occupancy = &Launchers<Sys>::occupancy;
+    using L = Launchers<Sys>;
+    k.step = &L::template launch<StepParams, step_kernel<Sys>, step_varied_kernel<Sys>>;
+    k.p2 = &L::template launch<P2Params, p2_kernel<Sys>, p2_varied_kernel<Sys>>;
+    k.lin = &L::template launch<LinParams, lin_kernel<Sys>, lin_varied_kernel<Sys>>;
+    k.proj = &L::template launch<ProjParams, project_kernel<Sys>, project_varied_kernel<Sys>>;
+    k.occupancy = &L::occupancy;
     k.d2 = &LaunchersD2<Sys>::run;
     k.d2_occupancy = &LaunchersD2<Sys>::occupancy;
-    k.step_v = &Launchers<Sys>::step_v;
-    k.p2_v = &Launchers<Sys>::p2_v;
-    k.lin_v = &Launchers<Sys>::lin_v;
-    k.proj_v = &Launchers<Sys>::proj_v;
-    k.occupancy_v = &Launchers<Sys>::occupancy_v;
     return k;
 }
 #endif  // __CUDACC__

@@ -165,20 +165,11 @@ _lib.trepb_event_pair_destroy.restype = None
 _lib.trepb_measure_fp64_peak.argtypes = [C.c_int, _dp]
 _vp = C.POINTER(Varied)
 _lib.trepb_varied_check.argtypes = [C.c_void_p, _vp]
-_lib.trepb_step_varied_batch.argtypes = [C.c_void_p, C.POINTER(StepArgs), _vp]
-_lib.trepb_step_varied_batch_dev.argtypes = [C.c_void_p, C.POINTER(StepArgs), _vp, C.c_void_p]
-_lib.trepb_project_varied_batch.argtypes = [C.c_void_p, C.POINTER(ProjectArgs), _vp]
-_lib.trepb_project_varied_batch_dev.argtypes = [C.c_void_p, C.POINTER(ProjectArgs), _vp, C.c_void_p]
-_lib.trepb_linearize_varied_batch.argtypes = [C.c_void_p, C.POINTER(LinArgs), _vp]
-_lib.trepb_linearize_varied_batch_dev.argtypes = [C.c_void_p, C.POINTER(LinArgs), _vp, C.c_void_p]
-_lib.trepb_calc_p2_varied_batch.argtypes = [C.c_void_p, C.c_int64, C.c_double] + [C.c_void_p] * 3 + [_vp]
-_lib.trepb_calc_p2_varied_batch_dev.argtypes = [C.c_void_p, C.c_int64, C.c_double] + [C.c_void_p] * 3 + [_vp, C.c_void_p]
-_lib.trepb_calc_f_varied_batch.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 6 + [_vp]
-_lib.trepb_calc_f_varied_batch_dev.argtypes = ([C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 6 +
-                                               [_vp, C.c_void_p])
-_lib.trepb_discrete_fm2_varied_batch.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 4 + [_vp]
-_lib.trepb_discrete_fm2_varied_batch_dev.argtypes = ([C.c_void_p, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 4 +
-                                                     [_vp, C.c_void_p])
+# trepb_<call>_varied_batch[_dev]: the arguments of trepb_<call>_batch, then the trepb_varied (and the stream)
+for _call in ("step", "project", "linearize", "calc_p2", "calc_f", "discrete_fm2"):
+    _plain = getattr(_lib, "trepb_%s_batch" % _call).argtypes
+    getattr(_lib, "trepb_%s_varied_batch" % _call).argtypes = _plain + [_vp]
+    getattr(_lib, "trepb_%s_varied_batch_dev" % _call).argtypes = _plain + [_vp, C.c_void_p]
 _lib.trepb_sincos_batch.argtypes = [C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
 
 EXPORTS = [
@@ -543,6 +534,17 @@ class System:
 
     # ---- raw calls: every array argument is a pointer-like (numpy => host entry point,
     #      anything with data_ptr() => device entry point); the caller owns shapes/dtypes ----------
+    def _call(self, call, on_device, params, stream, *args):
+        """trepb_<call>[_varied]_batch[_dev](handle, *args[, varied][, stream])."""
+        tail = []
+        if params is not None:
+            v, keep = _varied(params)   # keep: the arrays v points into, alive until the call returns
+            tail.append(C.byref(v))
+        if on_device:
+            tail.append(stream)
+        name = "trepb_%s%s_batch%s" % (call, "" if params is None else "_varied", "_dev" if on_device else "")
+        _check(getattr(_lib, name)(self._h, *args, *tail))
+
     def step_raw(self, on_device, batch, nsteps, t0, dt, q1, p1, u1, k2, q2_guess, lambda_guess,
                  q2, p2, lambda1, iters, status, tolerance=1e-10, max_iterations=200,
                  sample_every=0, traj_q=None, traj_p=None, stream=None, times=None, params=None):
@@ -552,16 +554,7 @@ class System:
                      q2_guess=_ptr(q2_guess), lambda_guess=_ptr(lambda_guess), q2=_ptr(q2),
                      p2=_ptr(p2), lambda1=_ptr(lambda1), iters=_ptr(iters), status=_ptr(status),
                      sample_every=sample_every, traj_q=_ptr(traj_q), traj_p=_ptr(traj_p))
-        if params is not None:
-            v, keep = _varied(params)
-            if on_device:
-                _check(_lib.trepb_step_varied_batch_dev(self._h, C.byref(a), C.byref(v), stream))
-            else:
-                _check(_lib.trepb_step_varied_batch(self._h, C.byref(a), C.byref(v)))
-        elif on_device:
-            _check(_lib.trepb_step_batch_dev(self._h, C.byref(a), stream))
-        else:
-            _check(_lib.trepb_step_batch(self._h, C.byref(a)))
+        self._call("step", on_device, params, stream, C.byref(a))
 
     @staticmethod
     def _lin_args(batch, q1, p1, u1, k2, status, t1=None, t2=None, t1_scalar=0.0, dt_scalar=0.0,
@@ -579,16 +572,7 @@ class System:
     def linearize_raw(self, on_device, batch, q1, p1, u1, k2, status, stream=None, params=None, **kw):
         """params: None, or (refs, values) with one row per instance, or per trajectory when traj_len >= 2."""
         a = self._lin_args(batch, q1, p1, u1, k2, status, **kw)
-        if params is not None:
-            v, keep = _varied(params)
-            if on_device:
-                _check(_lib.trepb_linearize_varied_batch_dev(self._h, C.byref(a), C.byref(v), stream))
-            else:
-                _check(_lib.trepb_linearize_varied_batch(self._h, C.byref(a), C.byref(v)))
-        elif on_device:
-            _check(_lib.trepb_linearize_batch_dev(self._h, C.byref(a), stream))
-        else:
-            _check(_lib.trepb_linearize_batch(self._h, C.byref(a)))
+        self._call("linearize", on_device, params, stream, C.byref(a))
 
     def deriv2_raw(self, on_device, batch, q1, p1, u1, k2, status, d2, stream=None, z=None,
                    fdxdx=None, fdxdu=None, fdudu=None, **kw):
@@ -612,56 +596,17 @@ class System:
                         bX=_ptr(bX), bU=_ptr(bU), Kfb=_ptr(Kfb), k_per_instance=1 if k_per_instance else 0,
                         use_hint=1 if use_hint else 0, X=_ptr(X), U=_ptr(U), iters=_ptr(iters), status=_ptr(status),
                         fail_step=_ptr(fail_step))
-        if params is not None:
-            v, keep = _varied(params)
-            if on_device:
-                _check(_lib.trepb_project_varied_batch_dev(self._h, C.byref(a), C.byref(v), stream))
-            else:
-                _check(_lib.trepb_project_varied_batch(self._h, C.byref(a), C.byref(v)))
-        elif on_device:
-            _check(_lib.trepb_project_batch_dev(self._h, C.byref(a), stream))
-        else:
-            _check(_lib.trepb_project_batch(self._h, C.byref(a)))
+        self._call("project", on_device, params, stream, C.byref(a))
 
     def calc_p2_raw(self, on_device, batch, dt, q0, q1, p, stream=None, params=None):
-        if params is not None:
-            v, keep = _varied(params)
-            if on_device:
-                _check(_lib.trepb_calc_p2_varied_batch_dev(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p), C.byref(v), stream))
-            else:
-                _check(_lib.trepb_calc_p2_varied_batch(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p), C.byref(v)))
-        elif on_device:
-            _check(_lib.trepb_calc_p2_batch_dev(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p), stream))
-        else:
-            _check(_lib.trepb_calc_p2_batch(self._h, batch, dt, _ptr(q0), _ptr(q1), _ptr(p)))
+        self._call("calc_p2", on_device, params, stream, batch, dt, _ptr(q0), _ptr(q1), _ptr(p))
 
     def calc_f_raw(self, on_device, batch, t1, t2, q1, q2, p1, u1, lambda1, f, stream=None, params=None):
-        if params is not None:
-            v, keep = _varied(params)
-            args = (self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(p1), _ptr(u1), _ptr(lambda1), _ptr(f), C.byref(v))
-            if on_device:
-                _check(_lib.trepb_calc_f_varied_batch_dev(*args, stream))
-            else:
-                _check(_lib.trepb_calc_f_varied_batch(*args))
-        elif on_device:
-            _check(_lib.trepb_calc_f_batch_dev(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(p1), _ptr(u1),
-                                               _ptr(lambda1), _ptr(f), stream))
-        else:
-            _check(_lib.trepb_calc_f_batch(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(p1), _ptr(u1),
-                                           _ptr(lambda1), _ptr(f)))
+        self._call("calc_f", on_device, params, stream, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(p1), _ptr(u1),
+                   _ptr(lambda1), _ptr(f))
 
     def discrete_fm2_raw(self, on_device, batch, t1, t2, q1, q2, u1, fm2, stream=None, params=None):
-        if params is not None:
-            v, keep = _varied(params)
-            args = (self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(u1), _ptr(fm2), C.byref(v))
-            if on_device:
-                _check(_lib.trepb_discrete_fm2_varied_batch_dev(*args, stream))
-            else:
-                _check(_lib.trepb_discrete_fm2_varied_batch(*args))
-        elif on_device:
-            _check(_lib.trepb_discrete_fm2_batch_dev(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(u1), _ptr(fm2), stream))
-        else:
-            _check(_lib.trepb_discrete_fm2_batch(self._h, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(u1), _ptr(fm2)))
+        self._call("discrete_fm2", on_device, params, stream, batch, t1, t2, _ptr(q1), _ptr(q2), _ptr(u1), _ptr(fm2))
 
     # ---- numpy convenience (host entry points) ---------------------------------------------------
     def _f(self, x, shape):
