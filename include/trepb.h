@@ -400,7 +400,8 @@ int trepb_deriv2_batch_dev(trepb_system* sys, const trepb_d2_args* args, void* s
  * other entry keeps the description's value): Monte Carlo over uncertain masses / lengths / gains, one candidate
  * parameter set per instance in system identification, K plausible models in robust trajectory optimisation.
  *   rows       one per instance; trepb_linearize_varied_batch* with traj_len >= 2: one per trajectory r (all
- *              traj_len - 1 steps of a rollout share its physics).
+ *              traj_len - 1 steps of a rollout share its physics).  trepb_deriv2_varied_batch* takes one row per
+ *              instance only: args->lin.traj_len must be 0 (TREPB_ERR_INVALID otherwise).
  *   entries    only run-time parameters can vary: an entry whose description value is exactly 0, or +-1 in
  *              frame_se3, is structure (it folds away in the specialised kernels and in trepb_struct_hash), and
  *              so are the spline x-points of a NonlinearConfigSpring and a Gravity component whose sum over all
@@ -409,7 +410,9 @@ int trepb_deriv2_batch_dev(trepb_system* sys, const trepb_d2_args* args, void* s
  *              gravity sum per instance.  A row value of exactly 0 is not checked and keeps the entry's role.
  *   kernels    specialised and table-driven thread kernels (a handle built for an all-literal instantiation runs
  *              the run-time-parameter kernels of its structure); cooperative handles are TREPB_ERR_UNSUPPORTED
- *              (create the handle with TREPB_FLAG_NO_COOP).  No second-derivative entry point varies.
+ *              (create the handle with TREPB_FLAG_NO_COOP).  Second derivatives vary through the same kernels
+ *              and schemes as the plain call (the per-pair kernel, or the per-parameter scheme on the tables);
+ *              its linearize launch runs on the same rows.
  * Results equal those of a handle created from each instance's own description, run through the plain entry
  * point. */
 #define TREPB_PAR_FRAME_VALUE 0   /* index f           */
@@ -449,6 +452,8 @@ int trepb_discrete_fm2_varied_batch(trepb_system* sys, int64_t batch, double t1,
 int trepb_discrete_fm2_varied_batch_dev(trepb_system* sys, int64_t batch, double t1, double t2, const double* q1,
                                         const double* q2, const double* u1, double* fm2, const trepb_varied* v,
                                         void* stream);
+int trepb_deriv2_varied_batch(trepb_system* sys, const trepb_d2_args* args, const trepb_varied* v);
+int trepb_deriv2_varied_batch_dev(trepb_system* sys, const trepb_d2_args* args, const trepb_varied* v, void* stream);
 
 /* ---- multi-GPU: one process per GPU ---------------------------------------------------------
  * Instances are independent, so a batch shards over ranks with no exchange during compute (each

@@ -47,6 +47,15 @@ struct DevBuf {
 size_t coop_smem(int blob_bytes, int teams, const trepb::CoopLayout& lay) {
     return (size_t)(((blob_bytes + 7) / 8 + 1) & ~1) * 8 + (size_t)teams * lay.total * 8;
 }
+
+// Second derivatives by the per-parameter scheme on the tables (trepb_d2jac.cuh) instead of the per-pair kernel of
+// `ks`: always for table-driven kernels; for a specialised per-pair kernel whose hyper-dual workspace is far beyond
+// the register file (info: its plain d2_kernel).  Measured (evaluations/s, per-pair vs per-parameter): 5-link
+// pendulum (31 KB of local memory per thread) 8.1e6 vs 1.1e7, wrench arm (19 KB) 7.8e6 vs 1.2e7; dual pendulums
+// (12 KB) 1.05e8 vs 6.8e7, pend-on-cart (10 KB) 1.0e8 vs 6.2e7
+bool d2_prefers_jac(const trepb::KernelSet* ks, const trepb::KernelInfo& info) {
+    return !ks->specialized || info.local_bytes > 16384;
+}
 }  // namespace
 
 #if defined(TREPB_PHASE_TIMING)
@@ -142,7 +151,10 @@ struct trepb_system {
     bool vinit = false;
     int vbps[4] = {1, 1, 1, 1};
     int vlin_bps_staged = 0;
-    DevBuf vmap, vslots;
+    bool vd2_use_jac = false;    // second derivatives on vks: as d2_use_jac for a handle built on vks
+    int vbps_d2 = 1, vbps_d2jac = 1;
+    // vmap_tab: the table-driven layout of the map, for pass A of the per-parameter scheme on a specialised handle
+    DevBuf vmap, vmap_tab, vslots;
     std::mutex mu;       // serialises launches on this handle
     std::mutex mu_host;  // serialises the host-pointer entry points (they share staging buffers)
 };
@@ -284,28 +296,25 @@ int trepb_system_create(const trepb_sysdesc* desc, int device, int flags, trepb_
         s->bps[w] = b > 0 ? b : 1;
     }
     s->ws_hd_elems = s->wsl_hd.layout(ps.nf, ps.nd, ps.nk, ps.nu, ps.nc, 1);
-    bool d2_spills = false;
     {
         int b = 0;
         KernelInfo ki{};
-        CUS(s->ks->d2_occupancy(s->block, base_smem, &b, &ki));
+        CUS(s->ks->d2_occupancy(false, s->block, base_smem, &b, &ki));
         s->bps_d2 = b > 0 ? b : 1;
-        // a specialised per-pair kernel whose hyper-dual workspace is far beyond the register file loses to
-        // the per-parameter scheme on the tables.  Measured (evaluations/s, per-pair vs per-parameter):
-        // 5-link pendulum (31 KB of local memory per thread) 8.1e6 vs 1.1e7, wrench arm (19 KB) 7.8e6 vs
-        // 1.2e7; dual pendulums (12 KB) 1.05e8 vs 6.8e7, pend-on-cart (10 KB) 1.0e8 vs 6.2e7
-        d2_spills = ki.local_bytes > 16384;
+        s->d2_use_jac = d2_prefers_jac(s->ks, ki);
     }
-    s->d2_use_jac = !s->ks->specialized || d2_spills;
-    if (s->d2_use_jac) {
-        s->ws_du_elems = s->wsl_du.layout(ps.nf, ps.nd, ps.nk, ps.nu, ps.nc, 2);
-        int b = 0;
-        CUS(d2jac_occupancy(s->block, d2jac_smem(s->blob_bytes, s->block, ps.nd, ps.nk), &b, nullptr));
-        s->bps_d2jac = b > 0 ? b : 1;
+    // the per-parameter scheme's shape data (also what a per-instance-parameter call on vks may need)
+    s->ws_du_elems = s->wsl_du.layout(ps.nf, ps.nd, ps.nk, ps.nu, ps.nc, 2);
+    {
         AuxLayout al;
         al.set(ps.nd, ps.nc);
         const int nx = 2 * (ps.nd + ps.nk) + ps.nu;
         s->d2jac_ok = nx <= 1024 && d2solve_smem_needed(ps.nd, ps.nk, ps.nc, nx, al.size) <= (size_t)prop.sharedMemPerBlockOptin;
+    }
+    if (s->d2_use_jac) {
+        int b = 0;
+        CUS(d2jac_occupancy(false, s->block, d2jac_smem(s->blob_bytes, s->block, ps.nd, ps.nk), &b, nullptr));
+        s->bps_d2jac = b > 0 ? b : 1;
     }
     if (s->ks->specialized) {
         const int nq = ps.nd + ps.nk, nX = 2 * nq, nU = ps.nu + ps.nk;
@@ -334,6 +343,7 @@ void trepb_system_destroy(trepb_system* s) {
     s->ws_du.release();
     s->coop_ext.release();
     s->vmap.release();
+    s->vmap_tab.release();
     s->vslots.release();
     s->d2g.release();
     for (auto& b : s->d2s) b.release();
@@ -493,8 +503,32 @@ struct Timed {
     ~Timed() { cudaEventRecord(s->ev1, st); s->timed = true; }
 };
 
-// Per-instance parameters: checks `v` against the handle's description, uploads its map (trepb_varied.h) to handle
-// scratch and fills va (slots: see varied_slots).  The caller holds s->mu and a ScratchGuard on `stream`.
+// Uploads the map of a checked `v` (trepb_varied.h) in the specialised (`slots`) or the table-driven layout to `buf`
+// and fills va (slots: see varied_slots).
+int varied_upload(trepb_system* s, const trepb_varied* v, bool slots, DevBuf& buf_d, cudaStream_t stream, VariedArgs* va) {
+    VariedHost H;
+    varied_map(s->P, v->n, v->table, v->index, slots, &H);
+    // one upload: base, gbase (doubles), then src, gcol (ints)
+    const size_t nb = H.base.size(), ng = H.gbase.size();
+    std::vector<double> buf(nb + ng + (H.src.size() + H.gcol.size() + 1) / 2 + 1, 0.0);
+    memcpy(buf.data(), H.base.data(), nb * sizeof(double));
+    if (ng) memcpy(buf.data() + nb, H.gbase.data(), ng * sizeof(double));
+    int* ib = (int*)(buf.data() + nb + ng);
+    if (!H.src.empty()) memcpy(ib, H.src.data(), H.src.size() * sizeof(int));
+    if (!H.gcol.empty()) memcpy(ib + H.src.size(), H.gcol.data(), H.gcol.size() * sizeof(int));
+    CU(buf_d.ensure(buf.size() * sizeof(double)));
+    // pageable source: returns once the bytes are staged, so `buf` may go out of scope
+    CU(cudaMemcpyAsync(buf_d.p, buf.data(), buf.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
+    const double* d = (const double*)buf_d.p;
+    const int* di = (const int*)(d + nb + ng);
+    va->map = H.view(di, d, di + H.src.size(), d + nb);
+    va->values = v->values;
+    va->slots = nullptr;
+    return TREPB_OK;
+}
+
+// Per-instance parameters: checks `v` against the handle's description, uploads its map in the layout of vks to
+// handle scratch and fills va.  The caller holds s->mu and a ScratchGuard on `stream`.
 int varied_setup(trepb_system* s, const trepb_varied* v, cudaStream_t stream, VariedArgs* va) {
     if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
     if (s->coop)
@@ -513,27 +547,21 @@ int varied_setup(trepb_system* s, const trepb_varied* v, cudaStream_t stream, Va
             s->vbps[w] = b > 0 ? b : 1;
         }
         if (s->lin_stage_bytes) CU(s->vks->occupancy(2, true, s->block, s->lin_stage_bytes, &s->vlin_bps_staged, nullptr));
+        // second derivatives: the scheme a handle built on vks would pick, and the varied kernels' occupancy
+        int b = 0;
+        KernelInfo ki{};
+        CU(s->vks->d2_occupancy(false, s->block, smem, &b, &ki));
+        s->vd2_use_jac = d2_prefers_jac(s->vks, ki);
+        CU(s->vks->d2_occupancy(true, s->block, smem, &b, nullptr));
+        s->vbps_d2 = b > 0 ? b : 1;
+        if (s->vd2_use_jac) {
+            const RtSys& ps = s->P.proto;
+            CU(d2jac_occupancy(true, s->block, d2jac_smem(s->blob_bytes, s->block, ps.nd, ps.nk), &b, nullptr));
+            s->vbps_d2jac = b > 0 ? b : 1;
+        }
         s->vinit = true;
     }
-    VariedHost H;
-    varied_map(s->P, v->n, v->table, v->index, s->vks->specialized != 0, &H);
-    // one upload: base, gbase (doubles), then src, gcol (ints)
-    const size_t nb = H.base.size(), ng = H.gbase.size();
-    std::vector<double> buf(nb + ng + (H.src.size() + H.gcol.size() + 1) / 2 + 1, 0.0);
-    memcpy(buf.data(), H.base.data(), nb * sizeof(double));
-    if (ng) memcpy(buf.data() + nb, H.gbase.data(), ng * sizeof(double));
-    int* ib = (int*)(buf.data() + nb + ng);
-    if (!H.src.empty()) memcpy(ib, H.src.data(), H.src.size() * sizeof(int));
-    if (!H.gcol.empty()) memcpy(ib + H.src.size(), H.gcol.data(), H.gcol.size() * sizeof(int));
-    CU(s->vmap.ensure(buf.size() * sizeof(double)));
-    // pageable source: returns once the bytes are staged, so `buf` may go out of scope
-    CU(cudaMemcpyAsync(s->vmap.p, buf.data(), buf.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
-    const double* d = (const double*)s->vmap.p;
-    const int* di = (const int*)(d + nb + ng);
-    va->map = H.view(di, d, di + H.src.size(), d + nb);
-    va->values = v->values;
-    va->slots = nullptr;
-    return TREPB_OK;
+    return varied_upload(s, v, s->vks->specialized != 0, s->vmap, stream, va);
 }
 
 // table-driven kernels: one expanded parameter vector per launched thread
@@ -547,10 +575,11 @@ int varied_slots(trepb_system* s, const LaunchCfg& c, VariedArgs* va) {
 // Launches one call (which: 0 step, 1 p2, 2 lin, 3 project) on the kernels `v` and the handle select: the
 // run-time-parameter kernels for per-instance parameters, else the cooperative kernels of a cooperative handle,
 // else one thread per instance.  thread(ks, cfg, va) and coop(cl) launch the call's kernel.  stage (linearize with
-// A or B, else null): set to 1 when the outputs are staged through shared memory.  The caller holds s->mu.
+// A or B, else null): set to 1 when the outputs are staged through shared memory.  vset: the map of `v` when the
+// caller has set it up already (varied_setup).  The caller holds s->mu.
 template <class Thread, class Coop>
 int dispatch(trepb_system* s, int which, long long batch, cudaStream_t stream, const trepb_varied* v, int* stage,
-             Thread thread, Coop coop) {
+             Thread thread, Coop coop, const VariedArgs* vset = nullptr) {
     if (!v && s->coop) {
         CoopLaunch cl;
         make_coop(s, batch, stream, &cl, which != 2);
@@ -562,7 +591,8 @@ int dispatch(trepb_system* s, int which, long long batch, cudaStream_t stream, c
     }
     ScratchGuard sg(s, stream, v || !s->ks->specialized);
     VariedArgs va;
-    if (v)
+    if (v && vset) va = *vset;
+    else if (v)
         if (int rc = varied_setup(s, v, stream, &va)) return rc;
     const int bps_staged = v ? s->vlin_bps_staged : s->lin_bps_staged;
     const bool staged = stage && s->lin_stage_bytes > 0 && bps_staged > 0;
@@ -668,8 +698,8 @@ int discrete_fm2_dev(trepb_system* s, int64_t batch, double t1, double t2, const
 }
 
 // validates + launches the linearize kernel; the caller holds s->mu
-int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, double* aux, int aux_size,
-               const trepb_varied* v = nullptr) {
+// argument checks of a linearize call (also run by deriv2 before it sets anything up)
+int lin_check(const trepb_system* s, const trepb_lin_args* a) {
     const RtSys& ps = s->P.proto;
     if (a->batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
     if (!a->q1 || !a->p1 || !a->status) return fail(TREPB_ERR_INVALID, "q1, p1 and status are required");
@@ -678,6 +708,13 @@ int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, do
     if (!a->t2 && !(a->dt_scalar != 0.0)) return fail(TREPB_ERR_INVALID, "dt must be non-zero");
     if (a->traj_len < 0 || a->traj_len == 1 || (a->traj_len > 1 && a->batch % (a->traj_len - 1) != 0))
         return fail(TREPB_ERR_INVALID, "traj_len must be 0 or >= 2 with batch a multiple of traj_len - 1");
+    return TREPB_OK;
+}
+
+int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, double* aux, int aux_size,
+               const trepb_varied* v = nullptr, const VariedArgs* vset = nullptr) {
+    const RtSys& ps = s->P.proto;
+    if (int rc = lin_check(s, a)) return rc;
     if (a->batch == 0) return TREPB_OK;
     CU(cudaSetDevice(s->device));
     LinParams p;
@@ -699,7 +736,7 @@ int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, do
                         AuxLayout al;
                         al.set(ps.nd, ps.nc);
                         return s->cks->lin(cl, p, al);
-                    });
+                    }, vset);
 }
 
 int lin_dev(trepb_system* s, const trepb_lin_args* a, void* stream, const trepb_varied* v) {
@@ -794,18 +831,32 @@ int trepb_linearize_varied_batch_dev(trepb_system* s, const trepb_lin_args* a, c
     return lin_dev(s, a, stream, v);
 }
 
-int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream_) {
-    TREPB_NVTX("trepb_deriv2_batch_dev");
+// deriv1 (the linearize kernel, exporting the factorizations) + second derivatives.  Per-instance parameters (v): one
+// row per instance, the map uploaded once (varied_setup) and used by both launches, on the run-time-parameter kernels
+// of the structure (vks).  Every launch-geometry and scratch decision is made before the first launch, so that the
+// table-driven slots are sized once for both.
+static int d2_dev(trepb_system* s, const trepb_d2_args* a, cudaStream_t stream, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     const RtSys& ps = s->P.proto;
     const int nd = ps.nd, nk = ps.nk, nq = nd + nk, nu = ps.nu, nc = ps.nc;
     const long long B = a->lin.batch;
     if (B < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
+    if (v && a->lin.traj_len != 0)
+        return fail(TREPB_ERR_INVALID, "per-instance parameters of second derivatives take one row per instance: "
+                                       "traj_len must be 0");
     if (B == 0) return TREPB_OK;
-    cudaStream_t stream = (cudaStream_t)stream_;
+    if (int rc = lin_check(s, &a->lin)) return rc;   // before any scratch, zeroing or launch of this call
     std::lock_guard<std::mutex> lk(s->mu);
     CU(cudaSetDevice(s->device));
     ScratchGuard sg(s, stream, true);   // covers the linearize launch below and both second-derivative passes
+    VariedArgs va{};
+    const KernelSet* ks = s->ks;
+    bool use_jac = s->d2_use_jac;
+    if (v) {
+        if (int rc = varied_setup(s, v, stream, &va)) return rc;
+        ks = s->vks;
+        use_jac = s->vd2_use_jac;
+    }
     // deriv1 products this kernel consumes: use the caller's arrays where given, scratch otherwise
     trepb_lin_args la = a->lin;
     const size_t cnt[4] = {(size_t)nq, (size_t)nd, (size_t)nu, (size_t)nk};
@@ -826,9 +877,6 @@ int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream
     al.set(nd, nc);
     CU(s->d2s[k].ensure((size_t)B * al.size * sizeof(double)));
     double* aux = (double*)s->d2s[k].p;
-    int rc = lin_launch(s, &la, stream, aux, al.size);
-    if (rc) return rc;
-    // ---- second-derivative kernel: one thread per (instance, pair)
     D2Params p;
     p.batch = B;
     p.nx = nq + nd + nu + nk;
@@ -848,11 +896,24 @@ int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream
         if (p.zuu && nU) CU(cudaMemsetAsync(p.zuu, 0, (size_t)B * nU * nU * sizeof(double), stream));
         if (nU == 0) { p.zxu = nullptr; p.zuu = nullptr; }
     }
-    if (s->d2_use_jac && !(s->flags & TREPB_FLAG_D2_PAIRWISE) && s->d2jac_ok) {
+    // ---- launch geometry of the second-derivative pass(es)
+    const bool jac = use_jac && !(s->flags & TREPB_FLAG_D2_PAIRWISE) && s->d2jac_ok;
+    LaunchCfg c;
+    c.ws = s->wsl;
+    c.dblob = s->dblob; c.blob_bytes = s->blob_bytes; c.stream = stream;
+    c.block = s->block;
+    // per-instance parameters of pass A / of the per-pair kernel: the map of the linearize launch, except on a
+    // specialised handle that takes the per-parameter scheme (pass A is table-driven there: its own map layout)
+    VariedArgs vd = va;
+    long long d2_threads = 0;   // threads that need a table-driven slot
+    JacLayout jl;
+    long long nb = 0, jgrid = 0;
+    WsStridedT<Dual> wd = s->wsl_du;
+    WsStridedT<HDG> w = s->wsl_hd;
+    if (jac) {
         // pass A: one dual evaluation of the Jacobian tables per (instance, parameter);
         // pass B: contraction + solves per pair (trepb_d2jac.cuh).  The batch is processed in
         // chunks so that the table records stay within a few GB.
-        JacLayout jl;
         jl.set(nd, nk, nu, nc);
         size_t free_b = 0, total_b = 0;
         CU(cudaMemGetInfo(&free_b, &total_b));
@@ -860,52 +921,69 @@ int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream
         const size_t per_inst = (size_t)p.nx * jl.size * sizeof(double);
         size_t gbudget = avail / 4;
         if (gbudget > ((size_t)4 << 30)) gbudget = (size_t)4 << 30;
-        long long nb = (long long)(gbudget / per_inst);
+        nb = (long long)(gbudget / per_inst);
         if (nb < 1) return fail(TREPB_ERR_CUDA, "not enough device memory for the second-derivative table records");
         if (nb > B) nb = B;
-        const int block = s->block;
-        long long grid = (nb * p.nx + block - 1) / block;
-        if (int rc = slab_grid(&grid, (long long)s->sms * s->bps_d2jac, s->ws_du_elems, sizeof(Dual), block,
-                               s->ws_du.cap + s->d2g.cap, s->ws_du, "second-derivative workspace"))
+        jgrid = (nb * p.nx + c.block - 1) / c.block;
+        if (int rc = slab_grid(&jgrid, (long long)s->sms * (v ? s->vbps_d2jac : s->bps_d2jac), s->ws_du_elems, sizeof(Dual),
+                               c.block, s->ws_du.cap + s->d2g.cap, s->ws_du, "second-derivative workspace"))
             return rc;
         CU(s->d2g.ensure((size_t)nb * per_inst));
-        WsStridedT<Dual> wd = s->wsl_du;
         wd.base = (Dual*)s->ws_du.p; wd.stride = 0;
-        LaunchCfg c;
         c.spec_params = nullptr;
-        c.block = block; c.smem = d2jac_smem(s->blob_bytes, block, nd, nk); c.stream = stream;
-        c.sys = &s->dview; c.dblob = s->dblob; c.blob_bytes = s->blob_bytes; c.ws = s->wsl;
-        Timed t(s, stream);
+        c.smem = d2jac_smem(s->blob_bytes, c.block, nd, nk);
+        c.sys = &s->dview;
+        if (v && ks->specialized)
+            if (int rc = varied_upload(s, v, false, s->vmap_tab, stream, &vd)) return rc;
+        if (v) d2_threads = jgrid * c.block;
+    } else {
+        // one thread per (instance, parameter s, block of kD2Dirs directions t)
+        const long long threads = B * (long long)d2_blocks(p.nx, ks->specialized ? 1 : kD2Dirs);
+        long long grid = (threads + c.block - 1) / c.block;
+        w.base = nullptr; w.stride = 0;
+        if (!ks->specialized) {
+            if (int rc = slab_grid(&grid, (long long)s->sms * (v ? s->vbps_d2 : s->bps_d2), s->ws_hd_elems, sizeof(HDG),
+                                   c.block, s->ws_hd.cap, s->ws_hd, "second-derivative workspace"))
+                return rc;
+            w.base = (HDG*)s->ws_hd.p;
+            if (v) d2_threads = grid * c.block;
+        } else if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;
+        c.spec_params = s->spec_params.empty() ? nullptr : s->spec_params.data();
+        c.grid = (int)grid;
+        c.smem = ks->specialized ? 0 : (size_t)s->blob_bytes;
+        c.sys = ks->specialized ? nullptr : &s->dview;
+    }
+    // table-driven slots for the larger of the two launches: this call's linearize launch may still grow vslots
+    // (varied_slots) before it runs, never between it and the launches below
+    if (d2_threads) CU(s->vslots.ensure((size_t)d2_threads * vd.map.n_out * sizeof(double)));
+    if (int rc = lin_launch(s, &la, stream, aux, al.size, v, v ? &va : nullptr)) return rc;
+    if (d2_threads) vd.slots = (double*)s->vslots.p;
+    const VariedArgs* vp = v ? &vd : nullptr;
+    Timed t(s, stream);
+    if (jac) {
         for (long long b0 = 0; b0 < B; b0 += nb) {
             const long long cnt_b = B - b0 < nb ? B - b0 : nb;
-            long long g = (cnt_b * p.nx + block - 1) / block;
-            c.grid = (int)(g < grid ? g : grid);
-            CU(d2jac_run(c, wd, p, (double*)s->d2g.p, jl, (long)b0, (long)cnt_b));
+            long long g = (cnt_b * p.nx + c.block - 1) / c.block;
+            c.grid = (int)(g < jgrid ? g : jgrid);
+            CU(d2jac_run(c, wd, p, (double*)s->d2g.p, jl, (long)b0, (long)cnt_b, vp));
+            // pass B reads deriv1's factors, the table records and the tangents, not the system: no varied flavour
             CU(d2solve_run(stream, p, (const double*)s->d2g.p, jl, nd, nk, nu, nc, (long)b0, (long)cnt_b));
         }
         return TREPB_OK;
     }
-    // one thread per (instance, parameter s, block of kD2Dirs directions t)
-    const long long threads = B * (long long)d2_blocks(p.nx, s->ks->specialized ? 1 : kD2Dirs);
-    int block = s->block;
-    const size_t smem = s->ks->specialized ? 0 : (size_t)s->blob_bytes;
-    long long grid = (threads + block - 1) / block;
-    WsStridedT<HDG> w = s->wsl_hd;
-    w.base = nullptr; w.stride = 0;
-    if (!s->ks->specialized) {
-        if (int rc = slab_grid(&grid, (long long)s->sms * s->bps_d2, s->ws_hd_elems, sizeof(HDG), block, s->ws_hd.cap,
-                               s->ws_hd, "second-derivative workspace"))
-            return rc;
-        w.base = (HDG*)s->ws_hd.p;
-    } else if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;
-    LaunchCfg c;
-    c.spec_params = s->spec_params.empty() ? nullptr : s->spec_params.data();
-    c.grid = (int)grid; c.block = block; c.smem = smem; c.stream = stream;
-    c.sys = s->ks->specialized ? nullptr : &s->dview;
-    c.dblob = s->dblob; c.blob_bytes = s->blob_bytes; c.ws = s->wsl;
-    Timed t(s, stream);
-    CU(s->ks->d2(c, w, p));
+    CU(ks->d2(c, w, p, vp));
     return TREPB_OK;
+}
+
+int trepb_deriv2_batch_dev(trepb_system* s, const trepb_d2_args* a, void* stream) {
+    TREPB_NVTX("trepb_deriv2_batch_dev");
+    return d2_dev(s, a, (cudaStream_t)stream, nullptr);
+}
+
+int trepb_deriv2_varied_batch_dev(trepb_system* s, const trepb_d2_args* a, const trepb_varied* v, void* stream) {
+    TREPB_NVTX("trepb_deriv2_varied_batch_dev");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return d2_dev(s, a, (cudaStream_t)stream, v);
 }
 
 int trepb_last_kernel_ms(trepb_system* s, float* ms) {
@@ -1297,8 +1375,7 @@ void stage_lin(Stager& st, const trepb_system* s, const trepb_lin_args* a, trepb
 }  // namespace
 extern "C" {
 
-int trepb_deriv2_batch(trepb_system* s, const trepb_d2_args* a) {
-    TREPB_NVTX("trepb_deriv2_batch");
+static int d2_host(trepb_system* s, const trepb_d2_args* a, const trepb_varied* v) {
     if (!s || !a) return fail(TREPB_ERR_INVALID, "null argument");
     std::lock_guard<std::mutex> hlk(s->mu_host);
     if (a->lin.batch < 0) return fail(TREPB_ERR_INVALID, "batch must be >= 0");
@@ -1320,10 +1397,22 @@ int trepb_deriv2_batch(trepb_system* s, const trepb_d2_args* a) {
         d.fdxdu = st.out(a->fdxdu, B * nX * nU);
         d.fdudu = st.out(a->fdudu, B * nU * nU);
     }
+    const trepb_varied* dv = st.varied(v, B);   // one row per instance
     if (st.err) return st.err;
-    int rc = trepb_deriv2_batch_dev(s, &d, nullptr);
+    int rc = d2_dev(s, &d, nullptr, dv);
     if (rc) return rc;
     return st.finish();
+}
+
+int trepb_deriv2_batch(trepb_system* s, const trepb_d2_args* a) {
+    TREPB_NVTX("trepb_deriv2_batch");
+    return d2_host(s, a, nullptr);
+}
+
+int trepb_deriv2_varied_batch(trepb_system* s, const trepb_d2_args* a, const trepb_varied* v) {
+    TREPB_NVTX("trepb_deriv2_varied_batch");
+    if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
+    return d2_host(s, a, v);
 }
 
 static int lin_host(trepb_system* s, const trepb_lin_args* a, const trepb_varied* v) {

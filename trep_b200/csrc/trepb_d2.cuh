@@ -234,10 +234,12 @@ struct CtxHD<Sys, false> {
     }
 };
 
-template <class Sys>
-__global__ void __launch_bounds__(128)
-d2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<HDG> wsp, const D2Params p,
-          const typename Sys::Params par) {
+// kVaried: work item (b, s, block of t) runs on row b of the per-instance parameters.  The items of one instance land
+// on different threads, so each item loads its row (load_params, trepb_kernels.cuh).
+template <class Sys, bool kVaried>
+__device__ __forceinline__ void
+d2_body(const RtSys& rsys, const char* dblob, int blob_bytes, const WsStridedT<HDG>& wsp, const D2Params& p,
+        const typename Sys::Params& par, const VariedArgs& va) {
     const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
     const long nth = (long)gridDim.x * blockDim.x;
     CtxHD<Sys> c(rsys, dblob, blob_bytes, wsp, tid, nth, par);
@@ -253,6 +255,7 @@ d2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<
     for (long g = tid; g < total; g += nth) {
         const long b = g / nblk;
         if (p.status && p.status[b] != 0) continue;
+        load_params<Sys, kVaried>(c, va, b, tid);
         int pr = (int)(g - b * nblk), s = 0;
         for (;;) {
             const int nb = (p.nx - s + N - 1) / N;
@@ -267,28 +270,34 @@ d2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<
 }
 
 template <class Sys>
+__global__ void __launch_bounds__(128)
+d2_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<HDG> wsp, const D2Params p,
+          const typename Sys::Params par) {
+    d2_body<Sys, false>(rsys, dblob, blob_bytes, wsp, p, par, VariedArgs{});
+}
+template <class Sys>
+__global__ void __launch_bounds__(128)
+d2_varied_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<HDG> wsp, const D2Params p,
+                 const VariedArgs va) {
+    d2_body<Sys, true>(rsys, dblob, blob_bytes, wsp, p, typename Sys::Params{}, va);
+}
+
+template <class Sys>
 struct LaunchersD2 {
-    static cudaError_t run(const LaunchCfg& c, const WsStridedT<HDG>& w, const D2Params& p) {
+    // d2_kernel for plain launches, d2_varied_kernel for per-instance parameters
+    static cudaError_t run(const LaunchCfg& c, const WsStridedT<HDG>& w, const D2Params& p, const VariedArgs* va) {
         RtSys rs{};
         if (c.sys) rs = *c.sys;
-        if (c.smem > 48 * 1024) {
-            cudaError_t e = cudaFuncSetAttribute((const void*)d2_kernel<Sys>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem);
-            if (e != cudaSuccess) return e;
-        }
-        d2_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, w, p, Launchers<Sys>::spec_params(c));
+        const void* fn = va ? (const void*)d2_varied_kernel<Sys> : (const void*)d2_kernel<Sys>;
+        cudaError_t e = Launchers<Sys>::prep(fn, c.smem);
+        if (e != cudaSuccess) return e;
+        if (va) d2_varied_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, w, p, *va);
+        else d2_kernel<Sys><<<c.grid, c.block, c.smem, c.stream>>>(rs, c.dblob, c.blob_bytes, w, p, Launchers<Sys>::spec_params(c));
         return cudaGetLastError();
     }
-    static cudaError_t occupancy(int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
-        const void* fn = (const void*)d2_kernel<Sys>;
-        cudaFuncAttributes a;
-        cudaError_t e = cudaFuncGetAttributes(&a, fn);
-        if (e != cudaSuccess) return e;
-        if (info) { info->regs = a.numRegs; info->max_threads = a.maxThreadsPerBlock; info->static_smem = a.sharedSizeBytes; info->local_bytes = a.localSizeBytes; }
-        if (smem > 48 * 1024) {
-            e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, fn, block, smem);
+    static cudaError_t occupancy(bool varied, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
+        return Launchers<Sys>::occupancy_of(varied ? (const void*)d2_varied_kernel<Sys> : (const void*)d2_kernel<Sys>,
+                                            block, smem, blocks_per_sm, info);
     }
 };
 #endif

@@ -32,9 +32,13 @@ struct TileSink {
 #ifndef TREPB_D2JAC_MINB
 #define TREPB_D2JAC_MINB 4   // measured on the marionette (B200): 4 CTAs per SM at 128 registers (some spills) 40.8 ms per 4096 instances, 3 at 168: 43.3, 5 at 96: 42.2, 2 at 232: 49.0
 #endif
-__global__ void __launch_bounds__(128, TREPB_D2JAC_MINB)
-d2jac_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<Dual> wsp, const D2Params p,
-             double* __restrict__ G, const JacLayout jl, long b0, long nb) {
+// kVaried: each (instance, s) item expands its instance's parameter row into this thread's slot and points the numeric
+// tables of the thread's RtSys copy at it (varied_point).  The integer tables and NzMaps stay in shared memory: NzMaps
+// depends on structure only, and an entry that may vary is never a structural zero (varied_check).
+template <bool kVaried>
+__device__ __forceinline__ void
+d2jac_body(const RtSys& rsys, const char* dblob, int blob_bytes, const WsStridedT<Dual>& wsp, const D2Params& p,
+           double* __restrict__ G, const JacLayout& jl, long b0, long nb, const VariedArgs& va) {
     extern __shared__ double smem_[];
     const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
     const long nth = (long)gridDim.x * blockDim.x;
@@ -44,7 +48,7 @@ d2jac_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStride
         for (int i = threadIdx.x; i < (blob_bytes + 7) / 8; i += blockDim.x) smem_[i] = src[i];
         __syncthreads();
     }
-    const RtSys sys = rsys.rebased(dblob, (const char*)smem_);
+    std::conditional_t<kVaried, RtSys, const RtSys> sys = rsys.rebased(dblob, (const char*)smem_);
     WsStridedT<Dual> ws = wsp;
     ws.base = wsp.base + tid;
     ws.stride = (unsigned)nth;
@@ -62,6 +66,9 @@ d2jac_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStride
         const long b = b0 + (in ? g / p.nx : 0);
         const int s = in ? (int)(g % p.nx) : 0;
         const bool act = in && !(p.status && p.status[b] != 0);
+        if constexpr (kVaried) {
+            if (act) varied_point(sys, va.map, va.values + b * va.map.n, va.slots + tid * (long)va.map.n_out);
+        }
         if (act) d2jac_eval(sys, ws, nz, p, b, s);
         __syncwarp();
         const double t1 = p.t1 ? p.t1[b] : p.t1s;
@@ -72,6 +79,17 @@ d2jac_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStride
         d2jac_emit(sys, ws, nz, t2 - t1, out);
         if (out.k) out.flush();
     }
+}
+
+__global__ void __launch_bounds__(128, TREPB_D2JAC_MINB)
+d2jac_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<Dual> wsp, const D2Params p,
+             double* __restrict__ G, const JacLayout jl, long b0, long nb) {
+    d2jac_body<false>(rsys, dblob, blob_bytes, wsp, p, G, jl, b0, nb, VariedArgs{});
+}
+__global__ void __launch_bounds__(128, TREPB_D2JAC_MINB)
+d2jac_varied_kernel(const RtSys rsys, const char* dblob, int blob_bytes, const WsStridedT<Dual> wsp, const D2Params p,
+                    double* __restrict__ G, const JacLayout jl, long b0, long nb, const VariedArgs va) {
+    d2jac_body<true>(rsys, dblob, blob_bytes, wsp, p, G, jl, b0, nb, va);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -408,8 +426,8 @@ size_t d2jac_smem(int blob_bytes, int block, int nd, int nk) {
     const int n8 = ((blob_bytes + 7) / 8 + 1) & ~1;
     return sizeof(double) * ((size_t)n8 + (size_t)(block / 32) * 32 * 33) + (size_t)NzMaps::bytes(nd, nk);
 }
-cudaError_t d2jac_occupancy(int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
-    const void* fn = (const void*)d2jac_kernel;
+cudaError_t d2jac_occupancy(bool varied, int block, size_t smem, int* blocks_per_sm, KernelInfo* info) {
+    const void* fn = varied ? (const void*)d2jac_varied_kernel : (const void*)d2jac_kernel;
     cudaFuncAttributes a;
     cudaError_t e = cudaFuncGetAttributes(&a, fn);
     if (e != cudaSuccess) return e;
@@ -421,12 +439,14 @@ cudaError_t d2jac_occupancy(int block, size_t smem, int* blocks_per_sm, KernelIn
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, fn, block, smem);
 }
 cudaError_t d2jac_run(const LaunchCfg& c, const WsStridedT<Dual>& w, const D2Params& p, double* G, const JacLayout& jl,
-                      long b0, long nb) {
+                      long b0, long nb, const VariedArgs* va) {
+    const void* fn = va ? (const void*)d2jac_varied_kernel : (const void*)d2jac_kernel;
     if (c.smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute((const void*)d2jac_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem);
+        cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem);
         if (e != cudaSuccess) return e;
     }
-    d2jac_kernel<<<c.grid, c.block, c.smem, c.stream>>>(*c.sys, c.dblob, c.blob_bytes, w, p, G, jl, b0, nb);
+    if (va) d2jac_varied_kernel<<<c.grid, c.block, c.smem, c.stream>>>(*c.sys, c.dblob, c.blob_bytes, w, p, G, jl, b0, nb, *va);
+    else d2jac_kernel<<<c.grid, c.block, c.smem, c.stream>>>(*c.sys, c.dblob, c.blob_bytes, w, p, G, jl, b0, nb);
     return cudaGetLastError();
 }
 size_t d2solve_smem_needed(int nd, int nk, int nc, int nx, int aux_size) {

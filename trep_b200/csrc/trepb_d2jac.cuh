@@ -357,10 +357,11 @@ TREPB_HD void d2_pair(const D2Pair& P, const D2Params& p, long b, int nd, int nk
 
 #if defined(__CUDACC__)
 // launchers (trepb_d2jac.cu)
-cudaError_t d2jac_occupancy(int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
+// pass A: d2jac_kernel, or d2jac_varied_kernel for a non-null VariedArgs / `varied` (table-driven map and slots)
+cudaError_t d2jac_occupancy(bool varied, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
 size_t d2jac_smem(int blob_bytes, int block, int nd, int nk);
 cudaError_t d2jac_run(const LaunchCfg& c, const WsStridedT<Dual>& w, const D2Params& p, double* G, const JacLayout& jl,
-                      long b0, long nb);
+                      long b0, long nb, const VariedArgs* va);
 size_t d2solve_smem(int nd, int nk, int nc, int aux_size, int T);
 // shared memory pass B needs for this shape (compile-time-size flavour where one exists)
 size_t d2solve_smem_needed(int nd, int nk, int nc, int nx, int aux_size);

@@ -140,8 +140,9 @@ struct KernelSet {
     cudaError_t (*proj)(const LaunchCfg&, const ProjParams&, const VariedArgs*);
     // which: 0 step, 1 p2, 2 lin, 3 project, of the *_varied_kernel set when `varied`.  blocks_per_sm at (block, smem).
     cudaError_t (*occupancy)(int which, bool varied, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
-    cudaError_t (*d2)(const LaunchCfg&, const WsStridedT<HDG>&, const D2Params&);
-    cudaError_t (*d2_occupancy)(int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
+    // second derivatives, per-pair scheme: d2_kernel, or d2_varied_kernel for a non-null VariedArgs / `varied`
+    cudaError_t (*d2)(const LaunchCfg&, const WsStridedT<HDG>&, const D2Params&, const VariedArgs*);
+    cudaError_t (*d2_occupancy)(bool varied, int block, size_t smem, int* blocks_per_sm, KernelInfo* info);
 };
 
 // factorizations and tables of deriv1 that the second-derivative kernel reuses (AuxLayout)
@@ -181,8 +182,10 @@ struct SpecRegistry {
 SpecRegistry& spec_registry();
 // Layout fingerprint of everything a specialisation unit shares with the library (kernel parameter structs,
 // the kernel-set table).  A plug-in compiled against other headers registers with another fingerprint and is
-// refused by spec_register (which lives in the library), instead of being called with mismatched structs.
-constexpr unsigned kSpecAbi = 0x20000u + (unsigned)(sizeof(RtSys) * 131 + sizeof(StepParams) * 31 + sizeof(LinParams) * 17 +
+// refused by spec_register (which lives in the library), instead of being called with mismatched structs.  The base
+// constant changes whenever a member of KernelSet changes meaning without changing size (0x30000: d2 / d2_occupancy
+// gained their per-instance-parameter argument).
+constexpr unsigned kSpecAbi = 0x30000u + (unsigned)(sizeof(RtSys) * 131 + sizeof(StepParams) * 31 + sizeof(LinParams) * 17 +
                                                     sizeof(ProjParams) * 13 + sizeof(P2Params) * 7 + sizeof(D2Params) * 5 +
                                                     sizeof(LaunchCfg) * 3 + sizeof(KernelSet));
 bool spec_register(const KernelSet* ks, unsigned abi);

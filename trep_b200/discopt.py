@@ -34,6 +34,7 @@ class DSystem:
         self._nQ, self._np, self._nv, self._nu, self._nrho = v.nq, v.nd, v.nk, v.nu, v.nk
         self._nX = self._nQ + self._np + self._nv
         self._nU = self._nu + self._nrho
+        self._params = None
 
     nX = property(lambda s: s._nX)
     nU = property(lambda s: s._nU)
@@ -41,6 +42,40 @@ class DSystem:
 
     def kf(self):
         return len(self._time) - 1
+
+    # ---- per-rollout physical parameters -----------------------------------------------------------------
+    def set_parameters(self, refs, values):
+        """Physical parameters per rollout for robust trajectory optimisation over several plausible models: refs a
+        list of SystemDesc.param_ref entries, values [R][len(refs)] (one row per rollout) or one row ([n] / [1, n])
+        for every rollout and instance.  set_parameters(None, None) goes back to the description's numbers.
+        Trajectory-level calls with R rollouts (linearize_trajectory, calc_feedback_controller, calc_newton_model,
+        project, simulate) run rollout r on row r at every step; instance-level calls (f, linearize,
+        second_derivatives) take one row per instance; the check_* helpers need a single row.  Any other row count
+        raises ValueError."""
+        if refs is None:
+            self._params = None
+            return
+        from . import lib
+        refs = [tuple(r) for r in refs]
+        lib.check_params(self.varint.desc, refs)
+        values = np.asarray(values, dtype=np.float64)
+        if values.ndim > 2 or values.size == 0 or values.shape[-1] != len(refs):
+            raise ValueError("parameter values must be [R][%d] or [%d]" % (len(refs), len(refs)))
+        self._params = (refs, np.ascontiguousarray(values.reshape(-1, len(refs))))
+
+    def _rows(self, n, per=1):
+        """(refs, values [n][len(refs)]) for n instances, consecutive runs of `per` instances sharing a row (the steps
+        of one rollout), or None without parameters."""
+        if self._params is None:
+            return None
+        refs, V = self._params
+        if V.shape[0] == 1:
+            return refs, np.ascontiguousarray(np.repeat(V, n, axis=0))
+        if V.shape[0] * per != n:
+            raise ValueError("parameters have %d rows; this call needs %s or a single row"
+                             % (V.shape[0], "%d (one per instance)" % n if per == 1 else
+                                "%d (one per rollout)" % (n // per)))
+        return refs, (V if per == 1 else np.ascontiguousarray(np.repeat(V, per, axis=0)))
 
     # ---- state packing (dsystem.py:118-226) -----------------------------------------------------------
     def build_state(self, Q=None, p=None, v=None):
@@ -162,14 +197,20 @@ class DSystem:
         q1, p1, _ = self.split_state(X)
         u1, rho = self.split_input(U)
         out = self.varint.sys.step(q1, p1, t1, t2 - t1, nsteps=1, u1=u1[:, None, :] if self._nu else None,
-                                   k2=rho[:, None, :] if self._nv else None, tolerance=self.varint.tolerance)
+                                   k2=rho[:, None, :] if self._nv else None, tolerance=self.varint.tolerance,
+                                   params=self._rows(X.shape[0]))
         bad = np.flatnonzero(out["status"] != 0)
         if bad.size:
             raise ConvergenceError("%d of %d steps failed" % (bad.size, X.shape[0]), out["status"])
         v2 = (out["q2"][:, self._np:] - q1[:, self._np:]) / (t2 - t1)
         return self.build_state(out["q2"], out["p2"], v2)
 
+    def _single_row(self):
+        if self._params is not None and self._params[1].shape[0] != 1:
+            raise ValueError("the check_* helpers need a single parameter row (set_parameters)")
+
     def _lin_at(self, X, U, k):
+        self._single_row()
         n = X.shape[0]
         return self.linearize(X, U, np.full(n, self._time[k]), np.full(n, self._time[k + 1]))
 
@@ -202,6 +243,7 @@ class DSystem:
     def _second(self, xk, uk, k):
         """fdxdx(e_i), fdxdu(e_i), fdudu(e_i) for every unit vector e_i of the state space: one batch of nX
         instances of the z-contracted second-derivative kernel."""
+        self._single_row()
         nX = self._nX
         t1, t2 = np.full(nX, self._time[k]), np.full(nX, self._time[k + 1])
         return self.second_derivatives(np.tile(xk, (nX, 1)), np.tile(uk, (nX, 1)), np.eye(nX), t1, t2)
@@ -240,6 +282,10 @@ class DSystem:
         everywhere=True) device to device: gather="nccl" (ncclSend/Recv or ncclAllGather on the finished
         slabs) or gather="peer" (rank 0's slab is mapped into every rank and the linearize kernel writes
         its block straight into it).  Ranks that do not receive the result return None."""
+        return self._linearize(X, U, t1, t2, X_hint, group, gather, everywhere, 1)
+
+    def _linearize(self, X, U, t1, t2, X_hint, group, gather, everywhere, per):
+        """linearize, consecutive runs of `per` instances sharing a parameter row (the steps of one rollout)."""
         X, U = np.asarray(X, float), np.asarray(U, float)
         n = X.shape[0]
         world = 1 if group is None else group.world
@@ -250,11 +296,16 @@ class DSystem:
         hint = None if X_hint is None else np.asarray(X_hint, float)[lo:hi, :self._np]
         t1 = np.broadcast_to(np.asarray(t1, float), (n,))[lo:hi]
         t2 = np.broadcast_to(np.asarray(t2, float), (n,))[lo:hi]
+        params = self._rows(n, per)
+        if params is not None:
+            params = (params[0], np.ascontiguousarray(params[1][lo:hi]))
         if world == 1:
-            out = self.varint.sys.linearize(q1, p1, u1, rho2, t1=t1, t2=t2, q2_guess=hint, tolerance=self.varint.tolerance)
+            out = self.varint.sys.linearize(q1, p1, u1, rho2, t1=t1, t2=t2, q2_guess=hint, tolerance=self.varint.tolerance,
+                                            params=params)
             A, B, status = out["A"], out["B"], out["status"]
         else:
-            A, B, status = self._linearize_sharded(q1, p1, u1, rho2, t1, t2, hint, n, lo, hi, group, gather, everywhere)
+            A, B, status = self._linearize_sharded(q1, p1, u1, rho2, t1, t2, hint, n, lo, hi, group, gather, everywhere,
+                                                   params)
             if A is None:
                 return None
         bad = np.flatnonzero(status != 0)
@@ -263,14 +314,17 @@ class DSystem:
                                    % (bad.size, n, bad[0], status[bad[0]]), status)
         return self.linearization_return(A, B)
 
-    def _linearize_sharded(self, q1, p1, u1, rho2, t1, t2, hint, n, lo, hi, group, gather, everywhere):
-        """This rank's block on its GPU, results collected on rank 0 without leaving device memory."""
+    def _linearize_sharded(self, q1, p1, u1, rho2, t1, t2, hint, n, lo, hi, group, gather, everywhere, params=None):
+        """This rank's block on its GPU, results collected on rank 0 without leaving device memory.  params: this
+        block's parameter rows."""
         from . import dist, lib
         sys_, dev = self.varint.sys, self.varint.sys.device
         nX, nU, cnt = self._nX, self._nU, hi - lo
         up = lambda a: lib.DeviceBuffer(dev, a.shape, np.float64).upload(np.ascontiguousarray(a, dtype=np.float64))
         ins = dict(q1=up(q1), p1=up(p1), u1=up(u1) if self._nu else None, k2=up(rho2) if self._nv else None,
-                   t1=up(t1), t2=up(t2), hint=None if hint is None else up(hint))
+                   t1=up(t1), t2=up(t2), hint=None if hint is None else up(hint),
+                   params=None if params is None else up(params[1]))
+        dpar = None if params is None else (params[0], ins["params"])
         rowA, rowB = nX * nX * 8, nX * nU * 8
         root = group.rank == 0
         slabs = []
@@ -282,7 +336,8 @@ class DSystem:
                 slabs.append(slab)
                 sys_.linearize_raw(True, cnt, ins["q1"], ins["p1"], ins["u1"], ins["k2"], slab.at(offS + lo * 4),
                                    t1=ins["t1"], t2=ins["t2"], q2_guess=ins["hint"], A=slab.at(lo * rowA),
-                                   B=slab.at(offB + lo * rowB) if nU else None, tolerance=self.varint.tolerance)
+                                   B=slab.at(offB + lo * rowB) if nU else None, tolerance=self.varint.tolerance,
+                                   params=dpar)
                 lib.synchronize(dev)
                 group.barrier()          # every rank's stores have reached rank 0's HBM
                 res = None
@@ -299,7 +354,8 @@ class DSystem:
             dS = lib.DeviceBuffer(dev, (max(cnt, 1),), np.int32)
             slabs += [dA, dB, dS]
             sys_.linearize_raw(True, cnt, ins["q1"], ins["p1"], ins["u1"], ins["k2"], dS, t1=ins["t1"], t2=ins["t2"],
-                               q2_guess=ins["hint"], A=dA, B=dB if nU else None, tolerance=self.varint.tolerance)
+                               q2_guess=ins["hint"], A=dA, B=dB if nU else None, tolerance=self.varint.tolerance,
+                               params=dpar)
             out = []
             for buf, rb, dt, shape in ((dA, rowA, np.float64, (n, nX, nX)), (dB, rowB, np.float64, (n, nX, nU)),
                                        (dS, 4, np.int32, (n,))):
@@ -323,6 +379,10 @@ class DSystem:
         fdxdx(z), fdxdu(z), fdudu(z) (dsystem.py:320-386) return after set(X[i], U[i], k).
         X [n,nX], U [n,nU], Z [n,nX], t1/t2 [n].  Returns (fdxdx [n,nX,nX], fdxdu [n,nX,nU],
         fdudu [n,nU,nU]); the full 30 tensors are never materialised."""
+        return self._second_derivatives(X, U, Z, t1, t2, X_hint, 1)
+
+    def _second_derivatives(self, X, U, Z, t1, t2, X_hint, per):
+        """second_derivatives, consecutive runs of `per` instances sharing a parameter row (the steps of one rollout)."""
         X, U, Z = np.asarray(X, float), np.asarray(U, float), np.asarray(Z, float)
         n = X.shape[0]
         q1, p1, _ = self.split_state(X)
@@ -330,7 +390,7 @@ class DSystem:
         hint = None if X_hint is None else np.asarray(X_hint, float)[:, :self._np]
         out = self.varint.sys.deriv2(q1, p1, u1, rho2, t1=np.broadcast_to(np.asarray(t1, float), (n,)),
                                      t2=np.broadcast_to(np.asarray(t2, float), (n,)), q2_guess=hint,
-                                     tolerance=self.varint.tolerance, z=Z, tensors=False)
+                                     tolerance=self.varint.tolerance, z=Z, tensors=False, params=self._rows(n, per))
         bad = np.flatnonzero(out["status"] != 0)
         if bad.size:
             raise ConvergenceError("%d of %d instances failed" % (bad.size, n), out["status"])
@@ -356,8 +416,8 @@ class DSystem:
             Acl = A[:, k] - np.einsum("rxu,ruy->rxy", B[:, k], K[:, k])
             Z[:, k] = l_dx[:, k] - np.einsum("ru,rux->rx", l_du[:, k], K[:, k]) + np.einsum("rx,rxy->ry", Z[:, k + 1], Acl)
         t1, t2 = np.tile(self._time[:n], R), np.tile(self._time[1:n + 1], R)
-        xx, xu, uu = self.second_derivatives(X[:, :n].reshape(R * n, -1), U[:, :n].reshape(R * n, -1),
-                                             Z[:, 1:].reshape(R * n, -1), t1, t2, X_hint=X[:, 1:].reshape(R * n, -1))
+        xx, xu, uu = self._second_derivatives(X[:, :n].reshape(R * n, -1), U[:, :n].reshape(R * n, -1),
+                                              Z[:, 1:].reshape(R * n, -1), t1, t2, X[:, 1:].reshape(R * n, -1), n)
         xx = xx.reshape(R, n, self._nX, self._nX); xu = xu.reshape(R, n, self._nX, self._nU)
         uu = uu.reshape(R, n, self._nU, self._nU)
         if single:
@@ -377,8 +437,8 @@ class DSystem:
         assert U.shape[1] >= K and len(self._time) >= K + 1
         t1 = np.tile(self._time[:K], R)
         t2 = np.tile(self._time[1:K + 1], R)
-        res = self.linearize(X[:, :K].reshape(R * K, -1), U[:, :K].reshape(R * K, -1), t1, t2,
-                             X_hint=X[:, 1:K + 1].reshape(R * K, -1), group=group, gather=gather, everywhere=everywhere)
+        res = self._linearize(X[:, :K].reshape(R * K, -1), U[:, :K].reshape(R * K, -1), t1, t2,
+                              X[:, 1:K + 1].reshape(R * K, -1), group, gather, everywhere, K)
         if res is None:
             return None
         A, B = res
@@ -415,11 +475,13 @@ class DSystem:
         dst = lib.DeviceBuffer(dev, (n,), np.int32)
         dQ, dR = up(Q), up(R)
         dK, dls = lib.DeviceBuffer(dev, (Rn, K, nU, nX)), lib.DeviceBuffer(dev, (Rn,), np.int32)
-        bufs = [b for b in (dq1, dp1, du1, dk2, dhint, dt1, dt2, dA, dB, dst, dQ, dR, dK, dls) if b is not None]
+        params = self._rows(n, K)
+        dpar = None if params is None else up(params[1])
+        bufs = [b for b in (dq1, dp1, du1, dk2, dhint, dt1, dt2, dA, dB, dst, dQ, dR, dK, dls, dpar) if b is not None]
         try:
             # linearize -> Riccati sweep without the A / B slabs leaving the GPU
             sys_.linearize_raw(True, n, dq1, dp1, du1, dk2, dst, t1=dt1, t2=dt2, q2_guess=dhint, A=dA, B=dB,
-                               tolerance=self.varint.tolerance)
+                               tolerance=self.varint.tolerance, params=None if dpar is None else (params[0], dpar))
             lib.lqr_raw(True, dev, Rn, K, nX, nU, dA, dB, dQ, dR, dK, dls, q_per_step=Q.ndim == 3, r_per_step=R.ndim == 3)
             lib.synchronize(dev)
             status, ls = dst.download(), dls.download()
@@ -458,7 +520,8 @@ class DSystem:
         # the kernel steps on this system's own time grid, uniform or not (dsystem.py:426-457 uses self._time[k])
         out = self.varint.sys.project(bX, bU[:, :K], np.asarray(Kproj, float), self._time[0],
                                       float(self._time[1] - self._time[0]), use_hint=use_hint,
-                                      tolerance=self.varint.tolerance, times=self._time[:K + 1])
+                                      tolerance=self.varint.tolerance, times=self._time[:K + 1],
+                                      params=self._rows(bX.shape[0]))
         self.last_project = out
         bad = np.flatnonzero(out["status"] != 0)
         if bad.size:
@@ -471,7 +534,9 @@ class DSystem:
 
     def simulate(self, X0, U):
         """Rollouts X[k+1] = f(X[k], U[k], k) from X0 [R, nX] with U [R, K, nU] in one launch
-        (what repeated DSystem.step calls do, dsystem.py:253-281).  Returns X [R, K+1, nX]."""
+        (what repeated DSystem.step calls do, dsystem.py:253-281).  Returns X [R, K+1, nX].  With set_parameters,
+        rollout r runs on row r; the MidpointVI is left at the final states reached on those rows, while its own
+        parameters (none) stay as they were."""
         X0, U = np.atleast_2d(np.asarray(X0, float)), np.asarray(U, float)
         if U.ndim == 2:
             U = U[None]
@@ -482,9 +547,12 @@ class DSystem:
         q0, p0, _ = self.split_state(X0)
         u, rho = self.split_input(U)
         v = self.varint
+        params = self._rows(X0.shape[0])   # rollout r on row r
+        if params is not None and v._params is not None:
+            raise ValueError("parameters are set on both the DSystem and its MidpointVI: clear one of them")
         v.initialize_from_state(self._time[0], q0, p0)
         out = v.simulate(K, float(dts[0]), u=u if self._nu else None, k=rho if self._nv else None, sample_every=1,
-                         times=self._time[:K + 1])
+                         times=self._time[:K + 1], params=params)
         Q = np.concatenate([q0[:, None, :], out["traj_q"]], axis=1)
         P = np.concatenate([p0[:, None, :], out["traj_p"]], axis=1)
         X = np.zeros((R, K + 1, self._nX))

@@ -166,7 +166,7 @@ _lib.trepb_measure_fp64_peak.argtypes = [C.c_int, _dp]
 _vp = C.POINTER(Varied)
 _lib.trepb_varied_check.argtypes = [C.c_void_p, _vp]
 # trepb_<call>_varied_batch[_dev]: the arguments of trepb_<call>_batch, then the trepb_varied (and the stream)
-for _call in ("step", "project", "linearize", "calc_p2", "calc_f", "discrete_fm2"):
+for _call in ("step", "project", "linearize", "calc_p2", "calc_f", "discrete_fm2", "deriv2"):
     _plain = getattr(_lib, "trepb_%s_batch" % _call).argtypes
     getattr(_lib, "trepb_%s_varied_batch" % _call).argtypes = _plain + [_vp]
     getattr(_lib, "trepb_%s_varied_batch_dev" % _call).argtypes = _plain + [_vp, C.c_void_p]
@@ -189,6 +189,7 @@ EXPORTS = [
     "trepb_linearize_varied_batch_dev", "trepb_project_varied_batch", "trepb_project_varied_batch_dev",
     "trepb_calc_p2_varied_batch", "trepb_calc_p2_varied_batch_dev", "trepb_calc_f_varied_batch",
     "trepb_calc_f_varied_batch_dev", "trepb_discrete_fm2_varied_batch", "trepb_discrete_fm2_varied_batch_dev",
+    "trepb_deriv2_varied_batch", "trepb_deriv2_varied_batch_dev",
 ]
 
 
@@ -575,19 +576,17 @@ class System:
         self._call("linearize", on_device, params, stream, C.byref(a))
 
     def deriv2_raw(self, on_device, batch, q1, p1, u1, k2, status, d2, stream=None, z=None,
-                   fdxdx=None, fdxdu=None, fdudu=None, **kw):
+                   fdxdx=None, fdxdu=None, fdudu=None, params=None, **kw):
         """d2: {"q2_dq1dq1": array, ...} any subset of D2_WHICH x D2_KINDS; z + fdxdx/fdxdu/fdudu:
-        the z-contracted forms of DSystem.fdxdx(z) / fdxdu(z) / fdudu(z)."""
+        the z-contracted forms of DSystem.fdxdx(z) / fdxdu(z) / fdudu(z).  params: None, or (refs, values) with one
+        row per instance (trepb_deriv2_varied_batch*)."""
         a = D2Args()
         a.lin = self._lin_args(batch, q1, p1, u1, k2, status, **kw)
         a.z, a.fdxdx, a.fdxdu, a.fdudu = _ptr(z), _ptr(fdxdx), _ptr(fdxdu), _ptr(fdudu)
         for n, v in d2.items():
             w, kd = n.split("_")
             a.d2[10 * D2_WHICH.index(w) + D2_KINDS.index(kd)] = _ptr(v)
-        if on_device:
-            _check(_lib.trepb_deriv2_batch_dev(self._h, C.byref(a), stream))
-        else:
-            _check(_lib.trepb_deriv2_batch(self._h, C.byref(a)))
+        self._call("deriv2", on_device, params, stream, C.byref(a))
 
     def project_raw(self, on_device, batch, nsteps, t0, dt, bX, bU, Kfb, X, U, status, k_per_instance=False,
                     use_hint=True, iters=None, fail_step=None, tolerance=1e-10, max_iterations=200, stream=None,
@@ -754,9 +753,10 @@ class System:
         return out
 
     def deriv2(self, q1, p1, u1=None, k2=None, t1=0.0, t2=None, dt=None, q2_guess=None,
-               lambda_guess=None, tolerance=1e-10, max_iterations=200, z=None, tensors=True):
+               lambda_guess=None, tolerance=1e-10, max_iterations=200, z=None, tensors=True, params=None):
         """solve + first derivatives + every second-derivative tensor (reference layout
-        [B][wrt A][wrt B][out]); returns the dict of `linearize(want_raw=True)` plus the tensors."""
+        [B][wrt A][wrt B][out]); returns the dict of `linearize(want_raw=True)` plus the tensors.
+        params: None, or (refs, values [B][len(refs)]) per-instance parameters."""
         q1 = np.atleast_2d(np.asarray(q1, float))
         B = q1.shape[0]
         q1, p1 = self._f(q1, (B, self.nq)), self._f(p1, (B, self.nd))
@@ -784,7 +784,7 @@ class System:
                         lambda_guess=lg, q2=out["q2"], p2=out["p2"],
                         lambda1=out["lambda1"] if self.nc else None, iters=out["iters"], A=out["A"],
                         B=out["B"] if self.nU else None, raw={k: v for k, v in rawbufs.items() if v.size},
-                        tolerance=tolerance, max_iterations=max_iterations)
+                        tolerance=tolerance, max_iterations=max_iterations, params=self._params(params, B))
         out.update(rawbufs)
         out.update(d2)
         return out

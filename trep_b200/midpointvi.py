@@ -51,8 +51,9 @@ class MidpointVI:
     def set_parameters(self, refs, values):
         """Per-instance physical parameters for every later initialize_from_*, step, simulate, calc_f,
         discrete_fm2 and first-derivative call: refs a list of SystemDesc.param_ref entries, values [B][len(refs)]
-        (instance b runs on row b).  set_parameters(None, None) goes back to the description's numbers.  Second
-        derivatives have no per-instance form: they raise while parameters are set."""
+        (instance b runs on row b).  set_parameters(None, None) goes back to the description's numbers.  The
+        second-derivative getters raise while parameters are set (lib.System.deriv2(params=...) and
+        DSystem.set_parameters take per-instance parameters)."""
         if refs is None:
             self._params = None
         else:
@@ -128,15 +129,22 @@ class MidpointVI:
         self._check(out["status"])
         return out["iters"]
 
-    def simulate(self, nsteps, dt, u=None, k=None, max_iterations=200, sample_every=0, times=None):
+    def simulate(self, nsteps, dt, u=None, k=None, max_iterations=200, sample_every=0, times=None, params=None):
         """`nsteps` steps inside one kernel launch (the Monte-Carlo / rollout path): of length dt, or on
         the grid `times` [nsteps+1] (times[0] = the current t2; any spacing).
         u: [B, nsteps, nu], k: [B, nsteps, nk] (kinematic configs at the END of each step).
+        params: (refs, values [B][len(refs)]) for this call only, instead of set_parameters' (ValueError when both
+        are set); the state it leaves was reached on those rows, later calls run on set_parameters' again.
         Returns dict(iters, traj_q, traj_p) - trajectories only if sample_every > 0."""
+        if params is not None and self._params is not None:
+            raise ValueError("parameters are set on this MidpointVI and passed to simulate: clear one of them")
+        if params is not None:
+            refs = [tuple(r) for r in params[0]]
+            params = (refs, np.ascontiguousarray(np.asarray(params[1], dtype=np.float64).reshape(self.batch, len(refs))))
         out = self.sys.step(self.q2, self.p2, self.t2, float(dt), nsteps=nsteps, u1=u, k2=k,
                             lambda_guess=self.lambda1 if self.nc else None, tolerance=self.tolerance,
                             max_iterations=max_iterations, sample_every=sample_every, times=times,
-                            params=self._p(self.batch))
+                            params=self._p(self.batch) if params is None else params)
         # state before the last step is only known when a trajectory was captured
         self.q1 = self.p1 = None
         t = self.t2
@@ -202,8 +210,9 @@ class MidpointVI:
     #      [B][wrt A][wrt B][out]  (trep.h:439-473), e.g. q2_dq1dq1()[b, i, j, :] = d2 q2 / dq1_i dq1_j
     def _calc_deriv2(self):
         if self._params is not None:
-            raise NotImplementedError("second derivatives have no per-instance-parameter form: "
-                                      "call set_parameters(None, None) first")
+            raise NotImplementedError("MidpointVI's second-derivative getters have no per-instance-parameter form: "
+                                      "call set_parameters(None, None) first, or use lib.System.deriv2(params=...) "
+                                      "or DSystem.set_parameters")
         if getattr(self, "_d2", None) is None or self._lin is None:
             assert self.q1 is not None and self.p1 is not None, "derivatives need the state before the step"
             out = self.sys.deriv2(self.q1, self.p1, self.u1, self.q2[:, self.nd:], t1=self.t1, t2=self.t2,
