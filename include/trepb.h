@@ -23,7 +23,11 @@
  *                            (trep/discopt/dsystem.py:426-457, doptimizer.py:405-428).
  *   trepb_lqr_batch*         discopt.dlqr.solve_tv_lqr (trep/discopt/dlqr.py:9-38), the Riccati sweep of
  *                            DSystem.calc_feedback_controller (trep/discopt/dsystem.py:474-494).
- *   trepb_linearize_batch*   DSystem.set + fdx + fdu for every k of
+ *   trepb_tangent_batch*     DSystem.dproject (trep/discopt/dsystem.py:460-471): the forward sweep of a
+ *                            descent direction, on the slabs the two calls above leave in HBM.
+ *   trepb_adjoint_batch*     the costate recursion of DOptimizer.calc_newton_model
+ *                            (trep/discopt/doptimizer.py:319-345).
+ *   trepb_linearize_batch*  DSystem.set + fdx + fdu for every k of
  *                            DSystem.linearize_trajectory (trep/discopt/dsystem.py:229-250,
  *                            284-317, 406-423) == solve_DEL + MidpointVI_calc_deriv1
  *                            (trep/_trep/midpointvi.c:1100-1120).
@@ -315,6 +319,58 @@ int trepb_lq_batch_dev(int device, const trepb_lq_args* args, void* stream); /* 
  * (mma.sync m8n8k4, 16 x 40 warp tiles, ragged edges read as zero), below that on 4 x 4 register tiles; the
  * gamma solve is a Gauss-Jordan elimination by the whole CTA (nU (nU + nX + 1) <= 2048).                  */
 int trepb_lqr_last_kernel_ms(int device, float* ms);
+
+/* Tangent (forward) sweep about a linearization, batched over rollouts: DSystem.dproject
+ * (trep/discopt/dsystem.py:460-471) and the last loop of DOptimizer.calc_descent_direction
+ * (trep/discopt/doptimizer.py:348-402):
+ *     dX[0] = x0 (NULL: bdX[0], or zero when bdX is NULL);
+ *     dU[k] = bdU[k] - K[k] (dX[k] - bdX[k]);   dX[k+1] = A[k] dX[k] + B[k] dU[k]
+ * It reads the A / B slabs trepb_linearize_batch_dev writes and the gains of trepb_lqr_batch_dev /
+ * trepb_lq_batch_dev as they are.  No system handle is needed.  One team of lanes per rollout streams
+ * each step through shared memory; every output element is summed in a fixed order, so a rollout gives
+ * the same bits alone and inside any batch.  nU = 0 is allowed (B, K, bdU and dU may then be NULL).  */
+typedef struct trepb_tangent_args {
+    int64_t batch;            /* rollouts                                              */
+    int32_t nsteps;           /* K                                                     */
+    int32_t nX, nU;
+    int32_t _pad;
+    const double* A;          /* [batch][K][nX][nX]                                    */
+    const double* B;          /* [batch][K][nX][nU]                                    */
+    const double* K;          /* [batch][K][nU][nX]                                    */
+    const double* bdX;        /* [batch][K+1][nX], NULL = zero                         */
+    const double* bdU;        /* [batch][K][nU], NULL = zero                           */
+    const double* x0;         /* [batch][nX] dX[0], NULL = bdX[0] (zero without bdX)   */
+    double* dX;               /* [batch][K+1][nX] out                                  */
+    double* dU;               /* [batch][K][nU] out                                    */
+} trepb_tangent_args;
+
+int trepb_tangent_batch(int device, const trepb_tangent_args* args);                   /* host pointers   */
+int trepb_tangent_batch_dev(int device, const trepb_tangent_args* args, void* stream); /* device pointers */
+
+/* Adjoint (backward) sweep, batched over rollouts: the costate recursion of DOptimizer.calc_newton_model
+ * (trep/discopt/doptimizer.py:319-345),
+ *     z[K] = m_dx;   z[k] = l_dx[k] - K[k]^T l_du[k] + A[k]^T z[k+1] - K[k]^T (B[k]^T z[k+1]),
+ * evaluated as l_dx[k] + A[k]^T z[k+1] - K[k]^T (l_du[k] + B[k]^T z[k+1]) (A - B K is never formed).
+ * K NULL gives the open-loop costate z[k] = l_dx[k] + A[k]^T z[k+1].  Same layouts and team scheme as
+ * trepb_tangent_batch.  z1, if given, receives z[k+1] for k < K, packed [batch][K][nX]: the costate each step's
+ * z-contracted second derivatives take (trepb_deriv2_batch_dev's z over the batch x K step instances).  */
+typedef struct trepb_adjoint_args {
+    int64_t batch;            /* rollouts                                              */
+    int32_t nsteps;           /* K                                                     */
+    int32_t nX, nU;
+    int32_t _pad;
+    const double* A;          /* [batch][K][nX][nX]                                    */
+    const double* B;          /* [batch][K][nX][nU], needed with K                     */
+    const double* K;          /* [batch][K][nU][nX], NULL = open loop                  */
+    const double* l_dx;       /* [batch][K][nX], NULL = zero                           */
+    const double* l_du;       /* [batch][K][nU], NULL = zero                           */
+    const double* m_dx;       /* [batch][nX]                                           */
+    double* z;                /* [batch][K+1][nX] out                                  */
+    double* z1;               /* [batch][K][nX] out (z[k+1]), may be NULL              */
+} trepb_adjoint_args;
+
+int trepb_adjoint_batch(int device, const trepb_adjoint_args* args);                   /* host pointers   */
+int trepb_adjoint_batch_dev(int device, const trepb_adjoint_args* args, void* stream); /* device pointers */
 
 /* p2 from two consecutive configurations (initialize_from_configs). q0,q1: [B][nq] -> p: [B][nd] */
 int trepb_calc_p2_batch(trepb_system* sys, int64_t batch, double dt,

@@ -22,6 +22,7 @@
 #include "../../include/trepb.h"
 #include "trepb_coop_math.cuh"
 #include "trepb_err.h"
+#include "trepb_sweep.cuh"
 
 namespace trepb {
 namespace {
@@ -580,4 +581,137 @@ extern "C" int trepb_lqr_batch(int device, const trepb_lqr_args* a) {
 #undef LQ
     cudaFree(dA); cudaFree(dB); cudaFree(dQ); cudaFree(dR); cudaFree(dK); cudaFree(dP); cudaFree(dS);
     return rc;
+}
+
+// ---- tangent / adjoint sweeps (trepb_sweep.cuh) ----------------------------------------------------------------
+namespace {
+int sweep_launch(int device, SweepParams& p, bool tangent, cudaStream_t stream) {
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    // one team of lanes per rollout, a power of two covering the longer of a state row / an input row
+    const int rows = p.nX > p.nU ? p.nX : p.nU;
+    int team = 1;
+    while (team < rows && team < 128) team <<= 1;   // rows beyond 128 are strided over the team
+    const int block = team < 64 ? 64 : team, teams = block / team;
+    int smem_optin = 0;
+    e = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    // the deepest ring that fits: small states prefetch 7 steps ahead, the marionette's 74 KB steps one
+    int stages = 8;
+    while (stages >= 2 && (size_t)teams * sweep_team_doubles(p.nX, p.nU, stages) * 8 > (size_t)smem_optin) stages /= 2;
+    if (stages < 2) return lqr_fail(TREPB_ERR_UNSUPPORTED, "state dimension too large for the shared-memory sweep");
+    const size_t smem = (size_t)teams * sweep_team_doubles(p.nX, p.nU, stages) * 8;
+    p.team = team; p.stages = stages;
+    const void* fn = tangent ? (const void*)sweep_kernel<true> : (const void*)sweep_kernel<false>;
+    e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    long long grid = (p.batch + teams - 1) / teams;
+    if (grid > (1LL << 24)) grid = 1LL << 24;   // the kernel strides over the rest
+    if (tangent) sweep_kernel<true><<<(unsigned)grid, block, smem, stream>>>(p);
+    else sweep_kernel<false><<<(unsigned)grid, block, smem, stream>>>(p);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    return TREPB_OK;
+}
+
+// the checks every tangent / adjoint entry point makes before any CUDA call; -1 = go on
+int tangent_check(const trepb_tangent_args* a) {
+    if (!a) return lqr_fail(TREPB_ERR_INVALID, "null argument");
+    if (a->batch < 0 || a->nsteps < 1 || a->nX < 1 || a->nU < 0) return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    if (!a->A || !a->dX || (a->nU > 0 && (!a->B || !a->K || !a->dU)))
+        return lqr_fail(TREPB_ERR_INVALID, "A and dX are required, and B, K and dU when nU > 0");
+    if (a->batch == 0) return TREPB_OK;
+    return -1;
+}
+int adjoint_check(const trepb_adjoint_args* a) {
+    if (!a) return lqr_fail(TREPB_ERR_INVALID, "null argument");
+    if (a->batch < 0 || a->nsteps < 1 || a->nX < 1 || a->nU < 0) return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    if (!a->A || !a->m_dx || !a->z || (a->K && a->nU > 0 && !a->B))
+        return lqr_fail(TREPB_ERR_INVALID, "A, m_dx and z are required, and B when K is given");
+    if (a->batch == 0) return TREPB_OK;
+    return -1;
+}
+
+// host -> device staging of n_in inputs and n_out outputs around `run(device pointers)` (null / empty arrays
+// stay null); synchronous, like trepb_lq_batch
+template <int NI, int NO, class Run>
+int sweep_staged(int device, const void* const (&src)[NI], const size_t (&in_n)[NI], void* const (&dst)[NO],
+                 const size_t (&out_n)[NO], Run run) {
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    double* din[NI] = {nullptr};
+    double* dout[NO] = {nullptr};
+    int rc = TREPB_OK;
+#define SW(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess && rc == TREPB_OK) rc = lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e_)); } while (0)
+    for (int i = 0; i < NI; ++i)
+        if (src[i] && in_n[i]) {
+            SW(cudaMalloc(&din[i], in_n[i] * 8));
+            if (rc == TREPB_OK) SW(cudaMemcpy(din[i], src[i], in_n[i] * 8, cudaMemcpyHostToDevice));
+        }
+    for (int i = 0; i < NO; ++i) if (dst[i] && out_n[i]) SW(cudaMalloc(&dout[i], out_n[i] * 8));
+    if (rc == TREPB_OK) rc = run(din, dout);
+    if (rc == TREPB_OK) SW(cudaStreamSynchronize(nullptr));
+    if (rc == TREPB_OK)
+        for (int i = 0; i < NO; ++i) if (dout[i]) SW(cudaMemcpy(dst[i], dout[i], out_n[i] * 8, cudaMemcpyDeviceToHost));
+#undef SW
+    for (int i = 0; i < NI; ++i) cudaFree(din[i]);
+    for (int i = 0; i < NO; ++i) cudaFree(dout[i]);
+    return rc;
+}
+}  // namespace
+
+extern "C" int trepb_tangent_batch_dev(int device, const trepb_tangent_args* a, void* stream) {
+    TREPB_NVTX("trepb_tangent_batch_dev");
+    const int c = tangent_check(a);
+    if (c >= 0) return c;
+    SweepParams p{};
+    p.batch = a->batch; p.K = a->nsteps; p.nX = a->nX; p.nU = a->nU;
+    p.A = a->A; p.B = a->nU ? a->B : nullptr; p.Kfb = a->nU ? a->K : nullptr;
+    p.vx = a->bdX; p.vu = a->nU ? a->bdU : nullptr; p.x0 = a->x0;
+    p.ox = a->dX; p.ou = a->nU ? a->dU : nullptr;
+    return sweep_launch(device, p, true, (cudaStream_t)stream);
+}
+
+extern "C" int trepb_adjoint_batch_dev(int device, const trepb_adjoint_args* a, void* stream) {
+    TREPB_NVTX("trepb_adjoint_batch_dev");
+    const int c = adjoint_check(a);
+    if (c >= 0) return c;
+    SweepParams p{};
+    p.batch = a->batch; p.K = a->nsteps; p.nX = a->nX; p.nU = a->nU;
+    p.A = a->A; p.B = a->nU && a->K ? a->B : nullptr; p.Kfb = a->nU ? a->K : nullptr;
+    p.vx = a->l_dx; p.vu = a->nU && a->K ? a->l_du : nullptr; p.x0 = a->m_dx;
+    p.ox = a->z; p.ou = a->z1;
+    return sweep_launch(device, p, false, (cudaStream_t)stream);
+}
+
+extern "C" int trepb_tangent_batch(int device, const trepb_tangent_args* a) {
+    TREPB_NVTX("trepb_tangent_batch");
+    const int c = tangent_check(a);
+    if (c >= 0) return c;
+    const size_t Rn = (size_t)a->batch, K = (size_t)a->nsteps, nX = (size_t)a->nX, nU = (size_t)a->nU;
+    const void* const src[6] = {a->A, a->B, a->K, a->bdX, a->bdU, a->x0};
+    const size_t in_n[6] = {Rn * K * nX * nX, Rn * K * nX * nU, Rn * K * nU * nX, Rn * (K + 1) * nX, Rn * K * nU, Rn * nX};
+    void* const dst[2] = {a->dX, a->dU};
+    const size_t out_n[2] = {Rn * (K + 1) * nX, Rn * K * nU};
+    return sweep_staged(device, src, in_n, dst, out_n, [&](double* const* d, double* const* o) {
+        trepb_tangent_args x = *a;
+        x.A = d[0]; x.B = d[1]; x.K = d[2]; x.bdX = d[3]; x.bdU = d[4]; x.x0 = d[5]; x.dX = o[0]; x.dU = o[1];
+        return trepb_tangent_batch_dev(device, &x, nullptr);
+    });
+}
+
+extern "C" int trepb_adjoint_batch(int device, const trepb_adjoint_args* a) {
+    TREPB_NVTX("trepb_adjoint_batch");
+    const int c = adjoint_check(a);
+    if (c >= 0) return c;
+    const size_t Rn = (size_t)a->batch, K = (size_t)a->nsteps, nX = (size_t)a->nX, nU = (size_t)a->nU;
+    const void* const src[6] = {a->A, a->B, a->K, a->l_dx, a->l_du, a->m_dx};
+    const size_t in_n[6] = {Rn * K * nX * nX, Rn * K * nX * nU, Rn * K * nU * nX, Rn * K * nX, Rn * K * nU, Rn * nX};
+    void* const dst[2] = {a->z, a->z1};
+    const size_t out_n[2] = {Rn * (K + 1) * nX, Rn * K * nX};
+    return sweep_staged(device, src, in_n, dst, out_n, [&](double* const* d, double* const* o) {
+        trepb_adjoint_args x = *a;
+        x.A = d[0]; x.B = d[1]; x.K = d[2]; x.l_dx = d[3]; x.l_du = d[4]; x.m_dx = d[5]; x.z = o[0]; x.z1 = o[1];
+        return trepb_adjoint_batch_dev(device, &x, nullptr);
+    });
 }

@@ -448,6 +448,65 @@ class DSystem:
             A, B = A[0], B[0]
         return self.linearization_return(A, B)
 
+    def _feedback_on_device(self, Xb, Ub, Q, R):
+        """linearize -> Riccati sweep for Rn rollouts (Xb [Rn,K+1,nX], Ub [Rn,K,nU]), enqueued on the device without
+        the A / B slabs leaving the GPU.  Q / R as calc_feedback_controller.  Returns a dict of device buffers:
+        the linearization's inputs (q1, p1, u1, k2, hint, t1, t2, params), its outputs A, B, status, and the gains K
+        with their status lqr_status; the caller synchronizes, calls _check_feedback and frees them (_free)."""
+        from . import lib
+        Rn, K = Xb.shape[0], Xb.shape[1] - 1
+        Q = np.eye(self._nX) if Q is None else (np.stack([Q(k) for k in range(K + 1)]) if callable(Q) else np.asarray(Q, float))
+        R = np.eye(self._nU) if R is None else (np.stack([R(k) for k in range(K)]) if callable(R) else np.asarray(R, float))
+        sys_, dev = self.varint.sys, self.varint.sys.device
+        nX, nU, nq, nd = self._nX, self._nU, self._nQ, self._np
+        n = Rn * K
+        up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, a.shape, dt).upload(np.ascontiguousarray(a, dtype=dt))
+        Xk = Xb[:, :K].reshape(n, nX)
+        d = {}
+        try:
+            # inputs of the n = rollouts x steps independent linearizations, resident in HBM
+            d["q1"], d["p1"] = up(Xk[:, :nq]), up(Xk[:, nq:nq + nd])
+            d["u1"] = up(Ub[:, :K, :self._nu].reshape(n, -1)) if self._nu else None
+            d["k2"] = up(Ub[:, :K, self._nu:].reshape(n, -1)) if self._nv else None
+            d["hint"] = up(Xb[:, 1:K + 1, :nd].reshape(n, nd))
+            d["t1"], d["t2"] = up(np.tile(self._time[:K], Rn)), up(np.tile(self._time[1:K + 1], Rn))
+            d["A"], d["B"] = lib.DeviceBuffer(dev, (n, nX, nX)), lib.DeviceBuffer(dev, (n, nX, nU))
+            d["status"] = lib.DeviceBuffer(dev, (n,), np.int32)
+            d["Q"], d["R"] = up(Q), up(R)
+            d["K"], d["lqr_status"] = lib.DeviceBuffer(dev, (Rn, K, nU, nX)), lib.DeviceBuffer(dev, (Rn,), np.int32)
+            params = self._rows(n, K)
+            d["params"] = None if params is None else up(params[1])
+            d["refs"] = None if params is None else params[0]
+            # linearize -> Riccati sweep without the A / B slabs leaving the GPU
+            sys_.linearize_raw(True, n, d["q1"], d["p1"], d["u1"], d["k2"], d["status"], t1=d["t1"], t2=d["t2"],
+                               q2_guess=d["hint"], A=d["A"], B=d["B"], tolerance=self.varint.tolerance,
+                               params=self._dev_params(d))
+            lib.lqr_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["Q"], d["R"], d["K"], d["lqr_status"],
+                        q_per_step=Q.ndim == 3, r_per_step=R.ndim == 3)
+        except BaseException:
+            self._free(d)
+            raise
+        return d
+
+    @staticmethod
+    def _dev_params(d):
+        return None if d["params"] is None else (d["refs"], d["params"])
+
+    @staticmethod
+    def _free(d):
+        for b in d.values():
+            if hasattr(b, "free"):
+                b.free()
+
+    @staticmethod
+    def _check_feedback(d):
+        """After a synchronize: raise ConvergenceError for a failed linearization or a singular Riccati step."""
+        status, ls = d["status"].download(), d["lqr_status"].download()
+        if np.any(status != 0):
+            raise ConvergenceError("%d of %d linearizations failed" % (int(np.sum(status != 0)), status.size), status)
+        if np.any(ls != 0):
+            raise ConvergenceError("singular gamma in the Riccati sweep", ls)
+
     def calc_feedback_controller(self, X, U, Q=None, R=None, return_linearization=False):
         """DSystem.calc_feedback_controller (dsystem.py:474-494): linearize about (X, U), then the
         time-varying LQR gains (discopt.dlqr.solve_tv_lqr, dlqr.py:9-38) - both on the GPU, for one
@@ -458,49 +517,109 @@ class DSystem:
         single = X.ndim == 2
         Xb, Ub = (X[None], U[None]) if single else (X, U)
         Rn, K = Xb.shape[0], Xb.shape[1] - 1
-        Q = np.eye(self._nX) if Q is None else (np.stack([Q(k) for k in range(K + 1)]) if callable(Q) else np.asarray(Q, float))
-        R = np.eye(self._nU) if R is None else (np.stack([R(k) for k in range(K)]) if callable(R) else np.asarray(R, float))
-        sys_, dev = self.varint.sys, self.varint.sys.device
-        nX, nU, nq, nd = self._nX, self._nU, self._nQ, self._np
-        n = Rn * K
-        up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, a.shape, dt).upload(np.ascontiguousarray(a, dtype=dt))
-        Xk = Xb[:, :K].reshape(n, nX)
-        # inputs of the n = rollouts x steps independent linearizations, resident in HBM
-        dq1, dp1 = up(Xk[:, :nq]), up(Xk[:, nq:nq + nd])
-        du1 = up(Ub[:, :K, :self._nu].reshape(n, -1)) if self._nu else None
-        dk2 = up(Ub[:, :K, self._nu:].reshape(n, -1)) if self._nv else None
-        dhint = up(Xb[:, 1:K + 1, :nd].reshape(n, nd))
-        dt1, dt2 = up(np.tile(self._time[:K], Rn)), up(np.tile(self._time[1:K + 1], Rn))
-        dA, dB = lib.DeviceBuffer(dev, (n, nX, nX)), lib.DeviceBuffer(dev, (n, nX, nU))
-        dst = lib.DeviceBuffer(dev, (n,), np.int32)
-        dQ, dR = up(Q), up(R)
-        dK, dls = lib.DeviceBuffer(dev, (Rn, K, nU, nX)), lib.DeviceBuffer(dev, (Rn,), np.int32)
-        params = self._rows(n, K)
-        dpar = None if params is None else up(params[1])
-        bufs = [b for b in (dq1, dp1, du1, dk2, dhint, dt1, dt2, dA, dB, dst, dQ, dR, dK, dls, dpar) if b is not None]
+        nX, nU = self._nX, self._nU
+        d = self._feedback_on_device(Xb, Ub, Q, R)
         try:
-            # linearize -> Riccati sweep without the A / B slabs leaving the GPU
-            sys_.linearize_raw(True, n, dq1, dp1, du1, dk2, dst, t1=dt1, t2=dt2, q2_guess=dhint, A=dA, B=dB,
-                               tolerance=self.varint.tolerance, params=None if dpar is None else (params[0], dpar))
-            lib.lqr_raw(True, dev, Rn, K, nX, nU, dA, dB, dQ, dR, dK, dls, q_per_step=Q.ndim == 3, r_per_step=R.ndim == 3)
-            lib.synchronize(dev)
-            status, ls = dst.download(), dls.download()
-            if np.any(status != 0):
-                raise ConvergenceError("%d of %d linearizations failed" % (int(np.sum(status != 0)), n), status)
-            if np.any(ls != 0):
-                raise ConvergenceError("singular gamma in the Riccati sweep", ls)
-            Kfb = dK.download()
-            A = dA.download().reshape(Rn, K, nX, nX) if return_linearization else None
-            B = dB.download().reshape(Rn, K, nX, nU) if return_linearization else None
+            lib.synchronize(self.varint.sys.device)
+            self._check_feedback(d)
+            Kfb = d["K"].download()
+            A = d["A"].download().reshape(Rn, K, nX, nX) if return_linearization else None
+            B = d["B"].download().reshape(Rn, K, nX, nU) if return_linearization else None
         finally:
-            for b in bufs:
-                b.free()
+            self._free(d)
         if single:
             Kfb = Kfb[0]
             A, B = (A[0], B[0]) if return_linearization else (None, None)
         if return_linearization:
             return Kfb, A, B
         return Kfb
+
+    def calc_descent_direction(self, X, U, q, r, Q, S, R, Qproj=None, Rproj=None, newton=False, dx0=None,
+                               return_linearization=False):
+        """The descent direction of DOptimizer.calc_descent_direction (doptimizer.py:348-402) for one trajectory or
+        R rollouts sharing `time`, as one chain of device launches:
+            linearize -> LQR (Kproj, with Qproj / Rproj as calc_feedback_controller)
+            [newton: adjoint sweep z (K = Kproj, l_dx = q[:K], l_du = r, m_dx = q[K]) -> z-contracted second
+             derivatives, added to Q[:K] / S / R]
+            -> LQ (trepb_lq_batch: K, C) -> tangent sweep dX[0] = dx0, dU[k] = -K[k] dX[k] - C[k],
+               dX[k+1] = A[k] dX[k] + B[k] dU[k].
+        q [K+1,nX], r [K,nU], Q [K+1,nX,nX], S [K,nX,nU] or None, R [K,nU,nU]: the LQ model (the cost's gradients
+        and second derivatives along (X, U)), shared by the rollouts or one set per rollout (one more leading axis),
+        as for lib.solve_tv_lq.  dx0: [nX] or [R,nX], default zero.  A, B, Kproj, K and C stay on the device; only
+        (X, U), the cost terms and dx0 go in.  With newton=True the three z-contracted blocks are downloaded, added to
+        Q / S / R on the host and uploaded again.
+        Returns (Kproj, dX, dU), then z [..,K+1,nX] with newton=True, then A, B with return_linearization=True.
+        With set_parameters, rollout r runs on row r in every launch."""
+        from . import lib
+        X, U = np.asarray(X, float), np.asarray(U, float)
+        single = X.ndim == 2
+        Xb, Ub = (X[None], U[None]) if single else (X, U)
+        Rn, K = Xb.shape[0], Xb.shape[1] - 1
+        nX, nU = self._nX, self._nU
+        sys_, dev = self.varint.sys, self.varint.sys.device
+        f = lambda a: None if a is None else np.asarray(a, float)
+        q, r, Q, S, R = f(q), f(r), f(Q), f(S), f(R)
+        # one cost per rollout when any term has the rollout axis, or when the Newton terms make it so
+        per = newton or Q.ndim == 4 or q.ndim == 3 or r.ndim == 3 or R.ndim == 4 or (S is not None and S.ndim == 4)
+        if per:
+            roll = lambda a, sh: None if a is None else np.ascontiguousarray(np.broadcast_to(a, (Rn,) + sh))
+            q, r, Q, R = roll(q, (K + 1, nX)), roll(r, (K, nU)), roll(Q, (K + 1, nX, nX)), roll(R, (K, nU, nU))
+            S = roll(S, (K, nX, nU))
+        up = lambda a: lib.DeviceBuffer(dev, a.shape, np.float64).upload(np.ascontiguousarray(a, dtype=np.float64))
+        n = Rn * K
+        d = self._feedback_on_device(Xb, Ub, Qproj, Rproj)
+        try:
+            z = None
+            if newton:
+                # costate on the device (step k's second derivatives contract with z[k+1] = z1[k]), then one launch
+                # of the z-contracted second-derivative kernel over every step of every rollout
+                d["l_dx"], d["l_du"], d["m_dx"] = up(q[:, :K]), up(r), up(q[:, K])
+                d["z"], d["z1"] = lib.DeviceBuffer(dev, (Rn, K + 1, nX)), lib.DeviceBuffer(dev, (n, nX))
+                lib.adjoint_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["m_dx"], d["z"], K=d["K"], l_dx=d["l_dx"],
+                                l_du=d["l_du"], z1=d["z1"])
+                d["fdxdx"], d["fdxdu"] = lib.DeviceBuffer(dev, (n, nX, nX)), lib.DeviceBuffer(dev, (n, nX, nU))
+                d["fdudu"], d["d2_status"] = lib.DeviceBuffer(dev, (n, nU, nU)), lib.DeviceBuffer(dev, (n,), np.int32)
+                sys_.deriv2_raw(True, n, d["q1"], d["p1"], d["u1"], d["k2"], d["d2_status"], {}, z=d["z1"],
+                                fdxdx=d["fdxdx"], fdxdu=d["fdxdu"], fdudu=d["fdudu"], t1=d["t1"], t2=d["t2"],
+                                q2_guess=d["hint"], tolerance=self.varint.tolerance, params=self._dev_params(d))
+                lib.synchronize(dev)
+                self._check_feedback(d)
+                st = d["d2_status"].download()
+                if np.any(st != 0):
+                    raise ConvergenceError("%d of %d instances failed" % (int(np.sum(st != 0)), n), st)
+                # the Newton terms are summed on the host (download, add, upload)
+                Q = Q.copy()
+                Q[:, :K] += d["fdxdx"].download().reshape(Rn, K, nX, nX)
+                xu = d["fdxdu"].download().reshape(Rn, K, nX, nU)
+                S = xu if S is None else S + xu
+                R = R + d["fdudu"].download().reshape(Rn, K, nU, nU)
+                z = d["z"].download()
+            d["Qm"], d["Rm"], d["qm"], d["rm"] = up(Q), up(R), up(q), up(r)
+            d["Sm"] = None if S is None else up(S)
+            d["Klq"], d["C"] = lib.DeviceBuffer(dev, (Rn, K, nU, nX)), lib.DeviceBuffer(dev, (Rn, K, nU))
+            d["lq_status"] = lib.DeviceBuffer(dev, (Rn,), np.int32)
+            lib.lq_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["Qm"], d["Sm"], d["Rm"], d["qm"], d["rm"], d["Klq"],
+                       d["C"], d["lq_status"], cost_per_rollout=per)
+            # the tangent sweep runs with bdU = +C and x0 = -dx0: by linearity it returns exactly -dX, -dU (negation
+            # is exact in floating point), which spares a device-side negation of C
+            x0 = None
+            if dx0 is not None:
+                d["x0"] = x0 = up(-np.broadcast_to(np.asarray(dx0, float), (Rn, nX)))
+            d["dX"], d["dU"] = lib.DeviceBuffer(dev, (Rn, K + 1, nX)), lib.DeviceBuffer(dev, (Rn, K, nU))
+            lib.tangent_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["Klq"], d["dX"], d["dU"], bdU=d["C"], x0=x0)
+            lib.synchronize(dev)
+            self._check_feedback(d)
+            ls = d["lq_status"].download()
+            if np.any(ls != 0):
+                raise ConvergenceError("singular gamma in the LQ solve", ls)
+            out = [d["K"].download(), -d["dX"].download(), -d["dU"].download()]
+            if newton:
+                out.append(z)
+            if return_linearization:
+                out += [d["A"].download().reshape(Rn, K, nX, nX), d["B"].download().reshape(Rn, K, nX, nU)]
+        finally:
+            self._free(d)
+        return tuple(o[0] for o in out) if single else tuple(out)
 
     def project(self, bX, bU, Kproj, use_hint=True):
         """DSystem.project (dsystem.py:426-457) for one candidate or a batch of candidates in one

@@ -59,6 +59,18 @@ class LqArgs(C.Structure):
                 ("b0", C.c_void_p), ("status", C.c_void_p)]
 
 
+class TangentArgs(C.Structure):
+    _fields_ = [("batch", C.c_int64), ("nsteps", C.c_int32), ("nX", C.c_int32), ("nU", C.c_int32), ("_pad", C.c_int32),
+                ("A", C.c_void_p), ("B", C.c_void_p), ("K", C.c_void_p), ("bdX", C.c_void_p), ("bdU", C.c_void_p),
+                ("x0", C.c_void_p), ("dX", C.c_void_p), ("dU", C.c_void_p)]
+
+
+class AdjointArgs(C.Structure):
+    _fields_ = [("batch", C.c_int64), ("nsteps", C.c_int32), ("nX", C.c_int32), ("nU", C.c_int32), ("_pad", C.c_int32),
+                ("A", C.c_void_p), ("B", C.c_void_p), ("K", C.c_void_p), ("l_dx", C.c_void_p), ("l_du", C.c_void_p),
+                ("m_dx", C.c_void_p), ("z", C.c_void_p), ("z1", C.c_void_p)]
+
+
 RAW = ["q2_dq1", "q2_dp1", "q2_du1", "q2_dk2", "p2_dq1", "p2_dp1", "p2_du1", "p2_dk2",
        "l1_dq1", "l1_dp1", "l1_du1", "l1_dk2"]
 
@@ -124,6 +136,10 @@ _lib.trepb_lqr_batch.argtypes = [C.c_int, C.POINTER(LqrArgs)]
 _lib.trepb_lqr_batch_dev.argtypes = [C.c_int, C.POINTER(LqrArgs), C.c_void_p]
 _lib.trepb_lq_batch.argtypes = [C.c_int, C.POINTER(LqArgs)]
 _lib.trepb_lq_batch_dev.argtypes = [C.c_int, C.POINTER(LqArgs), C.c_void_p]
+_lib.trepb_tangent_batch.argtypes = [C.c_int, C.POINTER(TangentArgs)]
+_lib.trepb_tangent_batch_dev.argtypes = [C.c_int, C.POINTER(TangentArgs), C.c_void_p]
+_lib.trepb_adjoint_batch.argtypes = [C.c_int, C.POINTER(AdjointArgs)]
+_lib.trepb_adjoint_batch_dev.argtypes = [C.c_int, C.POINTER(AdjointArgs), C.c_void_p]
 _lib.trepb_lqr_last_kernel_ms.argtypes = [C.c_int, C.POINTER(C.c_float)]
 _lib.trepb_linearize_batch.argtypes = [C.c_void_p, C.POINTER(LinArgs)]
 _lib.trepb_linearize_batch_dev.argtypes = [C.c_void_p, C.POINTER(LinArgs), C.c_void_p]
@@ -189,7 +205,8 @@ EXPORTS = [
     "trepb_linearize_varied_batch_dev", "trepb_project_varied_batch", "trepb_project_varied_batch_dev",
     "trepb_calc_p2_varied_batch", "trepb_calc_p2_varied_batch_dev", "trepb_calc_f_varied_batch",
     "trepb_calc_f_varied_batch_dev", "trepb_discrete_fm2_varied_batch", "trepb_discrete_fm2_varied_batch_dev",
-    "trepb_deriv2_varied_batch", "trepb_deriv2_varied_batch_dev",
+    "trepb_deriv2_varied_batch", "trepb_deriv2_varied_batch_dev", "trepb_tangent_batch", "trepb_tangent_batch_dev",
+    "trepb_adjoint_batch", "trepb_adjoint_batch_dev",
 ]
 
 
@@ -326,6 +343,65 @@ def solve_tv_lq(A, B, q, r, Q, S, R, device=0):
     if np.any(status != 0):
         raise TrepbError(0, "singular gamma in the Riccati sweep of rollout(s) %s" % np.flatnonzero(status != 0)[:8])
     return (Kfb[0], Cff[0], P0[0], b0[0]) if single else (Kfb, Cff, P0, b0)
+
+
+def tangent_raw(on_device, device, batch, nsteps, nX, nU, A, B, K, dX, dU, bdX=None, bdU=None, x0=None, stream=None):
+    a = TangentArgs(batch=batch, nsteps=nsteps, nX=nX, nU=nU, A=_ptr(A), B=_ptr(B), K=_ptr(K), bdX=_ptr(bdX),
+                    bdU=_ptr(bdU), x0=_ptr(x0), dX=_ptr(dX), dU=_ptr(dU))
+    if on_device:
+        _check(_lib.trepb_tangent_batch_dev(device, C.byref(a), stream))
+    else:
+        _check(_lib.trepb_tangent_batch(device, C.byref(a)))
+
+
+def adjoint_raw(on_device, device, batch, nsteps, nX, nU, A, B, m_dx, z, K=None, l_dx=None, l_du=None, z1=None,
+                stream=None):
+    a = AdjointArgs(batch=batch, nsteps=nsteps, nX=nX, nU=nU, A=_ptr(A), B=_ptr(B), K=_ptr(K), l_dx=_ptr(l_dx),
+                    l_du=_ptr(l_du), m_dx=_ptr(m_dx), z=_ptr(z), z1=_ptr(z1))
+    if on_device:
+        _check(_lib.trepb_adjoint_batch_dev(device, C.byref(a), stream))
+    else:
+        _check(_lib.trepb_adjoint_batch(device, C.byref(a)))
+
+
+def _sweep_in(A, B, single, *more):
+    """float64 contiguous copies, a leading rollout axis added to a single trajectory's arrays (None stays None)."""
+    f = lambda x: None if x is None else np.ascontiguousarray(np.asarray(x, float))
+    out = [f(x) for x in (A, B) + more]
+    return [None if x is None else (x[None] if single else x) for x in out]
+
+
+def tangent_sweep(A, B, K, bdX, bdU, x0=None, device=0):
+    """Batched DSystem.dproject (trep/discopt/dsystem.py:460-471) on the GPU:
+    dX[0] = x0 (default bdX[0]); dU[k] = bdU[k] - K[k] (dX[k] - bdX[k]); dX[k+1] = A[k] dX[k] + B[k] dU[k].
+    One trajectory: A [K,nX,nX], B [K,nX,nU], K [K,nU,nX], bdX [K+1,nX], bdU [K,nU], x0 [nX]; a batch: one more
+    leading axis on every array.  bdX / bdU / x0 may be None (zero; x0 then defaults to bdX[0]).
+    Returns (dX, dU)."""
+    A = np.asarray(A)
+    single = A.ndim == 3
+    A, B, K, bdX, bdU, x0 = _sweep_in(A, B, single, K, bdX, bdU, x0)
+    Rn, n, nX = A.shape[0], A.shape[1], A.shape[2]
+    nU = B.shape[3]
+    dX, dU = np.zeros((Rn, n + 1, nX)), np.zeros((Rn, n, nU))
+    tangent_raw(False, device, Rn, n, nX, nU, A, B if nU else None, K if nU else None, dX, dU if nU else None,
+                bdX=bdX, bdU=bdU if nU else None, x0=x0)
+    return (dX[0], dU[0]) if single else (dX, dU)
+
+
+def adjoint_sweep(A, B, m_dx, l_dx=None, l_du=None, K=None, device=0):
+    """The costate recursion of DOptimizer.calc_newton_model (trep/discopt/doptimizer.py:319-345) on the GPU:
+    z[K] = m_dx; z[k] = l_dx[k] - K[k]^T l_du[k] + (A[k] - B[k] K[k])^T z[k+1] (K None: z[k] = l_dx[k] + A[k]^T z[k+1]).
+    One trajectory: A [K,nX,nX], B [K,nX,nU], m_dx [nX], l_dx [K,nX], l_du [K,nU], K [K,nU,nX]; a batch: one more
+    leading axis on every array.  l_dx / l_du may be None (zero).  Returns z [..,K+1,nX]."""
+    A = np.asarray(A)
+    single = A.ndim == 3
+    A, B, m_dx, l_dx, l_du, K = _sweep_in(A, B, single, m_dx, l_dx, l_du, K)
+    Rn, n, nX = A.shape[0], A.shape[1], A.shape[2]
+    nU = B.shape[3]
+    z = np.zeros((Rn, n + 1, nX))
+    adjoint_raw(False, device, Rn, n, nX, nU, A, B if nU else None, m_dx, z, K=K if nU else None, l_dx=l_dx,
+                l_du=l_du if nU else None)
+    return z[0] if single else z
 
 
 def specialized_names():
