@@ -27,6 +27,9 @@
  *                            descent direction, on the slabs the two calls above leave in HBM.
  *   trepb_adjoint_batch*     the costate recursion of DOptimizer.calc_newton_model
  *                            (trep/discopt/doptimizer.py:319-345).
+ *   trepb_track_batch*       DCost (trep/discopt/dcost.py) summed as DOptimizer.calc_cost / calc_dcost, and the
+ *                            LQ model of DOptimizer's steepest / quasi / newton directions.
+ *   trepb_candidates_batch*  the step-size candidates of DOptimizer.armijo_search.
  *   trepb_linearize_batch*  DSystem.set + fdx + fdu for every k of
  *                            DSystem.linearize_trajectory (trep/discopt/dsystem.py:229-250,
  *                            284-317, 406-423) == solve_DEL + MidpointVI_calc_deriv1
@@ -371,6 +374,75 @@ typedef struct trepb_adjoint_args {
 
 int trepb_adjoint_batch(int device, const trepb_adjoint_args* args);                   /* host pointers   */
 int trepb_adjoint_batch_dev(int device, const trepb_adjoint_args* args, void* stream); /* device pointers */
+
+/* Quadratic tracking cost and its LQ model, batched over trajectories: trep.discopt.DCost (dcost.py) as
+ * DOptimizer.calc_cost / calc_dcost sum it (doptimizer.py).  With dx_k = X[k] - Xd[k], du_k = U[k] - Ud[k]:
+ *     cost  = sum_{k<K} (dx_k^T Q dx_k + du_k^T R du_k) / 2 + dx_K^T Q dx_K / 2
+ *     q[k]  = dx_k^T Q (k = 0..K),   r[k] = du_k^T R
+ *     dcost = sum_{k<K} (q[k] . dX[k] + r[k] . dU[k]) + q[K] . dX[K]
+ *     Qm[k] = Q (+ fdxdx[k] for k < K),   Sm[k] = 0 (+ fdxdu[k]),   Rm[k] = R (+ fdudu[k])
+ * Trajectory b tracks reference ref_index[b] (NULL: every trajectory tracks reference 0).  Every output is
+ * optional; q, r, Qm, Sm and Rm are in the per-rollout layout trepb_lq_batch_dev reads (cost_per_rollout = 1),
+ * l_dx / m_dx in the layout trepb_adjoint_batch_dev reads, and the three Newton blocks in the layout
+ * trepb_deriv2_batch_dev writes over the batch x K step instances.  Every sum runs in ascending index order with
+ * separately rounded products and additions, so a trajectory gives the same bits alone and inside any batch, and
+ * each Newton sum is one IEEE addition.  No system handle is needed.  nU = 0 is allowed.                     */
+typedef struct trepb_track_args {
+    int64_t batch;            /* trajectories                                          */
+    int32_t nsteps;           /* K                                                     */
+    int32_t nX, nU;
+    int32_t nref;             /* references in Xd / Ud (>= 1)                          */
+    const double* X;          /* [batch][K+1][nX]                                      */
+    const double* U;          /* [batch][K][nU]                                        */
+    const double* Xd;         /* [nref][K+1][nX]                                       */
+    const double* Ud;         /* [nref][K][nU]                                         */
+    const double* Q;          /* [nX][nX]                                              */
+    const double* R;          /* [nU][nU]                                              */
+    const int32_t* ref_index; /* [batch], NULL = reference 0 for all                   */
+    const double* dX;         /* [batch][K+1][nX], needed with dcost                   */
+    const double* dU;         /* [batch][K][nU], needed with dcost                     */
+    const double* fdxdx;      /* [batch*K][nX][nX] Newton blocks: all three or none    */
+    const double* fdxdu;      /* [batch*K][nX][nU]                                     */
+    const double* fdudu;      /* [batch*K][nU][nU]                                     */
+    double* cost;             /* [batch] out                                           */
+    double* dcost;            /* [batch] out                                           */
+    double* q;                /* [batch][K+1][nX] out                                  */
+    double* r;                /* [batch][K][nU] out                                    */
+    double* l_dx;             /* [batch][K][nX] out (q[:K])                            */
+    double* m_dx;             /* [batch][nX] out (q[K])                                */
+    double* Qm;               /* [batch][K+1][nX][nX] out                              */
+    double* Sm;               /* [batch][K][nX][nU] out                                */
+    double* Rm;               /* [batch][K][nU][nU] out                                */
+} trepb_track_args;
+
+int trepb_track_batch(int device, const trepb_track_args* args);                   /* host pointers   */
+int trepb_track_batch_dev(int device, const trepb_track_args* args, void* stream); /* device pointers */
+
+/* Armijo line-search candidates of DOptimizer.armijo_search (doptimizer.py), ncand step sizes for each of `groups`
+ * rollouts at once: for group g (rollout rows[g], NULL = g) and step size lam[m],
+ *     bX[g][m] = X + lam[m] dX,   bU[g][m] = U + lam[m] dU   (product and sum rounded separately)
+ *     Kc[g][m] = Kproj                                        (per-candidate gains for trepb_project_batch_dev
+ *                                                              with k_per_instance = 1)                         */
+typedef struct trepb_candidates_args {
+    int64_t groups;           /* rollouts searched                                     */
+    int32_t ncand;            /* M step sizes per rollout (>= 1)                       */
+    int32_t nsteps;           /* K                                                     */
+    int32_t nX, nU;
+    int64_t nrollouts;        /* rollouts in X .. Kproj (host form with rows only)     */
+    const int32_t* rows;      /* [groups], NULL = identity                             */
+    const double* lam;        /* [ncand]                                               */
+    const double* X;          /* [R][K+1][nX]                                          */
+    const double* U;          /* [R][K][nU]                                            */
+    const double* dX;         /* [R][K+1][nX]                                          */
+    const double* dU;         /* [R][K][nU]                                            */
+    const double* Kproj;      /* [R][K][nU][nX]                                        */
+    double* bX;               /* [groups][ncand][K+1][nX] out                          */
+    double* bU;               /* [groups][ncand][K][nU] out                            */
+    double* Kc;               /* [groups][ncand][K][nU][nX] out                        */
+} trepb_candidates_args;
+
+int trepb_candidates_batch(int device, const trepb_candidates_args* args);                   /* host pointers   */
+int trepb_candidates_batch_dev(int device, const trepb_candidates_args* args, void* stream); /* device pointers */
 
 /* p2 from two consecutive configurations (initialize_from_configs). q0,q1: [B][nq] -> p: [B][nd] */
 int trepb_calc_p2_batch(trepb_system* sys, int64_t batch, double dt,

@@ -23,6 +23,7 @@
 #include "trepb_coop_math.cuh"
 #include "trepb_err.h"
 #include "trepb_sweep.cuh"
+#include "trepb_track.cuh"
 
 namespace trepb {
 namespace {
@@ -713,5 +714,181 @@ extern "C" int trepb_adjoint_batch(int device, const trepb_adjoint_args* a) {
         trepb_adjoint_args x = *a;
         x.A = d[0]; x.B = d[1]; x.K = d[2]; x.l_dx = d[3]; x.l_du = d[4]; x.m_dx = d[5]; x.z = o[0]; x.z1 = o[1];
         return trepb_adjoint_batch_dev(device, &x, nullptr);
+    });
+}
+
+// ---- tracking cost, LQ model and line-search candidates (trepb_track.cuh) ----------------------------------------
+namespace {
+// the checks every track / candidates entry point makes before any CUDA call; -1 = go on
+int track_check(const trepb_track_args* a) {
+    if (!a) return lqr_fail(TREPB_ERR_INVALID, "null argument");
+    if (a->batch < 0 || a->nsteps < 1 || a->nX < 1 || a->nU < 0 || a->nref < 1) return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    const long long nX = a->nX, nU = a->nU, K = a->nsteps;
+    if ((K + 1) * nX * nX + K * nX * nU + K * nU * nU > 0x7fffffffLL || (K + 1) * (nX + nU) > 0x7fffffffLL)
+        return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    const bool grad = a->cost || a->dcost || a->q || a->r || a->l_dx || a->m_dx;
+    const bool model = a->Qm || a->Sm || a->Rm;
+    if (grad && (!a->X || !a->Xd || !a->Q || (nU > 0 && (!a->U || !a->Ud || !a->R))))
+        return lqr_fail(TREPB_ERR_INVALID, "X, Xd and Q are required for the cost outputs, and U, Ud and R when nU > 0");
+    if (a->dcost && (!a->dX || (nU > 0 && !a->dU))) return lqr_fail(TREPB_ERR_INVALID, "dcost needs dX and dU");
+    const int newton = (a->fdxdx != nullptr) + (nU > 0 && a->fdxdu != nullptr) + (nU > 0 && a->fdudu != nullptr);
+    if (newton != 0 && newton != (nU > 0 ? 3 : 1))
+        return lqr_fail(TREPB_ERR_INVALID, "fdxdx, fdxdu and fdudu go together");
+    if ((model || newton) && (!a->Qm || !a->Q || (nU > 0 && (!a->Rm || !a->R))))
+        return lqr_fail(TREPB_ERR_INVALID, "the model needs Qm and Q, and Rm and R when nU > 0");
+    if (a->batch == 0) return TREPB_OK;
+    return -1;
+}
+int candidates_check(const trepb_candidates_args* a) {
+    if (!a) return lqr_fail(TREPB_ERR_INVALID, "null argument");
+    if (a->groups < 0 || a->ncand < 1 || a->nsteps < 1 || a->nX < 1 || a->nU < 0 || a->nrollouts < 0)
+        return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    const long long nX = a->nX, nU = a->nU, K = a->nsteps;
+    if ((K + 1) * nX + K * nU + K * nU * nX > 0x7fffffffLL) return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    if (!a->lam || !a->X || !a->dX || !a->bX || (nU > 0 && (!a->U || !a->dU || !a->Kproj || !a->bU || !a->Kc)))
+        return lqr_fail(TREPB_ERR_INVALID, "lam, X, dX and bX are required, and U, dU, Kproj, bU and Kc when nU > 0");
+    if (a->groups == 0) return TREPB_OK;
+    return -1;
+}
+
+// host -> device staging of inputs and outputs given in bytes around `run(device pointers)` (null / empty arrays
+// stay null); synchronous, like the sweeps' host-pointer calls
+template <int NI, int NO, class Run>
+int stage_bytes(int device, const void* const (&src)[NI], const size_t (&in_b)[NI], void* const (&dst)[NO],
+                const size_t (&out_b)[NO], Run run) {
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    void* din[NI] = {nullptr};
+    void* dout[NO] = {nullptr};
+    int rc = TREPB_OK;
+#define SB(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess && rc == TREPB_OK) rc = lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e_)); } while (0)
+    for (int i = 0; i < NI; ++i)
+        if (src[i] && in_b[i]) {
+            SB(cudaMalloc(&din[i], in_b[i]));
+            if (rc == TREPB_OK) SB(cudaMemcpyAsync(din[i], src[i], in_b[i], cudaMemcpyHostToDevice, nullptr));
+        }
+    for (int i = 0; i < NO; ++i) if (dst[i] && out_b[i]) SB(cudaMalloc(&dout[i], out_b[i]));
+    if (rc == TREPB_OK) rc = run(din, dout);
+    if (rc == TREPB_OK)
+        for (int i = 0; i < NO; ++i) if (dout[i]) SB(cudaMemcpyAsync(dst[i], dout[i], out_b[i], cudaMemcpyDeviceToHost, nullptr));
+    SB(cudaStreamSynchronize(nullptr));
+#undef SB
+    for (int i = 0; i < NI; ++i) cudaFree(din[i]);
+    for (int i = 0; i < NO; ++i) cudaFree(dout[i]);
+    return rc;
+}
+}  // namespace
+
+extern "C" int trepb_track_batch_dev(int device, const trepb_track_args* a, void* stream) {
+    TREPB_NVTX("trepb_track_batch_dev");
+    const int c = track_check(a);
+    if (c >= 0) return c;
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    TrackParams p{};
+    const int nU = a->nU;
+    p.batch = a->batch; p.K = a->nsteps; p.nX = a->nX; p.nU = nU;
+    p.X = a->X; p.U = nU ? a->U : nullptr; p.Xd = a->Xd; p.Ud = nU ? a->Ud : nullptr; p.Q = a->Q; p.R = nU ? a->R : nullptr;
+    p.ref = a->ref_index; p.dX = a->dX; p.dU = nU ? a->dU : nullptr;
+    p.fxx = a->fdxdx; p.fxu = nU ? a->fdxdu : nullptr; p.fuu = nU ? a->fdudu : nullptr;
+    p.cost = a->cost; p.dcost = a->dcost; p.q = a->q; p.r = nU ? a->r : nullptr; p.l_dx = a->l_dx; p.m_dx = a->m_dx;
+    p.Qm = a->Qm; p.Sm = nU ? a->Sm : nullptr; p.Rm = nU ? a->Rm : nullptr;
+    const bool grad = p.cost || p.dcost || p.q || p.r || p.l_dx || p.m_dx;
+    const int block = 256;
+    // cost role: one CTA per trajectory (strided beyond 2^20); a tile of about 2048 staged doubles per CTA
+    const int cols = a->nX + nU;
+    int tile = 2048 / cols;
+    tile = tile < 1 ? 1 : tile > 256 ? 256 : tile;
+    p.tile = tile;
+    p.cost_blocks = grad ? (int)(p.batch < (1LL << 20) ? p.batch : (1LL << 20)) : 0;
+    const size_t smem = grad ? (size_t)track_smem_doubles(a->nX, nU, tile) * 8 : 0;
+    // model role: CTAs per trajectory such that each lane streams about four elements of the model
+    long long model_blocks = 0;
+    if (p.Qm) {
+        const long long per = (p.K + 1LL) * a->nX * a->nX + (p.Sm ? (long long)p.K * a->nX * nU : 0) +
+                              (p.Rm ? (long long)p.K * nU * nU : 0);
+        p.model_bpt = (int)((per + 4LL * block - 1) / (4LL * block));
+        model_blocks = p.batch * p.model_bpt;
+        if (model_blocks > (1LL << 22)) model_blocks = 1LL << 22;
+    }
+    if (smem > 48 * 1024) {
+        e = cudaFuncSetAttribute((const void*)track_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    }
+    const long long grid = p.cost_blocks + model_blocks;
+    if (grid == 0) return TREPB_OK;
+    track_kernel<<<(unsigned)grid, block, smem, (cudaStream_t)stream>>>(p);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    return TREPB_OK;
+}
+
+extern "C" int trepb_track_batch(int device, const trepb_track_args* a) {
+    TREPB_NVTX("trepb_track_batch");
+    const int c = track_check(a);
+    if (c >= 0) return c;
+    const size_t Rn = (size_t)a->batch, K = (size_t)a->nsteps, nX = (size_t)a->nX, nU = (size_t)a->nU, nr = (size_t)a->nref;
+    const size_t d = 8;
+    const void* const src[12] = {a->X, a->U, a->Xd, a->Ud, a->Q, a->R, a->ref_index, a->dX, a->dU,
+                                 a->fdxdx, a->fdxdu, a->fdudu};
+    const size_t in_b[12] = {Rn * (K + 1) * nX * d, Rn * K * nU * d, nr * (K + 1) * nX * d, nr * K * nU * d, nX * nX * d,
+                             nU * nU * d, Rn * 4, Rn * (K + 1) * nX * d, Rn * K * nU * d, Rn * K * nX * nX * d,
+                             Rn * K * nX * nU * d, Rn * K * nU * nU * d};
+    void* const dst[9] = {a->cost, a->dcost, a->q, a->r, a->l_dx, a->m_dx, a->Qm, a->Sm, a->Rm};
+    const size_t out_b[9] = {Rn * d, Rn * d, Rn * (K + 1) * nX * d, Rn * K * nU * d, Rn * K * nX * d, Rn * nX * d,
+                             Rn * (K + 1) * nX * nX * d, Rn * K * nX * nU * d, Rn * K * nU * nU * d};
+    return stage_bytes(device, src, in_b, dst, out_b, [&](void* const* i, void* const* o) {
+        trepb_track_args x = *a;
+        x.X = (const double*)i[0]; x.U = (const double*)i[1]; x.Xd = (const double*)i[2]; x.Ud = (const double*)i[3];
+        x.Q = (const double*)i[4]; x.R = (const double*)i[5]; x.ref_index = (const int32_t*)i[6];
+        x.dX = (const double*)i[7]; x.dU = (const double*)i[8]; x.fdxdx = (const double*)i[9];
+        x.fdxdu = (const double*)i[10]; x.fdudu = (const double*)i[11];
+        x.cost = (double*)o[0]; x.dcost = (double*)o[1]; x.q = (double*)o[2]; x.r = (double*)o[3];
+        x.l_dx = (double*)o[4]; x.m_dx = (double*)o[5]; x.Qm = (double*)o[6]; x.Sm = (double*)o[7]; x.Rm = (double*)o[8];
+        return trepb_track_batch_dev(device, &x, nullptr);
+    });
+}
+
+extern "C" int trepb_candidates_batch_dev(int device, const trepb_candidates_args* a, void* stream) {
+    TREPB_NVTX("trepb_candidates_batch_dev");
+    const int c = candidates_check(a);
+    if (c >= 0) return c;
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    CandParams p{};
+    const int nU = a->nU;
+    p.G = a->groups; p.M = a->ncand; p.K = a->nsteps; p.nX = a->nX; p.nU = nU;
+    p.rows = a->rows; p.lam = a->lam; p.X = a->X; p.U = nU ? a->U : nullptr; p.dX = a->dX; p.dU = nU ? a->dU : nullptr;
+    p.Kp = nU ? a->Kproj : nullptr; p.bX = a->bX; p.bU = nU ? a->bU : nullptr; p.Kc = nU ? a->Kc : nullptr;
+    const long long per = (p.K + 1LL) * p.nX + (long long)p.K * nU * (1LL + p.nX);
+    const int block = 256;
+    long long gx = (per + 4LL * block - 1) / (4LL * block);   // about four elements per lane
+    if (gx > 4096) gx = 4096;
+    long long gy = p.G * p.M;
+    if (gy > 65535) gy = 65535;                               // the kernel strides over the rest
+    candidates_kernel<<<dim3((unsigned)gx, (unsigned)gy), block, 0, (cudaStream_t)stream>>>(p);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    return TREPB_OK;
+}
+
+extern "C" int trepb_candidates_batch(int device, const trepb_candidates_args* a) {
+    TREPB_NVTX("trepb_candidates_batch");
+    const int c = candidates_check(a);
+    if (c >= 0) return c;
+    const size_t G = (size_t)a->groups, M = (size_t)a->ncand, K = (size_t)a->nsteps, nX = (size_t)a->nX, nU = (size_t)a->nU;
+    // the rollouts the groups read: rows[] indexes nrollouts of them (without rows, one per group)
+    const size_t Rn = a->rows ? (size_t)a->nrollouts : G, d = 8;
+    const void* const src[7] = {a->rows, a->lam, a->X, a->U, a->dX, a->dU, a->Kproj};
+    const size_t in_b[7] = {G * 4, M * d, Rn * (K + 1) * nX * d, Rn * K * nU * d, Rn * (K + 1) * nX * d, Rn * K * nU * d,
+                            Rn * K * nU * nX * d};
+    void* const dst[3] = {a->bX, a->bU, a->Kc};
+    const size_t out_b[3] = {G * M * (K + 1) * nX * d, G * M * K * nU * d, G * M * K * nU * nX * d};
+    return stage_bytes(device, src, in_b, dst, out_b, [&](void* const* i, void* const* o) {
+        trepb_candidates_args x = *a;
+        x.rows = (const int32_t*)i[0]; x.lam = (const double*)i[1]; x.X = (const double*)i[2]; x.U = (const double*)i[3];
+        x.dX = (const double*)i[4]; x.dU = (const double*)i[5]; x.Kproj = (const double*)i[6];
+        x.bX = (double*)o[0]; x.bU = (double*)o[1]; x.Kc = (double*)o[2];
+        return trepb_candidates_batch_dev(device, &x, nullptr);
     });
 }

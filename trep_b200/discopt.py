@@ -547,59 +547,58 @@ class DSystem:
         and second derivatives along (X, U)), shared by the rollouts or one set per rollout (one more leading axis),
         as for lib.solve_tv_lq.  dx0: [nX] or [R,nX], default zero.  A, B, Kproj, K and C stay on the device; only
         (X, U), the cost terms and dx0 go in.  With newton=True the three z-contracted blocks are downloaded, added to
-        Q / S / R on the host and uploaded again.
+        Q / S / R on the host and uploaded again (discopt.DOptimizer builds its model on the device instead).
         Returns (Kproj, dX, dU), then z [..,K+1,nX] with newton=True, then A, B with return_linearization=True.
         With set_parameters, rollout r runs on row r in every launch."""
-        from . import lib
         X, U = np.asarray(X, float), np.asarray(U, float)
         single = X.ndim == 2
         Xb, Ub = (X[None], U[None]) if single else (X, U)
         Rn, K = Xb.shape[0], Xb.shape[1] - 1
         nX, nU = self._nX, self._nU
+        d = self._descent_on_device(Xb, Ub, Qproj, Rproj, newton, dx0, _HostModel(self, Rn, K, newton, q, r, Q, S, R))
+        try:
+            out = [d["K"].download(), -d["dX"].download(), -d["dU"].download()]
+            if newton:
+                out.append(d["z"].download())
+            if return_linearization:
+                out += [d["A"].download().reshape(Rn, K, nX, nX), d["B"].download().reshape(Rn, K, nX, nU)]
+        finally:
+            self._free(d)
+        return tuple(o[0] for o in out) if single else tuple(out)
+
+    def _descent_on_device(self, Xb, Ub, Qproj, Rproj, newton, dx0, model):
+        """The device chain of calc_descent_direction for Rn rollouts (Xb [Rn,K+1,nX], Ub [Rn,K,nU]):
+            linearize -> LQR (Kproj) -> model.gradients [-> adjoint -> deriv2] -> model.hessians -> LQ -> tangent sweep.
+        `model` supplies the LQ model: gradients(d) puts q / r in d["qm"] / d["rm"] (and, for the adjoint, l_dx / m_dx in
+        d["l_dx"] / d["m_dx"]); hessians(d, newton) puts Q / S / R in d["Qm"] / d["Sm"] / d["Rm"], adding the z-contracted
+        blocks d["fdxdx"], d["fdxdu"], d["fdudu"] with newton=True, and returns cost_per_rollout.  Synchronizes and
+        raises ConvergenceError on a failed launch; otherwise returns the dict of device buffers (the caller frees it
+        with _free), whose d["dX"] / d["dU"] hold -dX / -dU (see below) and d["K"] the gains Kproj."""
+        from . import lib
+        Rn, K = Xb.shape[0], Xb.shape[1] - 1
+        nX, nU = self._nX, self._nU
         sys_, dev = self.varint.sys, self.varint.sys.device
-        f = lambda a: None if a is None else np.asarray(a, float)
-        q, r, Q, S, R = f(q), f(r), f(Q), f(S), f(R)
-        # one cost per rollout when any term has the rollout axis, or when the Newton terms make it so
-        per = newton or Q.ndim == 4 or q.ndim == 3 or r.ndim == 3 or R.ndim == 4 or (S is not None and S.ndim == 4)
-        if per:
-            roll = lambda a, sh: None if a is None else np.ascontiguousarray(np.broadcast_to(a, (Rn,) + sh))
-            q, r, Q, R = roll(q, (K + 1, nX)), roll(r, (K, nU)), roll(Q, (K + 1, nX, nX)), roll(R, (K, nU, nU))
-            S = roll(S, (K, nX, nU))
         up = lambda a: lib.DeviceBuffer(dev, a.shape, np.float64).upload(np.ascontiguousarray(a, dtype=np.float64))
         n = Rn * K
         d = self._feedback_on_device(Xb, Ub, Qproj, Rproj)
         try:
-            z = None
+            model.gradients(d)
             if newton:
                 # costate on the device (step k's second derivatives contract with z[k+1] = z1[k]), then one launch
                 # of the z-contracted second-derivative kernel over every step of every rollout
-                d["l_dx"], d["l_du"], d["m_dx"] = up(q[:, :K]), up(r), up(q[:, K])
                 d["z"], d["z1"] = lib.DeviceBuffer(dev, (Rn, K + 1, nX)), lib.DeviceBuffer(dev, (n, nX))
                 lib.adjoint_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["m_dx"], d["z"], K=d["K"], l_dx=d["l_dx"],
-                                l_du=d["l_du"], z1=d["z1"])
+                                l_du=d["rm"], z1=d["z1"])
                 d["fdxdx"], d["fdxdu"] = lib.DeviceBuffer(dev, (n, nX, nX)), lib.DeviceBuffer(dev, (n, nX, nU))
                 d["fdudu"], d["d2_status"] = lib.DeviceBuffer(dev, (n, nU, nU)), lib.DeviceBuffer(dev, (n,), np.int32)
                 sys_.deriv2_raw(True, n, d["q1"], d["p1"], d["u1"], d["k2"], d["d2_status"], {}, z=d["z1"],
                                 fdxdx=d["fdxdx"], fdxdu=d["fdxdu"], fdudu=d["fdudu"], t1=d["t1"], t2=d["t2"],
                                 q2_guess=d["hint"], tolerance=self.varint.tolerance, params=self._dev_params(d))
-                lib.synchronize(dev)
-                self._check_feedback(d)
-                st = d["d2_status"].download()
-                if np.any(st != 0):
-                    raise ConvergenceError("%d of %d instances failed" % (int(np.sum(st != 0)), n), st)
-                # the Newton terms are summed on the host (download, add, upload)
-                Q = Q.copy()
-                Q[:, :K] += d["fdxdx"].download().reshape(Rn, K, nX, nX)
-                xu = d["fdxdu"].download().reshape(Rn, K, nX, nU)
-                S = xu if S is None else S + xu
-                R = R + d["fdudu"].download().reshape(Rn, K, nU, nU)
-                z = d["z"].download()
-            d["Qm"], d["Rm"], d["qm"], d["rm"] = up(Q), up(R), up(q), up(r)
-            d["Sm"] = None if S is None else up(S)
+            per = model.hessians(d, newton)
             d["Klq"], d["C"] = lib.DeviceBuffer(dev, (Rn, K, nU, nX)), lib.DeviceBuffer(dev, (Rn, K, nU))
             d["lq_status"] = lib.DeviceBuffer(dev, (Rn,), np.int32)
-            lib.lq_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["Qm"], d["Sm"], d["Rm"], d["qm"], d["rm"], d["Klq"],
-                       d["C"], d["lq_status"], cost_per_rollout=per)
+            lib.lq_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["Qm"], d.get("Sm"), d["Rm"], d["qm"], d["rm"],
+                       d["Klq"], d["C"], d["lq_status"], cost_per_rollout=per)
             # the tangent sweep runs with bdU = +C and x0 = -dx0: by linearity it returns exactly -dX, -dU (negation
             # is exact in floating point), which spares a device-side negation of C
             x0 = None
@@ -609,17 +608,21 @@ class DSystem:
             lib.tangent_raw(True, dev, Rn, K, nX, nU, d["A"], d["B"], d["Klq"], d["dX"], d["dU"], bdU=d["C"], x0=x0)
             lib.synchronize(dev)
             self._check_feedback(d)
+            if newton:
+                self._check_d2(d, n)
             ls = d["lq_status"].download()
             if np.any(ls != 0):
                 raise ConvergenceError("singular gamma in the LQ solve", ls)
-            out = [d["K"].download(), -d["dX"].download(), -d["dU"].download()]
-            if newton:
-                out.append(z)
-            if return_linearization:
-                out += [d["A"].download().reshape(Rn, K, nX, nX), d["B"].download().reshape(Rn, K, nX, nU)]
-        finally:
+        except BaseException:
             self._free(d)
-        return tuple(o[0] for o in out) if single else tuple(out)
+            raise
+        return d
+
+    @staticmethod
+    def _check_d2(d, n):
+        st = d["d2_status"].download()
+        if np.any(st != 0):
+            raise ConvergenceError("%d of %d instances failed" % (int(np.sum(st != 0)), n), st)
 
     def project(self, bX, bU, Kproj, use_hint=True):
         """DSystem.project (dsystem.py:426-457) for one candidate or a batch of candidates in one
@@ -681,3 +684,428 @@ class DSystem:
             X[:, 0, self._nQ + self._np:] = X0[:, self._nQ + self._np:]
             X[:, 1:, self._nQ + self._np:] = (Q[:, 1:, self._np:] - Q[:, :-1, self._np:]) / dts[None, :, None]
         return X
+
+
+class _HostModel:
+    """The LQ model of DSystem.calc_descent_direction given as host arrays: uploaded as they are, and with newton=True
+    the z-contracted blocks are downloaded, summed into Q / S / R on the host and uploaded again."""
+
+    def __init__(self, dsys, Rn, K, newton, q, r, Q, S, R):
+        f = lambda a: None if a is None else np.asarray(a, float)
+        q, r, Q, S, R = f(q), f(r), f(Q), f(S), f(R)
+        nX, nU = dsys.nX, dsys.nU
+        # one cost per rollout when any term has the rollout axis, or when the Newton terms make it so
+        self.per = newton or Q.ndim == 4 or q.ndim == 3 or r.ndim == 3 or R.ndim == 4 or (S is not None and S.ndim == 4)
+        if self.per:
+            roll = lambda a, sh: None if a is None else np.ascontiguousarray(np.broadcast_to(a, (Rn,) + sh))
+            q, r, Q, R = roll(q, (K + 1, nX)), roll(r, (K, nU)), roll(Q, (K + 1, nX, nX)), roll(R, (K, nU, nU))
+            S = roll(S, (K, nX, nU))
+        self.dsys, self.Rn, self.K, self.q, self.r, self.Q, self.S, self.R = dsys, Rn, K, q, r, Q, S, R
+
+    def _up(self, a):
+        from . import lib
+        return lib.DeviceBuffer(self.dsys.varint.sys.device, a.shape, np.float64).upload(np.ascontiguousarray(a))
+
+    def gradients(self, d):
+        d["qm"], d["rm"] = self._up(self.q), self._up(self.r)
+        if self.per:
+            d["l_dx"], d["m_dx"] = self._up(self.q[:, :self.K]), self._up(self.q[:, self.K])
+
+    def hessians(self, d, newton):
+        from . import lib
+        Q, S, R, Rn, K, ds = self.Q, self.S, self.R, self.Rn, self.K, self.dsys
+        if newton:
+            lib.synchronize(ds.varint.sys.device)
+            ds._check_feedback(d)
+            ds._check_d2(d, Rn * K)
+            # the Newton terms are summed on the host (download, add, upload)
+            nX, nU = ds.nX, ds.nU
+            Q = Q.copy()
+            Q[:, :K] += d["fdxdx"].download().reshape(Rn, K, nX, nX)
+            xu = d["fdxdu"].download().reshape(Rn, K, nX, nU)
+            S = xu if S is None else S + xu
+            R = R + d["fdudu"].download().reshape(Rn, K, nU, nU)
+        d["Qm"], d["Rm"] = self._up(Q), self._up(R)
+        d["Sm"] = None if S is None else self._up(S)
+        return self.per
+
+
+# ---- the tracking cost and the batched optimiser -------------------------------------------------------------------
+class DCost:
+    """The quadratic tracking cost of trep.discopt.DCost (dcost.py):
+        l(x, u, k) = (dx^T Q dx + du^T R du) / 2,  m(x) = dx_K^T Q dx_K / 2,  dx = x - xd[k],  du = u - ud[k].
+    xd [K+1,nX] and ud [K,nU] are one reference, or [R,K+1,nX] / [R,K,nU] one per rollout.  The methods take one state
+    / input, or one per rollout with a leading axis; DOptimizer evaluates the same cost on the GPU
+    (lib.track_cost)."""
+
+    def __init__(self, xd, ud, Q, R):
+        self.xd, self.ud = np.array(xd, dtype=float), np.array(ud, dtype=float)
+        self.Q, self.R = np.array(Q, dtype=float), np.array(R, dtype=float)
+
+    @property
+    def per_rollout(self):
+        return self.xd.ndim == 3
+
+    def l(self, xk, uk, k):
+        dx, du = np.asarray(xk, float) - self.xd[..., k, :], np.asarray(uk, float) - self.ud[..., k, :]
+        return 0.5 * (np.sum(dx * (dx @ self.Q.T), axis=-1) + np.sum(du * (du @ self.R.T), axis=-1))
+
+    def m(self, xf):
+        dx = np.asarray(xf, float) - self.xd[..., -1, :]
+        return 0.5 * np.sum(dx * (dx @ self.Q.T), axis=-1)
+
+    def l_dx(self, xk, uk, k):
+        return (np.asarray(xk, float) - self.xd[..., k, :]) @ self.Q
+
+    def l_du(self, xk, uk, k):
+        return (np.asarray(uk, float) - self.ud[..., k, :]) @ self.R
+
+    def m_dx(self, xf):
+        return (np.asarray(xf, float) - self.xd[..., -1, :]) @ self.Q
+
+    def l_dxdx(self, xk, uk, k):
+        return self.Q
+
+    def l_dudu(self, xk, uk, k):
+        return self.R
+
+    def l_dxdu(self, xk, uk, k):
+        return np.zeros((self.Q.shape[0], self.R.shape[0]))
+
+    def m_dxdx(self, xf):
+        return self.Q
+
+
+STEP_ACCEPTED = 0       # a step size passed the Armijo test (DOptimizer.last_status)
+STEP_CONVERGED = 1      # |dcost| < descent_tolerance
+ARMIJO_FAILED = -1      # no step size passed within armijo_max_iterations; the trajectory was kept
+
+
+class _TrackModel:
+    """The LQ model of a DOptimizer step built on the device by the track kernel (trepb_track_batch_dev): q / r /
+    l_dx / m_dx and cost0 from the DCost along (X, U), then Q / S / R per rollout in the layout the LQ solve reads:
+    identity weights for "steepest", the DCost weights for "quasi", and for "newton" those plus the z-contracted
+    blocks, each sum one IEEE addition."""
+
+    def __init__(self, opt, Xb, Ub, ref_rows, method):
+        self.opt, self.Xb, self.Ub, self.ref_rows, self.method = opt, Xb, Ub, ref_rows, method
+
+    def gradients(self, d):
+        from . import lib
+        opt = self.opt
+        ds, dev = opt.dsys, opt.dsys.varint.sys.device
+        Rn, K = self.Xb.shape[0], self.Xb.shape[1] - 1
+        nX, nU = ds.nX, ds.nU
+        opt._upload_cost(d, self.Xb, self.Ub, self.ref_rows)
+        d["qm"], d["rm"] = lib.DeviceBuffer(dev, (Rn, K + 1, nX)), lib.DeviceBuffer(dev, (Rn, K, nU))
+        d["l_dx"], d["m_dx"] = lib.DeviceBuffer(dev, (Rn, K, nX)), lib.DeviceBuffer(dev, (Rn, nX))
+        d["cost"] = lib.DeviceBuffer(dev, (Rn,))
+        model = {}
+        if self.method == "quasi":
+            d["Qm"], d["Rm"] = lib.DeviceBuffer(dev, (Rn, K + 1, nX, nX)), lib.DeviceBuffer(dev, (Rn, K, nU, nU))
+            model = dict(Qm=d["Qm"], Rm=d["Rm"])
+        lib.track_raw(True, dev, Rn, K, nX, nU, nref=d["nref"], X=d["X"], U=d["U"], Xd=d["Xd"], Ud=d["Ud"], Q=d["Qc"],
+                      R=d["Rc"], ref_index=d.get("ref_index"), q=d["qm"], r=d["rm"], l_dx=d["l_dx"], m_dx=d["m_dx"],
+                      cost=d["cost"], **model)
+
+    def hessians(self, d, newton):
+        from . import lib
+        if self.method == "quasi":
+            return True
+        ds, dev = self.opt.dsys, self.opt.dsys.varint.sys.device
+        Rn, K = self.Xb.shape[0], self.Xb.shape[1] - 1
+        nX, nU = ds.nX, ds.nU
+        d["Qm"], d["Rm"] = lib.DeviceBuffer(dev, (Rn, K + 1, nX, nX)), lib.DeviceBuffer(dev, (Rn, K, nU, nU))
+        if newton:
+            d["Sm"] = lib.DeviceBuffer(dev, (Rn, K, nX, nU))
+            lib.track_raw(True, dev, Rn, K, nX, nU, Q=d["Qc"], R=d["Rc"], fdxdx=d["fdxdx"], fdxdu=d["fdxdu"],
+                          fdudu=d["fdudu"], Qm=d["Qm"], Sm=d["Sm"], Rm=d["Rm"])
+        else:   # steepest: Q = I, R = I, S = 0
+            up = lambda a: lib.DeviceBuffer(dev, a.shape).upload(a)
+            d["I_x"], d["I_u"] = up(np.eye(nX)), up(np.eye(nU))
+            lib.track_raw(True, dev, Rn, K, nX, nU, Q=d["I_x"], R=d["I_u"], Qm=d["Qm"], Rm=d["Rm"])
+        return True
+
+
+class DOptimizer:
+    """A batched trep.discopt.DOptimizer (doptimizer.py) for a DCost: R independent trajectory-optimisation problems
+    (multi-start guesses, or plausible models through DSystem.set_parameters) per launch.  Every method takes one
+    trajectory (X [K+1,nX], U [K,nU]) or R rollouts with a leading axis.  The cost, its gradient, the LQ model with
+    the Newton terms, the Armijo candidates and their costs stay on the GPU; the host sees the costs, the statuses and
+    the accepted trajectories.
+
+    The defaults are believed to be the reference's (beta 0.7, alpha 1e-5, 30 Armijo iterations, descent tolerance
+    1e-6, 10 first-method iterations, "quasi" then "newton"); they were not checked against its source.
+    optimize_ic=True (a solve against P(0) inside the chain) and monitors are not supported."""
+    descent_return = namedtuple("descent", "Kproj dX dU")
+    armijo_search_return = namedtuple("armijo_search", "nX nU cost")
+    step_return = namedtuple("step", "converged X U dcost cost")
+
+    def __init__(self, dsys, cost, first_method_iterations=10, armijo_batch=8):
+        self.dsys, self.cost = dsys, cost
+        self.optimize_ic = False
+        self.Qproj = self.Rproj = None
+        self.armijo_beta = 0.7
+        self.armijo_alpha = 0.00001
+        self.armijo_max_iterations = 30
+        self.descent_tolerance = 1e-6
+        self.first_method_iterations = first_method_iterations
+        self.first_method = "quasi"
+        self.second_method = "newton"
+        self.armijo_batch = armijo_batch
+        self.last_status = None        # per rollout, after step / armijo_search / optimize
+        self.last_armijo_m = None      # per rollout: the accepted m of the last search, -1 if none
+
+    # ---- helpers -----------------------------------------------------------------------------------------------
+    def _batch(self, X, U):
+        X, U = np.asarray(X, float), np.asarray(U, float)
+        single = X.ndim == 2
+        return single, np.ascontiguousarray(X[None] if single else X), np.ascontiguousarray(U[None] if single else U)
+
+    def _ref_rows(self, rows):
+        """ref_index of the trajectories of rollouts `rows` (None: every rollout tracks the one reference)."""
+        return np.asarray(rows, np.int32) if self.cost.per_rollout else None
+
+    def _upload_cost(self, d, Xb, Ub, ref_rows):
+        """X, U, the references, the weights and the reference index on the device, in d."""
+        from . import lib
+        dev = self.dsys.varint.sys.device
+        up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, np.shape(a), dt).upload(np.ascontiguousarray(a, dtype=dt))
+        K = Xb.shape[1] - 1
+        xd = self.cost.xd if self.cost.per_rollout else self.cost.xd[None]
+        ud = self.cost.ud if self.cost.per_rollout else self.cost.ud[None]
+        if xd.shape[1] < K + 1 or ud.shape[1] < K:
+            raise ValueError("the reference has %d states, the trajectory %d" % (xd.shape[1], K + 1))
+        d["X"], d["U"] = up(Xb), up(Ub)
+        d["Xd"], d["Ud"] = up(xd[:, :K + 1]), up(ud[:, :K])
+        d["Qc"], d["Rc"] = up(self.cost.Q), up(self.cost.R)
+        d["nref"] = xd.shape[0]
+        d["ref_index"] = None if ref_rows is None else up(ref_rows, np.int32)
+
+    def _costs(self, Xb, Ub, dX=None, dU=None):
+        from . import lib
+        rows = self._ref_rows(np.arange(Xb.shape[0]))
+        K = Xb.shape[1] - 1
+        xd, ud = self.cost.xd[..., :K + 1, :], self.cost.ud[..., :K, :]
+        return lib.track_cost(Xb, Ub, xd, ud, self.cost.Q, self.cost.R, ref_index=rows, dX=dX, dU=dU,
+                              outputs=("cost", "dcost") if dX is not None else ("cost",),
+                              device=self.dsys.varint.sys.device)
+
+    def _params_for(self, rows):
+        """DSystem parameters restricted to rollouts `rows` (None when they are not per rollout)."""
+        p = self.dsys._params
+        if p is None or p[1].shape[0] == 1:
+            return None
+        return p[0], np.ascontiguousarray(p[1][rows])
+
+    # ---- the reference's interface -------------------------------------------------------------------------------
+    def calc_cost(self, X, U):
+        """DOptimizer.calc_cost: sum_k l(X[k], U[k], k) + m(X[K]), on the GPU."""
+        single, Xb, Ub = self._batch(X, U)
+        c = self._costs(Xb, Ub)["cost"]
+        return float(c[0]) if single else c
+
+    def calc_dcost(self, X, U, dX, dU):
+        """DOptimizer.calc_dcost: sum_k l_dx . dX[k] + l_du . dU[k] + m_dx . dX[K], on the GPU."""
+        single, Xb, Ub = self._batch(X, U)
+        _, dXb, dUb = self._batch(dX, dU)
+        c = self._costs(Xb, Ub, dXb, dUb)["dcost"]
+        return float(c[0]) if single else c
+
+    def _direction(self, Xb, Ub, rows, method):
+        """The device chain of one descent direction for rollouts `rows`; returns its buffers (caller frees)."""
+        if self.optimize_ic:
+            raise ValueError("optimize_ic=True is not supported")
+        if method not in ("steepest", "quasi", "newton"):
+            raise ValueError("Invalid descent direction method: %r" % (method,))
+        ds = self.dsys
+        saved = ds._params
+        sub = self._params_for(rows)
+        if sub is not None:
+            ds._params = sub
+        try:
+            return ds._descent_on_device(Xb, Ub, self.Qproj, self.Rproj, method == "newton", None,
+                                         _TrackModel(self, Xb, Ub, self._ref_rows(rows), method))
+        finally:
+            ds._params = saved
+
+    def calc_descent_direction(self, X, U, method="steepest"):
+        """DOptimizer.calc_descent_direction: (Kproj, dX, dU).  The model (Q, R, S) stays on the device and is not
+        returned."""
+        single, Xb, Ub = self._batch(X, U)
+        d = self._direction(Xb, Ub, np.arange(Xb.shape[0]), method)
+        try:
+            out = (d["K"].download(), -d["dX"].download(), -d["dU"].download())
+        finally:
+            self.dsys._free(d)
+        return self.descent_return(*(o[0] for o in out)) if single else self.descent_return(*out)
+
+    def _dcost_on_device(self, d, Rn, K):
+        """dcost0 of the chain's direction: the track kernel on d["dX"] / d["dU"], which hold -dX / -dU (every
+        product and sum is then exactly negated)."""
+        from . import lib
+        dev = self.dsys.varint.sys.device
+        d["dcost"] = lib.DeviceBuffer(dev, (Rn,))
+        lib.track_raw(True, dev, Rn, K, self.dsys.nX, self.dsys.nU, nref=d["nref"], X=d["X"], U=d["U"], Xd=d["Xd"],
+                      Ud=d["Ud"], Q=d["Qc"], R=d["Rc"], ref_index=d.get("ref_index"), dX=d["dX"], dU=d["dU"],
+                      dcost=d["dcost"])
+        return -d["dcost"].download()
+
+    def _search(self, d, Xb, Ub, rows, active, cost0, dcost0):
+        """Armijo search of DOptimizer.armijo_search for the rollouts at positions `active` of this batch (rows: their
+        rollout indices in the problem), on the buffers d holds: X, U, Xd, Ud, Qc, Rc, ref_index, dX / dU (= -dX /
+        -dU) and K (Kproj).  Step sizes beta^m in batches of armijo_batch: one candidates launch, one project launch
+        over the searching rollouts x M and one track launch for the candidates' costs; each rollout accepts the first
+        m with cost1 < cost0 + alpha beta^m dcost0.  Returns (X, U, cost, status, m)."""
+        from . import lib
+        ds = self.dsys
+        sys_, dev = ds.varint.sys, ds.varint.sys.device
+        Rn, K = Xb.shape[0], Xb.shape[1] - 1
+        nX, nU = ds.nX, ds.nU
+        Xn, Un, cost = Xb.copy(), Ub.copy(), np.array(cost0, float)
+        status = np.zeros(Rn, np.int32)
+        macc = np.full(Rn, -1)
+        up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, np.shape(a), dt).upload(np.ascontiguousarray(a, dtype=dt))
+        times = up(ds.time[:K + 1])
+        par = ds._params
+        try:
+            g = np.asarray(active, dtype=np.int64)
+            m0 = 0
+            while g.size and m0 < self.armijo_max_iterations:
+                ms = list(range(m0, min(m0 + self.armijo_batch, self.armijo_max_iterations)))
+                lam = np.array([self.armijo_beta ** m for m in ms])
+                M, G = len(ms), g.size
+                n = G * M
+                b = {}
+                try:
+                    b["rows"] = None if G == Rn else up(g, np.int32)
+                    b["lam"] = up(-lam)   # -lam times -dX is exactly lam dX
+                    b["bX"], b["bU"] = lib.DeviceBuffer(dev, (n, K + 1, nX)), lib.DeviceBuffer(dev, (n, K, nU))
+                    b["Kc"] = lib.DeviceBuffer(dev, (n, K, nU, nX))
+                    lib.candidates_raw(True, dev, G, M, K, nX, nU, b["lam"], d["X"], d["U"], d["dX"], d["dU"], d["K"],
+                                       b["bX"], b["bU"], b["Kc"], rows=b["rows"])
+                    b["pX"], b["pU"] = lib.DeviceBuffer(dev, (n, K + 1, nX)), lib.DeviceBuffer(dev, (n, K, nU))
+                    b["st"], b["cost"] = lib.DeviceBuffer(dev, (n,), np.int32), lib.DeviceBuffer(dev, (n,))
+                    params = None
+                    if par is not None:
+                        V = par[1] if par[1].shape[0] == 1 else par[1][np.repeat(rows[g], M)]
+                        b["params"] = up(np.ascontiguousarray(np.broadcast_to(V, (n, V.shape[1]))))
+                        params = (par[0], b["params"])
+                    sys_.project_raw(True, n, K, float(ds.time[0]), float(ds.time[1] - ds.time[0]), b["bX"], b["bU"],
+                                     b["Kc"], b["pX"], b["pU"], b["st"], k_per_instance=True, use_hint=False,
+                                     tolerance=ds.varint.tolerance, times=times, params=params)
+                    ref = self._ref_rows(np.repeat(rows[g], M))
+                    b["ref"] = None if ref is None else up(ref, np.int32)
+                    lib.track_raw(True, dev, n, K, nX, nU, nref=d["nref"], X=b["pX"], U=b["pU"], Xd=d["Xd"], Ud=d["Ud"],
+                                  Q=d["Qc"], R=d["Rc"], ref_index=b["ref"], cost=b["cost"])
+                    st, c1 = b["st"].download(), b["cost"].download()
+                    left = []
+                    for gi, r in enumerate(g):
+                        for i, m in enumerate(ms):
+                            j = gi * M + i
+                            if st[j] != 0:
+                                continue      # a failed simulation is skipped, as armijo_simulate's exception is
+                            if c1[j] < cost0[r] + self.armijo_alpha * lam[i] * dcost0[r]:
+                                Xn[r], Un[r] = b["pX"].download_row(j), b["pU"].download_row(j)
+                                cost[r], macc[r] = c1[j], m
+                                break
+                        else:
+                            left.append(r)
+                    g = np.asarray(left, dtype=np.int64)
+                    m0 += M
+                finally:
+                    ds._free(b)
+            status[g] = ARMIJO_FAILED
+        finally:
+            times.free()
+        return Xn, Un, cost, status, macc
+
+    def armijo_search(self, X, U, Kproj, dX, dU):
+        """DOptimizer.armijo_search on the GPU.  One trajectory: (nX, nU, cost), ConvergenceError when no step size
+        passes.  R rollouts: (nX, nU, cost [R]); a rollout whose search fails keeps its trajectory and cost0, and
+        last_status marks it ARMIJO_FAILED (last_armijo_m holds the accepted m, -1 for none)."""
+        from . import lib
+        single, Xb, Ub = self._batch(X, U)
+        _, dXb, dUb = self._batch(dX, dU)
+        Rn, K = Xb.shape[0], Xb.shape[1] - 1
+        Kp = np.asarray(Kproj, float)
+        Kp = np.ascontiguousarray(np.broadcast_to(Kp, (Rn,) + Kp.shape[-3:]))
+        dev = self.dsys.varint.sys.device
+        rows = np.arange(Rn)
+        d = {}
+        try:
+            self._upload_cost(d, Xb, Ub, self._ref_rows(rows))
+            up = lambda a: lib.DeviceBuffer(dev, a.shape).upload(np.ascontiguousarray(a))
+            d["dX"], d["dU"], d["K"] = up(-dXb), up(-dUb), up(Kp)
+            d["cost"] = lib.DeviceBuffer(dev, (Rn,))
+            lib.track_raw(True, dev, Rn, K, self.dsys.nX, self.dsys.nU, nref=d["nref"], X=d["X"], U=d["U"], Xd=d["Xd"],
+                          Ud=d["Ud"], Q=d["Qc"], R=d["Rc"], ref_index=d["ref_index"], cost=d["cost"])
+            dcost0 = self._dcost_on_device(d, Rn, K)
+            cost0 = d["cost"].download()
+            Xn, Un, cost, status, macc = self._search(d, Xb, Ub, rows, rows, cost0, dcost0)
+        finally:
+            self.dsys._free(d)
+        self.last_status, self.last_armijo_m = status, macc
+        if single:
+            if status[0] != 0:
+                raise ConvergenceError("Armijo Failed to Converge", status)
+            return self.armijo_search_return(Xn[0], Un[0], float(cost[0]))
+        return self.armijo_search_return(Xn, Un, cost)
+
+    def _step(self, Xb, Ub, rows, method):
+        """One step of rollouts `rows` (their trajectories Xb / Ub): (converged, X, U, dcost0, cost, status, m)."""
+        Rn, K = Xb.shape[0], Xb.shape[1] - 1
+        d = self._direction(Xb, Ub, rows, method)
+        try:
+            dcost0 = self._dcost_on_device(d, Rn, K)
+            cost0 = d["cost"].download()
+            conv = np.abs(dcost0) < self.descent_tolerance
+            Xn, Un, cost, status, macc = self._search(d, Xb, Ub, rows, np.flatnonzero(~conv), cost0, dcost0)
+        finally:
+            self.dsys._free(d)
+        status[conv] = STEP_CONVERGED
+        return conv, Xn, Un, dcost0, cost, status, macc
+
+    def step(self, iteration, X, U, method="steepest"):
+        """DOptimizer.step: the descent direction, cost0 and dcost0, then (unless |dcost0| < descent_tolerance) the
+        Armijo search.  Returns (converged, X, U, dcost0, cost); with R rollouts each is per rollout, and last_status
+        holds STEP_ACCEPTED, STEP_CONVERGED or ARMIJO_FAILED (the trajectory kept).  One trajectory raises
+        ConvergenceError when its search fails."""
+        single, Xb, Ub = self._batch(X, U)
+        conv, Xn, Un, dcost0, cost, status, macc = self._step(Xb, Ub, np.arange(Xb.shape[0]), method)
+        self.last_status, self.last_armijo_m = status, macc
+        if single:
+            if status[0] == ARMIJO_FAILED:
+                raise ConvergenceError("Armijo Failed to Converge", status)
+            return self.step_return(bool(conv[0]), Xn[0], Un[0], float(dcost0[0]), float(cost[0]))
+        return self.step_return(conv, Xn, Un, dcost0, cost)
+
+    def optimize(self, X, U, max_steps=50):
+        """DOptimizer.optimize: project (X, U) onto a trajectory of the system, then steps with first_method for
+        first_method_iterations steps and second_method afterwards.  Each rollout is frozen once it converges or its
+        Armijo search fails; last_status holds STEP_CONVERGED, ARMIJO_FAILED or STEP_ACCEPTED (max_steps reached).
+        Returns (converged, X, U); one trajectory raises ConvergenceError when its search fails."""
+        if self.optimize_ic:
+            raise ValueError("optimize_ic=True is not supported")
+        single, Xb, Ub = self._batch(X, U)
+        Xb, Ub = self.dsys.project(Xb, Ub, self.dsys.calc_feedback_controller(Xb, Ub))
+        Xb, Ub = Xb.copy(), Ub.copy()
+        status = np.zeros(Xb.shape[0], np.int32)
+        live = np.arange(Xb.shape[0])
+        method = self.first_method
+        for i in range(max_steps):
+            if i == self.first_method_iterations:
+                method = self.second_method
+            if not live.size:
+                break
+            _, Xn, Un, _, _, st, _ = self._step(Xb[live], Ub[live], live, method)
+            Xb[live], Ub[live] = Xn, Un
+            status[live] = st
+            live = live[st == STEP_ACCEPTED]
+        self.last_status = status
+        converged = status == STEP_CONVERGED
+        if single:
+            if status[0] == ARMIJO_FAILED:
+                raise ConvergenceError("Armijo Failed to Converge", status)
+            return bool(converged[0]), Xb[0], Ub[0]
+        return converged, Xb, Ub

@@ -71,6 +71,18 @@ class AdjointArgs(C.Structure):
                 ("m_dx", C.c_void_p), ("z", C.c_void_p), ("z1", C.c_void_p)]
 
 
+class TrackArgs(C.Structure):
+    _fields_ = [("batch", C.c_int64), ("nsteps", C.c_int32), ("nX", C.c_int32), ("nU", C.c_int32), ("nref", C.c_int32)]\
+        + [(n, C.c_void_p) for n in ("X", "U", "Xd", "Ud", "Q", "R", "ref_index", "dX", "dU", "fdxdx", "fdxdu", "fdudu",
+                                     "cost", "dcost", "q", "r", "l_dx", "m_dx", "Qm", "Sm", "Rm")]
+
+
+class CandidatesArgs(C.Structure):
+    _fields_ = [("groups", C.c_int64), ("ncand", C.c_int32), ("nsteps", C.c_int32), ("nX", C.c_int32), ("nU", C.c_int32),
+                ("nrollouts", C.c_int64)] \
+        + [(n, C.c_void_p) for n in ("rows", "lam", "X", "U", "dX", "dU", "Kproj", "bX", "bU", "Kc")]
+
+
 RAW = ["q2_dq1", "q2_dp1", "q2_du1", "q2_dk2", "p2_dq1", "p2_dp1", "p2_du1", "p2_dk2",
        "l1_dq1", "l1_dp1", "l1_du1", "l1_dk2"]
 
@@ -140,6 +152,10 @@ _lib.trepb_tangent_batch.argtypes = [C.c_int, C.POINTER(TangentArgs)]
 _lib.trepb_tangent_batch_dev.argtypes = [C.c_int, C.POINTER(TangentArgs), C.c_void_p]
 _lib.trepb_adjoint_batch.argtypes = [C.c_int, C.POINTER(AdjointArgs)]
 _lib.trepb_adjoint_batch_dev.argtypes = [C.c_int, C.POINTER(AdjointArgs), C.c_void_p]
+_lib.trepb_track_batch.argtypes = [C.c_int, C.POINTER(TrackArgs)]
+_lib.trepb_track_batch_dev.argtypes = [C.c_int, C.POINTER(TrackArgs), C.c_void_p]
+_lib.trepb_candidates_batch.argtypes = [C.c_int, C.POINTER(CandidatesArgs)]
+_lib.trepb_candidates_batch_dev.argtypes = [C.c_int, C.POINTER(CandidatesArgs), C.c_void_p]
 _lib.trepb_lqr_last_kernel_ms.argtypes = [C.c_int, C.POINTER(C.c_float)]
 _lib.trepb_linearize_batch.argtypes = [C.c_void_p, C.POINTER(LinArgs)]
 _lib.trepb_linearize_batch_dev.argtypes = [C.c_void_p, C.POINTER(LinArgs), C.c_void_p]
@@ -206,7 +222,8 @@ EXPORTS = [
     "trepb_calc_p2_varied_batch", "trepb_calc_p2_varied_batch_dev", "trepb_calc_f_varied_batch",
     "trepb_calc_f_varied_batch_dev", "trepb_discrete_fm2_varied_batch", "trepb_discrete_fm2_varied_batch_dev",
     "trepb_deriv2_varied_batch", "trepb_deriv2_varied_batch_dev", "trepb_tangent_batch", "trepb_tangent_batch_dev",
-    "trepb_adjoint_batch", "trepb_adjoint_batch_dev",
+    "trepb_adjoint_batch", "trepb_adjoint_batch_dev", "trepb_track_batch", "trepb_track_batch_dev",
+    "trepb_candidates_batch", "trepb_candidates_batch_dev",
 ]
 
 
@@ -404,6 +421,60 @@ def adjoint_sweep(A, B, m_dx, l_dx=None, l_du=None, K=None, device=0):
     return z[0] if single else z
 
 
+TRACK_OUTPUTS = ("cost", "dcost", "q", "r", "l_dx", "m_dx", "Qm", "Sm", "Rm")
+
+
+def track_raw(on_device, device, batch, nsteps, nX, nU, nref=1, stream=None, **arrays):
+    """trepb_track_batch[_dev]: arrays by field name of trepb_track_args (X, U, Xd, Ud, Q, R, ref_index, dX, dU, fdxdx,
+    fdxdu, fdudu and the outputs TRACK_OUTPUTS); missing ones are NULL."""
+    a = TrackArgs(batch=batch, nsteps=nsteps, nX=nX, nU=nU, nref=nref)
+    for n, v in arrays.items():
+        setattr(a, n, _ptr(v))
+    if on_device:
+        _check(_lib.trepb_track_batch_dev(device, C.byref(a), stream))
+    else:
+        _check(_lib.trepb_track_batch(device, C.byref(a)))
+
+
+def candidates_raw(on_device, device, groups, ncand, nsteps, nX, nU, lam, X, U, dX, dU, Kproj, bX, bU, Kc, rows=None,
+                   nrollouts=0, stream=None):
+    a = CandidatesArgs(groups=groups, ncand=ncand, nsteps=nsteps, nX=nX, nU=nU, nrollouts=nrollouts, rows=_ptr(rows),
+                       lam=_ptr(lam), X=_ptr(X), U=_ptr(U), dX=_ptr(dX), dU=_ptr(dU), Kproj=_ptr(Kproj), bX=_ptr(bX),
+                       bU=_ptr(bU), Kc=_ptr(Kc))
+    if on_device:
+        _check(_lib.trepb_candidates_batch_dev(device, C.byref(a), stream))
+    else:
+        _check(_lib.trepb_candidates_batch(device, C.byref(a)))
+
+
+def track_cost(X, U, Xd, Ud, Q, R, ref_index=None, dX=None, dU=None, newton=None, outputs=TRACK_OUTPUTS, device=0):
+    """The tracking cost of DCost (trep/discopt/dcost.py) and its LQ model on the GPU (trepb_track_batch).
+    X [B,K+1,nX], U [B,K,nU]; Xd [K+1,nX] / Ud [K,nU] (one reference) or [nref,..] with ref_index [B] naming each
+    trajectory's reference; Q [nX,nX], R [nU,nU]; dX / dU as X / U for dcost; newton = (fdxdx [B,K,nX,nX], fdxdu
+    [B,K,nX,nU], fdudu [B,K,nU,nU]) added to the model.  Returns a dict of the requested outputs (cost and dcost [B],
+    q [B,K+1,nX], r [B,K,nU], l_dx [B,K,nX], m_dx [B,nX], Qm [B,K+1,nX,nX], Sm [B,K,nX,nU], Rm [B,K,nU,nU]); dcost
+    only when dX is given."""
+    f = lambda x: None if x is None else np.ascontiguousarray(np.asarray(x, float))
+    X, U, Xd, Ud, Q, R, dX, dU = (f(x) for x in (X, U, Xd, Ud, Q, R, dX, dU))
+    Bn, K, nX = X.shape[0], X.shape[1] - 1, X.shape[2]
+    nU = U.shape[2]
+    if Xd.ndim == 2:
+        Xd, Ud = Xd[None], Ud[None]
+    shapes = dict(cost=(Bn,), dcost=(Bn,), q=(Bn, K + 1, nX), r=(Bn, K, nU), l_dx=(Bn, K, nX), m_dx=(Bn, nX),
+                  Qm=(Bn, K + 1, nX, nX), Sm=(Bn, K, nX, nU), Rm=(Bn, K, nU, nU))
+    out = {n: np.zeros(shapes[n]) for n in outputs if n != "dcost" or dX is not None}
+    arrays = dict(X=X, U=U, Xd=Xd, Ud=Ud, Q=Q, R=R, dX=dX, dU=dU)
+    if ref_index is not None:
+        arrays["ref_index"] = np.ascontiguousarray(ref_index, dtype=np.int32)
+    if newton is not None:
+        arrays.update(zip(("fdxdx", "fdxdu", "fdudu"), (f(x) for x in newton)))
+    if nU == 0:
+        arrays = {n: v for n, v in arrays.items() if n not in ("U", "Ud", "R", "dU", "fdxdu", "fdudu")}
+    arrays.update({n: v for n, v in out.items() if nU or n not in ("r", "Sm", "Rm")})
+    track_raw(False, device, Bn, K, nX, nU, nref=Xd.shape[0], **arrays)
+    return out
+
+
 def specialized_names():
     return [_lib.trepb_specialized_name(i).decode() for i in range(_lib.trepb_num_specialized())]
 
@@ -502,6 +573,12 @@ class DeviceBuffer:
         if out is None:
             out = np.empty(self.shape, self.dtype)
         _check(_lib.trepb_memcpy_d2h(self.device, out.ctypes.data, self.ptr, self.nbytes))
+        return out
+
+    def download_row(self, i):
+        """Element i of the first axis, as an array of shape shape[1:]."""
+        out = np.empty(self.shape[1:], self.dtype)
+        _check(_lib.trepb_memcpy_d2h(self.device, out.ctypes.data, self.ptr + i * out.nbytes, out.nbytes))
         return out
 
     def zero(self):
