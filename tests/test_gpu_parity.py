@@ -15,6 +15,7 @@ import numpy as np
 import pytest
 
 import golden_util as G
+from test_lq_reference import lq_pinned_cases, lqr_pinned_cases
 
 pytestmark = pytest.mark.gpu
 
@@ -451,46 +452,29 @@ def test_project_puppet_kinematic_feedback(lib):
 
 
 def test_lqr_sweep_matches_reference(lib):
-    """trepb_lqr_batch against the reference's discopt.dlqr.solve_tv_lqr (dlqr.py:9-38): random
-    stabilisable problems of the marionette's size and of pend-on-cart's, constant and per-step
-    weights, several rollouts in one launch."""
-    rng = np.random.default_rng(21)
-    # (37, 5): odd sizes on the tensor-core path (every tile ragged, no vector loads); (40, 6): partial 16 x 40 tiles
-    for nX, nU, K, R_, per_step in ((4, 1, 60, 3, False), (80, 18, 25, 2, True), (7, 3, 40, 5, True),
-                                    (37, 5, 12, 2, True), (40, 6, 12, 3, False)):
-        A = np.eye(nX)[None, None] + rng.normal(0, 0.3 / np.sqrt(nX), (R_, K, nX, nX))
-        B = rng.normal(0, 1.0, (R_, K, nX, nU))
-        if per_step:
-            Qs = np.stack([np.eye(nX) * (1 + 0.1 * k) for k in range(K + 1)])
-            Rs = np.stack([np.eye(nU) * (2 + 0.05 * k) for k in range(K)])
-        else:
-            M = rng.normal(0, 1, (nX, nX)); Qs = M @ M.T + np.eye(nX)
-            Rs = np.eye(nU) * 0.5
+    """trepb_lqr_batch against its own results pinned at f731ca3 (golden_util.expected), which were checked against
+    the reference's discopt.dlqr.solve_tv_lqr (dlqr.py:9-38) run live: random stabilisable problems of the
+    marionette's size and of pend-on-cart's, constant and per-step weights, several rollouts in one launch.  The inputs
+    come from test_lq_reference, which holds the long-double reference of tests/lqref.py to the same pins."""
+    for key, A, B, Qs, Rs in lqr_pinned_cases():
+        nX = A.shape[2]
         Kg, Pg = lib.solve_tv_lqr(A, B, Qs, Rs)
-        want = G.expected("lqr_%d_%d" % (nX, nU), lambda: {"K": Kg, "P": Pg})
-        for r in range(R_):
+        want = G.expected(key, lambda: {"K": Kg, "P": Pg})
+        for r in range(A.shape[0]):
             G.assert_close(Kg[r], want["K"][r], "lqr gains nX=%d rollout %d" % (nX, r), rtol=1e-9)
             G.assert_close(Pg[r], want["P"][r], "lqr P0 nX=%d rollout %d" % (nX, r), rtol=1e-9)
 
 
 def test_lq_sweep_matches_reference(lib):
-    """trepb_lq_batch against the reference's discopt.dlqr.solve_tv_lq (dlqr.py:41-81): linear and
-    cross cost terms, costs shared by the batch and one set per rollout, with and without S."""
-    rng = np.random.default_rng(22)
-    for nX, nU, K, R_, per_rollout, with_s in ((4, 1, 50, 3, False, True), (80, 18, 20, 2, True, True),
-                                               (7, 3, 30, 4, True, False), (5, 2, 10, 1, False, False),
-                                               (37, 5, 10, 2, True, True)):
-        A = np.eye(nX)[None, None] + rng.normal(0, 0.3 / np.sqrt(nX), (R_, K, nX, nX))
-        B = rng.normal(0, 1.0, (R_, K, nX, nU))
-        nc = R_ if per_rollout else 1
-        Qs = np.stack([np.stack([np.eye(nX) * (1 + 0.1 * k + 0.3 * c) for k in range(K + 1)]) for c in range(nc)])
-        Rs = np.stack([np.stack([np.eye(nU) * (2 + 0.05 * k + 0.2 * c) for k in range(K)]) for c in range(nc)])
-        Ss = rng.normal(0, 0.05, (nc, K, nX, nU)) if with_s else None
-        q = rng.normal(0, 1, (nc, K + 1, nX)); r = rng.normal(0, 1, (nc, K, nU))
-        sq = (lambda x: x) if per_rollout else (lambda x: None if x is None else x[0])
-        Kg, Cg, Pg, bg = lib.solve_tv_lq(A, B, sq(q), sq(r), sq(Qs), sq(Ss), sq(Rs))
-        want = G.expected("lq_%d_%d" % (nX, nU), lambda: {"K": Kg, "C": Cg, "P": Pg, "b": bg})
-        for i in range(R_):
+    """trepb_lq_batch against its own results pinned at f731ca3 (golden_util.expected), which were checked against
+    the reference's discopt.dlqr.solve_tv_lq (dlqr.py:41-81) run live: linear and cross cost terms, costs shared by the
+    batch and one set per rollout, with and without S.  The inputs come from test_lq_reference, which holds the
+    long-double reference of tests/lqref.py to the same pins."""
+    for key, A, B, q, r, Qs, Ss, Rs, _ in lq_pinned_cases():
+        nX = A.shape[2]
+        Kg, Cg, Pg, bg = lib.solve_tv_lq(A, B, q, r, Qs, Ss, Rs)
+        want = G.expected(key, lambda: {"K": Kg, "C": Cg, "P": Pg, "b": bg})
+        for i in range(A.shape[0]):
             G.assert_close(Kg[i], want["K"][i], "lq gains nX=%d rollout %d" % (nX, i), rtol=1e-9)
             G.assert_close(Cg[i], want["C"][i], "lq affine term nX=%d rollout %d" % (nX, i), rtol=1e-9)
             G.assert_close(Pg[i], want["P"][i], "lq P0 nX=%d rollout %d" % (nX, i), rtol=1e-9)

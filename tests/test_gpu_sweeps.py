@@ -3,6 +3,9 @@ DSystem.calc_descent_direction, the chain linearize -> LQR -> (adjoint -> deriv2
 
 - The sweeps against DSystem.dproject and the costate recursion of DSystem.calc_newton_model on random
   linearizations, with every optional array NULL in turn and without inputs.
+- The sweeps against the long-double recurrences of tests/lqref.py at every branch of sweep_launch: each team width
+  (1 to 128 lanes, rows beyond 128 strided), each ring depth (8, 4, 2) with nsteps around it, a last CTA with idle
+  teams, and the refusal one state past the shared-memory limit.
 - A rollout alone and inside larger batches gives the same bits, in the host-pointer and the _dev forms.
 - The open-loop costate of a real system equals the central difference of a tracking cost through DSystem.simulate.
 - calc_descent_direction against the composition of the existing calls it replaces, and with per-rollout parameters
@@ -11,6 +14,7 @@ import numpy as np
 import pytest
 
 import golden_util as G
+import lqref
 from test_gpu_varied_deriv2 import _refs, _traj
 from trep_b200 import discopt, lib as L, midpointvi as MV
 
@@ -156,6 +160,141 @@ def test_a_rollout_gives_the_same_bits_alone_and_in_a_batch(lib, nX, nU):
         for got, want, what in ((t[0], full_t[0], "dX"), (t[1], full_t[1], "dU"), (a, full_a, "z"),
                                 (dv[0], full_t[0], "dX dev"), (dv[1], full_t[1], "dU dev"), (dv[2], full_a, "z dev")):
             assert got.tobytes() == want[s].tobytes(), "%s rollouts %d:%d" % (what, lo, hi)
+
+
+# ---- sweep_launch's branches against the long-double recurrences (tests/lqref.py) ------------------------------
+
+def sweep_stage(nX, nU):
+    """Doubles of one staged step (trepb_sweep.cuh): A, B, K in rows padded to an odd length, two vectors."""
+    s = nX * (nX | 1) + nX * (nU | 1) + nU * (nX | 1) + nX + nU
+    return (s + 1) & ~1
+
+
+def sweep_geometry(nX, nU, optin):
+    """(team, teams per CTA, ring depth) as sweep_launch picks them; depth 0: refused."""
+    team = 1
+    while team < max(nX, nU) and team < 128:
+        team <<= 1
+    teams = max(64, team) // team
+    stages = 8
+    while stages >= 2 and teams * (stages * sweep_stage(nX, nU) + 2 * nX + nU + 2) * 8 > optin:
+        stages //= 2
+    return team, teams, stages if stages >= 2 else 0
+
+
+def _optin():
+    import torch
+    return torch.cuda.get_device_properties(0).shared_memory_per_block_optin
+
+
+def ring_shape(spec, optin):
+    """"ringD": the largest nX (nU = 2) whose ring is D steps deep; "ring_max+1": one past the largest nX that fits."""
+    depth = lambda x: sweep_geometry(x, 2, optin)[2]
+    if spec == "ring_max+1":
+        return max(x for x in range(1, 1024) if depth(x)) + 1, 2
+    return max(x for x in range(1, 1024) if depth(x) == int(spec[4:])), 2
+
+
+# team 1 / 8; 32 -> 64 lanes; 64 -> 128 lanes (one team per CTA); rows beyond 128 strided; each ring depth at its
+# largest state (depth 2: the largest state that fits)
+SWEEP_SHAPES = [(1, 1), (2, 5), (32, 1), (33, 1), (64, 3), (65, 3), (4, 130), "ring8", "ring4", "ring2"]
+
+
+def _sweep_cases():
+    # nsteps in {1, stages - 1, stages, stages + 1}: the prologue with fewer steps than the ring holds, a full ring,
+    # one wrap; resolved at run time (the depth depends on the device's shared memory)
+    return [(s, j) for s in SWEEP_SHAPES for j in range(4)]
+
+
+@gpu
+@pytest.mark.parametrize("spec,which", _sweep_cases(),
+                         ids=["%s-%s" % (s if isinstance(s, str) else "%dx%d" % s, ("1", "S-1", "S", "S+1")[j])
+                              for s, j in _sweep_cases()])
+def test_sweeps_match_the_long_double_recurrences_at_every_team_width_and_ring_depth(lib, spec, which):
+    """teams x 3 + 1 rollouts (the last CTA has idle teams), every rollout against lqref.tangent_ld / adjoint_ld at
+    1e-12, with all optional arrays and with each left out: tangent without bdX / x0 / bdU; adjoint with z1, without
+    K (open loop) and without l_dx / l_du.  The last rollout and one inside the batch give the same bits alone."""
+    optin = _optin()
+    nX, nU = ring_shape(spec, optin) if isinstance(spec, str) else spec
+    team, teams, S = sweep_geometry(nX, nU, optin)
+    n = (1, S - 1, S, S + 1)[which]
+    if which == 1 and n == 1:
+        pytest.skip("a ring of 2: stages - 1 = 1 is the nsteps = 1 case")
+    R = teams * 3 + 1
+    A, B, Kf, rng = linearization(R, n, nX, nU, 1000 * nX + nU + n)
+    bdX, bdU, x0 = rng.normal(size=(R, n + 1, nX)), rng.normal(size=(R, n, nU)), rng.normal(size=(R, nX))
+    l_dx, l_du, m_dx = rng.normal(size=(R, n, nX)), rng.normal(size=(R, n, nU)), rng.normal(size=(R, nX))
+    what = "%dx%d team %d x %d, ring %d, K=%d" % (nX, nU, team, teams, S, n)
+    ld = lambda f, *a: np.stack([f(*(None if x is None else x[i] for x in a)).astype(float) for i in range(R)])
+
+    def tangent(s, bx, bu, x):
+        sub = lambda v: None if v is None else np.ascontiguousarray(v[s])
+        m = len(range(R)[s])
+        dX, dU = np.zeros((m, n + 1, nX)), np.zeros((m, n, nU))
+        lib.tangent_raw(False, 0, m, n, nX, nU, sub(A), sub(B), sub(Kf), dX, dU, bdX=sub(bx), bdU=sub(bu), x0=sub(x))
+        return dX, dU
+
+    def adjoint(s, K, lx, lu):
+        sub = lambda v: None if v is None else np.ascontiguousarray(v[s])
+        m = len(range(R)[s])
+        z, z1 = np.zeros((m, n + 1, nX)), np.zeros((m, n, nX))
+        lib.adjoint_raw(False, 0, m, n, nX, nU, sub(A), sub(B), sub(m_dx), z, K=sub(K), l_dx=sub(lx), l_du=sub(lu),
+                        z1=z1)
+        return z, z1
+
+    full = slice(0, R)
+    for bx, bu, x in ((bdX, bdU, x0), (bdX, bdU, None), (None, bdU, None), (None, None, x0)):
+        dX, dU = tangent(full, bx, bu, x)
+        want = [ld(lambda *a: lqref.tangent_ld(*a)[j], A, B, Kf, bx, bu, x) for j in range(2)]
+        tag = "%s tangent bdX %s bdU %s x0 %s" % (what, bx is not None, bu is not None, x is not None)
+        assert_rollouts_close(dX, want[0], tag + " dX")
+        assert_rollouts_close(dU, want[1], tag + " dU")
+    for K, lx, lu in ((Kf, l_dx, l_du), (None, l_dx, l_du), (Kf, None, l_du), (Kf, l_dx, None)):
+        z, z1 = adjoint(full, K, lx, lu)
+        want = ld(lambda a, m, b, k, x, u: lqref.adjoint_ld(a, m, b, k, x, u), A, m_dx, B, K, lx, lu)
+        tag = "%s adjoint K %s l_dx %s l_du %s" % (what, K is not None, lx is not None, lu is not None)
+        assert_rollouts_close(z, want, tag + " z")
+        assert z1.tobytes() == np.ascontiguousarray(z[:, 1:]).tobytes(), tag + " z1 = z[1:]"
+    fX, fU = tangent(full, bdX, bdU, x0)
+    fz, fz1 = adjoint(full, Kf, l_dx, l_du)
+    for i in sorted({R - 1, R // 2}):
+        s = slice(i, i + 1)
+        for got, want, name in zip(tangent(s, bdX, bdU, x0) + adjoint(s, Kf, l_dx, l_du), (fX, fU, fz, fz1),
+                                   ("dX", "dU", "z", "z1")):
+            assert got.tobytes() == want[s].tobytes(), "%s rollout %d alone: %s" % (what, i, name)
+
+
+@gpu
+@pytest.mark.parametrize("spec", [(1, 0), (33, 0), "ring2"], ids=["1x0", "33x0", "ring2x0"])
+def test_sweeps_without_inputs_match_the_long_double_recurrences(lib, spec):
+    optin = _optin()
+    nX = ring_shape(spec, optin)[0] if isinstance(spec, str) else spec[0]
+    team, teams, S = sweep_geometry(nX, 0, optin)
+    assert S >= 2
+    R, n = teams * 3 + 1, S + 1
+    A, _, _, rng = linearization(R, n, nX, 1, 9 + nX)
+    bdX, l_dx, m_dx = rng.normal(size=(R, n + 1, nX)), rng.normal(size=(R, n, nX)), rng.normal(size=(R, nX))
+    dX = np.zeros((R, n + 1, nX))
+    lib.tangent_raw(False, 0, R, n, nX, 0, A, None, None, dX, None, bdX=bdX)
+    assert_rollouts_close(dX, np.stack([lqref.tangent_ld(A[i], bdX=bdX[i])[0].astype(float) for i in range(R)]),
+                          "%dx0 dX" % nX)
+    z = np.zeros((R, n + 1, nX))
+    lib.adjoint_raw(False, 0, R, n, nX, 0, A, None, m_dx, z, l_dx=l_dx)
+    assert_rollouts_close(z, np.stack([lqref.adjoint_ld(A[i], m_dx[i], l_dx=l_dx[i]).astype(float) for i in range(R)]),
+                          "%dx0 z" % nX)
+
+
+@gpu
+def test_sweep_refuses_the_state_one_past_the_shared_memory_limit(lib):
+    nX, nU = ring_shape("ring_max+1", _optin())
+    A, B, Kf = np.zeros((1, 1, nX, nX)), np.zeros((1, 1, nX, nU)), np.zeros((1, 1, nU, nX))
+    dX, dU, z = np.full((1, 2, nX), 0.5), np.full((1, 1, nU), 0.5), np.full((1, 2, nX), 0.5)
+    for call in (lambda: lib.tangent_raw(False, 0, 1, 1, nX, nU, A, B, Kf, dX, dU),
+                 lambda: lib.adjoint_raw(False, 0, 1, 1, nX, nU, A, B, np.zeros((1, nX)), z, K=Kf)):
+        with pytest.raises(lib.TrepbError) as e:
+            call()
+        assert e.value.code == 4 and "state dimension too large for the shared-memory sweep" in str(e.value)
+    assert np.all(dX == 0.5) and np.all(dU == 0.5) and np.all(z == 0.5)
 
 
 def _dsys(d, t, params=None, **kw):

@@ -442,6 +442,7 @@ int lqr_launch(int device, LqrParams& p, cudaStream_t stream) {
     if (block < 64) block = 64;
     if (mma) block = 512;   // the tensor-core schedule assigns products to warps 0-9 and 10-14
     // the elimination deals the nU x (nU + nX + 1) elements of [gamma | Kp | c] out to the threads, at most 4 each
+    // the limit below already refuses every nU >= 45; this one is what makes cta_gauss_jordan's 64-bit `used` mask safe
     if (nU > 64) return lqr_fail(TREPB_ERR_UNSUPPORTED, "more than 64 inputs");
     while (block < 512 && (long long)nU * (nU + nX + 1) > 4LL * block) block += 32;
     if ((long long)nU * (nU + nX + 1) > 4LL * block)
