@@ -142,6 +142,10 @@ typedef struct trepb_system trepb_system; /* opaque */
                                        batches that do not fill the GPU (name ".../pair") */
 #define TREPB_FLAG_NO_LITERAL 16     /* specialised systems: skip an all-literal instantiation built for exactly this
                                        description and use the run-time-parameter kernel of its structure */
+#define TREPB_FLAG_COOP_VARIED 128   /* cooperative handles: the *_varied_batch* entry points run on the varied
+                                       cooperative kernels of the handle's flavour instead of being refused; plain
+                                       calls are unchanged.  Ignored on other handles.  See "per-instance physical
+                                       parameters" below. */
 
 /* Loads a plug-in built by trep_b200/build.py:build_plugin from a system description: ahead-of-time specialised
  * (register-resident) kernels for a structure the library was not built with - the role the reference gives to
@@ -537,12 +541,18 @@ int trepb_deriv2_batch_dev(trepb_system* sys, const trepb_d2_args* args, void* s
  *              TREPB_ERR_INVALID (trepb_last_error names it).  A varied Gravity component re-forms the
  *              gravity sum per instance.  A row value of exactly 0 is not checked and keeps the entry's role.
  *   kernels    specialised and table-driven thread kernels (a handle built for an all-literal instantiation runs
- *              the run-time-parameter kernels of its structure); cooperative handles are TREPB_ERR_UNSUPPORTED
- *              (create the handle with TREPB_FLAG_NO_COOP).  Second derivatives vary through the same kernels
+ *              the run-time-parameter kernels of its structure).  Cooperative handles run the varied cooperative
+ *              kernels of their flavour when created with TREPB_FLAG_COOP_VARIED (each team re-evaluates its own
+ *              copy of the link tables from its row) and are TREPB_ERR_UNSUPPORTED without it (or create the handle
+ *              with TREPB_FLAG_NO_COOP for the thread kernels).  Second derivatives vary through the same kernels
  *              and schemes as the plain call (the per-pair kernel, or the per-parameter scheme on the tables);
- *              its linearize launch runs on the same rows.
+ *              its linearize launch runs on the same rows (on a flagged cooperative handle: the varied cooperative
+ *              linearize kernel).
  * Results equal those of a handle created from each instance's own description, run through the plain entry
- * point. */
+ * point, bit for bit - with one exception on cooperative handles: a varied angle of a constant rotation frame
+ * (TREPB_PAR_FRAME_VALUE of an RX / RY / RZ frame without a config) takes its cos / sin from the device math
+ * library, a handle built on the host from the C library; they may differ in the last bit, and the results
+ * then agree to the project's parity tolerance, not bit for bit. */
 #define TREPB_PAR_FRAME_VALUE 0   /* index f           */
 #define TREPB_PAR_FRAME_SE3 1     /* index 12 f + k    */
 #define TREPB_PAR_FRAME_MASS 2    /* index 4 f + k     */

@@ -155,6 +155,9 @@ struct trepb_system {
     int vbps_d2 = 1, vbps_d2jac = 1;
     // vmap_tab: the table-driven layout of the map, for pass A of the per-parameter scheme on a specialised handle
     DevBuf vmap, vmap_tab, vslots;
+    // ... on a cooperative handle with TREPB_FLAG_COOP_VARIED: the plan of the link tables' numeric entries and one
+    // slot per team of the persistent grid (CoopVaried), allocated at the first varied call
+    DevBuf cplan, cvscratch;
     std::mutex mu;       // serialises launches on this handle
     std::mutex mu_host;  // serialises the host-pointer entry points (they share staging buffers)
 };
@@ -345,6 +348,8 @@ void trepb_system_destroy(trepb_system* s) {
     s->vmap.release();
     s->vmap_tab.release();
     s->vslots.release();
+    s->cplan.release();
+    s->cvscratch.release();
     s->d2g.release();
     for (auto& b : s->d2s) b.release();
     for (auto& b : s->hb) b.release();
@@ -531,7 +536,7 @@ int varied_upload(trepb_system* s, const trepb_varied* v, bool slots, DevBuf& bu
 // handle scratch and fills va.  The caller holds s->mu and a ScratchGuard on `stream`.
 int varied_setup(trepb_system* s, const trepb_varied* v, cudaStream_t stream, VariedArgs* va) {
     if (!v) return fail(TREPB_ERR_INVALID, "null trepb_varied");
-    if (s->coop)
+    if (s->coop && !(s->flags & TREPB_FLAG_COOP_VARIED))
         return fail(TREPB_ERR_UNSUPPORTED, "per-instance parameters are not supported by the cooperative kernels (their "
                                            "link tables are built on the host from the description): create the handle "
                                            "with TREPB_FLAG_NO_COOP");
@@ -572,14 +577,34 @@ int varied_slots(trepb_system* s, const LaunchCfg& c, VariedArgs* va) {
     return TREPB_OK;
 }
 
+// Varied cooperative launch: the plan on the device (uploaded once) and the teams' slots, sized once for the widest
+// persistent grid of the handle.  The caller holds s->mu and a ScratchGuard on `stream`.
+int coop_varied_args(trepb_system* s, const VariedArgs& va, cudaStream_t stream, CoopVaried* cv) {
+    const CoopPlan& pl = s->CP.plan;
+    if (!s->cplan.p) {
+        CU(s->cplan.ensure(pl.ints.size() * sizeof(int32_t)));
+        CU(cudaMemcpyAsync(s->cplan.p, pl.ints.data(), pl.ints.size() * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
+    }
+    const long n8 = (s->coop_blob_bytes + 7) / 8;
+    cv->per_team = ((n8 + 1) & ~1L) + 12L * pl.nf;
+    const int teams = s->coop_warps > s->coop_warps_solve ? s->coop_warps : s->coop_warps_solve;
+    CU(s->cvscratch.ensure((size_t)s->sms * teams * cv->per_team * sizeof(double)));
+    cv->map = va.map;
+    cv->values = va.values;
+    cv->plan = pl.view((const int32_t*)s->cplan.p);
+    cv->scratch = (double*)s->cvscratch.p;
+    return TREPB_OK;
+}
+
 // Launches one call (which: 0 step, 1 p2, 2 lin, 3 project) on the kernels `v` and the handle select: the
-// run-time-parameter kernels for per-instance parameters, else the cooperative kernels of a cooperative handle,
-// else one thread per instance.  thread(ks, cfg, va) and coop(cl) launch the call's kernel.  stage (linearize with
+// cooperative kernels of a cooperative handle (for per-instance parameters only with TREPB_FLAG_COOP_VARIED: their
+// varied instantiations, coop_v(cl, cv)), else the run-time-parameter kernels for per-instance parameters, else one
+// thread per instance.  thread(ks, cfg, va) and coop(cl) launch the call's kernel.  stage (linearize with
 // A or B, else null): set to 1 when the outputs are staged through shared memory.  vset: the map of `v` when the
 // caller has set it up already (varied_setup).  The caller holds s->mu.
-template <class Thread, class Coop>
+template <class Thread, class Coop, class CoopV>
 int dispatch(trepb_system* s, int which, long long batch, cudaStream_t stream, const trepb_varied* v, int* stage,
-             Thread thread, Coop coop, const VariedArgs* vset = nullptr) {
+             Thread thread, Coop coop, CoopV coop_v, const VariedArgs* vset = nullptr) {
     if (!v && s->coop) {
         CoopLaunch cl;
         make_coop(s, batch, stream, &cl, which != 2);
@@ -587,6 +612,21 @@ int dispatch(trepb_system* s, int which, long long batch, cudaStream_t stream, c
         if (int rc = attach_slabs(s, &cl)) return rc;
         Timed t(s, cl.stream);
         CU(coop(cl));
+        return TREPB_OK;
+    }
+    if (v && s->coop && (s->flags & TREPB_FLAG_COOP_VARIED)) {
+        CoopLaunch cl;
+        make_coop(s, batch, stream, &cl, which != 2);
+        ScratchGuard sg(s, stream, true);   // the teams' slots (and ext slabs) are owned by the handle
+        VariedArgs va;
+        if (vset) va = *vset;
+        else if (int rc = varied_setup(s, v, stream, &va)) return rc;
+        CoopVaried cv;
+        if (int rc = coop_varied_args(s, va, stream, &cv)) return rc;
+        if (int rc = attach_slabs(s, &cl)) return rc;
+        if (stage) *stage = 0;
+        Timed t(s, cl.stream);
+        CU(coop_v(cl, cv));
         return TREPB_OK;
     }
     ScratchGuard sg(s, stream, v || !s->ks->specialized);
@@ -633,7 +673,8 @@ int step_launch(trepb_system* s, const trepb_step_args* a, void* stream, const t
     p.times = a->times;
     return dispatch(s, 0, a->batch, (cudaStream_t)stream, v, nullptr,
                     [&](const KernelSet* ks, const LaunchCfg& c, const VariedArgs* va) { return ks->step(c, p, va); },
-                    [&](const CoopLaunch& cl) { return s->cks->step(cl, p); });
+                    [&](const CoopLaunch& cl) { return s->cks->step(cl, p); },
+                    [&](const CoopLaunch& cl, const CoopVaried& cv) { return s->cks->step_v(cl, p, cv); });
 }
 
 int project_launch(trepb_system* s, const trepb_project_args* a, void* stream, const trepb_varied* v) {
@@ -655,7 +696,8 @@ int project_launch(trepb_system* s, const trepb_project_args* a, void* stream, c
     p.times = a->times;
     return dispatch(s, 3, a->batch, (cudaStream_t)stream, v, nullptr,
                     [&](const KernelSet* ks, const LaunchCfg& c, const VariedArgs* va) { return ks->proj(c, p, va); },
-                    [&](const CoopLaunch& cl) { return s->cks->proj(cl, p); });
+                    [&](const CoopLaunch& cl) { return s->cks->proj(cl, p); },
+                    [&](const CoopLaunch& cl, const CoopVaried& cv) { return s->cks->proj_v(cl, p, cv); });
 }
 
 // calc_p2 / calc_f / discrete_fm2 share one kernel (P2Params::mode); the caller has validated the pointers
@@ -665,7 +707,8 @@ int eval_launch(trepb_system* s, const P2Params& p, void* stream, const trepb_va
     CU(cudaSetDevice(s->device));
     return dispatch(s, 1, p.batch, (cudaStream_t)stream, v, nullptr,
                     [&](const KernelSet* ks, const LaunchCfg& c, const VariedArgs* va) { return ks->p2(c, p, va); },
-                    [&](const CoopLaunch& cl) { return s->cks->p2(cl, p); });
+                    [&](const CoopLaunch& cl) { return s->cks->p2(cl, p); },
+                    [&](const CoopLaunch& cl, const CoopVaried& cv) { return s->cks->p2_v(cl, p, cv); });
 }
 
 int calc_p2_dev(trepb_system* s, int64_t batch, double dt, const double* q0, const double* q1, double* pout,
@@ -736,6 +779,11 @@ int lin_launch(trepb_system* s, const trepb_lin_args* a, cudaStream_t stream, do
                         AuxLayout al;
                         al.set(ps.nd, ps.nc);
                         return s->cks->lin(cl, p, al);
+                    },
+                    [&](const CoopLaunch& cl, const CoopVaried& cv) {
+                        AuxLayout al;
+                        al.set(ps.nd, ps.nc);
+                        return s->cks->lin_v(cl, p, al, cv);
                     }, vset);
 }
 

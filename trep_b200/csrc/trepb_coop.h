@@ -34,6 +34,18 @@ struct CoopLaunch {
     double* ext;            // external slabs, grid x warps x lay.xtotal doubles (linearize kernels of ext flavours), or null
 };
 
+// What a varied launch (TREPB_FLAG_COOP_VARIED) hands the cooperative kernels besides their usual parameters.  Every
+// team of the persistent grid owns a slot of `scratch`: a copy of the blob whose numeric tables it re-evaluates from
+// its instance's row (coop_eval_level / coop_eval_tables, trepb_coop_sys.h) whenever the row changes, followed by the
+// frame poses of that evaluation.  The team's view of the system points at the slot instead of the shared-memory copy.
+struct CoopVaried {
+    VariedMap map;          // the table-driven layout (trepb_varied.h, slots = false)
+    const double* values;   // [rows][map.n]
+    CoopPlanView plan;      // device pointers
+    double* scratch;        // [grid x teams][per_team]
+    long per_team;          // doubles: blob (rounded up to an even count) + 12 x frames
+};
+
 // One set per size flavour: run-time sizes ("cooperative") or a CtDims instantiation that serves
 // every system of that shape (e.g. "cooperative/puppet").
 struct CoopKernelSet {
@@ -50,6 +62,11 @@ struct CoopKernelSet {
     cudaError_t (*lin)(const CoopLaunch&, const LinParams&, const AuxLayout&);
     cudaError_t (*proj)(const CoopLaunch&, const ProjParams&);
     cudaError_t (*info)(int which, KernelInfo*);   // 0 step, 1 p2, 2 lin, 3 project
+    // per-instance parameters: the *_varied_kernel instantiations of the same flavour and width
+    cudaError_t (*step_v)(const CoopLaunch&, const StepParams&, const CoopVaried&);
+    cudaError_t (*p2_v)(const CoopLaunch&, const P2Params&, const CoopVaried&);
+    cudaError_t (*lin_v)(const CoopLaunch&, const LinParams&, const AuxLayout&, const CoopVaried&);
+    cudaError_t (*proj_v)(const CoopLaunch&, const ProjParams&, const CoopVaried&);
 };
 
 struct CoopRegistry {
@@ -61,7 +78,7 @@ CoopRegistry& coop_registry();
 // layout fingerprint of what a cooperative specialisation unit shares with the library (see kSpecAbi)
 constexpr unsigned kCoopAbi = 0x20000u + (unsigned)(sizeof(CoopSys) * 131 + sizeof(CoopLayout) * 31 + sizeof(CoopLaunch) * 17 +
                                                     sizeof(CoopKernelSet) * 13 + sizeof(StepParams) * 7 + sizeof(LinParams) * 5 +
-                                                    sizeof(ProjParams) * 3 + sizeof(P2Params));
+                                                    sizeof(ProjParams) * 3 + sizeof(P2Params) + sizeof(CoopVaried) * 11);
 bool coop_register(const CoopKernelSet* ks, unsigned abi);
 struct CoopRegistrar {
     explicit CoopRegistrar(const CoopKernelSet* ks) { coop_register(ks, kCoopAbi); }

@@ -85,15 +85,62 @@ __device__ __forceinline__ Stage coop_stage(const CoopSys& gs, int blob_bytes, c
     return st;
 }
 
-template <class D, class Team, int TEAMS>
-__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
-coop_step_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const StepParams p, double* __restrict__ ext) {
+// Varied flavours (CoopVaried): the team's copy of the blob in its slot of scratch, the team's view of the system
+// (grav: its row's) and the row whose numbers the copy holds.  The integer tables are copied once per launch, the
+// numeric ones re-evaluated only when the team's row changes.
+struct TeamTables {
+    CoopSys S;
+    double* fx;
+    long row;
+};
+
+template <class Team>
+__device__ __forceinline__ void varied_init(TeamTables& tt, const Stage& st, int blob_bytes, const CoopVaried& v, const Team& tm) {
+    const long g = (long)blockIdx.x * (blockDim.x / Team::kSize) + team_index<Team>();
+    double* slot = v.scratch + g * v.per_team;
+    const int n8 = (blob_bytes + 7) / 8;
+    const double* src = (const double*)st.S.base;
+    for (int i = tm.lane(); i < n8; i += Team::kSize) slot[i] = src[i];
+    tt.S = st.S;
+    tt.S.base = (const char*)slot;
+    tt.fx = slot + ((n8 + 1) & ~1);
+    tt.row = -1;
+}
+
+// Points the team's tables at row r (the whole team calls it; the barriers order the slot's writes and reads).
+template <class Team>
+__device__ __forceinline__ void varied_row(TeamTables& tt, const CoopVaried& v, long r, const Team& tm) {
+    if (r == tt.row) return;
+    tm.sync();
+    const VariedX x{v.map, v.values + r * v.map.n};
+    for (int L = 0; L < v.plan.nlev; ++L) {
+        coop_eval_level(v.plan, x, tt.fx, L, tm.lane(), Team::kSize);
+        tm.sync();
+    }
+    coop_eval_tables(v.plan, x, tt.fx, (double*)tt.S.base, tm.lane(), Team::kSize);
+    for (int k = 0; k < 3; ++k) tt.S.grav[k] = x(v.plan.xg + k);
+    tt.row = r;
+    tm.sync();
+}
+
+template <bool kVaried>
+__device__ __forceinline__ const CoopSys& team_sys(const Stage& st, const TeamTables& tt) {
+    if constexpr (kVaried) return tt.S;
+    else return st.S;
+}
+
+template <class D, class Team, int TEAMS, bool kVaried>
+__device__ __forceinline__ void
+coop_step_body(const CoopSys& gs, const int blob_bytes, const CoopLayout& lay_, const StepParams& p, double* __restrict__ ext,
+               const CoopVaried* v) {
     CoopLayout lay = lay_;
     if constexpr (D::kStatic) lay = static_layout<D>(gs, true);
     Stage st = coop_stage<Team>(gs, blob_bytes, lay);
-    const CoopSys& S = st.S;
-    double* w = st.w;
     const Team tm = make_team<Team>();
+    TeamTables tt;
+    if constexpr (kVaried) varied_init(tt, st, blob_bytes, *v, tm);
+    const CoopSys& S = team_sys<kVaried>(st, tt);
+    double* w = st.w;
     constexpr int TS = Team::kSize;
     Coop<Team, D> c(S, lay, w, tm, team_slab<D, Team>(ext, lay));
     const int lane = tm.lane(), wpc = blockDim.x / TS;
@@ -103,6 +150,7 @@ coop_step_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, 
         const long b = b0 + team_index<Team>();
         const bool live = b < p.batch;
         if (live) {
+            if constexpr (kVaried) varied_row(tt, *v, b, tm);
             for (int i = lane; i < nq; i += TS) {
                 const double v = p.q1[b * nq + i];
                 w[lay.q1 + i] = v;
@@ -154,18 +202,33 @@ coop_step_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, 
     }
 }
 
+template <class D, class Team, int TEAMS>
+__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
+coop_step_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const StepParams p, double* __restrict__ ext) {
+    coop_step_body<D, Team, TEAMS, false>(gs, blob_bytes, lay_, p, ext, nullptr);
+}
+template <class D, class Team, int TEAMS>
+__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
+coop_step_varied_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const StepParams p, double* __restrict__ ext,
+                        const CoopVaried v) {
+    coop_step_body<D, Team, TEAMS, true>(gs, blob_bytes, lay_, p, ext, &v);
+}
+
 // DSystem.project / armijo_simulate (trep/discopt/dsystem.py:426-457): closed-loop rollouts, one warp per
 // candidate, the affine feedback U[k] = bU[k] - K[k](X[k] - bX[k]) evaluated by the lanes (one input
 // component each) inside the time loop.
-template <class D, class Team, int TEAMS>
-__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
-coop_project_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const ProjParams p, double* __restrict__ ext) {
+template <class D, class Team, int TEAMS, bool kVaried>
+__device__ __forceinline__ void
+coop_project_body(const CoopSys& gs, const int blob_bytes, const CoopLayout& lay_, const ProjParams& p, double* __restrict__ ext,
+                  const CoopVaried* v) {
     CoopLayout lay = lay_;
     if constexpr (D::kStatic) lay = static_layout<D>(gs, true);
     Stage st = coop_stage<Team>(gs, blob_bytes, lay);
-    const CoopSys& S = st.S;
-    double* w = st.w;
     const Team tm = make_team<Team>();
+    TeamTables tt;
+    if constexpr (kVaried) varied_init(tt, st, blob_bytes, *v, tm);
+    const CoopSys& S = team_sys<kVaried>(st, tt);
+    double* w = st.w;
     constexpr int TS = Team::kSize;
     Coop<Team, D> c(S, lay, w, tm, team_slab<D, Team>(ext, lay));
     const int lane = tm.lane(), wpc = blockDim.x / TS;
@@ -180,6 +243,7 @@ coop_project_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay
         double* Xo = p.X + b * (long)(K + 1) * nX;
         double* Uo = p.U + b * (long)K * nU;
         if (live) {
+            if constexpr (kVaried) varied_row(tt, *v, b, tm);
             for (int i = lane; i < nq; i += TS) { const double v = bX[i]; w[lay.q2 + i] = v; Xo[i] = v; }
             for (int i = lane; i < nd; i += TS) { const double v = bX[nq + i]; w[lay.p2 + i] = v; Xo[nq + i] = v; }
             for (int i = lane; i < nk; i += TS) { const double v = bX[nq + nd + i]; w[lay.vk + i] = v; Xo[nq + nd + i] = v; }
@@ -235,18 +299,34 @@ coop_project_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay
 
 template <class D, class Team, int TEAMS>
 __global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
-coop_p2_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const P2Params p, double* __restrict__ ext) {
+coop_project_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const ProjParams p, double* __restrict__ ext) {
+    coop_project_body<D, Team, TEAMS, false>(gs, blob_bytes, lay_, p, ext, nullptr);
+}
+template <class D, class Team, int TEAMS>
+__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
+coop_project_varied_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const ProjParams p,
+                           double* __restrict__ ext, const CoopVaried v) {
+    coop_project_body<D, Team, TEAMS, true>(gs, blob_bytes, lay_, p, ext, &v);
+}
+
+template <class D, class Team, int TEAMS, bool kVaried>
+__device__ __forceinline__ void
+coop_p2_body(const CoopSys& gs, const int blob_bytes, const CoopLayout& lay_, const P2Params& p, double* __restrict__ ext,
+             const CoopVaried* v) {
     CoopLayout lay = lay_;
     if constexpr (D::kStatic) lay = static_layout<D>(gs, true);
     Stage st = coop_stage<Team>(gs, blob_bytes, lay);
-    const CoopSys& S = st.S;
-    double* w = st.w;
     const Team tm = make_team<Team>();
+    TeamTables tt;
+    if constexpr (kVaried) varied_init(tt, st, blob_bytes, *v, tm);
+    const CoopSys& S = team_sys<kVaried>(st, tt);
+    double* w = st.w;
     constexpr int TS = Team::kSize;
     Coop<Team, D> c(S, lay, w, tm, team_slab<D, Team>(ext, lay));
     const int lane = tm.lane(), wpc = blockDim.x / TS;
     const int nd = c.ND(), nq = c.NQ(), nu = c.NU(), nc = c.NC();
     for (long b = (long)blockIdx.x * wpc + team_index<Team>(); b < p.batch; b += (long)gridDim.x * wpc) {
+        if constexpr (kVaried) varied_row(tt, *v, b, tm);
         for (int i = lane; i < nq; i += TS) {
             w[lay.q1 + i] = p.q0[b * nq + i];
             w[lay.q2 + i] = p.q1[b * nq + i];
@@ -273,14 +353,28 @@ coop_p2_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, co
 
 template <class D, class Team, int TEAMS>
 __global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
-coop_lin_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const LinParams p, const AuxLayout al,
-                double* __restrict__ ext) {
+coop_p2_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const P2Params p, double* __restrict__ ext) {
+    coop_p2_body<D, Team, TEAMS, false>(gs, blob_bytes, lay_, p, ext, nullptr);
+}
+template <class D, class Team, int TEAMS>
+__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
+coop_p2_varied_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const P2Params p, double* __restrict__ ext,
+                      const CoopVaried v) {
+    coop_p2_body<D, Team, TEAMS, true>(gs, blob_bytes, lay_, p, ext, &v);
+}
+
+template <class D, class Team, int TEAMS, bool kVaried>
+__device__ __forceinline__ void
+coop_lin_body(const CoopSys& gs, const int blob_bytes, const CoopLayout& lay_, const LinParams& p, const AuxLayout& al,
+              double* __restrict__ ext, const CoopVaried* v) {
     CoopLayout lay = lay_;
     if constexpr (D::kStatic) lay = static_layout<D>(gs, false);
     Stage st = coop_stage<Team>(gs, blob_bytes, lay);
-    const CoopSys& S = st.S;
-    double* w = st.w;
     const Team tm = make_team<Team>();
+    TeamTables tt;
+    if constexpr (kVaried) varied_init(tt, st, blob_bytes, *v, tm);
+    const CoopSys& S = team_sys<kVaried>(st, tt);
+    double* w = st.w;
     constexpr int TS = Team::kSize;
     Coop<Team, D> c(S, lay, w, tm, team_slab<D, Team>(ext, lay));
     const int lane = tm.lane(), wpc = blockDim.x / TS;
@@ -295,6 +389,7 @@ coop_lin_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, c
     for (long b0 = (long)blockIdx.x * wpc; b0 < p.batch; b0 += (long)gridDim.x * wpc, TREPB_LOCKSTEP()) {
         const long b = b0 + team_index<Team>();
         if (b >= p.batch) continue;
+        if constexpr (kVaried) varied_row(tt, *v, p.traj_len > 1 ? b / (p.traj_len - 1) : b, tm);
         const long r = p.traj_len > 1 ? b + b / (p.traj_len - 1) : b;   // state row (trepb_lin_args.traj_len)
         for (int i = lane; i < nq; i += TS) {
             const double v = p.q1[r * nq + i];
@@ -339,6 +434,19 @@ coop_lin_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, c
         }
         tm.sync();
     }
+}
+
+template <class D, class Team, int TEAMS>
+__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
+coop_lin_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const LinParams p, const AuxLayout al,
+                double* __restrict__ ext) {
+    coop_lin_body<D, Team, TEAMS, false>(gs, blob_bytes, lay_, p, al, ext, nullptr);
+}
+template <class D, class Team, int TEAMS>
+__global__ void __launch_bounds__(TEAMS * Team::kSize, 1)
+coop_lin_varied_kernel(const CoopSys gs, const int blob_bytes, const CoopLayout lay_, const LinParams p, const AuxLayout al,
+                       double* __restrict__ ext, const CoopVaried v) {
+    coop_lin_body<D, Team, TEAMS, true>(gs, blob_bytes, lay_, p, al, ext, &v);
 }
 
 template <class K>
@@ -411,6 +519,34 @@ struct Launch {
         coop_project_kernel<typename D::Solve, WarpTeam, kSolve><<<c.grid, 32 * c.warps, c.smem, c.stream>>>(c.sys, c.blob_bytes, c.lay, p, c.ext);
         return cudaGetLastError();
     }
+    template <class K, class... A>
+    static cudaError_t go(K kernel, const CoopLaunch& c, int threads, const A&... args) {
+        cudaError_t e = prep(kernel, c.smem);
+        if (e != cudaSuccess) return e;
+        kernel<<<c.grid, threads, c.smem, c.stream>>>(args...);
+        return cudaGetLastError();
+    }
+    // per-instance parameters: the varied instantiations, selected as above
+    static cudaError_t step_v(const CoopLaunch& c, const StepParams& p, const CoopVaried& v) {
+        if constexpr (kWide) if (c.warps > kSolve)
+            return go(coop_step_varied_kernel<typename D::Solve, WarpTeam, kWideTeams>, c, 32 * c.warps, c.sys, c.blob_bytes, c.lay, p, c.ext, v);
+        return go(coop_step_varied_kernel<typename D::Solve, WarpTeam, kSolve>, c, 32 * c.warps, c.sys, c.blob_bytes, c.lay, p, c.ext, v);
+    }
+    static cudaError_t p2_v(const CoopLaunch& c, const P2Params& p, const CoopVaried& v) {
+        if constexpr (kWide) if (c.warps > kSolve)
+            return go(coop_p2_varied_kernel<typename D::Solve, WarpTeam, kWideTeams>, c, 32 * c.warps, c.sys, c.blob_bytes, c.lay, p, c.ext, v);
+        return go(coop_p2_varied_kernel<typename D::Solve, WarpTeam, kSolve>, c, 32 * c.warps, c.sys, c.blob_bytes, c.lay, p, c.ext, v);
+    }
+    static cudaError_t lin_v(const CoopLaunch& c, const LinParams& p, const AuxLayout& al, const CoopVaried& v) {
+        if constexpr (kWide) if (c.warps > kLin)
+            return go(coop_lin_varied_kernel<D, Team, kWideTeams>, c, Team::kSize * c.warps, c.sys, c.blob_bytes, c.lay, p, al, c.ext, v);
+        return go(coop_lin_varied_kernel<D, Team, kLin>, c, Team::kSize * c.warps, c.sys, c.blob_bytes, c.lay, p, al, c.ext, v);
+    }
+    static cudaError_t proj_v(const CoopLaunch& c, const ProjParams& p, const CoopVaried& v) {
+        if constexpr (kWide) if (c.warps > kSolve)
+            return go(coop_project_varied_kernel<typename D::Solve, WarpTeam, kWideTeams>, c, 32 * c.warps, c.sys, c.blob_bytes, c.lay, p, c.ext, v);
+        return go(coop_project_varied_kernel<typename D::Solve, WarpTeam, kSolve>, c, 32 * c.warps, c.sys, c.blob_bytes, c.lay, p, c.ext, v);
+    }
     // which: 0 step, 1 p2, 2 lin, 3 project; + 4 for the wide instantiation
     static cudaError_t info(int which, KernelInfo* ki) {
         const void* fn = nullptr;
@@ -460,6 +596,10 @@ CoopKernelSet make_coop_kernelset(const char* name) {
     k.lin = &coopk::Launch<D, Team>::lin;
     k.proj = &coopk::Launch<D, Team>::proj;
     k.info = &coopk::Launch<D, Team>::info;
+    k.step_v = &coopk::Launch<D, Team>::step_v;
+    k.p2_v = &coopk::Launch<D, Team>::p2_v;
+    k.lin_v = &coopk::Launch<D, Team>::lin_v;
+    k.proj_v = &coopk::Launch<D, Team>::proj_v;
     return k;
 }
 

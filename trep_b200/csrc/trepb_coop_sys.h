@@ -25,6 +25,7 @@
 #include <vector>
 #include "../../include/trepb.h"
 #include "trepb_sys.h"
+#include "trepb_varied.h"
 
 namespace trepb {
 
@@ -177,12 +178,171 @@ struct CoopSys {
     TREPB_HD bool wrl(int l) const { return (l_kind()[l] & 32) != 0; }
 };
 
+// ---- the numeric part of the condensation
+// coop_pack is a host-only PLAN - the topology, and which numbers of the description feed which numeric entry of the
+// blob, in which order - followed by coop_eval_level / coop_eval_tables, which evaluate those entries from the plan
+// and one numeric vector of the description: the table-driven kernels' expansion of a row (trepb_varied.h,
+// slots = false: the numeric region of the packed blob, then grav[3]).  coop_pack runs them on the description's own
+// vector; the varied cooperative kernels (TREPB_FLAG_COOP_VARIED) run them on a team's copy of the blob for the
+// team's row.  The integer tables depend on structure only, which a varied entry never changes (varied_check).
+//
+// Every product and sum is rounded on its own, in the order the host evaluates it (x86-64 does not contract
+// `a * b + c`; nvcc would, into an FMA), and every sum runs over its terms in ascending order, so the device gives
+// the host's bits.  The one exception is cos / sin of a constant rotation frame's angle (K_RX .. K_RZ): the device
+// math library and the C library may differ in the last bit.
+TREPB_HD double cp_mul(double a, double b) {
+#if defined(__CUDA_ARCH__)
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+TREPB_HD double cp_add(double a, double b) {
+#if defined(__CUDA_ARCH__)
+    return __dadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+
+// The plan: sizes, indices and integer lists (one relocatable int32 array, like the blob).
+struct CoopPlanView {
+    int nlev;                            // depth levels of the frame tree
+    int nl, np, nplane, nw, ncp, nsum;
+    int xv, xs, xm, xg;                  // index in the numeric vector of frame_value[0], frame_se3[0], frame_mass[0], grav[0]
+    int dRc, dpc, din, dpt, dcn, dwr;    // index (in doubles) in the blob of l_Rc, l_pc, l_in, pt_r, con_n, wr_d
+    const int32_t* fr;       // [nf][3] every frame, level by level: frame, parent, kind (-1: identity - the world or a
+                             // variable frame, whose link coordinates start at itself)
+    const int32_t* fr_off;   // [nlev + 1]
+    const int32_t* lk;       // [nl] the frame whose pose is link l's constant pre-transform (the parent of its frame)
+    const int32_t* ms_off;   // [nl + 1] / ms: the frames whose masses sum into link l's inertia, ascending
+    const int32_t* ms;
+    const int32_t* pt;       // [np] frame of each point
+    const int32_t* pl;       // [nplane][3] PointOnPlane constraint, plane frame, numeric index of its con_d[4 c]
+    const int32_t* wr;       // [nw] frame of each wrench
+    const int32_t* cp;       // [ncp][2] blob index <- numeric index
+    const int32_t* sum_off;  // [nsum + 1], sum_dst [nsum], sum_t [][2]: blob index <- 0 + x[a] (b < 0) or x[a] * x[b] + ...
+    const int32_t* sum_dst;
+    const int32_t* sum_t;
+};
+
+// fx[12 f]: the pose of frame f in the coordinates of its link (of the world for a frame fixed in it), R row-major
+// then p.  Level L of the frame tree; levels in order, each after the previous one is complete.
+template <class X>
+TREPB_HD void coop_eval_level(const CoopPlanView& pl, const X& x, double* fx, int L, int lane, int nlanes) {
+    for (int i = pl.fr_off[L] + lane; i < pl.fr_off[L + 1]; i += nlanes) {
+        const int f = pl.fr[3 * i], kind = pl.fr[3 * i + 2];
+        double* o = fx + 12 * f;
+        // local transform of a constant frame (trep/_trep/frame.c:839-1076)
+        double b[12];
+        for (int k = 0; k < 12; ++k) b[k] = (k < 9 && k % 4 == 0) ? 1.0 : 0.0;
+        if (kind < 0) {
+            for (int k = 0; k < 12; ++k) o[k] = b[k];
+            continue;
+        }
+        if (kind == K_CONST_SE3) {
+            for (int r = 0; r < 3; ++r) {
+                for (int c = 0; c < 3; ++c) b[r * 3 + c] = x(pl.xs + 12 * f + r * 4 + c);
+                b[9 + r] = x(pl.xs + 12 * f + r * 4 + 3);
+            }
+        } else if (kind >= K_TX && kind <= K_TZ) {
+            b[9 + kind - K_TX] = x(pl.xv + f);
+        } else if (kind >= K_RX && kind <= K_RZ) {
+            const int a = kind - K_RX, bb = (a + 1) % 3, c = (a + 2) % 3;
+            const double v = x(pl.xv + f), cs = cos(v), sn = sin(v);
+            b[bb * 3 + bb] = cs; b[bb * 3 + c] = -sn;
+            b[c * 3 + bb] = sn; b[c * 3 + c] = cs;
+        }
+        // parent then the local transform
+        const double* a = fx + 12 * pl.fr[3 * i + 1];
+        for (int r = 0; r < 3; ++r) {
+            for (int c = 0; c < 3; ++c)
+                o[r * 3 + c] = cp_add(cp_add(cp_mul(a[r * 3], b[c]), cp_mul(a[r * 3 + 1], b[3 + c])), cp_mul(a[r * 3 + 2], b[6 + c]));
+            o[9 + r] = cp_add(cp_add(cp_add(a[9 + r], cp_mul(a[r * 3], b[9])), cp_mul(a[r * 3 + 1], b[10])), cp_mul(a[r * 3 + 2], b[11]));
+        }
+    }
+}
+
+// Every numeric entry of the blob from the frame poses and the numeric vector; lanes split the destinations.
+template <class X>
+TREPB_HD void coop_eval_tables(const CoopPlanView& pl, const X& x, const double* fx, double* blob, int lane, int nlanes) {
+    for (int l = lane; l < pl.nl; l += nlanes) {
+        const double* xc = fx + 12 * pl.lk[l];
+        for (int k = 0; k < 9; ++k) blob[pl.dRc + 9 * l + k] = xc[k];
+        for (int k = 0; k < 3; ++k) blob[pl.dpc + 3 * l + k] = xc[9 + k];
+        // masses -> link inertia (about the link origin, link axes): m, h = m c, R diag(Ixx, Iyy, Izz) R^T + m (|p|^2 1 - p p^T)
+        double I[10];
+        for (int k = 0; k < 10; ++k) I[k] = 0.0;
+        for (int j = pl.ms_off[l]; j < pl.ms_off[l + 1]; ++j) {
+            const int f = pl.ms[j];
+            const double* R = fx + 12 * f;
+            const double* p = R + 9;
+            const double m = x(pl.xm + 4 * f);
+            I[0] = cp_add(I[0], m);
+            for (int k = 0; k < 3; ++k) I[1 + k] = cp_add(I[1 + k], cp_mul(m, p[k]));
+            const double pp = cp_add(cp_add(cp_mul(p[0], p[0]), cp_mul(p[1], p[1])), cp_mul(p[2], p[2]));
+            const int rr[6] = {0, 1, 2, 0, 0, 1}, cc[6] = {0, 1, 2, 1, 2, 2};
+            for (int e = 0; e < 6; ++e) {
+                const int r = rr[e], c = cc[e];
+                double v = 0.0;
+                for (int k = 0; k < 3; ++k) v = cp_add(v, cp_mul(cp_mul(R[r * 3 + k], x(pl.xm + 4 * f + 1 + k)), R[c * 3 + k]));
+                v = cp_add(v, cp_mul(cp_mul(-m, p[r]), p[c]));
+                if (r == c) v = cp_add(v, cp_mul(m, pp));
+                I[4 + e] = cp_add(I[4 + e], v);
+            }
+        }
+        for (int k = 0; k < 10; ++k) blob[pl.din + 10 * l + k] = I[k];
+    }
+    for (int i = lane; i < pl.np; i += nlanes)
+        for (int k = 0; k < 3; ++k) blob[pl.dpt + 3 * i + k] = fx[12 * pl.pt[i] + 9 + k];
+    // PointOnPlane: the normal, fixed in the plane frame, in the coordinates of the link the frame hangs on
+    for (int i = lane; i < pl.nplane; i += nlanes) {
+        const int c = pl.pl[3 * i], xn = pl.pl[3 * i + 2];
+        const double* R = fx + 12 * pl.pl[3 * i + 1];
+        const double n0 = x(xn), n1 = x(xn + 2), n2 = x(xn + 3);
+        for (int r = 0; r < 3; ++r)
+            blob[pl.dcn + 3 * c + r] = cp_add(cp_add(cp_mul(R[r * 3], n0), cp_mul(R[r * 3 + 1], n1)), cp_mul(R[r * 3 + 2], n2));
+    }
+    for (int i = lane; i < pl.nw; i += nlanes)
+        for (int k = 0; k < 9; ++k) blob[pl.dwr + 15 * i + 6 + k] = fx[12 * pl.wr[i] + k];
+    for (int i = lane; i < pl.ncp; i += nlanes) blob[pl.cp[2 * i]] = x(pl.cp[2 * i + 1]);
+    for (int i = lane; i < pl.nsum; i += nlanes) {
+        double v = 0.0;
+        for (int j = pl.sum_off[i]; j < pl.sum_off[i + 1]; ++j) {
+            const int a = pl.sum_t[2 * j], b = pl.sum_t[2 * j + 1];
+            v = cp_add(v, b < 0 ? x(a) : cp_mul(x(a), x(b)));
+        }
+        blob[pl.sum_dst[i]] = v;
+    }
+}
+
+// The numeric vector as an array (the host's).
+struct CoopXVec {
+    const double* v;
+    TREPB_HD double operator()(int i) const { return v[i]; }
+};
+
+struct CoopPlan {
+    std::vector<int32_t> ints;
+    CoopPlanView hdr;    // sizes and indices; view() fills the pointers
+    size_t o[12];        // offsets in ints of fr, fr_off, lk, ms_off, ms, pt, pl, wr, cp, sum_off, sum_dst, sum_t
+    int nf = 0;          // frames (the frame poses take 12 nf doubles)
+    CoopPlanView view(const int32_t* base) const {
+        CoopPlanView v = hdr;
+        const int32_t** p[12] = {&v.fr, &v.fr_off, &v.lk, &v.ms_off, &v.ms, &v.pt, &v.pl, &v.wr, &v.cp, &v.sum_off,
+                                 &v.sum_dst, &v.sum_t};
+        for (int k = 0; k < 12; ++k) *p[k] = base + o[k];
+        return v;
+    }
+};
+
 struct CoopPack {
     bool ok = false;
     std::string why;          // why the cooperative path does not apply
     std::vector<char> blob;
     CoopSys proto;
     size_t off[72];
+    CoopPlan plan;           // evaluates the numeric tables of the blob from a numeric vector of the description
 
     CoopSys view(const char* base) const {
         CoopSys s = proto;
@@ -233,75 +393,74 @@ struct CoopPack {
     }
 };
 
-namespace coop_detail {
-struct Se3 {
-    double R[9], p[3];
-};
-inline Se3 se3_identity() {
-    Se3 x;
-    for (int k = 0; k < 9; ++k) x.R[k] = (k % 4 == 0) ? 1.0 : 0.0;
-    x.p[0] = x.p[1] = x.p[2] = 0.0;
-    return x;
-}
-inline Se3 se3_mul(const Se3& a, const Se3& b) {  // a then b (b expressed in a's frame)
-    Se3 o;
-    for (int r = 0; r < 3; ++r) {
-        for (int c = 0; c < 3; ++c)
-            o.R[r * 3 + c] = a.R[r * 3] * b.R[c] + a.R[r * 3 + 1] * b.R[3 + c] + a.R[r * 3 + 2] * b.R[6 + c];
-        o.p[r] = a.p[r] + a.R[r * 3] * b.p[0] + a.R[r * 3 + 1] * b.p[1] + a.R[r * 3 + 2] * b.p[2];
-    }
-    return o;
-}
-// local transform of a constant frame (trep/_trep/frame.c:839-1076)
-inline Se3 se3_const_frame(int kind, double value, const double* se3) {
-    Se3 x = se3_identity();
-    if (kind == K_CONST_SE3) {
-        for (int r = 0; r < 3; ++r) {
-            for (int c = 0; c < 3; ++c) x.R[r * 3 + c] = se3[r * 4 + c];
-            x.p[r] = se3[r * 4 + 3];
-        }
-    } else if (kind >= K_TX && kind <= K_TZ) {
-        x.p[kind - K_TX] = value;
-    } else if (kind >= K_RX && kind <= K_RZ) {
-        const int a = kind - K_RX, b = (a + 1) % 3, c = (a + 2) % 3;
-        const double cs = cos(value), sn = sin(value);
-        x.R[b * 3 + b] = cs; x.R[b * 3 + c] = -sn;
-        x.R[c * 3 + b] = sn; x.R[c * 3 + c] = cs;
-    }
-    return x;
-}
-inline bool se3_is_identity(const Se3& x) {
-    for (int k = 0; k < 9; ++k) if (x.R[k] != ((k % 4 == 0) ? 1.0 : 0.0)) return false;
-    return x.p[0] == 0.0 && x.p[1] == 0.0 && x.p[2] == 0.0;
-}
-}  // namespace coop_detail
-
 // Builds the link-level tables.  Returns a pack with ok == false (and `why`) when the system uses
 // something the cooperative kernels do not implement (the thread-per-instance general kernels do).
+// P.plan evaluates the numeric tables for any numeric vector of the description (see above).
 inline CoopPack coop_pack(const trepb_sysdesc* d) {
-    using namespace coop_detail;
     CoopPack P;
     const int nf = d->n_frames, nd = d->nd, nk = d->nk, nq = nd + nk, nu = d->nu, nc = d->n_constraints;
     if (nq > 64) { P.why = "more than 64 configs"; return P; }
     for (int i = 0; i < d->n_forces; ++i)
         if (d->force_kind[i] == TREPB_FORCE_LINEAR_DAMPER && d->force_i[4 * i + 1] != 2) { P.why = "LinearDamper over more than one segment"; return P; }
+    // the description's numeric vector, laid out as the expansion of a row lays it out
+    std::vector<double> xv;
+    int toff[8];
+    {
+        PackedSys PS;
+        std::string err;
+        if (!pack_system(d, &PS, &err)) { P.why = err; return P; }
+        VariedHost H;
+        varied_map(PS, 0, nullptr, nullptr, false, &H);
+        xv = H.base;
+        for (int k = 0; k < 8; ++k) toff[k] = H.toff[k];
+    }
+    const CoopXVec X{xv.data()};
+    CoopPlan& PL = P.plan;
+    PL.nf = nf;
+    CoopPlanView& hd = PL.hdr;
+    memset(&hd, 0, sizeof(hd));
+    hd.xv = toff[0]; hd.xs = toff[1]; hd.xm = toff[2]; hd.xg = toff[7];
 
     // ---- frames -> links
     std::vector<int> flink(nf, -1);      // frame -> frame index of the link it belongs to (-1: world)
-    std::vector<Se3> fx(nf);             // frame pose in its link's coordinates (world coordinates when flink == -1)
     std::vector<int> lframes;            // variable frames in pre-order
-    fx[0] = se3_identity();
+    std::vector<int> fdepth(nf, 0);
+    int nfl = 1;
     for (int f = 1; f < nf; ++f) {
         const int par = d->frame_parent[f];
+        fdepth[f] = fdepth[par] + 1;
+        if (fdepth[f] + 1 > nfl) nfl = fdepth[f] + 1;
         if (d->frame_config[f] >= 0) {
             flink[f] = f;
-            fx[f] = se3_identity();
             lframes.push_back(f);
         } else {
             flink[f] = flink[par];
-            fx[f] = se3_mul(fx[par], se3_const_frame(d->frame_kind[f], d->frame_value[f], d->frame_se3 + 12 * f));
         }
     }
+    // frame poses in their links' coordinates, level by level of the frame tree
+    std::vector<int32_t> fr, fr_off;
+    for (int L = 0; L < nfl; ++L) {
+        fr_off.push_back((int32_t)(fr.size() / 3));
+        for (int f = 0; f < nf; ++f) {
+            if (fdepth[f] != L) continue;
+            fr.push_back(f);
+            fr.push_back(f == 0 ? 0 : d->frame_parent[f]);
+            fr.push_back(f == 0 || d->frame_config[f] >= 0 ? -1 : d->frame_kind[f]);
+        }
+    }
+    fr_off.push_back((int32_t)(fr.size() / 3));
+    hd.nlev = nfl;
+    std::vector<double> fxv((size_t)12 * nf);
+    {
+        CoopPlanView fv = hd;
+        fv.fr = fr.data(); fv.fr_off = fr_off.data();
+        for (int L = 0; L < nfl; ++L) coop_eval_level(fv, X, fxv.data(), L, 0, 1);
+    }
+    auto fx_identity = [&](int f) {
+        const double* x = &fxv[(size_t)12 * f];
+        for (int k = 0; k < 9; ++k) if (x[k] != ((k % 4 == 0) ? 1.0 : 0.0)) return false;
+        return x[9] == 0.0 && x[10] == 0.0 && x[11] == 0.0;
+    };
     const int nl = (int)lframes.size();
     if (nl < 1) { P.why = "no variable frame"; return P; }
     if (nl > 64) { P.why = "more than 64 variable frames"; return P; }
@@ -330,22 +489,28 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
     }
     lvl_off[nlevels] = (int32_t)order.size();
 
+    // numeric entries: (table of the blob in put order, element) <- one numeric-vector entry, or a sum of terms
+    struct Dst { int tab, pos; };
+    std::vector<std::pair<Dst, int>> copies;
+    std::vector<std::pair<Dst, std::vector<std::pair<int, int>>>> sums;
+    enum { T_DAMP = 11, T_KS = 12, T_KQ0 = 13, T_CON_DIST = 23, T_CON_TOL = 24, T_SP_K = 37, T_SP_X0 = 38, T_DA_C = 45,
+           T_NSP_D = 51, T_NSP_TAB = 52, T_WR_D = 54 };
+    const int xpot = toff[3], xforce = toff[4], xcon = toff[5], xpool = toff[6];
+
     std::vector<int32_t> l_par(nl), l_cfg(nl), l_kind(nl), l_child0(nl, 0), l_nchild(nl, 0);
-    std::vector<double> l_Rc(9 * nl), l_pc(3 * nl), l_in(10 * nl, 0.0);
+    std::vector<double> l_Rc(9 * nl, 0.0), l_pc(3 * nl, 0.0), l_in(10 * nl, 0.0);
     std::vector<uint64_t> l_anc(nl, 0);
-    std::vector<int32_t> cfg_link(nq > 0 ? nq : 1, -1);
+    std::vector<int32_t> cfg_link(nq > 0 ? nq : 1, -1), lk(nl);
     for (int l = 0; l < nl; ++l) {
         const int f = order[l];
         const int kind = d->frame_kind[f];
         l_par[l] = fpl[f] < 0 ? -1 : newidx[fpl[f]];
         l_cfg[l] = d->frame_config[f];
         cfg_link[l_cfg[l]] = l;
-        const Se3 xc = fx[d->frame_parent[f]];
+        lk[l] = d->frame_parent[f];
         int kbits = (kind >= K_RX ? (kind - K_RX) | 4 : (kind - K_TX));
-        if (!se3_is_identity(xc)) kbits |= 8;
+        if (!fx_identity(lk[l])) kbits |= 8;
         l_kind[l] = kbits;
-        for (int k = 0; k < 9; ++k) l_Rc[9 * l + k] = xc.R[k];
-        for (int k = 0; k < 3; ++k) l_pc[3 * l + k] = xc.p[k];
         l_anc[l] = (l_par[l] < 0 ? 0ull : l_anc[l_par[l]]) | (1ull << l);
     }
     for (int l = nl - 1; l >= 0; --l)
@@ -376,28 +541,14 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
         sl_off.push_back((int32_t)sl_head.size());
     }
 
-    // ---- masses -> link inertia (about the link origin, link axes)
+    // ---- masses -> link inertia: which frames, in ascending order
+    std::vector<std::vector<int32_t>> lmass(nl);
     for (int f = 1; f < nf; ++f) {
         const double* mm = d->frame_mass + 4 * f;
         if (mm[0] == 0.0 && mm[1] == 0.0 && mm[2] == 0.0 && mm[3] == 0.0) continue;
         if (flink[f] < 0) continue;  // fixed in the world: contributes nothing to the dynamics
         const int l = newidx[flink[f]];
-        const Se3& x = fx[f];
-        double* I = &l_in[10 * l];
-        const double m = mm[0];
-        I[0] += m;
-        for (int k = 0; k < 3; ++k) I[1 + k] += m * x.p[k];
-        // R diag(Ixx,Iyy,Izz) R^T + m (|p|^2 1 - p p^T)
-        const double pp = x.p[0] * x.p[0] + x.p[1] * x.p[1] + x.p[2] * x.p[2];
-        const int rr[6] = {0, 1, 2, 0, 0, 1}, cc[6] = {0, 1, 2, 1, 2, 2};
-        for (int e = 0; e < 6; ++e) {
-            const int r = rr[e], c = cc[e];
-            double v = 0.0;
-            for (int k = 0; k < 3; ++k) v += x.R[r * 3 + k] * mm[1 + k] * x.R[c * 3 + k];
-            v += -m * x.p[r] * x.p[c];
-            if (r == c) v += m * pp;
-            I[4 + e] += v;
-        }
+        lmass[l].push_back(f);
         for (int a = l; a >= 0; a = l_par[a]) l_kind[a] |= 16;
     }
 
@@ -412,29 +563,28 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
         pt_frame.push_back(f);
         const int l = flink[f] < 0 ? -1 : newidx[flink[f]];
         pt_link.push_back(l);
-        for (int k = 0; k < 3; ++k) pt_r.push_back(fx[f].p[k]);
+        for (int k = 0; k < 3; ++k) pt_r.push_back(0.0);
         for (int a = l; a >= 0; a = l_par[a]) l_kind[a] |= bit;
         return (int)pt_frame.size() - 1;
     };
     std::vector<int32_t> con_kind(nc > 0 ? nc : 1), con_a(nc > 0 ? nc : 1), con_b(nc > 0 ? nc : 1), con_third(nc > 0 ? nc : 1);
-    std::vector<double> con_dist(nc > 0 ? nc : 1), con_tol(nc > 0 ? nc : 1);
+    std::vector<double> con_dist(nc > 0 ? nc : 1, 0.0), con_tol(nc > 0 ? nc : 1, 0.0);
     std::vector<uint64_t> con_dep(nc > 0 ? nc : 1, 0);
     std::vector<double> con_n(nc > 0 ? 3 * nc : 3, 0.0);
+    std::vector<int32_t> planes;
     for (int c = 0; c < nc; ++c) {
         const int32_t* ii = d->con_i + 4 * c;
         con_kind[c] = d->con_kind[c];
         con_a[c] = point_of(ii[0]);
         con_b[c] = point_of(ii[1]);
         con_third[c] = ii[2];
-        con_dist[c] = d->con_d[4 * c];
-        con_tol[c] = d->con_d[4 * c + 1];
+        copies.push_back({{T_CON_TOL, c}, xcon + 4 * c + 1});
         if (con_kind[c] == TREPB_CON_PLANE) {
-            // normal fixed in the plane frame -> coordinates of the link the frame hangs on
-            const double n[3] = {d->con_d[4 * c], d->con_d[4 * c + 2], d->con_d[4 * c + 3]};
-            const Se3& x = fx[ii[0]];
-            for (int r = 0; r < 3; ++r) con_n[3 * c + r] = x.R[r * 3] * n[0] + x.R[r * 3 + 1] * n[1] + x.R[r * 3 + 2] * n[2];
+            // normal (con_d[0], con_d[2], con_d[3]) fixed in the plane frame; distance 0
+            planes.push_back(c); planes.push_back(ii[0]); planes.push_back(xcon + 4 * c);
             con_third[c] = -1;
-            con_dist[c] = 0.0;
+        } else {
+            copies.push_back({{T_CON_DIST, c}, xcon + 4 * c});
         }
         uint64_t m = 0;
         for (int e = 0; e < 2; ++e) {
@@ -455,8 +605,10 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
         for (int i = 0; i < d->n_potentials; ++i) {
             if (d->pot_kind[i] != TREPB_POT_LINEAR_SPRING) continue;
             const int a = point_of(d->pot_i[4 * i], (size_t)npc, 64), b = point_of(d->pot_i[4 * i + 1], (size_t)npc, 64);
+            copies.push_back({{T_SP_K, (int)sp_a.size()}, xpot + 4 * i});
+            copies.push_back({{T_SP_X0, (int)sp_a.size()}, xpot + 4 * i + 1});
             sp_a.push_back(a); sp_b.push_back(b);
-            sp_k.push_back(d->pot_d[4 * i]); sp_x0.push_back(d->pot_d[4 * i + 1]);
+            sp_k.push_back(0.0); sp_x0.push_back(0.0);
             uint64_t m = 0;
             for (int e = 0; e < 2; ++e) {
                 const int l = pt_link[e == 0 ? a : b];
@@ -472,7 +624,7 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
     // ---- LinearDamper end points and the configs that move exactly one end
     std::vector<int32_t> da_a, da_b, dp_off(1, 0), dp_cfg, xf_idx(nq > 0 ? nq : 1, -1), xf_cfg;
     std::vector<double> da_c, wr_d;
-    std::vector<int32_t> wr_i;
+    std::vector<int32_t> wr_i, wr_frame;
     std::vector<uint64_t> wr_dep;
     {
         uint64_t any = 0;
@@ -480,7 +632,8 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
             if (d->force_kind[i] != TREPB_FORCE_LINEAR_DAMPER) continue;
             const int off = d->force_i[4 * i];
             const int a = point_of(d->ipool[off], (size_t)npc, 64), b = point_of(d->ipool[off + 1], (size_t)npc, 64);
-            da_a.push_back(a); da_b.push_back(b); da_c.push_back(d->force_d[4 * i]);
+            copies.push_back({{T_DA_C, (int)da_a.size()}, xforce + 4 * i});
+            da_a.push_back(a); da_b.push_back(b); da_c.push_back(0.0);
             uint64_t ma = 0, mb = 0;
             for (int x = pt_link[a]; x >= 0; x = l_par[x]) ma |= 1ull << l_cfg[x];
             for (int x = pt_link[b]; x >= 0; x = l_par[x]) mb |= 1ull << l_cfg[x];
@@ -496,8 +649,9 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
             const int pt = point_of(f, (size_t)npc, 64);
             wr_i.push_back(kind); wr_i.push_back(pt);
             for (int k = 0; k < 6; ++k) wr_i.push_back(d->ipool[io + k]);
-            for (int k = 0; k < 6; ++k) wr_d.push_back(d->dpool[dof + k]);
-            for (int k = 0; k < 9; ++k) wr_d.push_back(fx[f].R[k]);
+            for (int k = 0; k < 6; ++k) copies.push_back({{T_WR_D, (int)wr_d.size() + k}, xpool + dof + k});
+            for (int k = 0; k < 15; ++k) wr_d.push_back(0.0);
+            wr_frame.push_back(f);
             uint64_t m = 0;
             for (int x = pt_link[pt]; x >= 0; x = l_par[x]) m |= 1ull << l_cfg[x];
             wr_dep.push_back(m);
@@ -513,8 +667,13 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
         if (d->pot_kind[i] != TREPB_POT_NONLINEAR_CONFIG_SPRING) continue;
         const int c = d->pot_i[4 * i], off = d->pot_i[4 * i + 1], n = d->pot_i[4 * i + 2];
         nsp_i.push_back(c); nsp_i.push_back((int32_t)nsp_tab.size()); nsp_i.push_back(n);
-        nsp_d.push_back(d->pot_d[4 * i]); nsp_d.push_back(d->pot_d[4 * i + 1]);
-        for (int e = 0; e < n + 6 * (n - 1); ++e) nsp_tab.push_back(d->dpool[off + e]);
+        copies.push_back({{T_NSP_D, (int)nsp_d.size()}, xpot + 4 * i});
+        copies.push_back({{T_NSP_D, (int)nsp_d.size() + 1}, xpot + 4 * i + 1});
+        nsp_d.push_back(0.0); nsp_d.push_back(0.0);
+        for (int e = 0; e < n + 6 * (n - 1); ++e) {
+            copies.push_back({{T_NSP_TAB, (int)nsp_tab.size()}, xpool + off + e});
+            nsp_tab.push_back(0.0);
+        }
     }
     const int nns = (int)nsp_i.size() / 3;
     const int np = (int)pt_link.size();
@@ -550,28 +709,30 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
     const int npairs = (int)pair_ij.size();
     if (npairs > 30000) { P.why = "too many chain pairs"; return P; }
 
-    // ---- potentials / forces folded into per-config constants
+    // ---- potentials / forces folded into per-config constants: sums in potential / force order
     std::vector<double> damp(nd > 0 ? nd : 1, 0.0), ks(nq > 0 ? nq : 1, 0.0), kq0(nq > 0 ? nq : 1, 0.0), Fu((size_t)(nd * nu > 0 ? nd * nu : 1), 0.0);
-    double grav[3] = {0, 0, 0};
+    std::vector<std::vector<std::pair<int, int>>> t_damp(nd > 0 ? nd : 1), t_ks(nq > 0 ? nq : 1), t_kq0(nq > 0 ? nq : 1);
     int has_grav = 0;
     for (int i = 0; i < d->n_potentials; ++i) {
         if (d->pot_kind[i] == TREPB_POT_GRAVITY) {
-            for (int k = 0; k < 3; ++k) grav[k] += d->pot_d[4 * i + k];
             has_grav = 1;
         } else if (d->pot_kind[i] == TREPB_POT_CONFIG_SPRING) {
             const int c = d->pot_i[4 * i];
-            ks[c] += d->pot_d[4 * i];
-            kq0[c] += d->pot_d[4 * i] * d->pot_d[4 * i + 1];
+            t_ks[c].push_back({xpot + 4 * i, -1});
+            t_kq0[c].push_back({xpot + 4 * i, xpot + 4 * i + 1});
         }
     }
     for (int i = 0; i < d->n_forces; ++i) {
         if (d->force_kind[i] == TREPB_FORCE_DAMPING) {
-            for (int j = 0; j < nd; ++j) damp[j] += d->dpool[d->force_i[4 * i] + j];
+            for (int j = 0; j < nd; ++j) t_damp[j].push_back({xpool + d->force_i[4 * i] + j, -1});
         } else if (d->force_kind[i] == TREPB_FORCE_CONFIG) {
             const int c = d->force_i[4 * i], u = d->force_i[4 * i + 1];
             if (c < nd) Fu[(size_t)c * nu + u] += 1.0;
         }
     }
+    for (int j = 0; j < nd; ++j) if (!t_damp[j].empty()) sums.push_back({{T_DAMP, j}, t_damp[j]});
+    for (int j = 0; j < nq; ++j) if (!t_ks[j].empty()) sums.push_back({{T_KS, j}, t_ks[j]});
+    for (int j = 0; j < nq; ++j) if (!t_kq0[j].empty()) sums.push_back({{T_KQ0, j}, t_kq0[j]});
 
     // ---- pack
     memset(&P.proto, 0, sizeof(P.proto));
@@ -581,7 +742,7 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
     P.proto.ns = ns; P.proto.nqs = nqs; P.proto.npc = npc;
     P.proto.nfd = nfd; P.proto.nqf = nqf; P.proto.nns = nns; P.proto.nw = nw;
     P.proto.has_gravity = has_grav;
-    for (int k = 0; k < 3; ++k) P.proto.grav[k] = grav[k];
+    for (int k = 0; k < 3; ++k) P.proto.grav[k] = X(hd.xg + k);
     int k = 0;
     auto put = [&](const void* src, size_t bytes) {
         size_t o = (P.blob.size() + 15) & ~size_t(15);
@@ -612,6 +773,30 @@ inline CoopPack coop_pack(const trepb_sysdesc* d) {
     put(nsp_i.data(), 4 * nsp_i.size()); put(nsp_d.data(), 8 * nsp_d.size()); put(nsp_tab.data(), 8 * nsp_tab.size());
     put(wr_i.data(), 4 * wr_i.size()); put(wr_d.data(), 8 * wr_d.size()); put(wr_dep.data(), 8 * wr_dep.size());
     P.blob.resize((P.blob.size() + 15) & ~size_t(15), 0);
+
+    // ---- the plan, with blob positions resolved
+    auto dst = [&](const Dst& t) { return (int32_t)(P.off[t.tab] / sizeof(double)) + t.pos; };
+    hd.nl = nl; hd.np = np; hd.nplane = (int)planes.size() / 3; hd.nw = nw;
+    hd.ncp = (int)copies.size(); hd.nsum = (int)sums.size();
+    hd.dRc = (int)(P.off[5] / 8); hd.dpc = (int)(P.off[6] / 8); hd.din = (int)(P.off[7] / 8);
+    hd.dpt = (int)(P.off[18] / 8); hd.dcn = (int)(P.off[34] / 8); hd.dwr = (int)(P.off[54] / 8);
+    std::vector<int32_t>& I = PL.ints;
+    I.clear();
+    int ko = 0;
+    auto add = [&](const std::vector<int32_t>& v) { PL.o[ko++] = I.size(); I.insert(I.end(), v.begin(), v.end()); };
+    std::vector<int32_t> ms_off(1, 0), ms, pts(pt_frame.begin(), pt_frame.end()), cps, sum_off(1, 0), sum_dst, sum_t;
+    for (int l = 0; l < nl; ++l) { ms.insert(ms.end(), lmass[l].begin(), lmass[l].end()); ms_off.push_back((int32_t)ms.size()); }
+    for (const auto& c : copies) { cps.push_back(dst(c.first)); cps.push_back(c.second); }
+    for (const auto& s : sums) {
+        sum_dst.push_back(dst(s.first));
+        for (const auto& t : s.second) { sum_t.push_back(t.first); sum_t.push_back(t.second); }
+        sum_off.push_back((int32_t)(sum_t.size() / 2));
+    }
+    add(fr); add(fr_off); add(lk); add(ms_off); add(ms); add(pts); add(planes); add(wr_frame); add(cps); add(sum_off);
+    add(sum_dst); add(sum_t);
+    I.push_back(0);   // keeps every offset inside the array
+    // ---- the numeric tables of the description
+    coop_eval_tables(PL.view(I.data()), X, fxv.data(), (double*)P.blob.data(), 0, 1);
     P.ok = true;
     return P;
 }

@@ -50,6 +50,14 @@ TREPB_HD double varied_value(const VariedMap& m, const double* row, int i) {
     return g;
 }
 
+// Element i of the expanded vector for one row, as a function object (the cooperative kernels' plan evaluation,
+// trepb_coop_sys.h, reads the elements it needs without expanding the whole vector).
+struct VariedX {
+    VariedMap m;
+    const double* row;
+    TREPB_HD double operator()(int i) const { return varied_value(m, row, i); }
+};
+
 // Table-driven: expand one row into `slot` and point the numeric tables of `sys` at it (the integer tables stay
 // where they are, e.g. in the CTA's shared-memory copy of the blob).
 TREPB_HD void varied_point(RtSys& sys, const VariedMap& m, const double* row, double* slot) {

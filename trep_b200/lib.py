@@ -617,11 +617,15 @@ def _ptr(x):
     return x.data_ptr()
 
 
+# trepb_system_create flag: per-instance parameters on a cooperative handle (trepb.h)
+FLAG_COOP_VARIED = 128
+
+
 class System:
     """Handle of a flattened system resident on one GPU (trepb_system)."""
 
     def __init__(self, desc: D.SystemDesc, device=0, specialize=True, cooperative=None, d2_pairwise=False, literal=True,
-                 coop_one_warp=False, coop_two_warps=False):
+                 coop_one_warp=False, coop_two_warps=False, coop_varied=False):
         """specialize=False: skip the ahead-of-time specialised kernels.  cooperative: None = let
         the library choose between one thread and one warp per instance for a table-driven system,
         False = always one thread, True = always the cooperative kernels (their compile-time-size
@@ -630,7 +634,9 @@ class System:
         pair instead of one dual evaluation of the Jacobian tables per parameter.  coop_one_warp /
         coop_two_warps: for shapes whose cooperative kernels were built in several flavours, the one-warp
         flavour with the whole workspace in shared memory / the two-warps-per-instance flavour instead of
-        the default (TREPB_FLAG_COOP_ONE_WARP, TREPB_FLAG_COOP_TWO_WARPS)."""
+        the default (TREPB_FLAG_COOP_ONE_WARP, TREPB_FLAG_COOP_TWO_WARPS).  coop_varied: on a cooperative handle,
+        per-instance parameters (params=...) run on the varied cooperative kernels instead of being refused
+        (TREPB_FLAG_COOP_VARIED); it changes nothing else."""
         self.desc = desc
         self.device = device
         cd, self._keep = D.to_c(desc)
@@ -646,6 +652,8 @@ class System:
             flags |= 32
         if coop_two_warps:
             flags |= 64
+        if coop_varied:
+            flags |= FLAG_COOP_VARIED
         if not literal:
             flags |= 16     # skip an all-literal instantiation: the run-time-parameter kernel of the structure
         _check(_lib.trepb_system_create(C.byref(cd), device, flags, C.byref(h)))

@@ -37,7 +37,8 @@ def as_desc(system) -> D.SystemDesc:
 class MidpointVI:
     def __init__(self, system, tolerance=1e-10, device=0, specialize=True):
         self.desc = as_desc(system)
-        self.sys = lib.System(self.desc, device=device, specialize=specialize)
+        # coop_varied: set_parameters works on a cooperative handle too (the marionette's); plain calls are unchanged
+        self.sys = lib.System(self.desc, device=device, specialize=specialize, coop_varied=True)
         self.tolerance = float(tolerance)
         d = self.desc
         self.nq, self.nd, self.nk, self.nu, self.nc = d.nq, d.nd, d.nk, d.nu, d.nc
