@@ -30,6 +30,8 @@
  *   trepb_track_batch*       DCost (trep/discopt/dcost.py) summed as DOptimizer.calc_cost / calc_dcost, and the
  *                            LQ model of DOptimizer's steepest / quasi / newton directions.
  *   trepb_candidates_batch*  the step-size candidates of DOptimizer.armijo_search.
+ *   trepb_dare_batch*        no counterpart: the stationary LQR gain at an equilibrium, which a user of the
+ *                            reference computes on the host with scipy.linalg.solve_discrete_are.
  *   trepb_linearize_batch*  DSystem.set + fdx + fdu for every k of
  *                            DSystem.linearize_trajectory (trep/discopt/dsystem.py:229-250,
  *                            284-317, 406-423) == solve_DEL + MidpointVI_calc_deriv1
@@ -447,6 +449,45 @@ typedef struct trepb_candidates_args {
 
 int trepb_candidates_batch(int device, const trepb_candidates_args* args);                   /* host pointers   */
 int trepb_candidates_batch_dev(int device, const trepb_candidates_args* args, void* stream); /* device pointers */
+
+/* Stationary discrete LQR, batched over models: the stabilizing solution P of the discrete algebraic Riccati equation
+ *     P = A^T P A - (A^T P B + S)(R + B^T P B)^-1 (B^T P A + S^T) + Q
+ * and the gain K = (R + B^T P B)^-1 (B^T P A + S^T) (u = -K x), what scipy.linalg.solve_discrete_are (with s = S) and
+ * one more solve give on the host.  No counterpart in the reference (discopt.dlqr is time-varying only).  A / B are in
+ * the layout trepb_linearize_batch_dev writes for `batch` single-step instances; K [batch][nU][nX] is the layout
+ * trepb_project_batch reads with k_per_instance = 1 for a one-step rollout (for K steps, repeat each model's gain K
+ * times).  Structure-preserving doubling (quadratic convergence, A need not be invertible), one CTA per model with
+ * every matrix in shared memory: 8 (4 n ((n + 1) | 1) + ...) bytes, so nX = 80 runs with any nU <= 39 and nX <= 82
+ * with nU = 1; larger shapes are TREPB_ERR_UNSUPPORTED.  Every output element is summed by one thread in a fixed
+ * order, so a model gives the same bits alone and inside any batch; P is symmetric bit for bit.  Q is read as
+ * (Q + Q^T) / 2.  The K / P rows of a model whose status is not TREPB_DARE_OK are unspecified.  No system handle is
+ * needed. */
+#define TREPB_DARE_OK 0
+#define TREPB_DARE_NOT_CONVERGED -1 /* ||H' - H||_F > tol ||H'||_F after max_iterations doublings, or the
+                                       doubling stalled on a P whose residual exceeds 1e-6 of the equation's terms */
+#define TREPB_DARE_SINGULAR -2      /* exact zero pivot in R, in I + G H or in R + B^T P B (the LQR kernel's code) */
+#define TREPB_DARE_NONFINITE -3     /* an iterate overflowed or went NaN (e.g. an unstable mode B cannot reach)   */
+typedef struct trepb_dare_args {
+    int64_t batch;            /* models                                                              */
+    int32_t nX, nU;
+    int32_t max_iterations;   /* doubling steps (64 is ample: the error squares every step)          */
+    int32_t q_per_rollout;    /* 0: Q is one [nX][nX] matrix, 1: [batch][nX][nX]                     */
+    int32_t r_per_rollout;    /* 0: R is one [nU][nU] matrix, 1: [batch][nU][nU]                     */
+    int32_t s_per_rollout;    /* 0: S is one [nX][nU] matrix, 1: [batch][nX][nU]                     */
+    double tol;               /* stop at ||H' - H||_F <= tol ||H'||_F (1e-13 is about 60 ulp)         */
+    const double* A;          /* [batch][nX][nX]                                                     */
+    const double* B;          /* [batch][nX][nU]                                                     */
+    const double* Q;
+    const double* R;
+    const double* S;          /* cross term, NULL = zero                                             */
+    double* K;                /* [batch][nU][nX] out, may be NULL                                    */
+    double* P;                /* [batch][nX][nX] out, may be NULL                                    */
+    int32_t* status;          /* [batch] TREPB_DARE_*                                                 */
+    int32_t* iterations;      /* [batch] doubling steps taken, may be NULL                           */
+} trepb_dare_args;
+
+int trepb_dare_batch(int device, const trepb_dare_args* args);                   /* host pointers   */
+int trepb_dare_batch_dev(int device, const trepb_dare_args* args, void* stream); /* device pointers */
 
 /* p2 from two consecutive configurations (initialize_from_configs). q0,q1: [B][nq] -> p: [B][nd] */
 int trepb_calc_p2_batch(trepb_system* sys, int64_t batch, double dt,

@@ -24,6 +24,7 @@
 #include "trepb_err.h"
 #include "trepb_sweep.cuh"
 #include "trepb_track.cuh"
+#include "trepb_dare.cuh"
 
 namespace trepb {
 namespace {
@@ -891,5 +892,82 @@ extern "C" int trepb_candidates_batch(int device, const trepb_candidates_args* a
         x.dX = (const double*)i[4]; x.dU = (const double*)i[5]; x.Kproj = (const double*)i[6];
         x.bX = (double*)o[0]; x.bU = (double*)o[1]; x.Kc = (double*)o[2];
         return trepb_candidates_batch_dev(device, &x, nullptr);
+    });
+}
+
+// ---- stationary LQR: the discrete algebraic Riccati equation (trepb_dare.cuh) -------------------------------------
+namespace {
+static_assert(TREPB_DARE_SINGULAR == ST_SINGULAR, "a singular DARE solve reports the LQR kernel's code");
+
+// the checks both DARE entry points make before any CUDA call; -1 = go on
+int dare_check(const trepb_dare_args* a) {
+    if (!a) return lqr_fail(TREPB_ERR_INVALID, "null argument");
+    if (a->batch < 0 || a->nX < 1 || a->nU < 1 || a->max_iterations < 1) return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    if (!(a->tol > 0.0)) return lqr_fail(TREPB_ERR_INVALID, "tol must be positive");
+    const void* req[5] = {a->A, a->B, a->Q, a->R, a->status};
+    const char* names[5] = {"A", "B", "Q", "R", "status"};
+    std::string miss;
+    for (int i = 0; i < 5; ++i)
+        if (!req[i]) miss += std::string(miss.empty() ? "" : ", ") + names[i];
+    if (!miss.empty()) return lqr_fail(TREPB_ERR_INVALID, "A, B, Q, R and status are required (missing: " + miss + ")");
+    if (a->batch == 0) return TREPB_OK;
+    return -1;
+}
+
+int dare_launch(int device, const DareParams& p, cudaStream_t stream) {
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    const DareLayout L = dare_layout(p.nX, p.nU);
+    const size_t smem = (size_t)L.total * sizeof(double);
+    int smem_optin = 0, sms = 0;
+    e = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    if (smem > (size_t)smem_optin)
+        return lqr_fail(TREPB_ERR_UNSUPPORTED, "state / input dimensions too large for the shared-memory DARE solve");
+    e = cudaFuncSetAttribute((const void*)dare_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    const int block = 32 * L.nw;
+    // small models: as many CTAs per SM as shared memory allows (one model per CTA at a time)
+    int occ = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, dare_kernel, block, smem) != cudaSuccess || occ < 1) occ = 1;
+    const long long slots = (long long)sms * occ;
+    const long long grid = p.batch < slots ? p.batch : slots;
+    dare_kernel<<<(int)grid, block, smem, stream>>>(p);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    return TREPB_OK;
+}
+}  // namespace
+
+extern "C" int trepb_dare_batch_dev(int device, const trepb_dare_args* a, void* stream) {
+    TREPB_NVTX("trepb_dare_batch_dev");
+    const int c = dare_check(a);
+    if (c >= 0) return c;
+    const long long nX = a->nX, nU = a->nU;
+    DareParams p{};
+    p.batch = a->batch; p.nX = a->nX; p.nU = a->nU; p.max_it = a->max_iterations; p.tol = a->tol;
+    p.A = a->A; p.B = a->B; p.Q = a->Q; p.R = a->R; p.S = a->S;
+    p.Qs = a->q_per_rollout ? nX * nX : 0; p.Rs = a->r_per_rollout ? nU * nU : 0; p.Ss = a->s_per_rollout ? nX * nU : 0;
+    p.K = a->K; p.P = a->P; p.status = a->status; p.iters = a->iterations;
+    return dare_launch(device, p, (cudaStream_t)stream);
+}
+
+extern "C" int trepb_dare_batch(int device, const trepb_dare_args* a) {
+    TREPB_NVTX("trepb_dare_batch");
+    const int c = dare_check(a);
+    if (c >= 0) return c;
+    const size_t Rn = (size_t)a->batch, nX = (size_t)a->nX, nU = (size_t)a->nU, d = 8;
+    const void* const src[5] = {a->A, a->B, a->Q, a->R, a->S};
+    const size_t in_b[5] = {Rn * nX * nX * d, Rn * nX * nU * d, (a->q_per_rollout ? Rn : 1) * nX * nX * d,
+                            (a->r_per_rollout ? Rn : 1) * nU * nU * d, (a->s_per_rollout ? Rn : 1) * nX * nU * d};
+    void* const dst[4] = {a->K, a->P, a->status, a->iterations};
+    const size_t out_b[4] = {Rn * nU * nX * d, Rn * nX * nX * d, Rn * 4, Rn * 4};
+    return stage_bytes(device, src, in_b, dst, out_b, [&](void* const* i, void* const* o) {
+        trepb_dare_args x = *a;
+        x.A = (const double*)i[0]; x.B = (const double*)i[1]; x.Q = (const double*)i[2]; x.R = (const double*)i[3];
+        x.S = (const double*)i[4];
+        x.K = (double*)o[0]; x.P = (double*)o[1]; x.status = (int32_t*)o[2]; x.iterations = (int32_t*)o[3];
+        return trepb_dare_batch_dev(device, &x, nullptr);
     });
 }

@@ -534,6 +534,73 @@ class DSystem:
             return Kfb, A, B
         return Kfb
 
+    def calc_stationary_controller(self, xk, uk, Q=None, R=None, k=0, S=None, tol=1e-13, max_iterations=64,
+                                   return_linearization=False):
+        """Stationary LQR about an equilibrium (no counterpart in the reference, whose dlqr is time-varying only):
+        linearize at (xk, uk) over the time step time[k] -> time[k+1], then the stabilizing solution P of the discrete
+        algebraic Riccati equation P = A^T P A - (A^T P B + S)(R + B^T P B)^-1 (B^T P A + S^T) + Q and the gain
+        K = (R + B^T P B)^-1 (B^T P A + S^T), so that u = uk - K (x - xk) - both on the GPU, A / B never leaving it.
+        xk [nX], uk [nU] for one equilibrium or [M,nX], [M,nU] for M of them; with set_parameters, model r runs on
+        row r (one equilibrium with M parameter rows: that equilibrium under each of the M models).  Q [nX,nX] and
+        R [nU,nU] (identity by default) and S [nX,nU] (None: zero) are shared by the models, or one per model with a
+        leading axis.  Returns (K [..,nU,nX], P [..,nX,nX]) - without the leading axis for one equilibrium and at most
+        one parameter row - and A, B as well with return_linearization=True.  Raises ConvergenceError with the
+        per-model status when a linearization or a DARE solve fails (lib.DARE_* for the latter)."""
+        from . import lib
+        xk, uk = np.asarray(xk, float), np.asarray(uk, float)
+        single = xk.ndim == 1
+        Xb, Ub = np.atleast_2d(xk), np.atleast_2d(uk)
+        rows = 1 if self._params is None else self._params[1].shape[0]
+        if Xb.shape[0] == 1 and rows > 1:
+            Xb, Ub, single = np.repeat(Xb, rows, axis=0), np.repeat(Ub, rows, axis=0), False
+        n = Xb.shape[0]
+        if Ub.shape[0] != n:
+            raise ValueError("xk has %d equilibria, uk %d" % (n, Ub.shape[0]))
+        nX, nU, nq, nd = self._nX, self._nU, self._nQ, self._np
+        Q = np.eye(nX) if Q is None else np.asarray(Q, float)
+        R = np.eye(nU) if R is None else np.asarray(R, float)
+        S = None if S is None else np.asarray(S, float)
+        sys_, dev = self.varint.sys, self.varint.sys.device
+        up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, a.shape, dt).upload(np.ascontiguousarray(a, dtype=dt))
+        d = {}
+        try:
+            d["q1"], d["p1"] = up(Xb[:, :nq]), up(Xb[:, nq:nq + nd])
+            d["u1"] = up(Ub[:, :self._nu]) if self._nu else None
+            d["k2"] = up(Ub[:, self._nu:]) if self._nv else None
+            d["hint"] = up(Xb[:, :nd])                     # at an equilibrium the dynamic configs stay where they are
+            d["t1"], d["t2"] = up(np.full(n, self._time[k])), up(np.full(n, self._time[k + 1]))
+            d["A"], d["B"] = lib.DeviceBuffer(dev, (n, nX, nX)), lib.DeviceBuffer(dev, (n, nX, nU))
+            d["status"] = lib.DeviceBuffer(dev, (n,), np.int32)
+            params = self._rows(n)
+            d["params"] = None if params is None else up(params[1])
+            d["refs"] = None if params is None else params[0]
+            d["Q"], d["R"] = up(Q), up(R)
+            d["S"] = None if S is None else up(S)
+            d["K"], d["P"] = lib.DeviceBuffer(dev, (n, nU, nX)), lib.DeviceBuffer(dev, (n, nX, nX))
+            d["dare_status"] = lib.DeviceBuffer(dev, (n,), np.int32)
+            # linearize -> DARE without the A / B slabs leaving the GPU
+            sys_.linearize_raw(True, n, d["q1"], d["p1"], d["u1"], d["k2"], d["status"], t1=d["t1"], t2=d["t2"],
+                               q2_guess=d["hint"], A=d["A"], B=d["B"], tolerance=self.varint.tolerance,
+                               params=self._dev_params(d))
+            lib.dare_raw(True, dev, n, nX, nU, d["A"], d["B"], d["Q"], d["R"], d["dare_status"], K=d["K"], P=d["P"],
+                         S=d["S"], q_per_rollout=Q.ndim == 3, r_per_rollout=R.ndim == 3,
+                         s_per_rollout=S is not None and S.ndim == 3, tol=tol, max_iterations=max_iterations)
+            lib.synchronize(dev)
+            status = d["status"].download()
+            if np.any(status != 0):
+                raise ConvergenceError("%d of %d linearizations failed" % (int(np.sum(status != 0)), n), status)
+            ds = d["dare_status"].download()
+            bad = np.flatnonzero(ds != lib.DARE_OK)
+            if bad.size:
+                raise ConvergenceError("the DARE solve failed for %d of %d models (first: model %d, %s)"
+                                       % (bad.size, n, bad[0], lib.DARE_STATUS.get(int(ds[bad[0]]), "?")), ds)
+            out = [d["K"].download(), d["P"].download()]
+            if return_linearization:
+                out += [d["A"].download(), d["B"].download()]
+        finally:
+            self._free(d)
+        return tuple(o[0] for o in out) if single else tuple(out)
+
     def calc_descent_direction(self, X, U, q, r, Q, S, R, Qproj=None, Rproj=None, newton=False, dx0=None,
                                return_linearization=False):
         """The descent direction of DOptimizer.calc_descent_direction (doptimizer.py:348-402) for one trajectory or

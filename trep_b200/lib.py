@@ -83,6 +83,13 @@ class CandidatesArgs(C.Structure):
         + [(n, C.c_void_p) for n in ("rows", "lam", "X", "U", "dX", "dU", "Kproj", "bX", "bU", "Kc")]
 
 
+class DareArgs(C.Structure):
+    _fields_ = [("batch", C.c_int64), ("nX", C.c_int32), ("nU", C.c_int32), ("max_iterations", C.c_int32),
+                ("q_per_rollout", C.c_int32), ("r_per_rollout", C.c_int32), ("s_per_rollout", C.c_int32),
+                ("tol", C.c_double)] \
+        + [(n, C.c_void_p) for n in ("A", "B", "Q", "R", "S", "K", "P", "status", "iterations")]
+
+
 RAW = ["q2_dq1", "q2_dp1", "q2_du1", "q2_dk2", "p2_dq1", "p2_dp1", "p2_du1", "p2_dk2",
        "l1_dq1", "l1_dp1", "l1_du1", "l1_dk2"]
 
@@ -156,6 +163,8 @@ _lib.trepb_track_batch.argtypes = [C.c_int, C.POINTER(TrackArgs)]
 _lib.trepb_track_batch_dev.argtypes = [C.c_int, C.POINTER(TrackArgs), C.c_void_p]
 _lib.trepb_candidates_batch.argtypes = [C.c_int, C.POINTER(CandidatesArgs)]
 _lib.trepb_candidates_batch_dev.argtypes = [C.c_int, C.POINTER(CandidatesArgs), C.c_void_p]
+_lib.trepb_dare_batch.argtypes = [C.c_int, C.POINTER(DareArgs)]
+_lib.trepb_dare_batch_dev.argtypes = [C.c_int, C.POINTER(DareArgs), C.c_void_p]
 _lib.trepb_lqr_last_kernel_ms.argtypes = [C.c_int, C.POINTER(C.c_float)]
 _lib.trepb_linearize_batch.argtypes = [C.c_void_p, C.POINTER(LinArgs)]
 _lib.trepb_linearize_batch_dev.argtypes = [C.c_void_p, C.POINTER(LinArgs), C.c_void_p]
@@ -223,7 +232,7 @@ EXPORTS = [
     "trepb_calc_f_varied_batch_dev", "trepb_discrete_fm2_varied_batch", "trepb_discrete_fm2_varied_batch_dev",
     "trepb_deriv2_varied_batch", "trepb_deriv2_varied_batch_dev", "trepb_tangent_batch", "trepb_tangent_batch_dev",
     "trepb_adjoint_batch", "trepb_adjoint_batch_dev", "trepb_track_batch", "trepb_track_batch_dev",
-    "trepb_candidates_batch", "trepb_candidates_batch_dev",
+    "trepb_candidates_batch", "trepb_candidates_batch_dev", "trepb_dare_batch", "trepb_dare_batch_dev",
 ]
 
 
@@ -360,6 +369,51 @@ def solve_tv_lq(A, B, q, r, Q, S, R, device=0):
     if np.any(status != 0):
         raise TrepbError(0, "singular gamma in the Riccati sweep of rollout(s) %s" % np.flatnonzero(status != 0)[:8])
     return (Kfb[0], Cff[0], P0[0], b0[0]) if single else (Kfb, Cff, P0, b0)
+
+
+DARE_OK, DARE_NOT_CONVERGED, DARE_SINGULAR, DARE_NONFINITE = 0, -1, -2, -3   # TREPB_DARE_* (trepb.h)
+DARE_STATUS = {DARE_NOT_CONVERGED: "not converged", DARE_SINGULAR: "singular R, I + G H or R + B^T P B",
+               DARE_NONFINITE: "non-finite iterate (no stabilizing solution?)"}
+
+
+def dare_raw(on_device, device, batch, nX, nU, A, B, Q, R, status, K=None, P=None, S=None, iterations=None,
+             q_per_rollout=False, r_per_rollout=False, s_per_rollout=False, tol=1e-13, max_iterations=64, stream=None):
+    """trepb_dare_batch[_dev]: the stationary LQR gain K [batch,nU,nX] (u = -K x) and the stabilizing DARE solution
+    P [batch,nX,nX] of `batch` models A [batch,nX,nX], B [batch,nX,nU]; Q / R / S one matrix or one per model."""
+    a = DareArgs(batch=batch, nX=nX, nU=nU, max_iterations=max_iterations, q_per_rollout=1 if q_per_rollout else 0,
+                 r_per_rollout=1 if r_per_rollout else 0, s_per_rollout=1 if s_per_rollout else 0, tol=tol,
+                 A=_ptr(A), B=_ptr(B), Q=_ptr(Q), R=_ptr(R), S=_ptr(S), K=_ptr(K), P=_ptr(P), status=_ptr(status),
+                 iterations=_ptr(iterations))
+    if on_device:
+        _check(_lib.trepb_dare_batch_dev(device, C.byref(a), stream))
+    else:
+        _check(_lib.trepb_dare_batch(device, C.byref(a)))
+
+
+def solve_dare(A, B, Q, R, S=None, tol=1e-13, max_iterations=64, device=0):
+    """Stationary discrete LQR on the GPU: the stabilizing solution P of
+        P = A^T P A - (A^T P B + S)(R + B^T P B)^-1 (B^T P A + S^T) + Q
+    (scipy.linalg.solve_discrete_are(A, B, Q, R, s=S)) and K = (R + B^T P B)^-1 (B^T P A + S^T), u = -K x.
+    One problem: A [nX,nX], B [nX,nU], Q [nX,nX], R [nU,nU], S [nX,nU] or None; a batch: one more leading axis on A and
+    B, and on each of Q / R / S either the same (one per model) or none (shared).  Returns (K, P, status, iterations);
+    a single problem whose status is not DARE_OK raises TrepbError."""
+    f = lambda x: None if x is None else np.ascontiguousarray(np.asarray(x, float))
+    A, B, Q, R, S = f(A), f(B), f(Q), f(R), f(S)
+    single = A.ndim == 2
+    if single:
+        A, B = A[None], B[None]
+    Rn, nX, nU = A.shape[0], A.shape[1], B.shape[2]
+    K, P = np.zeros((Rn, nU, nX)), np.zeros((Rn, nX, nX))
+    status, iters = np.zeros(Rn, np.int32), np.zeros(Rn, np.int32)
+    dare_raw(False, device, Rn, nX, nU, A, B, Q, R, status, K=K, P=P, S=S, iterations=iters,
+             q_per_rollout=Q.ndim == 3, r_per_rollout=R.ndim == 3, s_per_rollout=S is not None and S.ndim == 3,
+             tol=tol, max_iterations=max_iterations)
+    if single:
+        if status[0] != DARE_OK:
+            raise TrepbError(0, "DARE failed after %d doubling steps: %s (status %d)"
+                             % (iters[0], DARE_STATUS.get(int(status[0]), "?"), status[0]))
+        return K[0], P[0], int(status[0]), int(iters[0])
+    return K, P, status, iters
 
 
 def tangent_raw(on_device, device, batch, nsteps, nX, nU, A, B, K, dX, dU, bdX=None, bdU=None, x0=None, stream=None):
