@@ -32,6 +32,8 @@
  *   trepb_candidates_batch*  the step-size candidates of DOptimizer.armijo_search.
  *   trepb_dare_batch*        no counterpart: the stationary LQR gain at an equilibrium, which a user of the
  *                            reference computes on the host with scipy.linalg.solve_discrete_are.
+ *   trepb_dlyap_batch*       no counterpart: closed-loop cost and stability of stationary gains under a batch of
+ *                            models, which a user computes on the host with scipy.linalg.solve_discrete_lyapunov.
  *   trepb_linearize_batch*  DSystem.set + fdx + fdu for every k of
  *                            DSystem.linearize_trajectory (trep/discopt/dsystem.py:229-250,
  *                            284-317, 406-423) == solve_DEL + MidpointVI_calc_deriv1
@@ -488,6 +490,57 @@ typedef struct trepb_dare_args {
 
 int trepb_dare_batch(int device, const trepb_dare_args* args);                   /* host pointers   */
 int trepb_dare_batch_dev(int device, const trepb_dare_args* args, void* stream); /* device pointers */
+
+/* Closed-loop cost and stability of stationary gains, batched over (gain, model) pairs: the solution P of the discrete
+ * Lyapunov (Stein) equation
+ *     P = A_c^T P A_c + Q_c,   A_c = A - B K,   Q_c = Q - S K - K^T S^T + K^T R K
+ * for gain K under model (A, B), the infinite-horizon cost-to-go of u = -K x under the stage cost
+ * x^T Q x + 2 x^T S u + u^T R u, which exists exactly when rho(A_c) < 1: what scipy.linalg.solve_discrete_lyapunov
+ * (A_c^T, Q_c) gives on the host, with a stability verdict.  No counterpart in the reference.  Pair p evaluates gain
+ * gain_index[p] under model model_index[p] (either NULL: gain p / model p), so a G x M cross-evaluation of the gains
+ * trepb_dare_batch wrote under the models trepb_linearize_batch_dev wrote is one call.  Smith doubling
+ * (P <- P + F^T P F, F <- F F from P = Q_c, F = A_c) until ||dP||_F <= tol ||P||_F and ||F||_F <= tol, one CTA per
+ * pair with A_c, P, F and one work block in shared memory: 8 (4 n ((n + 1) | 1) + ...) bytes; every shape
+ * trepb_dare_batch admits is admitted (up to nX = 84 at nU = 1 on a 227 KB device), larger ones are
+ * TREPB_ERR_UNSUPPORTED.  Every output element is summed by one thread in a fixed order, so a pair gives the same bits
+ * alone and inside any batch; P is symmetric bit for bit.  Q and R are read as (Q + Q^T) / 2 and (R + R^T) / 2.  The
+ * P rows of a pair whose status is not TREPB_DLYAP_STABLE are unspecified and its cost is +inf.  The host entry
+ * refuses an index outside [0, gains) / [0, models); the _dev entry cannot read the indices before the launch and
+ * reports such a pair as TREPB_DLYAP_BAD_INDEX instead.  No system handle is needed. */
+#define TREPB_DLYAP_STABLE 0
+#define TREPB_DLYAP_NOT_CONVERGED -1 /* bounded but not shrinking F (rho(A_c) >= 1, e.g. on the unit circle), too slow
+                                        to converge within max_iterations, or a residual above 1e-6 of the terms */
+#define TREPB_DLYAP_NONFINITE -3     /* an iterate overflowed or went NaN (rho(A_c) > 1 usually ends here)        */
+#define TREPB_DLYAP_BAD_INDEX -4     /* _dev entry only: gain_index / model_index outside [0, gains) / [0, models)  */
+typedef struct trepb_dlyap_args {
+    int64_t pairs;            /* (gain, model) pairs evaluated                                        */
+    int64_t gains;            /* G: gains in K (>= pairs without gain_index)                          */
+    int64_t models;           /* M: models in A / B (>= pairs without model_index)                    */
+    int32_t nX, nU;
+    int32_t max_iterations;   /* doubling steps (64 is ample: F squares every step)                    */
+    int32_t q_per_model;      /* 0: Q is one [nX][nX] matrix, 1: [models][nX][nX]                     */
+    int32_t r_per_model;      /* 0: R is one [nU][nU] matrix, 1: [models][nU][nU]                     */
+    int32_t s_per_model;      /* 0: S is one [nX][nU] matrix, 1: [models][nX][nU]                     */
+    int32_t x0_per_pair;      /* 0: x0 is one [nX] vector, 1: [pairs][nX]                             */
+    double tol;               /* stop at ||dP||_F <= tol ||P||_F and ||F||_F <= tol                    */
+    const double* A;          /* [models][nX][nX]                                                     */
+    const double* B;          /* [models][nX][nU]                                                     */
+    const double* K;          /* [gains][nU][nX], u = -K x                                            */
+    const double* Q;
+    const double* R;
+    const double* S;          /* cross term, NULL = zero                                              */
+    const int32_t* gain_index;  /* [pairs], NULL = pair p evaluates gain p                             */
+    const int32_t* model_index; /* [pairs], NULL = pair p runs under model p                           */
+    const double* x0;         /* cost = x0^T P x0; NULL: see W                                        */
+    const double* W;          /* [nX][nX], cost = trace(P W) (x0 and W exclusive, one needed for cost) */
+    double* P;                /* [pairs][nX][nX] out, may be NULL                                     */
+    double* cost;             /* [pairs] out, may be NULL                                             */
+    int32_t* status;          /* [pairs] TREPB_DLYAP_*                                                 */
+    int32_t* iterations;      /* [pairs] doubling steps taken, may be NULL                            */
+} trepb_dlyap_args;
+
+int trepb_dlyap_batch(int device, const trepb_dlyap_args* args);                   /* host pointers   */
+int trepb_dlyap_batch_dev(int device, const trepb_dlyap_args* args, void* stream); /* device pointers */
 
 /* p2 from two consecutive configurations (initialize_from_configs). q0,q1: [B][nq] -> p: [B][nd] */
 int trepb_calc_p2_batch(trepb_system* sys, int64_t batch, double dt,

@@ -25,6 +25,7 @@
 #include "trepb_sweep.cuh"
 #include "trepb_track.cuh"
 #include "trepb_dare.cuh"
+#include "trepb_dlyap.cuh"
 
 namespace trepb {
 namespace {
@@ -969,5 +970,111 @@ extern "C" int trepb_dare_batch(int device, const trepb_dare_args* a) {
         x.S = (const double*)i[4];
         x.K = (double*)o[0]; x.P = (double*)o[1]; x.status = (int32_t*)o[2]; x.iterations = (int32_t*)o[3];
         return trepb_dare_batch_dev(device, &x, nullptr);
+    });
+}
+
+// ---- closed-loop cost and stability of stationary gains: the discrete Lyapunov equation (trepb_dlyap.cuh) --------
+namespace {
+// the checks both Lyapunov entry points make before any CUDA call; -1 = go on
+int dlyap_check(const trepb_dlyap_args* a) {
+    if (!a) return lqr_fail(TREPB_ERR_INVALID, "null argument");
+    if (a->pairs < 0 || a->gains < 0 || a->models < 0 || a->nX < 1 || a->nU < 1 || a->max_iterations < 1)
+        return lqr_fail(TREPB_ERR_INVALID, "bad sizes");
+    if (!(a->tol > 0.0)) return lqr_fail(TREPB_ERR_INVALID, "tol must be positive");
+    const void* req[6] = {a->A, a->B, a->K, a->Q, a->R, a->status};
+    const char* names[6] = {"A", "B", "K", "Q", "R", "status"};
+    std::string miss;
+    for (int i = 0; i < 6; ++i)
+        if (!req[i]) miss += std::string(miss.empty() ? "" : ", ") + names[i];
+    if (!miss.empty()) return lqr_fail(TREPB_ERR_INVALID, "A, B, K, Q, R and status are required (missing: " + miss + ")");
+    if (a->x0 && a->W) return lqr_fail(TREPB_ERR_INVALID, "x0 and W are exclusive");
+    if (a->cost && !a->x0 && !a->W) return lqr_fail(TREPB_ERR_INVALID, "cost needs x0 or W");
+    if (a->pairs == 0) return TREPB_OK;
+    if (!a->gain_index && a->gains < a->pairs)
+        return lqr_fail(TREPB_ERR_INVALID, "without gain_index pair p evaluates gain p: gains must be >= pairs");
+    if (!a->model_index && a->models < a->pairs)
+        return lqr_fail(TREPB_ERR_INVALID, "without model_index pair p runs under model p: models must be >= pairs");
+    return -1;
+}
+
+// the host form's index check (the _dev form's kernel reports TREPB_DLYAP_BAD_INDEX instead)
+int dlyap_check_index(const int32_t* idx, long long pairs, long long count, const char* name) {
+    if (!idx) return -1;
+    for (long long p = 0; p < pairs; ++p)
+        if (idx[p] < 0 || idx[p] >= count)
+            return lqr_fail(TREPB_ERR_INVALID, std::string(name) + "[" + std::to_string(p) + "] = " +
+                                                   std::to_string(idx[p]) + " is outside [0, " + std::to_string(count) + ")");
+    return -1;
+}
+
+int dlyap_launch(int device, const DlyapParams& p, cudaStream_t stream) {
+    cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    const DlyapLayout L = dlyap_layout(p.nX, p.nU);
+    const size_t smem = (size_t)L.total * sizeof(double);
+    int smem_optin = 0, sms = 0;
+    e = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    if (smem > (size_t)smem_optin)
+        return lqr_fail(TREPB_ERR_UNSUPPORTED, "state / input dimensions too large for the shared-memory Lyapunov solve: " +
+                                                   std::to_string(smem) + " bytes of shared memory needed, " +
+                                                   std::to_string(smem_optin) + " per block on this device");
+    e = cudaFuncSetAttribute((const void*)dlyap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    const int block = 32 * L.nw;
+    // small states: as many CTAs per SM as shared memory allows (one pair per CTA at a time)
+    int occ = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, dlyap_kernel, block, smem) != cudaSuccess || occ < 1) occ = 1;
+    const long long slots = (long long)sms * occ;
+    const long long grid = p.pairs < slots ? p.pairs : slots;
+    dlyap_kernel<<<(int)grid, block, smem, stream>>>(p);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return lqr_fail(TREPB_ERR_CUDA, cudaGetErrorString(e));
+    return TREPB_OK;
+}
+}  // namespace
+
+extern "C" int trepb_dlyap_batch_dev(int device, const trepb_dlyap_args* a, void* stream) {
+    TREPB_NVTX("trepb_dlyap_batch_dev");
+    const int c = dlyap_check(a);
+    if (c >= 0) return c;
+    const long long nX = a->nX, nU = a->nU;
+    DlyapParams p{};
+    p.pairs = a->pairs; p.G = a->gains; p.M = a->models;
+    p.nX = a->nX; p.nU = a->nU; p.max_it = a->max_iterations; p.tol = a->tol;
+    p.A = a->A; p.B = a->B; p.K = a->K; p.Q = a->Q; p.R = a->R; p.S = a->S;
+    p.Qs = a->q_per_model ? nX * nX : 0; p.Rs = a->r_per_model ? nU * nU : 0; p.Ss = a->s_per_model ? nX * nU : 0;
+    p.gidx = a->gain_index; p.midx = a->model_index;
+    p.x0 = a->cost ? a->x0 : nullptr; p.W = a->cost ? a->W : nullptr; p.xs = a->x0_per_pair ? nX : 0;
+    p.P = a->P; p.cost = a->cost; p.status = a->status; p.iters = a->iterations;
+    return dlyap_launch(device, p, (cudaStream_t)stream);
+}
+
+extern "C" int trepb_dlyap_batch(int device, const trepb_dlyap_args* a) {
+    TREPB_NVTX("trepb_dlyap_batch");
+    int c = dlyap_check(a);
+    if (c >= 0) return c;
+    if ((c = dlyap_check_index(a->gain_index, a->pairs, a->gains, "gain_index")) >= 0) return c;
+    if ((c = dlyap_check_index(a->model_index, a->pairs, a->models, "model_index")) >= 0) return c;
+    const size_t Pn = (size_t)a->pairs, d = 8, nX = (size_t)a->nX, nU = (size_t)a->nU;
+    // the arrays cover the gains / models the indices reach (without an index: the first `pairs`)
+    const size_t G = a->gain_index ? (size_t)a->gains : Pn, M = a->model_index ? (size_t)a->models : Pn;
+    const void* const src[10] = {a->A, a->B, a->K, a->Q, a->R, a->S, a->gain_index, a->model_index,
+                                 a->cost ? a->x0 : nullptr, a->cost ? a->W : nullptr};
+    const size_t in_b[10] = {M * nX * nX * d, M * nX * nU * d, G * nU * nX * d, (a->q_per_model ? M : 1) * nX * nX * d,
+                             (a->r_per_model ? M : 1) * nU * nU * d, (a->s_per_model ? M : 1) * nX * nU * d, Pn * 4,
+                             Pn * 4, (a->x0_per_pair ? Pn : 1) * nX * d, nX * nX * d};
+    void* const dst[4] = {a->P, a->cost, a->status, a->iterations};
+    const size_t out_b[4] = {Pn * nX * nX * d, Pn * d, Pn * 4, Pn * 4};
+    return stage_bytes(device, src, in_b, dst, out_b, [&](void* const* i, void* const* o) {
+        trepb_dlyap_args x = *a;
+        x.A = (const double*)i[0]; x.B = (const double*)i[1]; x.K = (const double*)i[2]; x.Q = (const double*)i[3];
+        x.R = (const double*)i[4]; x.S = (const double*)i[5];
+        x.gain_index = (const int32_t*)i[6]; x.model_index = (const int32_t*)i[7];
+        x.x0 = (const double*)i[8]; x.W = (const double*)i[9];
+        x.P = (double*)o[0]; x.cost = (double*)o[1]; x.status = (int32_t*)o[2]; x.iterations = (int32_t*)o[3];
+        x.gains = (int64_t)G; x.models = (int64_t)M;
+        return trepb_dlyap_batch_dev(device, &x, nullptr);
     });
 }

@@ -547,48 +547,26 @@ class DSystem:
         one parameter row - and A, B as well with return_linearization=True.  Raises ConvergenceError with the
         per-model status when a linearization or a DARE solve fails (lib.DARE_* for the latter)."""
         from . import lib
-        xk, uk = np.asarray(xk, float), np.asarray(uk, float)
-        single = xk.ndim == 1
-        Xb, Ub = np.atleast_2d(xk), np.atleast_2d(uk)
-        rows = 1 if self._params is None else self._params[1].shape[0]
-        if Xb.shape[0] == 1 and rows > 1:
-            Xb, Ub, single = np.repeat(Xb, rows, axis=0), np.repeat(Ub, rows, axis=0), False
-        n = Xb.shape[0]
-        if Ub.shape[0] != n:
-            raise ValueError("xk has %d equilibria, uk %d" % (n, Ub.shape[0]))
-        nX, nU, nq, nd = self._nX, self._nU, self._nQ, self._np
+        Xb, Ub, single = self._equilibria(xk, uk)
+        n, nX, nU = Xb.shape[0], self._nX, self._nU
         Q = np.eye(nX) if Q is None else np.asarray(Q, float)
         R = np.eye(nU) if R is None else np.asarray(R, float)
         S = None if S is None else np.asarray(S, float)
-        sys_, dev = self.varint.sys, self.varint.sys.device
+        dev = self.varint.sys.device
         up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, a.shape, dt).upload(np.ascontiguousarray(a, dtype=dt))
         d = {}
         try:
-            d["q1"], d["p1"] = up(Xb[:, :nq]), up(Xb[:, nq:nq + nd])
-            d["u1"] = up(Ub[:, :self._nu]) if self._nu else None
-            d["k2"] = up(Ub[:, self._nu:]) if self._nv else None
-            d["hint"] = up(Xb[:, :nd])                     # at an equilibrium the dynamic configs stay where they are
-            d["t1"], d["t2"] = up(np.full(n, self._time[k])), up(np.full(n, self._time[k + 1]))
-            d["A"], d["B"] = lib.DeviceBuffer(dev, (n, nX, nX)), lib.DeviceBuffer(dev, (n, nX, nU))
-            d["status"] = lib.DeviceBuffer(dev, (n,), np.int32)
-            params = self._rows(n)
-            d["params"] = None if params is None else up(params[1])
-            d["refs"] = None if params is None else params[0]
+            self._linearize_equilibria(Xb, Ub, k, d)
             d["Q"], d["R"] = up(Q), up(R)
             d["S"] = None if S is None else up(S)
             d["K"], d["P"] = lib.DeviceBuffer(dev, (n, nU, nX)), lib.DeviceBuffer(dev, (n, nX, nX))
             d["dare_status"] = lib.DeviceBuffer(dev, (n,), np.int32)
             # linearize -> DARE without the A / B slabs leaving the GPU
-            sys_.linearize_raw(True, n, d["q1"], d["p1"], d["u1"], d["k2"], d["status"], t1=d["t1"], t2=d["t2"],
-                               q2_guess=d["hint"], A=d["A"], B=d["B"], tolerance=self.varint.tolerance,
-                               params=self._dev_params(d))
             lib.dare_raw(True, dev, n, nX, nU, d["A"], d["B"], d["Q"], d["R"], d["dare_status"], K=d["K"], P=d["P"],
                          S=d["S"], q_per_rollout=Q.ndim == 3, r_per_rollout=R.ndim == 3,
                          s_per_rollout=S is not None and S.ndim == 3, tol=tol, max_iterations=max_iterations)
             lib.synchronize(dev)
-            status = d["status"].download()
-            if np.any(status != 0):
-                raise ConvergenceError("%d of %d linearizations failed" % (int(np.sum(status != 0)), n), status)
+            self._check_linearizations(d)
             ds = d["dare_status"].download()
             bad = np.flatnonzero(ds != lib.DARE_OK)
             if bad.size:
@@ -600,6 +578,116 @@ class DSystem:
         finally:
             self._free(d)
         return tuple(o[0] for o in out) if single else tuple(out)
+
+    def _equilibria(self, xk, uk):
+        """(Xb [n,nX], Ub [n,nU], single) for calc_stationary_controller / evaluate_stationary_controller: one
+        equilibrium with M parameter rows is repeated M times; single = one equilibrium and at most one row."""
+        xk, uk = np.asarray(xk, float), np.asarray(uk, float)
+        single = xk.ndim == 1
+        Xb, Ub = np.atleast_2d(xk), np.atleast_2d(uk)
+        rows = 1 if self._params is None else self._params[1].shape[0]
+        if Xb.shape[0] == 1 and rows > 1:
+            Xb, Ub, single = np.repeat(Xb, rows, axis=0), np.repeat(Ub, rows, axis=0), False
+        if Ub.shape[0] != Xb.shape[0]:
+            raise ValueError("xk has %d equilibria, uk %d" % (Xb.shape[0], Ub.shape[0]))
+        return Xb, Ub, single
+
+    def _linearize_equilibria(self, Xb, Ub, k, d):
+        """Launch the linearization at the equilibria (Xb, Ub) over time[k] -> time[k+1], model r on parameter row r:
+        A / B / status into d["A"], d["B"], d["status"] on the device (no synchronize; see _check_linearizations)."""
+        from . import lib
+        n, nX, nU, nq, nd = Xb.shape[0], self._nX, self._nU, self._nQ, self._np
+        sys_, dev = self.varint.sys, self.varint.sys.device
+        up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, a.shape, dt).upload(np.ascontiguousarray(a, dtype=dt))
+        d["q1"], d["p1"] = up(Xb[:, :nq]), up(Xb[:, nq:nq + nd])
+        d["u1"] = up(Ub[:, :self._nu]) if self._nu else None
+        d["k2"] = up(Ub[:, self._nu:]) if self._nv else None
+        d["hint"] = up(Xb[:, :nd])                     # at an equilibrium the dynamic configs stay where they are
+        d["t1"], d["t2"] = up(np.full(n, self._time[k])), up(np.full(n, self._time[k + 1]))
+        d["A"], d["B"] = lib.DeviceBuffer(dev, (n, nX, nX)), lib.DeviceBuffer(dev, (n, nX, nU))
+        d["status"] = lib.DeviceBuffer(dev, (n,), np.int32)
+        params = self._rows(n)
+        d["params"] = None if params is None else up(params[1])
+        d["refs"] = None if params is None else params[0]
+        sys_.linearize_raw(True, n, d["q1"], d["p1"], d["u1"], d["k2"], d["status"], t1=d["t1"], t2=d["t2"],
+                           q2_guess=d["hint"], A=d["A"], B=d["B"], tolerance=self.varint.tolerance,
+                           params=self._dev_params(d))
+
+    @staticmethod
+    def _check_linearizations(d):
+        """After a synchronize: raise ConvergenceError for a failed linearization of _linearize_equilibria."""
+        status = d["status"].download()
+        if np.any(status != 0):
+            raise ConvergenceError("%d of %d linearizations failed" % (int(np.sum(status != 0)), status.size), status)
+
+    def evaluate_stationary_controller(self, xk, uk, K, Q=None, R=None, k=0, S=None, x0=None, cross=True,
+                                       return_P=False, tol=1e-13, max_iterations=64):
+        """Closed-loop stability and infinite-horizon cost of stationary gains under every model (no counterpart in
+        the reference): linearize at the equilibrium (xk, uk) exactly as calc_stationary_controller does (model m on
+        parameter row m), then for each gain K_g and model m the solution P of the discrete Lyapunov equation
+        P = A_c^T P A_c + Q_c, A_c = A_m - B_m K_g, Q_c = Q - S K_g - K_g^T S^T + K_g^T R K_g (the cost-to-go of
+        u = uk - K_g (x - xk) under the stage cost dx^T Q dx + 2 dx^T S du + du^T R du), on the GPU with A / B never
+        leaving it.  K [nU,nX] or [G,nU,nX]; Q / R / S as for calc_stationary_controller.  cost = x0^T P x0 for the
+        initial deviation x0 [nX], or trace(P) without it (the expected cost from x0 ~ N(0, I)); +inf where the
+        closed loop is not certified stable.  cross=True evaluates every gain under every model: returns
+        (cost [G,M], status [G,M]); cross=False gain m under model m only (G = M): (cost [M], status [M]).  Without the
+        G axis for K [nU,nX], without the M axis for one equilibrium and at most one parameter row.  status is
+        lib.DLYAP_STABLE (0) exactly when the doubling certified rho(A_c) < 1, else lib.DLYAP_NOT_CONVERGED /
+        lib.DLYAP_NONFINITE.  With return_P=True P [.., nX, nX] comes third.  Raises ConvergenceError when a
+        linearization fails."""
+        from . import lib
+        Xb, Ub, single = self._equilibria(xk, uk)
+        M, nX, nU = Xb.shape[0], self._nX, self._nU
+        K = np.asarray(K, float)
+        one_gain = K.ndim == 2
+        Kb = np.ascontiguousarray(K[None] if one_gain else K)
+        if Kb.ndim != 3 or Kb.shape[1:] != (nU, nX):
+            raise ValueError("K must be [%d,%d] or [G,%d,%d]" % (nU, nX, nU, nX))
+        G = Kb.shape[0]
+        if not cross and not one_gain and G != M:
+            raise ValueError("cross=False pairs gain m with model m: %d gains, %d models" % (G, M))
+        Q = np.eye(nX) if Q is None else np.asarray(Q, float)
+        R = np.eye(nU) if R is None else np.asarray(R, float)
+        S = None if S is None else np.asarray(S, float)
+        if cross:
+            gi, mi = np.repeat(np.arange(G), M), np.tile(np.arange(M), G)
+        else:
+            gi, mi = np.zeros(M, int) if one_gain else np.arange(M), np.arange(M)
+        pairs = gi.size
+        dev = self.varint.sys.device
+        up = lambda a, dt=np.float64: lib.DeviceBuffer(dev, a.shape, dt).upload(np.ascontiguousarray(a, dtype=dt))
+        d = {}
+        try:
+            self._linearize_equilibria(Xb, Ub, k, d)
+            d["K"], d["Q"], d["R"] = up(Kb), up(Q), up(R)
+            d["S"] = None if S is None else up(S)
+            d["gi"], d["mi"] = up(gi, np.int32), up(mi, np.int32)
+            if x0 is None:
+                d["x0"], d["W"] = None, up(np.eye(nX))
+            else:
+                d["x0"], d["W"] = up(np.asarray(x0, float).reshape(nX)), None
+            d["cost"] = lib.DeviceBuffer(dev, (pairs,))
+            d["P"] = lib.DeviceBuffer(dev, (pairs, nX, nX)) if return_P else None
+            d["dlyap_status"] = lib.DeviceBuffer(dev, (pairs,), np.int32)
+            # linearize -> Lyapunov without the A / B slabs leaving the GPU
+            lib.dlyap_raw(True, dev, pairs, G, M, nX, nU, d["A"], d["B"], d["K"], d["Q"], d["R"], d["dlyap_status"],
+                          S=d["S"], gain_index=d["gi"], model_index=d["mi"], x0=d["x0"], W=d["W"], P=d["P"],
+                          cost=d["cost"], q_per_model=Q.ndim == 3, r_per_model=R.ndim == 3,
+                          s_per_model=S is not None and S.ndim == 3, tol=tol, max_iterations=max_iterations)
+            lib.synchronize(dev)
+            self._check_linearizations(d)
+            out = [d["cost"].download(), d["dlyap_status"].download()]
+            if return_P:
+                out.append(d["P"].download())
+        finally:
+            self._free(d)
+        lead = (G, M) if cross else (M,)
+        out = [o.reshape(lead + o.shape[1:]) for o in out]
+        if cross and one_gain:
+            out, lead = [o[0] for o in out], (M,)
+        if single:
+            out = [np.take(o, 0, axis=len(lead) - 1) for o in out]
+        return tuple(out)
 
     def calc_descent_direction(self, X, U, q, r, Q, S, R, Qproj=None, Rproj=None, newton=False, dx0=None,
                                return_linearization=False):

@@ -90,6 +90,15 @@ class DareArgs(C.Structure):
         + [(n, C.c_void_p) for n in ("A", "B", "Q", "R", "S", "K", "P", "status", "iterations")]
 
 
+class DlyapArgs(C.Structure):
+    _fields_ = [("pairs", C.c_int64), ("gains", C.c_int64), ("models", C.c_int64), ("nX", C.c_int32),
+                ("nU", C.c_int32), ("max_iterations", C.c_int32), ("q_per_model", C.c_int32),
+                ("r_per_model", C.c_int32), ("s_per_model", C.c_int32), ("x0_per_pair", C.c_int32),
+                ("tol", C.c_double)] \
+        + [(n, C.c_void_p) for n in ("A", "B", "K", "Q", "R", "S", "gain_index", "model_index", "x0", "W", "P",
+                                     "cost", "status", "iterations")]
+
+
 RAW = ["q2_dq1", "q2_dp1", "q2_du1", "q2_dk2", "p2_dq1", "p2_dp1", "p2_du1", "p2_dk2",
        "l1_dq1", "l1_dp1", "l1_du1", "l1_dk2"]
 
@@ -165,6 +174,8 @@ _lib.trepb_candidates_batch.argtypes = [C.c_int, C.POINTER(CandidatesArgs)]
 _lib.trepb_candidates_batch_dev.argtypes = [C.c_int, C.POINTER(CandidatesArgs), C.c_void_p]
 _lib.trepb_dare_batch.argtypes = [C.c_int, C.POINTER(DareArgs)]
 _lib.trepb_dare_batch_dev.argtypes = [C.c_int, C.POINTER(DareArgs), C.c_void_p]
+_lib.trepb_dlyap_batch.argtypes = [C.c_int, C.POINTER(DlyapArgs)]
+_lib.trepb_dlyap_batch_dev.argtypes = [C.c_int, C.POINTER(DlyapArgs), C.c_void_p]
 _lib.trepb_lqr_last_kernel_ms.argtypes = [C.c_int, C.POINTER(C.c_float)]
 _lib.trepb_linearize_batch.argtypes = [C.c_void_p, C.POINTER(LinArgs)]
 _lib.trepb_linearize_batch_dev.argtypes = [C.c_void_p, C.POINTER(LinArgs), C.c_void_p]
@@ -233,6 +244,7 @@ EXPORTS = [
     "trepb_deriv2_varied_batch", "trepb_deriv2_varied_batch_dev", "trepb_tangent_batch", "trepb_tangent_batch_dev",
     "trepb_adjoint_batch", "trepb_adjoint_batch_dev", "trepb_track_batch", "trepb_track_batch_dev",
     "trepb_candidates_batch", "trepb_candidates_batch_dev", "trepb_dare_batch", "trepb_dare_batch_dev",
+    "trepb_dlyap_batch", "trepb_dlyap_batch_dev",
 ]
 
 
@@ -414,6 +426,75 @@ def solve_dare(A, B, Q, R, S=None, tol=1e-13, max_iterations=64, device=0):
                              % (iters[0], DARE_STATUS.get(int(status[0]), "?"), status[0]))
         return K[0], P[0], int(status[0]), int(iters[0])
     return K, P, status, iters
+
+
+DLYAP_STABLE, DLYAP_NOT_CONVERGED, DLYAP_NONFINITE, DLYAP_BAD_INDEX = 0, -1, -3, -4   # TREPB_DLYAP_* (trepb.h)
+DLYAP_STATUS = {DLYAP_STABLE: "stable", DLYAP_NOT_CONVERGED: "not converged (rho(A - B K) >= 1?)",
+                DLYAP_NONFINITE: "non-finite iterate (unstable closed loop)",
+                DLYAP_BAD_INDEX: "gain or model index out of range"}
+
+
+def dlyap_raw(on_device, device, pairs, gains, models, nX, nU, A, B, K, Q, R, status, S=None, gain_index=None,
+              model_index=None, x0=None, W=None, P=None, cost=None, iterations=None, q_per_model=False,
+              r_per_model=False, s_per_model=False, x0_per_pair=False, tol=1e-13, max_iterations=64, stream=None):
+    """trepb_dlyap_batch[_dev]: for pair p, gain K[gain_index[p]] [nU,nX] (u = -K x) under model
+    A[model_index[p]] [nX,nX], B[model_index[p]] [nX,nU] (either index None: gain p / model p), the closed-loop
+    cost-to-go P [pairs,nX,nX] of P = A_c^T P A_c + Q_c, cost [pairs] = x0^T P x0 or trace(P W), and the stability
+    verdict status [pairs] (DLYAP_*); Q / R / S one matrix or one per model."""
+    a = DlyapArgs(pairs=pairs, gains=gains, models=models, nX=nX, nU=nU, max_iterations=max_iterations,
+                  q_per_model=1 if q_per_model else 0, r_per_model=1 if r_per_model else 0,
+                  s_per_model=1 if s_per_model else 0, x0_per_pair=1 if x0_per_pair else 0, tol=tol,
+                  A=_ptr(A), B=_ptr(B), K=_ptr(K), Q=_ptr(Q), R=_ptr(R), S=_ptr(S), gain_index=_ptr(gain_index),
+                  model_index=_ptr(model_index), x0=_ptr(x0), W=_ptr(W), P=_ptr(P), cost=_ptr(cost),
+                  status=_ptr(status), iterations=_ptr(iterations))
+    if on_device:
+        _check(_lib.trepb_dlyap_batch_dev(device, C.byref(a), stream))
+    else:
+        _check(_lib.trepb_dlyap_batch(device, C.byref(a)))
+
+
+def solve_closed_loop(A, B, K, Q, R, S=None, x0=None, W=None, gain_index=None, model_index=None, tol=1e-13,
+                      max_iterations=64, device=0):
+    """Closed-loop cost and stability of stationary gains on the GPU: for u = -K x under x+ = A x + B u, the solution
+    P of P = A_c^T P A_c + Q_c with A_c = A - B K and Q_c = Q - S K - K^T S^T + K^T R K
+    (scipy.linalg.solve_discrete_lyapunov(A_c.T, Q_c)), the infinite-horizon cost of the stage cost
+    x^T Q x + 2 x^T S u + u^T R u, which exists exactly when rho(A_c) < 1.
+    One problem: A [nX,nX], B [nX,nU], K [nU,nX].  A batch: A [M,nX,nX], B [M,nX,nU], K [G,nU,nX], and pair p
+    evaluates gain gain_index[p] under model model_index[p] (either None: gain p / model p; without both, G = M
+    pairs).  Q / R / S shared or one per model (leading axis M).  cost = x0^T P x0 (x0 [nX], or [pairs,nX] one per
+    pair) or trace(P W) (W [nX,nX]); None without either.  Returns (P, cost, status, iterations); the cost of a pair
+    that is not DLYAP_STABLE is +inf.  A single problem whose status is not DLYAP_STABLE raises TrepbError."""
+    f = lambda x: None if x is None else np.ascontiguousarray(np.asarray(x, float))
+    A, B, K, Q, R, S, x0, W = f(A), f(B), f(K), f(Q), f(R), f(S), f(x0), f(W)
+    single = A.ndim == 2
+    if single:
+        A, B, K = A[None], B[None], K[None]
+    M, nX, nU, G = A.shape[0], A.shape[1], B.shape[2], K.shape[0]
+    idx = lambda i: None if i is None else np.ascontiguousarray(np.asarray(i, dtype=np.int32).ravel())
+    gain_index, model_index = idx(gain_index), idx(model_index)
+    if gain_index is not None:
+        pairs = gain_index.size
+    elif model_index is not None:
+        pairs = model_index.size
+    elif G == M:
+        pairs = G
+    else:
+        raise ValueError("%d gains and %d models: pass gain_index / model_index" % (G, M))
+    if gain_index is not None and model_index is not None and model_index.size != pairs:
+        raise ValueError("gain_index has %d pairs, model_index %d" % (pairs, model_index.size))
+    P = np.zeros((pairs, nX, nX))
+    cost = np.zeros(pairs) if x0 is not None or W is not None else None
+    status, iters = np.zeros(pairs, np.int32), np.zeros(pairs, np.int32)
+    dlyap_raw(False, device, pairs, G, M, nX, nU, A, B, K, Q, R, status, S=S, gain_index=gain_index,
+              model_index=model_index, x0=x0, W=W, P=P, cost=cost, iterations=iters, q_per_model=Q.ndim == 3,
+              r_per_model=R.ndim == 3, s_per_model=S is not None and S.ndim == 3,
+              x0_per_pair=x0 is not None and x0.ndim == 2, tol=tol, max_iterations=max_iterations)
+    if single:
+        if status[0] != DLYAP_STABLE:
+            raise TrepbError(0, "closed-loop Lyapunov solve failed after %d doubling steps: %s (status %d)"
+                             % (iters[0], DLYAP_STATUS.get(int(status[0]), "?"), status[0]))
+        return P[0], None if cost is None else float(cost[0]), int(status[0]), int(iters[0])
+    return P, cost, status, iters
 
 
 def tangent_raw(on_device, device, batch, nsteps, nX, nU, A, B, K, dX, dU, bdX=None, bdU=None, x0=None, stream=None):
